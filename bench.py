@@ -2,7 +2,7 @@
 """bench.py — poses/s of the MPL lifter forward (BASELINE.json metric) on N B200s of one node.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--precision bf16|tf32|fp32]
-                    [--arch hm0|chosen|cmu0|kptok] [--views V] [--depth D] [--batch B]
+                    [--arch hm0|chosen|cmu0|kptok] [--views V] [--depth D] [--batch B] [--dump-outputs DIR]
 
 One "step" = one forward of the H36M 4-view 17-joint `hm_0` lifter (depth 12, D = 1088, 114 M parameters) over a
 batch of 65 536 synthetic poses per GPU (BASELINE.json configs[1]).  Ranks shard the pose index range; there is no
@@ -33,6 +33,7 @@ ARCH_NAMES = {"hm0": "H36M hm_0 (MultiSPT, Conf3rd, Raytoken, Add3dEncRays)", "c
 ARCH_DEPTH = {"hm0": 12, "chosen": 12, "kptok": 12, "cmu0": 2}
 ARCH_VIEWS = {"hm0": 4, "chosen": 4, "kptok": 4, "cmu0": 5}
 ARCH_RIG = {"hm0": "h36m", "chosen": "h36m", "kptok": "h36m", "cmu0": "cmu"}
+DUMP_LIMIT = 64 << 20          # bytes written by --dump-outputs at most
 
 
 def parse():
@@ -50,7 +51,14 @@ def parse():
     p.add_argument("--depth", type=int, default=None)
     p.add_argument("--parity-poses", type=int, default=512, help="poses of the step checked against the oracle (outside the timed regions)")
     p.add_argument("--no-extras", action="store_true", help="skip the latency_b256 and fp32-grade-mode side measurements")
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="write the output of the last timed step to DIR/output.npy (float32, rank 0's shard; above "
+                        f"{DUMP_LIMIT >> 20} MB a fixed seeded sample of its poses) so that two builds can be compared")
     a = p.parse_args()
+    if a.steps < 1:
+        p.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        p.error("--dump-outputs applies to --impl ours")
     a.views = a.views or ARCH_VIEWS[a.arch]
     a.depth = ARCH_DEPTH[a.arch] if a.depth is None else a.depth
     return a
@@ -130,7 +138,7 @@ def run_reference(args):
     if rank != 0:
         return
     cores = os.cpu_count() or 1
-    steps, warmup = max(1, min(args.steps, 100)), max(1, min(args.warmup, 5))   # K timed forwards, W untimed
+    steps, warmup = args.steps, max(1, min(args.warmup, 5))   # K timed forwards, W untimed
     times, kind = cpu_forward_timer(args, steps, warmup)
     total = sum(times)
     value = args.cpu_batch * len(times) / total
@@ -172,7 +180,7 @@ def run_reference_gpu(args):
     dev = torch.device("cuda", 0)
     model = mod.MultiView_MPL(**kw).eval().to(dev)
     V = cfg.V
-    steps, warmup = max(1, min(args.steps, 20)), max(2, min(args.warmup, 5))
+    steps, warmup = args.steps, max(2, min(args.warmup, 5))
     modes = {}
     for B in sorted({256, args.batch}):
         batch = synth.make_batch(B, synth.make_rig(V, ARCH_RIG[args.arch]), seed=1)
@@ -246,6 +254,21 @@ class ClockSampler:
         order = np.argsort(pw)[len(pw) // 2:]
         return {"sm_mhz": float(np.median(np.asarray(sm)[order])), "sm_max_mhz": float(max(mx)),
                 "power_w_max": float(max(pw)), "samples": len(sm), "reasons": sorted(reasons)}
+
+
+def dump_outputs(out_dir, out):
+    """Write a step's output (B, J, 3) to out_dir/output.npy; above DUMP_LIMIT bytes, the rows of a fixed seeded sample of
+    poses (in index order), so that runs with the same arguments write the same poses."""
+    host = out.cpu().numpy()
+    rows = len(host)
+    if host.nbytes > DUMP_LIMIT:
+        keep = DUMP_LIMIT // host[0].nbytes
+        host = host[np.sort(np.random.default_rng(0).choice(rows, size=keep, replace=False))]
+    os.makedirs(out_dir, exist_ok=True)
+    path = os.path.join(out_dir, "output.npy")
+    np.save(path, host)
+    return {"file": path, "shape": list(host.shape), "poses_of": rows,
+            "sample": None if len(host) == rows else "numpy default_rng(0).choice without replacement, sorted"}
 
 
 def run_ours(args):
@@ -334,13 +357,15 @@ def run_ours(args):
     launches = 0
     e0.record()
     for _ in range(args.steps):
-        step_device()
+        last = step_device()
         launches += model.last_launches
     e1.record()
     barrier()
     ms = mdist.max_over_ranks(e0.elapsed_time(e1), dev)
     clocks = sampler.stop() if sampler else None
     value = world * args.steps * B / (ms / 1000.0)
+    dump = dict(dump_outputs(args.dump_outputs, last), ranks=[0], world_size=world) if args.dump_outputs and rank == 0 else None
+    del last
 
     # ---- timed region 2: end to end through the module call with host buffers (e2e) ----
     for _ in range(2):
@@ -548,7 +573,7 @@ def run_ours(args):
             "breakdown_note": "per-launch CUDA events on the launch stream in a separate profiled pass (same launches, same order as "
                               "the timed step); with chunk_streams=2 the timed step overlaps two chunks and runs below the sum",
             "breakdown_sum_ms": tot_ms / prof_steps, "memory_bound_kernels": memory_kernels, "hbm_peak_gbs": pk.get("hbm_gbs"),
-            "cpu_baseline": cpu, "parity": parity, **extras,
+            "cpu_baseline": cpu, "parity": parity, **extras, **({"dump_outputs": dump} if dump else {}),
             "mpjpe_cm": {"absolute": res["mpjpe_abs"], "root_relative": res["mpjpe_rel"], "procrustes_aligned": pres["p_mpjpe"],
                          "poses": res["n"],
                          "note": "random-init weights: the values only exercise the accumulators + all-reduce"},
