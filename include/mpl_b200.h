@@ -12,6 +12,7 @@
  *   MPL/lib/utils/pose_utils.py:61-143       PoseUtils.procrustes (-> mpl_pmpjpe_accumulate)
  *   MPL/lib/dataset/joints_dataset_mpl.py:615-648,701-715,762-772,817-820,872-904
  *                                            per-sample input construction (-> mpl_build_inputs)
+ *   MPL/lib/multiviews/triangulate.py:59-115 linear triangulation baseline (-> mpl_triangulate)
  *
  * Conventions
  *   - plain pointers and sizes only; no torch / C++ types cross this boundary;
@@ -32,7 +33,7 @@
 extern "C" {
 #endif
 
-#define MPL_ABI_VERSION 2
+#define MPL_ABI_VERSION 3
 
 typedef enum MplStatus {
   MPL_OK = 0,
@@ -211,6 +212,18 @@ int mpl_build_inputs(const float* pix, const double* calib, int64_t batch, int n
  *   pix    [B, V, J, 3] fp32 raw pixels (u, v, conf) -- feed to mpl_build_inputs;  target [B, J, 3] fp32, metres. */
 int mpl_synth_project(uint64_t seed, int64_t start, int64_t batch, int num_views, int num_joints, const double* calib,
                       const double* room, int conf_ones, float* pix, float* target, mpl_stream_t stream);
+
+/* Linear multi-view triangulation of the same raw detections, the baseline a multi-view lifter is measured against
+ * (MPL/lib/multiviews/triangulate.py:59-115, which calls pymvg's find3d once per joint): per (pose, joint), view v takes
+ * part iff conf > min_conf and 0 < u < w - 1 and 0 < v < h - 1 (the comparisons of mpl_build_inputs, so with min_conf = 0
+ * the used views are those whose confidence the lifter sees as > 0).  Each used view contributes the unweighted pixel-space
+ * rows u P3 - P1 and v P3 - P2 with P = K [R | -R t] (no distortion); X~ is the right singular vector of the smallest
+ * singular value of the stacked 2n x 4 matrix (Hartley & Zisserman section 12.2), X = X~[:3] / X~[3].  fp64 throughout.
+ *   pix [B, V, J, 3] fp32 (u, v, conf), calib [V, 18] fp64 as in mpl_build_inputs, 1 <= V <= 16;
+ *   points [B, J, 3] fp32 in world units (NaN where fewer than 2 views are used), views_used [B, J] int32.
+ * Allocates nothing and never synchronises (graph-capturable).  batch == 0 returns MPL_OK without touching the pointers. */
+int mpl_triangulate(const float* pix, const double* calib, int64_t batch, int num_views, int num_joints, float min_conf,
+                    float* points, int32_t* views_used, mpl_stream_t stream);
 
 /* ---- unit-test hooks for the building blocks (used by tests/ only) ------------------------------------------- */
 /* Y[M,N] = epilogue(A[M,K] . W[N,K]^T): the tcgen05 projection kernel in isolation.

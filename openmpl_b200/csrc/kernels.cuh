@@ -206,5 +206,7 @@ int launch_build_inputs(const float* pix, const double* calib, int64_t B, int V,
                         float* centers, cudaStream_t s);
 int launch_synth_project(uint64_t seed, int64_t start, int64_t B, int V, int J, const double* calib, const double* room,
                          int conf_ones, float* pix, float* target, cudaStream_t s);
+int launch_triangulate(const float* pix, const double* calib, int64_t B, int V, int J, float min_conf, float* points,
+                       int32_t* views_used, cudaStream_t s);
 
 }  // namespace mpl

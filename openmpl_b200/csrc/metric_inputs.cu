@@ -1,6 +1,7 @@
 // K6: MPJPE accumulators (evaluate.py:91-125 + function_mpl.py:674-687), P-MPJPE accumulators (pose_utils.py:61-143)
 // and the batched input builder
-// (joints_dataset_mpl.py:615-648,701-715,762-772,817-820,872-904).  Both are HBM-bound streaming kernels.
+// (joints_dataset_mpl.py:615-648,701-715,762-772,817-820,872-904).  Both are HBM-bound streaming kernels.  Also the linear
+// multi-view triangulation of the same raw detections (multiviews/triangulate.py:59-115), the lifter's baseline.
 #include "kernels.cuh"
 
 namespace mpl {
@@ -354,6 +355,148 @@ __global__ void __launch_bounds__(256) build_inputs_kernel(const float* __restri
 #pragma unroll
     for (int k = 0; k < 3; ++k) centers[bv * 3 + k] = (float)c[9 + k];
   }
+}
+
+// ---- linear multi-view triangulation (MPL/lib/multiviews/triangulate.py:59-115, pymvg find3d) -----------------------
+// One thread per (pose, joint), fp64 throughout.  View v takes part iff conf > min_conf and the pixel lies strictly inside
+// the image, the comparisons build_inputs_kernel makes.  Each used view adds the two pixel-space rows u P3 - P1 and
+// v P3 - P2 of the DLT system A X~ = 0 (Hartley & Zisserman section 12.2) into the 4x4 Gram matrix A^T A, so A is never
+// stored; the right singular vector of A's smallest singular value is the eigenvector of A^T A's smallest eigenvalue,
+// found with cyclic Jacobi.  Fewer than two used views leave the point undetermined: NaN.
+// A block stages the pixels of its kTriTile (pose, joint) items for every view through shared memory: for a fixed view the
+// items of one pose are consecutive floats, so the copy is coalesced where per-thread reads would be 12-byte strided.
+constexpr int kTriTile = 128;
+
+// Cyclic Jacobi on the symmetric 4x4 S (upper triangle used): on return diag(S) holds the eigenvalues and the columns of
+// V the eigenvectors.  A pair is skipped once |S_pq| <= 1e-15 sqrt|S_pp S_qq|, the rule of svd3_one_sided.
+__device__ __forceinline__ void eig4_jacobi(double (&S)[4][4], double (&V)[4][4]) {
+#pragma unroll
+  for (int i = 0; i < 4; ++i)
+#pragma unroll
+    for (int k = 0; k < 4; ++k) V[i][k] = i == k ? 1.0 : 0.0;
+  for (int sweep = 0; sweep < 12; ++sweep) {              // <= 7 sweeps on the synthetic rigs with 2 px noise
+    bool rotated = false;
+#pragma unroll
+    for (int pq = 0; pq < 6; ++pq) {
+      const int p = pq < 3 ? 0 : (pq < 5 ? 1 : 2);
+      const int q = pq < 3 ? pq + 1 : (pq < 5 ? pq - 1 : 3);
+      const double g = S[p][q];
+      if (g * g <= 1e-30 * fabs(S[p][p] * S[q][q])) continue;
+      rotated = true;
+      const double zeta = (S[q][q] - S[p][p]) / (2.0 * g);
+      const double t = copysign(1.0, zeta) / (fabs(zeta) + sqrt(1.0 + zeta * zeta));
+      const double c = rsqrt(1.0 + t * t), sn = c * t;
+      S[p][p] -= t * g;
+      S[q][q] += t * g;
+      S[p][q] = 0.0;
+#pragma unroll
+      for (int r = 0; r < 4; ++r) {
+        if (r == p || r == q) continue;
+        double& srp = r < p ? S[r][p] : S[p][r];
+        double& srq = r < q ? S[r][q] : S[q][r];
+        const double a = srp, b = srq;
+        srp = c * a - sn * b;
+        srq = sn * a + c * b;
+      }
+#pragma unroll
+      for (int r = 0; r < 4; ++r) {
+        const double a = V[r][p], b = V[r][q];
+        V[r][p] = c * a - sn * b;
+        V[r][q] = sn * a + c * b;
+      }
+    }
+    if (!rotated) break;
+  }
+}
+
+__global__ void __launch_bounds__(kTriTile) triangulate_kernel(const float* __restrict__ pix, const double* __restrict__ calib,
+                                                               int64_t B, int V, int J, float min_conf,
+                                                               float* __restrict__ points, int32_t* __restrict__ views_used) {
+  __shared__ double sP[kMaxViews][12];                    // P_v = K_v [R_v | -R_v t_v], row-major 3x4
+  __shared__ double sWH[kMaxViews][2];
+  __shared__ float sx[kMaxViews][3 * kTriTile];           // per view: (u, v, conf) of the tile's items
+  const int tid = threadIdx.x;
+  if (tid < V) {
+    const double* c = calib + tid * 18;
+    const double fx = c[12], fy = c[13], cx = c[14], cy = c[15];
+    double Rt[3];
+#pragma unroll
+    for (int r = 0; r < 3; ++r) Rt[r] = c[3 * r] * c[9] + c[3 * r + 1] * c[10] + c[3 * r + 2] * c[11];
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+      sP[tid][k] = fx * c[k] + cx * c[6 + k];
+      sP[tid][4 + k] = fy * c[3 + k] + cy * c[6 + k];
+      sP[tid][8 + k] = c[6 + k];
+    }
+    sP[tid][3] = -(fx * Rt[0] + cx * Rt[2]);
+    sP[tid][7] = -(fy * Rt[1] + cy * Rt[2]);
+    sP[tid][11] = -Rt[2];
+    sWH[tid][0] = c[16];
+    sWH[tid][1] = c[17];
+  }
+  const int64_t i0 = (int64_t)blockIdx.x * kTriTile;      // first item; item i = (pose i / J, joint i % J)
+  const int n = (int)(B * J - i0 < kTriTile ? B * J - i0 : kTriTile);
+  const int row = 3 * n;
+  // float f of the tile in view v is coordinate f % 3 of item i0 + f / 3 = (pose b0 + jj / J, joint jj % J), jj = j0 + f / 3
+  const int64_t b0 = i0 / J;
+  const int j0 = (int)(i0 - b0 * J);
+  for (int e = tid; e < V * row; e += kTriTile) {
+    const int v = e / row, f = e - v * row;
+    const int jj = j0 + f / 3, db = jj / J;
+    sx[v][f] = pix[(((b0 + db) * V + v) * J + (jj - db * J)) * 3 + f % 3];
+  }
+  __syncthreads();
+  if (tid >= n) return;
+  // Gram matrix A^T A, upper triangle
+  double G[4][4] = {{0, 0, 0, 0}, {0, 0, 0, 0}, {0, 0, 0, 0}, {0, 0, 0, 0}};
+  int used = 0;
+  for (int v = 0; v < V; ++v) {
+    const float uf = sx[v][3 * tid], vf = sx[v][3 * tid + 1], conf = sx[v][3 * tid + 2];
+    const double u = uf, w = vf;
+    if (!(conf > min_conf) || !(0.0 < u) || !(u < sWH[v][0] - 1.0) || !(0.0 < w) || !(w < sWH[v][1] - 1.0)) continue;
+    ++used;
+    const double* P = sP[v];
+    double a[4], b[4];
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+      a[k] = fma(u, P[8 + k], -P[k]);
+      b[k] = fma(w, P[8 + k], -P[4 + k]);
+    }
+#pragma unroll
+    for (int r = 0; r < 4; ++r)
+#pragma unroll
+      for (int k = r; k < 4; ++k) G[r][k] = fma(a[r], a[k], fma(b[r], b[k], G[r][k]));
+  }
+  const int64_t i = i0 + tid;
+  float out[3] = {__int_as_float(0x7fc00000), __int_as_float(0x7fc00000), __int_as_float(0x7fc00000)};
+  if (used >= 2) {
+    double E[4][4];
+    eig4_jacobi(G, E);
+    // eigenvector of the smallest eigenvalue (compile-time indices only, so G and E stay in registers)
+    double lmin = G[0][0], x[4] = {E[0][0], E[1][0], E[2][0], E[3][0]};
+#pragma unroll
+    for (int m = 1; m < 4; ++m)
+      if (G[m][m] < lmin) {
+        lmin = G[m][m];
+#pragma unroll
+        for (int k = 0; k < 4; ++k) x[k] = E[k][m];
+      }
+#pragma unroll
+    for (int k = 0; k < 3; ++k) out[k] = (float)(x[k] / x[3]);
+  }
+#pragma unroll
+  for (int k = 0; k < 3; ++k) points[i * 3 + k] = out[k];
+  views_used[i] = used;
+}
+
+int launch_triangulate(const float* pix, const double* calib, int64_t B, int V, int J, float min_conf, float* points,
+                       int32_t* views_used, cudaStream_t s) {
+  const int64_t items = B * J;
+  if (items == 0) return MPL_OK;
+  triangulate_kernel<<<(unsigned)ceil_div(items, kTriTile), kTriTile, 0, s>>>(pix, calib, B, V, J, min_conf, points,
+                                                                               views_used);
+  MPL_LAUNCH_CHECK();
+  return MPL_OK;
 }
 
 // ---------------------------------------------------------------------------------------------------------------------

@@ -1334,6 +1334,21 @@ int mpl_synth_project(uint64_t seed, int64_t start, int64_t batch, int num_views
                               reinterpret_cast<cudaStream_t>(stream));
 }
 
+int mpl_triangulate(const float* pix, const double* calib, int64_t batch, int num_views, int num_joints, float min_conf,
+                    float* points, int32_t* views_used, mpl_stream_t stream) {
+  if (batch < 0 || num_views < 1 || num_views > kMaxViews || num_joints < 1) {
+    set_error("mpl_triangulate: bad argument (batch %lld, num_views %d, num_joints %d)", (long long)batch, num_views, num_joints);
+    return MPL_ERR_INVALID_ARGUMENT;
+  }
+  if (batch == 0) return MPL_OK;
+  if (pix == nullptr || calib == nullptr || points == nullptr || views_used == nullptr) {
+    set_error("mpl_triangulate: null pointer");
+    return MPL_ERR_INVALID_ARGUMENT;
+  }
+  return launch_triangulate(pix, calib, batch, num_views, num_joints, min_conf, points, views_used,
+                            reinterpret_cast<cudaStream_t>(stream));
+}
+
 int mpl_test_gemm(const void* A, const void* W, const float* bias, void* Y, int64_t M, int N, int K, int dtype, int epilogue,
                   int out_fp32, int cta_group, mpl_stream_t stream) {
   MPL_API_BEGIN

@@ -4,6 +4,7 @@
     python -m openmpl_b200.evaluate --arch hm0 --views 4 --poses 10000000               # config 5 on one GPU
     torchrun --nproc-per-node 8 -m openmpl_b200.evaluate --arch cmu0 --views 5 ...      # config 3: ranks shard the poses
     python -m openmpl_b200.evaluate --arch kptok --views 8 --depth 12 --poses 262144    # config 4: view sweep
+    python -m openmpl_b200.evaluate --arch hm0 --views 4 --triangulate                   # + the triangulation baseline
 
 Per micro-batch, entirely on the device: `mpl_synth_project` (3D poses from the counter-based generator keyed by the
 GLOBAL pose index, projected through the V calibrations) -> `mpl_build_inputs` (clip, confidence zeroing, screen
@@ -11,6 +12,10 @@ normalisation, rays) -> `mpl_forward` -> `mpl_mpjpe_accumulate` + `mpl_pmpjpe_ac
 ranks own contiguous slices of the index range, and one all-reduce of the 11 J + 1 (and J + 3 Procrustes) sums at the end
 gives the MPJPE the reference's `evaluate()` would log (`function_mpl.py:670-687`) and the P-MPJPE of
 `pose_utils.py:61-143`.  Prints one JSON line from rank 0.
+
+With `--triangulate`, each micro-batch's pixels are also triangulated (`mpl_triangulate`, the linear baseline of
+`MPL/lib/multiviews/triangulate.py:59-115`) and scored by a third MPJPE accumulator that masks joints seen by fewer than two
+views; the line gains a "triangulation" entry.  Without the flag nothing of this runs.
 """
 from __future__ import annotations
 
@@ -18,6 +23,7 @@ import argparse
 import json
 import sys
 
+import numpy as np
 import torch
 
 from . import dist as mdist, inputs, metric, spec, synth
@@ -33,7 +39,7 @@ DEFAULT_RIG = {"hm0": "h36m", "chosen": "h36m", "kptok": "h36m", "cmu0": "cmu"}
 
 
 def run(arch="hm0", views=4, depth=None, poses=1 << 20, micro_batch=65536, precision="bf16", rig=None, seed=1,
-        weight_seed=0, warmup=1):
+        weight_seed=0, warmup=1, triangulate=False):
     rank, world, local = mdist.init_from_env("nccl")
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
@@ -49,6 +55,7 @@ def run(arch="hm0", views=4, depth=None, poses=1 << 20, micro_batch=65536, preci
     start, stop = mdist.shard_range(poses, rank, world)
     acc = metric.MpjpeAccumulator(cfg.J, output_in_meter=True, device=dev)
     pacc = metric.PmpjpeAccumulator(cfg.J, output_in_meter=True, device=dev)
+    tacc = metric.MpjpeAccumulator(cfg.J, output_in_meter=True, device=dev) if triangulate else None
 
     def step(s0, n):
         pix, target, calib = inputs.synth_project(n, the_rig, seed=seed, start=s0, device=dev)
@@ -58,11 +65,16 @@ def run(arch="hm0", views=4, depth=None, poses=1 << 20, micro_batch=65536, preci
         out = out[0] if isinstance(out, tuple) else out
         acc.update(out, target)
         pacc.update(out, target)
+        if tacc is not None:
+            points, used = inputs.triangulate(pix, calib)
+            tacc.update(points, target, used >= 2)
 
     for _ in range(warmup):                            # allocate the workspace, pack the weights
         step(start, min(micro_batch, max(stop - start, 1)))
     acc.acc.zero_()
     pacc.acc.zero_()
+    if tacc is not None:
+        tacc.acc.zero_()
     if world > 1:
         torch.distributed.barrier()
     torch.cuda.synchronize()
@@ -72,6 +84,8 @@ def run(arch="hm0", views=4, depth=None, poses=1 << 20, micro_batch=65536, preci
         step(s0, min(micro_batch, stop - s0))
     acc.all_reduce()                                   # the only collectives of the whole job:
     pacc.all_reduce()                                  # 11 J + 1 and J + 3 doubles
+    if tacc is not None:
+        tacc.all_reduce()
     e1.record()
     torch.cuda.synchronize()
     ms = mdist.max_over_ranks(e0.elapsed_time(e1), dev)
@@ -88,11 +102,32 @@ def run(arch="hm0", views=4, depth=None, poses=1 << 20, micro_batch=65536, preci
                          "note": "random-init weights: exercises the metric path, not a trained accuracy"},
             "tflops": poses / (ms / 1000.0) * spec.flops_per_pose(cfg) / 1e12 / world,
         }
+        if tacc is not None:
+            line["triangulation"] = triangulation_summary(tacc.acc.detach().cpu().numpy(), cfg.J)
         print(json.dumps(line), flush=True)
     if world > 1:
         torch.distributed.barrier()
         torch.distributed.destroy_process_group()
     return line
+
+
+def triangulation_summary(acc, J):
+    """The triangulation entry of the JSON line from the MPJPE sums of triangulated points masked by views_used >= 2.
+
+    absolute / root_relative: the reference's masking convention (a masked joint adds zero error but counts as a pose).
+    triangulated_joints: per joint, the error sum over its triangulated instances divided by their number (the x-count
+    of the sums), averaged over the joints triangulated at least once.  dist_rel (NaN once a root is under-determined) and
+    P-MPJPE (its accumulator takes no mask) are not reported.
+    """
+    res = metric.finalize(acc, J)
+    cnt = np.asarray(acc[8 * J:11 * J:3], dtype=np.float64)
+    seen = cnt > 0
+    per_joint = np.asarray(acc[0:J], dtype=np.float64)[seen] / cnt[seen]
+    return {"mpjpe_cm": {"absolute": res["mpjpe_abs"], "root_relative": res["mpjpe_rel"],
+                         "triangulated_joints": float(per_joint.mean()) if seen.any() else float("nan")},
+            "under_determined_joints": int(round(res["n"] * J - float(cnt.sum()))),
+            "method": "linear DLT, pixel-space rows, views with conf > 0 inside the image",
+            "note": "ms_total includes the triangulation and its accumulator"}
 
 
 def main(argv=None):
@@ -105,8 +140,9 @@ def main(argv=None):
     p.add_argument("--precision", default="bf16", choices=["bf16", "tf32", "fp32"])
     p.add_argument("--rig", default=None, choices=[None, "h36m", "cmu"])
     p.add_argument("--seed", type=int, default=1)
+    p.add_argument("--triangulate", action="store_true", help="also score the linear triangulation of the same pixels")
     a = p.parse_args(argv)
-    run(a.arch, a.views, a.depth, a.poses, a.micro_batch, a.precision, a.rig, a.seed)
+    run(a.arch, a.views, a.depth, a.poses, a.micro_batch, a.precision, a.rig, a.seed, triangulate=a.triangulate)
 
 
 if __name__ == "__main__":

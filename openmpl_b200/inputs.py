@@ -38,6 +38,30 @@ def build_inputs(pix: torch.Tensor, calib) -> tuple:
     return poses, rays, centers
 
 
+def triangulate(pix: torch.Tensor, calib, min_conf: float = 0.0) -> tuple:
+    """Linear multi-view triangulation of raw detections (`mpl_triangulate`; the baseline of
+    `MPL/lib/multiviews/triangulate.py:59-115`), enqueued on the current stream.
+
+    pix [B, V, J, 3] fp32 (u, v, conf) pixels on the device; calib [V, 18] (numpy or tensor) as for `build_inputs`.
+    A view is used for a joint iff conf > min_conf and the pixel lies strictly inside the image.  Returns
+    (points [B, J, 3] fp32 world units, NaN where fewer than 2 views are used; views_used [B, J] int32).
+    """
+    B, V, J, _ = pix.shape
+    device = pix.device
+    pix = pix.to(torch.float32).contiguous()
+    if isinstance(calib, torch.Tensor):
+        calib = calib.to(device=device, dtype=torch.float64).contiguous()
+    else:
+        calib = torch.as_tensor(np.asarray(calib, dtype=np.float64)).to(device).contiguous()
+    points = torch.empty((B, J, 3), dtype=torch.float32, device=device)
+    views_used = torch.empty((B, J), dtype=torch.int32, device=device)
+    with torch.cuda.device(device):
+        stream = torch.cuda.current_stream(device).cuda_stream
+        _lib.check(_lib.lib().mpl_triangulate(pix.data_ptr(), calib.data_ptr(), B, V, J, float(min_conf), points.data_ptr(),
+                                              views_used.data_ptr(), stream))
+    return points, views_used
+
+
 def synth_project(batch: int, rig, seed: int = 0, start: int = 0, conf_mode: str = "uniform", device=None) -> tuple:
     """N3: MHP-style synthetic poses generated and projected ON THE DEVICE (`mpl_synth_project`).
 
