@@ -13,6 +13,8 @@
  *   MPL/lib/dataset/joints_dataset_mpl.py:615-648,701-715,762-772,817-820,872-904
  *                                            per-sample input construction (-> mpl_build_inputs)
  *   MPL/lib/multiviews/triangulate.py:59-115 linear triangulation baseline (-> mpl_triangulate)
+ * Defined here, with no counterpart in the reference: robust (RANSAC) triangulation (mpl_triangulate_robust) and a
+ * detector-error model for the synthetic data (mpl_synth_detector_noise).
  *
  * Conventions
  *   - plain pointers and sizes only; no torch / C++ types cross this boundary;
@@ -33,7 +35,7 @@
 extern "C" {
 #endif
 
-#define MPL_ABI_VERSION 3
+#define MPL_ABI_VERSION 4
 
 typedef enum MplStatus {
   MPL_OK = 0,
@@ -224,6 +226,38 @@ int mpl_synth_project(uint64_t seed, int64_t start, int64_t batch, int num_views
  * Allocates nothing and never synchronises (graph-capturable).  batch == 0 returns MPL_OK without touching the pointers. */
 int mpl_triangulate(const float* pix, const double* calib, int64_t batch, int num_views, int num_joints, float min_conf,
                     float* points, int32_t* views_used, mpl_stream_t stream);
+
+/* Outlier-robust triangulation of the same detections: exhaustive-pair RANSAC with the MSAC cost, then a
+ * confidence-weighted DLT refit (defined by this library; the reference has no robust triangulation).  Candidate views are
+ * those of mpl_triangulate.  Per (pose, joint), in fp64:
+ *   - every candidate pair (a, b), a < b in lexicographic order, gives the hypothesis X~_ab, the unweighted DLT of exactly
+ *     those two views (mpl_triangulate's solve);
+ *   - its cost is sum over all candidates c of min(e_c^2, inlier_px^2), e_c the pixel reprojection error through
+ *     P_c = K [R | -R t], infinite where the depth (P_c3 . X~) / X~_4 is not > 0 or not finite; the lowest cost wins, an
+ *     exact tie the earlier pair (no random sampling: deterministic for any batch split, graph-capturable);
+ *   - the inliers are the candidates with e_c < inlier_px; with at least two of them the point is the DLT over the inliers
+ *     with each view's two rows multiplied by its conf (the maximum-likelihood weighting when the pixel noise is
+ *     proportional to 1 / conf).  When every candidate is an inlier and every conf is 1 the point is bitwise mpl_triangulate's.
+ *   pix [B, V, J, 3] fp32 (u, v, conf), calib [V, 18] fp64 as in mpl_build_inputs, 1 <= V <= 16, inlier_px finite and > 0;
+ *   points [B, J, 3] fp32 (NaN where there are fewer than 2 candidates or fewer than 2 inliers), inliers [B, J] int32
+ *   bitmask of the inlier views (bit v; 0 where the point is NaN).
+ * Allocates nothing and never synchronises.  batch == 0 returns MPL_OK without touching the pointers. */
+int mpl_triangulate_robust(const float* pix, const double* calib, int64_t batch, int num_views, int num_joints,
+                           float min_conf, float inlier_px, float* points, int32_t* inliers, mpl_stream_t stream);
+
+/* Detector-error model for the synthetic pixels of mpl_synth_project, applied in place (defined by this library; the
+ * reference's data carries the errors of a real detector).  pix [B, V, J, 3] (u, v, conf) of poses [start, start + B);
+ * only w and h of calib [V, 18] are read.  Entries with conf == 0 are left alone.  Each other entry draws U0..U5 from the
+ * Philox4x64-10 stream of mpl_synth_project under key (seed, 1) (pose i owns counter blocks [i nb, (i + 1) nb),
+ * nb = ceil(6 V J / 4); uniform slot (v J + j) 6 + m is U_m), so the result depends only on (seed, global pose index):
+ *   U0 < p_miss:              a miss, conf = 0 and the pixel is kept;
+ *   U0 < p_miss + p_outlier:  a confident false detection, u = U3 (w - 1), v = U4 (h - 1), conf = 0.3 + 0.7 U5;
+ *   otherwise:                Gaussian noise of std sigma_px / conf: (u, v) += sigma_px / conf * r (cos t, sin t),
+ *                             r = sqrt(-2 ln max(U1, 1e-12)), t = 2 pi U2; conf unchanged.
+ * fp64, rounded once to fp32; all parameters 0 leave pix bitwise unchanged.  sigma_px finite and >= 0, p_outlier and
+ * p_miss in [0, 1] with a sum <= 1, 1 <= V <= 16, start >= 0.  batch == 0 returns MPL_OK without touching the pointers. */
+int mpl_synth_detector_noise(uint64_t seed, int64_t start, int64_t batch, int num_views, int num_joints, const double* calib,
+                             float sigma_px, float p_outlier, float p_miss, float* pix, mpl_stream_t stream);
 
 /* ---- unit-test hooks for the building blocks (used by tests/ only) ------------------------------------------- */
 /* Y[M,N] = epilogue(A[M,K] . W[N,K]^T): the tcgen05 projection kernel in isolation.

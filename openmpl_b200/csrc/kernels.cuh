@@ -208,5 +208,9 @@ int launch_synth_project(uint64_t seed, int64_t start, int64_t B, int V, int J, 
                          int conf_ones, float* pix, float* target, cudaStream_t s);
 int launch_triangulate(const float* pix, const double* calib, int64_t B, int V, int J, float min_conf, float* points,
                        int32_t* views_used, cudaStream_t s);
+int launch_triangulate_robust(const float* pix, const double* calib, int64_t B, int V, int J, float min_conf,
+                              float inlier_px, float* points, int32_t* inliers, cudaStream_t s);
+int launch_detector_noise(uint64_t seed, int64_t start, int64_t B, int V, int J, const double* calib, float sigma_px,
+                          float p_outlier, float p_miss, float* pix, cudaStream_t s);
 
 }  // namespace mpl

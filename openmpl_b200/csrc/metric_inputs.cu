@@ -1,7 +1,9 @@
 // K6: MPJPE accumulators (evaluate.py:91-125 + function_mpl.py:674-687), P-MPJPE accumulators (pose_utils.py:61-143)
 // and the batched input builder
 // (joints_dataset_mpl.py:615-648,701-715,762-772,817-820,872-904).  Both are HBM-bound streaming kernels.  Also the linear
-// multi-view triangulation of the same raw detections (multiviews/triangulate.py:59-115), the lifter's baseline.
+// multi-view triangulation of the same raw detections (multiviews/triangulate.py:59-115), the lifter's baseline, its
+// outlier-robust counterpart (pair RANSAC + weighted refit), the synthetic projector and a detector-error model for its
+// pixels (the last two have no reference counterpart).
 #include "kernels.cuh"
 
 namespace mpl {
@@ -409,12 +411,12 @@ __device__ __forceinline__ void eig4_jacobi(double (&S)[4][4], double (&V)[4][4]
   }
 }
 
-__global__ void __launch_bounds__(kTriTile) triangulate_kernel(const float* __restrict__ pix, const double* __restrict__ calib,
-                                                               int64_t B, int V, int J, float min_conf,
-                                                               float* __restrict__ points, int32_t* __restrict__ views_used) {
-  __shared__ double sP[kMaxViews][12];                    // P_v = K_v [R_v | -R_v t_v], row-major 3x4
-  __shared__ double sWH[kMaxViews][2];
-  __shared__ float sx[kMaxViews][3 * kTriTile];           // per view: (u, v, conf) of the tile's items
+// Stages a block's tile of kTriTile (pose, joint) items: P_v = K_v [R_v | -R_v t_v] (row-major 3x4) and (w, h) per view,
+// and per view the (u, v, conf) of the tile's items.  Sets i0 to the tile's first item (item i = (pose i / J, joint i % J))
+// and returns the number of items in the tile.  Every thread of the block must call it (it ends with a barrier).
+__device__ __forceinline__ int tri_stage_tile(const float* __restrict__ pix, const double* __restrict__ calib, int64_t B,
+                                              int V, int J, double (&sP)[kMaxViews][12], double (&sWH)[kMaxViews][2],
+                                              float (&sx)[kMaxViews][3 * kTriTile], int64_t& i0) {
   const int tid = threadIdx.x;
   if (tid < V) {
     const double* c = calib + tid * 18;
@@ -434,7 +436,7 @@ __global__ void __launch_bounds__(kTriTile) triangulate_kernel(const float* __re
     sWH[tid][0] = c[16];
     sWH[tid][1] = c[17];
   }
-  const int64_t i0 = (int64_t)blockIdx.x * kTriTile;      // first item; item i = (pose i / J, joint i % J)
+  i0 = (int64_t)blockIdx.x * kTriTile;
   const int n = (int)(B * J - i0 < kTriTile ? B * J - i0 : kTriTile);
   const int row = 3 * n;
   // float f of the tile in view v is coordinate f % 3 of item i0 + f / 3 = (pose b0 + jj / J, joint jj % J), jj = j0 + f / 3
@@ -446,41 +448,70 @@ __global__ void __launch_bounds__(kTriTile) triangulate_kernel(const float* __re
     sx[v][f] = pix[(((b0 + db) * V + v) * J + (jj - db * J)) * 3 + f % 3];
   }
   __syncthreads();
+  return n;
+}
+
+// The view takes part iff conf > min_conf and the pixel lies strictly inside the w x h image (build_inputs_kernel's tests).
+__device__ __forceinline__ bool tri_candidate(float conf, double u, double w, float min_conf, const double (&wh)[2]) {
+  return conf > min_conf && 0.0 < u && u < wh[0] - 1.0 && 0.0 < w && w < wh[1] - 1.0;
+}
+
+// Adds the DLT rows s (u P3 - P1) and s (w P3 - P2) of one view into the Gram matrix G (upper triangle).  s = 1 is an
+// exact multiply, so the unweighted sum has the same bits with or without it.
+__device__ __forceinline__ void gram_add_view(double (&G)[4][4], const double (&P)[12], double u, double w, double s) {
+  double a[4], b[4];
+#pragma unroll
+  for (int k = 0; k < 4; ++k) {
+    a[k] = s * fma(u, P[8 + k], -P[k]);
+    b[k] = s * fma(w, P[8 + k], -P[4 + k]);
+  }
+#pragma unroll
+  for (int r = 0; r < 4; ++r)
+#pragma unroll
+    for (int k = r; k < 4; ++k) G[r][k] = fma(a[r], a[k], fma(b[r], b[k], G[r][k]));
+}
+
+// x = eigenvector of G's smallest eigenvalue (G is overwritten), i.e. the homogeneous DLT solution.  Compile-time indices
+// only, so G and the eigenvectors stay in registers.
+__device__ __forceinline__ void gram_null_vector(double (&G)[4][4], double (&x)[4]) {
+  double E[4][4];
+  eig4_jacobi(G, E);
+  double lmin = G[0][0];
+#pragma unroll
+  for (int k = 0; k < 4; ++k) x[k] = E[k][0];
+#pragma unroll
+  for (int m = 1; m < 4; ++m)
+    if (G[m][m] < lmin) {
+      lmin = G[m][m];
+#pragma unroll
+      for (int k = 0; k < 4; ++k) x[k] = E[k][m];
+    }
+}
+
+__global__ void __launch_bounds__(kTriTile) triangulate_kernel(const float* __restrict__ pix, const double* __restrict__ calib,
+                                                               int64_t B, int V, int J, float min_conf,
+                                                               float* __restrict__ points, int32_t* __restrict__ views_used) {
+  __shared__ double sP[kMaxViews][12];
+  __shared__ double sWH[kMaxViews][2];
+  __shared__ float sx[kMaxViews][3 * kTriTile];
+  const int tid = threadIdx.x;
+  int64_t i0;
+  const int n = tri_stage_tile(pix, calib, B, V, J, sP, sWH, sx, i0);
   if (tid >= n) return;
   // Gram matrix A^T A, upper triangle
   double G[4][4] = {{0, 0, 0, 0}, {0, 0, 0, 0}, {0, 0, 0, 0}, {0, 0, 0, 0}};
   int used = 0;
   for (int v = 0; v < V; ++v) {
-    const float uf = sx[v][3 * tid], vf = sx[v][3 * tid + 1], conf = sx[v][3 * tid + 2];
-    const double u = uf, w = vf;
-    if (!(conf > min_conf) || !(0.0 < u) || !(u < sWH[v][0] - 1.0) || !(0.0 < w) || !(w < sWH[v][1] - 1.0)) continue;
+    const double u = sx[v][3 * tid], w = sx[v][3 * tid + 1];
+    if (!tri_candidate(sx[v][3 * tid + 2], u, w, min_conf, sWH[v])) continue;
     ++used;
-    const double* P = sP[v];
-    double a[4], b[4];
-#pragma unroll
-    for (int k = 0; k < 4; ++k) {
-      a[k] = fma(u, P[8 + k], -P[k]);
-      b[k] = fma(w, P[8 + k], -P[4 + k]);
-    }
-#pragma unroll
-    for (int r = 0; r < 4; ++r)
-#pragma unroll
-      for (int k = r; k < 4; ++k) G[r][k] = fma(a[r], a[k], fma(b[r], b[k], G[r][k]));
+    gram_add_view(G, sP[v], u, w, 1.0);
   }
   const int64_t i = i0 + tid;
   float out[3] = {__int_as_float(0x7fc00000), __int_as_float(0x7fc00000), __int_as_float(0x7fc00000)};
   if (used >= 2) {
-    double E[4][4];
-    eig4_jacobi(G, E);
-    // eigenvector of the smallest eigenvalue (compile-time indices only, so G and E stay in registers)
-    double lmin = G[0][0], x[4] = {E[0][0], E[1][0], E[2][0], E[3][0]};
-#pragma unroll
-    for (int m = 1; m < 4; ++m)
-      if (G[m][m] < lmin) {
-        lmin = G[m][m];
-#pragma unroll
-        for (int k = 0; k < 4; ++k) x[k] = E[k][m];
-      }
+    double x[4];
+    gram_null_vector(G, x);
 #pragma unroll
     for (int k = 0; k < 3; ++k) out[k] = (float)(x[k] / x[3]);
   }
@@ -499,6 +530,100 @@ int launch_triangulate(const float* pix, const double* calib, int64_t B, int V, 
   return MPL_OK;
 }
 
+// ---- robust multi-view triangulation: exhaustive-pair RANSAC with the MSAC cost, then a confidence-weighted DLT refit --
+// Same items, staging and candidate views as triangulate_kernel.  Every candidate pair (a < b, lexicographic) gives one
+// hypothesis, the unweighted two-view DLT; its MSAC cost is sum_c min(e_c^2, tau^2) over all candidates c, e_c the pixel
+// reprojection error (infinite where the hypothesis lies behind camera c or at infinity).  The cheapest hypothesis wins
+// (an exact tie keeps the earlier pair); its inliers are the candidates with e_c < tau, and with at least two of them the
+// point is the DLT over the inliers with each view's rows scaled by its confidence.  All pairs are searched -- at most 120
+// for V = 16 -- so the result is deterministic and independent of how the batch is split.  Per-view errors are recomputed
+// for the inlier mask rather than kept in a dynamically indexed array, which would live in local memory.
+
+// Squared reprojection error (pixels^2) of the homogeneous point x through P at pixel (u, w); +inf where the depth
+// (P3 . x) / x_4 is not > 0 or not finite.
+__device__ __forceinline__ double reproj_err2(const double (&P)[12], const double (&x)[4], double u, double w) {
+  const double z = P[8] * x[0] + P[9] * x[1] + P[10] * x[2] + P[11] * x[3];
+  const double depth = z / x[3];
+  if (!(depth > 0.0) || isinf(depth)) return __longlong_as_double(0x7ff0000000000000ll);
+  const double du = (P[0] * x[0] + P[1] * x[1] + P[2] * x[2] + P[3] * x[3]) / z - u;
+  const double dv = (P[4] * x[0] + P[5] * x[1] + P[6] * x[2] + P[7] * x[3]) / z - w;
+  return du * du + dv * dv;
+}
+
+__global__ void __launch_bounds__(kTriTile) triangulate_robust_kernel(const float* __restrict__ pix,
+                                                                      const double* __restrict__ calib, int64_t B, int V,
+                                                                      int J, float min_conf, float inlier_px,
+                                                                      float* __restrict__ points,
+                                                                      int32_t* __restrict__ inliers) {
+  __shared__ double sP[kMaxViews][12];
+  __shared__ double sWH[kMaxViews][2];
+  __shared__ float sx[kMaxViews][3 * kTriTile];
+  const int tid = threadIdx.x;
+  int64_t i0;
+  const int n = tri_stage_tile(pix, calib, B, V, J, sP, sWH, sx, i0);
+  if (tid >= n) return;
+  unsigned cand = 0;                                       // bit v: view v is a candidate
+  for (int v = 0; v < V; ++v)
+    if (tri_candidate(sx[v][3 * tid + 2], sx[v][3 * tid], sx[v][3 * tid + 1], min_conf, sWH[v])) cand |= 1u << v;
+  const double tau2 = (double)inlier_px * (double)inlier_px;
+  unsigned inl = 0;
+  float out[3] = {__int_as_float(0x7fc00000), __int_as_float(0x7fc00000), __int_as_float(0x7fc00000)};
+  if (__popc(cand) >= 2) {
+    double best = __longlong_as_double(0x7ff0000000000000ll), xb[4] = {0.0, 0.0, 0.0, 0.0};
+    for (unsigned ma = cand; ma; ma &= ma - 1) {
+      const int a = __ffs(ma) - 1;
+      for (unsigned mb = ma & (ma - 1); mb; mb &= mb - 1) {
+        const int b = __ffs(mb) - 1;
+        double G[4][4] = {{0, 0, 0, 0}, {0, 0, 0, 0}, {0, 0, 0, 0}, {0, 0, 0, 0}};
+        gram_add_view(G, sP[a], sx[a][3 * tid], sx[a][3 * tid + 1], 1.0);
+        gram_add_view(G, sP[b], sx[b][3 * tid], sx[b][3 * tid + 1], 1.0);
+        double x[4];
+        gram_null_vector(G, x);
+        double cost = 0.0;                                 // MSAC; fmin maps an infinite (or NaN) error to tau^2
+        for (unsigned mc = cand; mc; mc &= mc - 1) {
+          const int c = __ffs(mc) - 1;
+          cost += fmin(reproj_err2(sP[c], x, sx[c][3 * tid], sx[c][3 * tid + 1]), tau2);
+        }
+        if (cost < best) {
+          best = cost;
+#pragma unroll
+          for (int k = 0; k < 4; ++k) xb[k] = x[k];
+        }
+      }
+    }
+    for (unsigned mc = cand; mc; mc &= mc - 1) {
+      const int c = __ffs(mc) - 1;
+      if (reproj_err2(sP[c], xb, sx[c][3 * tid], sx[c][3 * tid + 1]) < tau2) inl |= 1u << c;
+    }
+    if (__popc(inl) >= 2) {
+      // refit in triangulate_kernel's view order, rows scaled by conf (the ML weighting when the pixel noise is sigma / conf)
+      double G[4][4] = {{0, 0, 0, 0}, {0, 0, 0, 0}, {0, 0, 0, 0}, {0, 0, 0, 0}};
+      for (int v = 0; v < V; ++v)
+        if ((inl >> v) & 1u) gram_add_view(G, sP[v], sx[v][3 * tid], sx[v][3 * tid + 1], (double)sx[v][3 * tid + 2]);
+      double x[4];
+      gram_null_vector(G, x);
+#pragma unroll
+      for (int k = 0; k < 3; ++k) out[k] = (float)(x[k] / x[3]);
+    } else {
+      inl = 0;
+    }
+  }
+  const int64_t i = i0 + tid;
+#pragma unroll
+  for (int k = 0; k < 3; ++k) points[i * 3 + k] = out[k];
+  inliers[i] = (int32_t)inl;
+}
+
+int launch_triangulate_robust(const float* pix, const double* calib, int64_t B, int V, int J, float min_conf,
+                              float inlier_px, float* points, int32_t* inliers, cudaStream_t s) {
+  const int64_t items = B * J;
+  if (items == 0) return MPL_OK;
+  triangulate_robust_kernel<<<(unsigned)ceil_div(items, kTriTile), kTriTile, 0, s>>>(pix, calib, B, V, J, min_conf,
+                                                                                      inlier_px, points, inliers);
+  MPL_LAUNCH_CHECK();
+  return MPL_OK;
+}
+
 // ---------------------------------------------------------------------------------------------------------------------
 // N3: MHP-style synthetic projector.  3D poses from a counter-based generator keyed by (seed, GLOBAL pose index) --
 // any sharding of the index range over ranks / micro-batches yields the same data -- pushed through V calibrations:
@@ -506,8 +631,8 @@ int launch_triangulate(const float* pix, const double* calib, int64_t B, int V, 
 // for mpl_build_inputs and the 3D target.  The generator is numpy's Philox4x64-10 stream, bit for bit (openmpl_b200/
 // synth.py draws the same uniforms on the host), so the device data can be checked against the host generator.
 // ---------------------------------------------------------------------------------------------------------------------
-__device__ __forceinline__ void philox4x64_10(uint64_t n, uint64_t key0, uint64_t (&out)[4]) {
-  uint64_t c0 = n, c1 = 0, c2 = 0, c3 = 0, k0 = key0, k1 = 0;
+__device__ __forceinline__ void philox4x64_10(uint64_t n, uint64_t key0, uint64_t key1, uint64_t (&out)[4]) {
+  uint64_t c0 = n, c1 = 0, c2 = 0, c3 = 0, k0 = key0, k1 = key1;
 #pragma unroll
   for (int r = 0; r < 10; ++r) {
     if (r > 0) { k0 += 0x9E3779B97F4A7C15ull; k1 += 0xBB67AE8584CAA73Bull; }
@@ -526,7 +651,7 @@ struct UniformCursor {  // sequential reader of one pose's uniform stream with a
   __device__ UniformCursor(uint64_t base_, uint64_t key_) : blk(-1), base(base_), key(key_) {}
   __device__ double get(int i) {
     const int64_t b = i >> 2;
-    if (b != blk) { philox4x64_10(base + (uint64_t)b + 1ull, key, v); blk = b; }  // numpy increments the counter before generating
+    if (b != blk) { philox4x64_10(base + (uint64_t)b + 1ull, key, 0ull, v); blk = b; }  // numpy increments the counter before generating
     const int k = i & 3;
     const uint64_t raw = k == 0 ? v[0] : (k == 1 ? v[1] : (k == 2 ? v[2] : v[3]));
     return (double)(raw >> 11) * (1.0 / 9007199254740992.0);
@@ -581,6 +706,67 @@ int launch_synth_project(uint64_t seed, int64_t start, int64_t B, int V, int J, 
                          int conf_ones, float* pix, float* target, cudaStream_t s) {
   if (B == 0) return MPL_OK;
   synth_project_kernel<<<(unsigned)ceil_div(B, 128), 128, 0, s>>>(seed, start, B, V, J, calib, room, conf_ones, pix, target);
+  MPL_LAUNCH_CHECK();
+  return MPL_OK;
+}
+
+// ---- detector-error model on raw pixels: misses, confident false detections, Gaussian noise of std sigma / conf -----------
+// One thread per (pose, view, joint) entry of pix [B, V, J, 3], in place; entries with conf == 0 (behind the camera) stay.
+// The six uniforms U0..U5 of an entry come from the Philox4x64-10 stream of synth_project_kernel under key (seed, 1), so
+// they are independent of the geometry's key (seed, 0): pose i owns counter blocks [i nb, (i + 1) nb), nb = ceil(6 V J / 4),
+// and uniform slot (v J + j) 6 + m is U_m.  openmpl_b200/synth.py (detector_noise) draws the same uniforms on the host.
+//   U0 < p_miss                       -> conf = 0, pixel kept
+//   U0 < p_miss + p_outlier           -> u = U3 (w - 1), v = U4 (h - 1), conf = 0.3 + 0.7 U5
+//   otherwise                         -> (u, v) += sigma / conf * r (cos t, sin t), r = sqrt(-2 ln max(U1, 1e-12)), t = 2 pi U2
+// fp64 throughout, rounded once to fp32.  The outlier and threshold arithmetic is written with explicit roundings so it
+// matches numpy bit for bit.
+__global__ void __launch_bounds__(256) detector_noise_kernel(uint64_t seed, int64_t start, int64_t B, int V, int J,
+                                                             const double* __restrict__ calib, float sigma_px,
+                                                             float p_outlier, float p_miss, float* __restrict__ pix) {
+  const int per = V * J;
+  const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= B * per) return;
+  float* p = pix + e * 3;
+  const float conf = p[2];
+  if (conf == 0.0f) return;
+  const int64_t b = e / per;
+  const int r = (int)(e - b * per);                        // v J + j
+  const uint64_t base = (uint64_t)(start + b) * (uint64_t)((6 * per + 3) / 4);
+  const int s0 = 6 * r;                                    // slot of U0; s0 % 4 is 0 or 2, so U0..U5 span two blocks
+  uint64_t lo[4], hi[4];
+  philox4x64_10(base + (uint64_t)(s0 >> 2) + 1ull, seed, 1ull, lo);  // numpy increments the counter before generating
+  philox4x64_10(base + (uint64_t)(s0 >> 2) + 2ull, seed, 1ull, hi);
+  const bool al = (s0 & 3) == 0;
+  const uint64_t raw[6] = {al ? lo[0] : lo[2], al ? lo[1] : lo[3], al ? lo[2] : hi[0],
+                           al ? lo[3] : hi[1], al ? hi[0] : hi[2], al ? hi[1] : hi[3]};
+  double U[6];
+#pragma unroll
+  for (int m = 0; m < 6; ++m) U[m] = (double)(raw[m] >> 11) * (1.0 / 9007199254740992.0);
+  const double pm = (double)p_miss;
+  if (U[0] < pm) {
+    p[2] = 0.0f;
+    return;
+  }
+  if (U[0] < __dadd_rn(pm, (double)p_outlier)) {
+    const double* c = calib + (r / J) * 18;
+    p[0] = (float)__dmul_rn(U[3], c[16] - 1.0);
+    p[1] = (float)__dmul_rn(U[4], c[17] - 1.0);
+    p[2] = (float)__dadd_rn(0.3, __dmul_rn(0.7, U[5]));
+    return;
+  }
+  const double s = (double)sigma_px / (double)conf * sqrt(-2.0 * log(fmax(U[1], 1e-12)));
+  double sn, cs;
+  sincospi(2.0 * U[2], &sn, &cs);                          // = sincos(2 pi U2) without sincos's reduction (a stack frame)
+  p[0] = (float)((double)p[0] + s * cs);
+  p[1] = (float)((double)p[1] + s * sn);
+}
+
+int launch_detector_noise(uint64_t seed, int64_t start, int64_t B, int V, int J, const double* calib, float sigma_px,
+                          float p_outlier, float p_miss, float* pix, cudaStream_t s) {
+  const int64_t total = B * V * J;
+  if (total == 0) return MPL_OK;
+  detector_noise_kernel<<<(unsigned)ceil_div(total, 256), 256, 0, s>>>(seed, start, B, V, J, calib, sigma_px, p_outlier,
+                                                                       p_miss, pix);
   MPL_LAUNCH_CHECK();
   return MPL_OK;
 }

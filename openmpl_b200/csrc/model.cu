@@ -1349,6 +1349,42 @@ int mpl_triangulate(const float* pix, const double* calib, int64_t batch, int nu
                             reinterpret_cast<cudaStream_t>(stream));
 }
 
+int mpl_triangulate_robust(const float* pix, const double* calib, int64_t batch, int num_views, int num_joints,
+                           float min_conf, float inlier_px, float* points, int32_t* inliers, mpl_stream_t stream) {
+  if (batch < 0 || num_views < 1 || num_views > kMaxViews || num_joints < 1 || !std::isfinite(inlier_px) || !(inlier_px > 0.0f)) {
+    set_error("mpl_triangulate_robust: bad argument (batch %lld, num_views %d, num_joints %d, inlier_px %g)", (long long)batch,
+              num_views, num_joints, (double)inlier_px);
+    return MPL_ERR_INVALID_ARGUMENT;
+  }
+  if (batch == 0) return MPL_OK;
+  if (pix == nullptr || calib == nullptr || points == nullptr || inliers == nullptr) {
+    set_error("mpl_triangulate_robust: null pointer");
+    return MPL_ERR_INVALID_ARGUMENT;
+  }
+  return launch_triangulate_robust(pix, calib, batch, num_views, num_joints, min_conf, inlier_px, points, inliers,
+                                   reinterpret_cast<cudaStream_t>(stream));
+}
+
+int mpl_synth_detector_noise(uint64_t seed, int64_t start, int64_t batch, int num_views, int num_joints, const double* calib,
+                             float sigma_px, float p_outlier, float p_miss, float* pix, mpl_stream_t stream) {
+  // the probabilities' sum in fp64, as the kernel forms it
+  if (batch < 0 || start < 0 || num_views < 1 || num_views > kMaxViews || num_joints < 1 || !std::isfinite(sigma_px) ||
+      !(sigma_px >= 0.0f) || !(p_outlier >= 0.0f && p_outlier <= 1.0f) || !(p_miss >= 0.0f && p_miss <= 1.0f) ||
+      !((double)p_outlier + (double)p_miss <= 1.0)) {
+    set_error("mpl_synth_detector_noise: bad argument (batch %lld, start %lld, num_views %d, num_joints %d, sigma_px %g, "
+              "p_outlier %g, p_miss %g)", (long long)batch, (long long)start, num_views, num_joints, (double)sigma_px,
+              (double)p_outlier, (double)p_miss);
+    return MPL_ERR_INVALID_ARGUMENT;
+  }
+  if (batch == 0) return MPL_OK;
+  if (calib == nullptr || pix == nullptr) {
+    set_error("mpl_synth_detector_noise: null pointer");
+    return MPL_ERR_INVALID_ARGUMENT;
+  }
+  return launch_detector_noise(seed, start, batch, num_views, num_joints, calib, sigma_px, p_outlier, p_miss, pix,
+                               reinterpret_cast<cudaStream_t>(stream));
+}
+
 int mpl_test_gemm(const void* A, const void* W, const float* bias, void* Y, int64_t M, int N, int K, int dtype, int epilogue,
                   int out_fp32, int cta_group, mpl_stream_t stream) {
   MPL_API_BEGIN

@@ -5,6 +5,8 @@
     torchrun --nproc-per-node 8 -m openmpl_b200.evaluate --arch cmu0 --views 5 ...      # config 3: ranks shard the poses
     python -m openmpl_b200.evaluate --arch kptok --views 8 --depth 12 --poses 262144    # config 4: view sweep
     python -m openmpl_b200.evaluate --arch hm0 --views 4 --triangulate                   # + the triangulation baseline
+    python -m openmpl_b200.evaluate --arch hm0 --views 4 --pixel-noise 2 --outlier-rate 0.1 --triangulate \
+        --triangulate-robust                                                            # noisy detections, both baselines
 
 Per micro-batch, entirely on the device: `mpl_synth_project` (3D poses from the counter-based generator keyed by the
 GLOBAL pose index, projected through the V calibrations) -> `mpl_build_inputs` (clip, confidence zeroing, screen
@@ -16,6 +18,12 @@ gives the MPJPE the reference's `evaluate()` would log (`function_mpl.py:670-687
 With `--triangulate`, each micro-batch's pixels are also triangulated (`mpl_triangulate`, the linear baseline of
 `MPL/lib/multiviews/triangulate.py:59-115`) and scored by a third MPJPE accumulator that masks joints seen by fewer than two
 views; the line gains a "triangulation" entry.  Without the flag nothing of this runs.
+
+`--pixel-noise PX`, `--outlier-rate P` and `--miss-rate P` corrupt each micro-batch's pixels right after they are generated
+(`mpl_synth_detector_noise`: Gaussian noise of std PX / conf, confident false detections, misses; keyed by the global pose
+index like the poses), so the lifter and the triangulations all see the same detections; the line's "data" entry records
+the three values.  `--triangulate-robust` adds a "triangulation_robust" entry for `mpl_triangulate_robust` (pair RANSAC
+with the MSAC cost at `--inlier-px`, then a confidence-weighted refit), masked where it finds fewer than two inliers.
 """
 from __future__ import annotations
 
@@ -39,7 +47,8 @@ DEFAULT_RIG = {"hm0": "h36m", "chosen": "h36m", "kptok": "h36m", "cmu0": "cmu"}
 
 
 def run(arch="hm0", views=4, depth=None, poses=1 << 20, micro_batch=65536, precision="bf16", rig=None, seed=1,
-        weight_seed=0, warmup=1, triangulate=False):
+        weight_seed=0, warmup=1, triangulate=False, pixel_noise=0.0, outlier_rate=0.0, miss_rate=0.0,
+        triangulate_robust=False, inlier_px=10.0):
     rank, world, local = mdist.init_from_env("nccl")
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
@@ -56,9 +65,13 @@ def run(arch="hm0", views=4, depth=None, poses=1 << 20, micro_batch=65536, preci
     acc = metric.MpjpeAccumulator(cfg.J, output_in_meter=True, device=dev)
     pacc = metric.PmpjpeAccumulator(cfg.J, output_in_meter=True, device=dev)
     tacc = metric.MpjpeAccumulator(cfg.J, output_in_meter=True, device=dev) if triangulate else None
+    racc = metric.MpjpeAccumulator(cfg.J, output_in_meter=True, device=dev) if triangulate_robust else None
+    noisy = pixel_noise != 0 or outlier_rate != 0 or miss_rate != 0
 
     def step(s0, n):
         pix, target, calib = inputs.synth_project(n, the_rig, seed=seed, start=s0, device=dev)
+        if noisy:
+            inputs.add_detector_noise(pix, calib, seed, s0, pixel_noise, outlier_rate, miss_rate)
         p, r, c = inputs.build_inputs(pix, calib)
         with torch.no_grad():
             out = model(p, rays=r, centers=c)
@@ -68,13 +81,17 @@ def run(arch="hm0", views=4, depth=None, poses=1 << 20, micro_batch=65536, preci
         if tacc is not None:
             points, used = inputs.triangulate(pix, calib)
             tacc.update(points, target, used >= 2)
+        if racc is not None:
+            points, inl = inputs.triangulate_robust(pix, calib, inlier_px=inlier_px)
+            racc.update(points, target, inl != 0)      # popcount >= 2: a non-zero inlier mask has at least two bits
 
     for _ in range(warmup):                            # allocate the workspace, pack the weights
         step(start, min(micro_batch, max(stop - start, 1)))
     acc.acc.zero_()
     pacc.acc.zero_()
-    if tacc is not None:
-        tacc.acc.zero_()
+    for a in (tacc, racc):
+        if a is not None:
+            a.acc.zero_()
     if world > 1:
         torch.distributed.barrier()
     torch.cuda.synchronize()
@@ -84,8 +101,9 @@ def run(arch="hm0", views=4, depth=None, poses=1 << 20, micro_batch=65536, preci
         step(s0, min(micro_batch, stop - s0))
     acc.all_reduce()                                   # the only collectives of the whole job:
     pacc.all_reduce()                                  # 11 J + 1 and J + 3 doubles
-    if tacc is not None:
-        tacc.all_reduce()
+    for a in (tacc, racc):
+        if a is not None:
+            a.all_reduce()
     e1.record()
     torch.cuda.synchronize()
     ms = mdist.max_over_ranks(e0.elapsed_time(e1), dev)
@@ -102,8 +120,17 @@ def run(arch="hm0", views=4, depth=None, poses=1 << 20, micro_batch=65536, preci
                          "note": "random-init weights: exercises the metric path, not a trained accuracy"},
             "tflops": poses / (ms / 1000.0) * spec.flops_per_pose(cfg) / 1e12 / world,
         }
+        if noisy:
+            line["data"] = {"source": line["data"], "pixel_noise_px": pixel_noise, "outlier_rate": outlier_rate,
+                            "miss_rate": miss_rate,
+                            "noise_model": "Gaussian of std pixel_noise_px / conf; outliers uniform in the image with conf "
+                                           "0.3-1; misses set conf 0"}
         if tacc is not None:
             line["triangulation"] = triangulation_summary(tacc.acc.detach().cpu().numpy(), cfg.J)
+        if racc is not None:
+            line["triangulation_robust"] = triangulation_summary(
+                racc.acc.detach().cpu().numpy(), cfg.J,
+                method=f"pair RANSAC, MSAC cost at {inlier_px:g} px, conf-weighted DLT refit over the inliers")
         print(json.dumps(line), flush=True)
     if world > 1:
         torch.distributed.barrier()
@@ -111,13 +138,14 @@ def run(arch="hm0", views=4, depth=None, poses=1 << 20, micro_batch=65536, preci
     return line
 
 
-def triangulation_summary(acc, J):
+def triangulation_summary(acc, J, method="linear DLT, pixel-space rows, views with conf > 0 inside the image"):
     """The triangulation entry of the JSON line from the MPJPE sums of triangulated points masked by views_used >= 2.
 
     absolute / root_relative: the reference's masking convention (a masked joint adds zero error but counts as a pose).
     triangulated_joints: per joint, the error sum over its triangulated instances divided by their number (the x-count
     of the sums), averaged over the joints triangulated at least once.  dist_rel (NaN once a root is under-determined) and
-    P-MPJPE (its accumulator takes no mask) are not reported.
+    P-MPJPE (its accumulator takes no mask) are not reported.  For the robust triangulation the mask is "at least two
+    inliers", so under_determined_joints counts the joints it rejected as well as those seen by fewer than two views.
     """
     res = metric.finalize(acc, J)
     cnt = np.asarray(acc[8 * J:11 * J:3], dtype=np.float64)
@@ -126,7 +154,7 @@ def triangulation_summary(acc, J):
     return {"mpjpe_cm": {"absolute": res["mpjpe_abs"], "root_relative": res["mpjpe_rel"],
                          "triangulated_joints": float(per_joint.mean()) if seen.any() else float("nan")},
             "under_determined_joints": int(round(res["n"] * J - float(cnt.sum()))),
-            "method": "linear DLT, pixel-space rows, views with conf > 0 inside the image",
+            "method": method,
             "note": "ms_total includes the triangulation and its accumulator"}
 
 
@@ -141,8 +169,18 @@ def main(argv=None):
     p.add_argument("--rig", default=None, choices=[None, "h36m", "cmu"])
     p.add_argument("--seed", type=int, default=1)
     p.add_argument("--triangulate", action="store_true", help="also score the linear triangulation of the same pixels")
+    p.add_argument("--triangulate-robust", action="store_true",
+                   help="also score the robust (pair RANSAC + conf-weighted refit) triangulation of the same pixels")
+    p.add_argument("--inlier-px", type=float, default=10.0, help="inlier threshold of --triangulate-robust, pixels")
+    p.add_argument("--pixel-noise", type=float, default=0.0, metavar="PX",
+                   help="detector noise: Gaussian pixel error of std PX / conf")
+    p.add_argument("--outlier-rate", type=float, default=0.0, metavar="P",
+                   help="detector noise: share of confident false detections")
+    p.add_argument("--miss-rate", type=float, default=0.0, metavar="P", help="detector noise: share of missed detections")
     a = p.parse_args(argv)
-    run(a.arch, a.views, a.depth, a.poses, a.micro_batch, a.precision, a.rig, a.seed, triangulate=a.triangulate)
+    run(a.arch, a.views, a.depth, a.poses, a.micro_batch, a.precision, a.rig, a.seed, triangulate=a.triangulate,
+        pixel_noise=a.pixel_noise, outlier_rate=a.outlier_rate, miss_rate=a.miss_rate,
+        triangulate_robust=a.triangulate_robust, inlier_px=a.inlier_px)
 
 
 if __name__ == "__main__":

@@ -62,6 +62,54 @@ def triangulate(pix: torch.Tensor, calib, min_conf: float = 0.0) -> tuple:
     return points, views_used
 
 
+def triangulate_robust(pix: torch.Tensor, calib, min_conf: float = 0.0, inlier_px: float = 10.0) -> tuple:
+    """Outlier-robust triangulation of raw detections (`mpl_triangulate_robust`), enqueued on the current stream.
+
+    Candidate views as in `triangulate`.  Every candidate pair gives a two-view DLT hypothesis scored by the MSAC cost
+    sum_c min(e_c^2, inlier_px^2) over the candidates' pixel reprojection errors; the cheapest one's inliers (e_c < inlier_px)
+    are refitted by a DLT with rows weighted by conf.  Returns (points [B, J, 3] fp32 world units, NaN where fewer than two
+    candidates or inliers; inliers [B, J] int32 bitmask of the inlier views, bit v for view v, 0 where the point is NaN).
+    """
+    B, V, J, _ = pix.shape
+    device = pix.device
+    pix = pix.to(torch.float32).contiguous()
+    calib = _device_calib(calib, device)
+    points = torch.empty((B, J, 3), dtype=torch.float32, device=device)
+    inliers = torch.empty((B, J), dtype=torch.int32, device=device)
+    with torch.cuda.device(device):
+        stream = torch.cuda.current_stream(device).cuda_stream
+        _lib.check(_lib.lib().mpl_triangulate_robust(pix.data_ptr(), calib.data_ptr(), B, V, J, float(min_conf),
+                                                     float(inlier_px), points.data_ptr(), inliers.data_ptr(), stream))
+    return points, inliers
+
+
+def add_detector_noise(pix: torch.Tensor, calib, seed: int, start: int, sigma_px: float, p_outlier: float,
+                       p_miss: float) -> torch.Tensor:
+    """Detector-error model (`mpl_synth_detector_noise`) applied IN PLACE to raw pixels of poses [start, start + B),
+    enqueued on the current stream; returns `pix`.
+
+    pix [B, V, J, 3] contiguous fp32 (u, v, conf) on the device, as `synth_project` returns it; calib [V, 18] (only w, h
+    are read).  Per entry with conf > 0: a miss (conf = 0) with probability p_miss, a confident false detection anywhere in
+    the image with probability p_outlier, otherwise Gaussian pixel noise of std sigma_px / conf.  The draws depend only on
+    (seed, global pose index), under a key separate from `synth_project`'s; `synth.detector_noise` is the numpy twin.
+    """
+    if pix.dtype != torch.float32 or not pix.is_contiguous() or pix.dim() != 4 or pix.shape[-1] != 3:
+        raise ValueError("add_detector_noise works in place on a contiguous float32 [B, V, J, 3] tensor")
+    B, V, J, _ = pix.shape
+    calib = _device_calib(calib, pix.device)
+    with torch.cuda.device(pix.device):
+        stream = torch.cuda.current_stream(pix.device).cuda_stream
+        _lib.check(_lib.lib().mpl_synth_detector_noise(int(seed), int(start), B, V, J, calib.data_ptr(), float(sigma_px),
+                                                       float(p_outlier), float(p_miss), pix.data_ptr(), stream))
+    return pix
+
+
+def _device_calib(calib, device) -> torch.Tensor:
+    if isinstance(calib, torch.Tensor):
+        return calib.to(device=device, dtype=torch.float64).contiguous()
+    return torch.as_tensor(np.asarray(calib, dtype=np.float64)).to(device).contiguous()
+
+
 def synth_project(batch: int, rig, seed: int = 0, start: int = 0, conf_mode: str = "uniform", device=None) -> tuple:
     """N3: MHP-style synthetic poses generated and projected ON THE DEVICE (`mpl_synth_project`).
 

@@ -69,10 +69,10 @@ def make_rig(num_views: int, kind: str = "h36m") -> Rig:
                image_size=(w, h), room=room)
 
 
-def _uniforms(seed: int, start: int, count: int, per_pose: int) -> np.ndarray:
-    """[count, per_pose] uniforms in [0,1); row i depends only on (seed, start+i)."""
+def _uniforms(seed: int, start: int, count: int, per_pose: int, key1: int = 0) -> np.ndarray:
+    """[count, per_pose] uniforms in [0,1); row i depends only on (seed, start+i).  Philox key (seed, key1)."""
     blocks = (per_pose + 3) // 4                      # Philox4x64: 4 outputs per counter step
-    bg = np.random.Philox(key=seed)
+    bg = np.random.Philox(key=seed if key1 == 0 else np.array([seed, key1], dtype=np.uint64))
     bg.advance(start * blocks)
     raw = bg.random_raw(count * blocks * 4).reshape(count, blocks * 4)[:, :per_pose]
     return (raw >> np.uint64(11)).astype(np.float64) * (1.0 / 9007199254740992.0)
@@ -127,6 +127,35 @@ def make_batch(batch: int, rig: Rig, seed: int = 0, start: int = 0, conf_mode: s
     poses = np.concatenate([xy, conf[..., None]], axis=-1)
     return {"poses": np.ascontiguousarray(poses, dtype=dtype), "rays": np.ascontiguousarray(rays, dtype=dtype),
             "centers": np.ascontiguousarray(centers, dtype=dtype), "target": np.ascontiguousarray(target, dtype=dtype)}
+
+
+def detector_noise(pix, image_size, seed: int, start: int, sigma_px: float, p_outlier: float, p_miss: float) -> np.ndarray:
+    """Host twin of `mpl_synth_detector_noise`: the detector-error model applied to raw pixels of poses [start, start+B).
+
+    pix [B,V,J,3] (u, v, conf) as `mpl_synth_project` writes them; image_size (w, h).  Returns a perturbed float32 copy.
+    Entries with conf == 0 are kept.  Every other entry draws U0..U5 from the Philox4x64-10 stream under key (seed, 1)
+    (pose i owns counter blocks [i nb, (i+1) nb), nb = ceil(6 V J / 4), slot (v J + j) 6 + m is U_m):
+    U0 < p_miss -> conf = 0; U0 < p_miss + p_outlier -> (u, v) = (U3 (w-1), U4 (h-1)), conf = 0.3 + 0.7 U5;
+    otherwise (u, v) += sigma_px / conf * sqrt(-2 ln max(U1, 1e-12)) (cos, sin)(2 pi U2).  The parameters are rounded to
+    float32 first, as the C call receives them.
+    """
+    pix = np.asarray(pix, dtype=np.float32)
+    B, V, J, _ = pix.shape
+    w, h = (float(x) for x in image_size)
+    sigma, po, pm = (float(np.float32(x)) for x in (sigma_px, p_outlier, p_miss))
+    U = _uniforms(seed, start, B, 6 * V * J, key1=1).reshape(B, V, J, 6)
+    u, v, conf = (pix[..., k].astype(np.float64) for k in range(3))
+    live = conf != 0
+    miss = live & (U[..., 0] < pm)
+    out = live & ~miss & (U[..., 0] < pm + po)
+    noisy = live & ~miss & ~out
+    s = sigma / np.where(noisy, conf, 1.0) * np.sqrt(-2.0 * np.log(np.maximum(U[..., 1], 1e-12)))
+    theta = 2 * math.pi * U[..., 2]
+    res = pix.copy()
+    res[..., 0] = np.where(out, U[..., 3] * (w - 1), np.where(noisy, u + s * np.cos(theta), u)).astype(np.float32)
+    res[..., 1] = np.where(out, U[..., 4] * (h - 1), np.where(noisy, v + s * np.sin(theta), v)).astype(np.float32)
+    res[..., 2] = np.where(miss, 0.0, np.where(out, 0.3 + 0.7 * U[..., 5], conf)).astype(np.float32)
+    return res
 
 
 def named_weights(shapes: dict, seed: int = 0, pos_std: float = 0.02) -> dict:
