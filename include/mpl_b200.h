@@ -13,8 +13,9 @@
  *   MPL/lib/dataset/joints_dataset_mpl.py:615-648,701-715,762-772,817-820,872-904
  *                                            per-sample input construction (-> mpl_build_inputs)
  *   MPL/lib/multiviews/triangulate.py:59-115 linear triangulation baseline (-> mpl_triangulate)
- * Defined here, with no counterpart in the reference: robust (RANSAC) triangulation (mpl_triangulate_robust) and a
- * detector-error model for the synthetic data (mpl_synth_detector_noise).
+ * Defined here, with no counterpart in the reference: robust (RANSAC) triangulation (mpl_triangulate_robust), a
+ * detector-error model for the synthetic data (mpl_synth_detector_noise) and a generator of random camera setups
+ * (mpl_synth_cameras).
  *
  * Conventions
  *   - plain pointers and sizes only; no torch / C++ types cross this boundary;
@@ -23,7 +24,14 @@
  *   - all work is enqueued on the caller's stream on the caller's current device; no hidden synchronisation;
  *   - every function returns MPL_OK (0) or a negative MplStatus; mpl_last_error() gives the thread-local message;
  *   - entry points are re-entrant; a handle may be used from one thread at a time (one handle per device replica,
- *     like one nn.Module replica per GPU in the reference's DataParallel, MPL/run/valid_mpl.py:177-178).
+ *     like one nn.Module replica per GPU in the reference's DataParallel, MPL/run/valid_mpl.py:177-178);
+ *   - calibrations: every entry point that reads `calib` has a *_strided variant with an int64_t calib_stride, the number
+ *     of doubles between the [V, 18] calibration blocks of consecutive poses (like the pose_stride / center_stride of
+ *     mpl_forward).  0 = one block for the whole batch (the plain entry point, which forwards with 0); >= 18 V = pose b
+ *     uses calib + b * calib_stride (a packed [B, V, 18] tensor: 18 V).  Any other value is MPL_ERR_INVALID_ARGUMENT,
+ *     before any CUDA call.  With the same block in every pose the results are bitwise those of stride 0.  A real
+ *     validation batch mixes calibrations (the reference reads each sample's camera from its own db record,
+ *     joints_dataset_mpl.py:499-512), so it needs no splitting by camera.
  */
 #ifndef MPL_B200_H_
 #define MPL_B200_H_
@@ -35,7 +43,7 @@
 extern "C" {
 #endif
 
-#define MPL_ABI_VERSION 4
+#define MPL_ABI_VERSION 5
 
 typedef enum MplStatus {
   MPL_OK = 0,
@@ -206,6 +214,9 @@ int mpl_pmpjpe_accumulate(const float* pred, const float* gt, int64_t batch, int
  *   poses / rays [B, V, J, 3], centers [B, V, 1, 3] fp32 (packed layout accepted by mpl_forward). */
 int mpl_build_inputs(const float* pix, const double* calib, int64_t batch, int num_views, int num_joints, float* poses,
                      float* rays, float* centers, mpl_stream_t stream);
+/* mpl_build_inputs with a calibration per pose: pose b reads calib + b * calib_stride (see Conventions). */
+int mpl_build_inputs_strided(const float* pix, const double* calib, int64_t calib_stride, int64_t batch, int num_views,
+                             int num_joints, float* poses, float* rays, float* centers, mpl_stream_t stream);
 
 /* MHP-style synthetic data on the device (what MHP/utils.py:261-318 + MPL/lib/utils/calib.py:42-77 do to AMASS poses:
  * place a 3D pose in the room, project it through every calibration).  Pose i of `seed` depends only on (seed, start + i)
@@ -214,6 +225,27 @@ int mpl_build_inputs(const float* pix, const double* calib, int64_t batch, int n
  *   pix    [B, V, J, 3] fp32 raw pixels (u, v, conf) -- feed to mpl_build_inputs;  target [B, J, 3] fp32, metres. */
 int mpl_synth_project(uint64_t seed, int64_t start, int64_t batch, int num_views, int num_joints, const double* calib,
                       const double* room, int conf_ones, float* pix, float* target, mpl_stream_t stream);
+/* mpl_synth_project through a calibration per pose (calib + b * calib_stride for pose start + b; see Conventions).  The 3D
+ * poses and confidences do not depend on the calibrations. */
+int mpl_synth_project_strided(uint64_t seed, int64_t start, int64_t batch, int num_views, int num_joints, const double* calib,
+                              int64_t calib_stride, const double* room, int conf_ones, float* pix, float* target,
+                              mpl_stream_t stream);
+
+/* Random camera setups for the synthetic data (defined by this library; no reference counterpart): calib_out [B, V, 18] fp64
+ * in the row layout of mpl_build_inputs for poses [start, start + B), to be used with calib_stride 18 V.  Per (pose i,
+ * view v), U0..U5 come from the Philox4x64-10 stream of mpl_synth_project under key (seed, 2) (pose i owns counter blocks
+ * [i nb, (i + 1) nb), nb = ceil(6 V / 4); slot 6 v + m is U_m), so the result depends only on (seed, global pose index):
+ *   azimuth                 a = 2 pi (v + 0.8 (U0 - 0.5)) / V + 0.3   (each camera stays in its own sector)
+ *   horizontal distance     4.5 (0.75 + 0.5 U1) m from the look-at point;  height 0.9 + 1.2 U2 m
+ *   look-at point           room centre ((min_x + max_x) / 2, (min_y + max_y) / 2, 0.9) + (0.5 (U3 - 0.5), 0.5 (U4 - 0.5), 0)
+ *   intrinsics              fx = fy = f0 (0.8 + 0.4 U5), principal point (w / 2, h / 2), image w x h
+ *   R                       rows x, y, z: z the unit optical axis towards the look-at point, x = z x (0, 0, 1) normalised,
+ *                           y = z x x (image y down);  t = the camera position
+ * Every U = 0.5 gives the ring camera of openmpl_b200/synth.py make_rig.  fp64; room [4] fp64 on the device as in
+ * mpl_synth_project.  1 <= V <= 16, start >= 0, f0, w, h finite, f0 > 0, w > 1, h > 1.  Allocates nothing and never
+ * synchronises.  batch == 0 returns MPL_OK without touching the pointers. */
+int mpl_synth_cameras(uint64_t seed, int64_t start, int64_t batch, int num_views, double f0, double w, double h,
+                      const double* room, double* calib_out, mpl_stream_t stream);
 
 /* Linear multi-view triangulation of the same raw detections, the baseline a multi-view lifter is measured against
  * (MPL/lib/multiviews/triangulate.py:59-115, which calls pymvg's find3d once per joint): per (pose, joint), view v takes
@@ -226,6 +258,9 @@ int mpl_synth_project(uint64_t seed, int64_t start, int64_t batch, int num_views
  * Allocates nothing and never synchronises (graph-capturable).  batch == 0 returns MPL_OK without touching the pointers. */
 int mpl_triangulate(const float* pix, const double* calib, int64_t batch, int num_views, int num_joints, float min_conf,
                     float* points, int32_t* views_used, mpl_stream_t stream);
+/* mpl_triangulate with a calibration per pose (see Conventions); same argument checks plus calib_stride. */
+int mpl_triangulate_strided(const float* pix, const double* calib, int64_t calib_stride, int64_t batch, int num_views,
+                            int num_joints, float min_conf, float* points, int32_t* views_used, mpl_stream_t stream);
 
 /* Outlier-robust triangulation of the same detections: exhaustive-pair RANSAC with the MSAC cost, then a
  * confidence-weighted DLT refit (defined by this library; the reference has no robust triangulation).  Candidate views are
@@ -244,6 +279,10 @@ int mpl_triangulate(const float* pix, const double* calib, int64_t batch, int nu
  * Allocates nothing and never synchronises.  batch == 0 returns MPL_OK without touching the pointers. */
 int mpl_triangulate_robust(const float* pix, const double* calib, int64_t batch, int num_views, int num_joints,
                            float min_conf, float inlier_px, float* points, int32_t* inliers, mpl_stream_t stream);
+/* mpl_triangulate_robust with a calibration per pose (see Conventions); same argument checks plus calib_stride. */
+int mpl_triangulate_robust_strided(const float* pix, const double* calib, int64_t calib_stride, int64_t batch, int num_views,
+                                   int num_joints, float min_conf, float inlier_px, float* points, int32_t* inliers,
+                                   mpl_stream_t stream);
 
 /* Detector-error model for the synthetic pixels of mpl_synth_project, applied in place (defined by this library; the
  * reference's data carries the errors of a real detector).  pix [B, V, J, 3] (u, v, conf) of poses [start, start + B);
@@ -258,6 +297,10 @@ int mpl_triangulate_robust(const float* pix, const double* calib, int64_t batch,
  * p_miss in [0, 1] with a sum <= 1, 1 <= V <= 16, start >= 0.  batch == 0 returns MPL_OK without touching the pointers. */
 int mpl_synth_detector_noise(uint64_t seed, int64_t start, int64_t batch, int num_views, int num_joints, const double* calib,
                              float sigma_px, float p_outlier, float p_miss, float* pix, mpl_stream_t stream);
+/* mpl_synth_detector_noise with a calibration per pose (only its w, h are read; see Conventions). */
+int mpl_synth_detector_noise_strided(uint64_t seed, int64_t start, int64_t batch, int num_views, int num_joints,
+                                     const double* calib, int64_t calib_stride, float sigma_px, float p_outlier, float p_miss,
+                                     float* pix, mpl_stream_t stream);
 
 /* ---- unit-test hooks for the building blocks (used by tests/ only) ------------------------------------------- */
 /* Y[M,N] = epilogue(A[M,K] . W[N,K]^T): the tcgen05 projection kernel in isolation.

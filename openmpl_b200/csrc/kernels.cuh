@@ -202,15 +202,18 @@ int launch_mpjpe_accumulate(const float* pred, const float* gt, const float* con
                             const float* room_affine, double* acc, cudaStream_t s);
 int launch_pmpjpe_accumulate(const float* pred, const float* gt, int64_t B, int J, float unit_scale, int scaling,
                              int reflection, double* acc, cudaStream_t s);
-int launch_build_inputs(const float* pix, const double* calib, int64_t B, int V, int J, float* poses, float* rays,
-                        float* centers, cudaStream_t s);
-int launch_synth_project(uint64_t seed, int64_t start, int64_t B, int V, int J, const double* calib, const double* room,
-                         int conf_ones, float* pix, float* target, cudaStream_t s);
-int launch_triangulate(const float* pix, const double* calib, int64_t B, int V, int J, float min_conf, float* points,
-                       int32_t* views_used, cudaStream_t s);
-int launch_triangulate_robust(const float* pix, const double* calib, int64_t B, int V, int J, float min_conf,
-                              float inlier_px, float* points, int32_t* inliers, cudaStream_t s);
-int launch_detector_noise(uint64_t seed, int64_t start, int64_t B, int V, int J, const double* calib, float sigma_px,
-                          float p_outlier, float p_miss, float* pix, cudaStream_t s);
+// calib_stride: 0 = one calib [V, 18] for every pose; else pose b reads calib + b * calib_stride (>= 18 V, checked by the caller)
+int launch_build_inputs(const float* pix, const double* calib, int64_t calib_stride, int64_t B, int V, int J, float* poses,
+                        float* rays, float* centers, cudaStream_t s);
+int launch_synth_project(uint64_t seed, int64_t start, int64_t B, int V, int J, const double* calib, int64_t calib_stride,
+                         const double* room, int conf_ones, float* pix, float* target, cudaStream_t s);
+int launch_triangulate(const float* pix, const double* calib, int64_t calib_stride, int64_t B, int V, int J, float min_conf,
+                       float* points, int32_t* views_used, cudaStream_t s);
+int launch_triangulate_robust(const float* pix, const double* calib, int64_t calib_stride, int64_t B, int V, int J,
+                              float min_conf, float inlier_px, float* points, int32_t* inliers, cudaStream_t s);
+int launch_detector_noise(uint64_t seed, int64_t start, int64_t B, int V, int J, const double* calib, int64_t calib_stride,
+                          float sigma_px, float p_outlier, float p_miss, float* pix, cudaStream_t s);
+int launch_synth_cameras(uint64_t seed, int64_t start, int64_t B, int V, double f0, double w, double h, const double* room,
+                         double* calib, cudaStream_t s);
 
 }  // namespace mpl

@@ -2,8 +2,9 @@
 // and the batched input builder
 // (joints_dataset_mpl.py:615-648,701-715,762-772,817-820,872-904).  Both are HBM-bound streaming kernels.  Also the linear
 // multi-view triangulation of the same raw detections (multiviews/triangulate.py:59-115), the lifter's baseline, its
-// outlier-robust counterpart (pair RANSAC + weighted refit), the synthetic projector and a detector-error model for its
-// pixels (the last two have no reference counterpart).
+// outlier-robust counterpart (pair RANSAC + weighted refit), the synthetic projector, a detector-error model for its
+// pixels and a generator of random camera setups (the last three have no reference counterpart).  Every kernel that reads
+// calibrations is instantiated twice: one [V, 18] block for the batch (kPerPose = false) or one per pose (true).
 #include "kernels.cuh"
 
 namespace mpl {
@@ -320,15 +321,17 @@ int launch_pmpjpe_accumulate(const float* pred, const float* gt, int64_t B, int 
 
 // One thread per (pose, view, joint).  Double arithmetic in the order numpy applies it (the dataset code works in
 // float64 and casts to float32 at the end), so results are bit-identical to the reference's per-sample path.
+// kPerPose: pose b reads its calibration at calib + b * cstride; otherwise every pose reads calib [V, 18].
+template <bool kPerPose>
 __global__ void __launch_bounds__(256) build_inputs_kernel(const float* __restrict__ pix, const double* __restrict__ calib,
-                                                           int64_t B, int V, int J, float* __restrict__ poses,
+                                                           int64_t cstride, int64_t B, int V, int J, float* __restrict__ poses,
                                                            float* __restrict__ rays, float* __restrict__ centers) {
   const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   const int64_t total = B * V * J;
   if (idx >= total) return;
   const int j = (int)(idx % J);
   const int v = (int)((idx / J) % V);
-  const double* c = calib + v * 18;
+  const double* c = (kPerPose ? calib + idx / ((int64_t)V * J) * cstride : calib) + v * 18;
   const double w = c[16], h = c[17];
   double u = pix[idx * 3], vv = pix[idx * 3 + 1], conf = pix[idx * 3 + 2];
   // clip + confidence zeroing (joints_dataset_mpl.py:709-715)
@@ -411,44 +414,82 @@ __device__ __forceinline__ void eig4_jacobi(double (&S)[4][4], double (&V)[4][4]
   }
 }
 
-// Stages a block's tile of kTriTile (pose, joint) items: P_v = K_v [R_v | -R_v t_v] (row-major 3x4) and (w, h) per view,
-// and per view the (u, v, conf) of the tile's items.  Sets i0 to the tile's first item (item i = (pose i / J, joint i % J))
-// and returns the number of items in the tile.  Every thread of the block must call it (it ends with a barrier).
-__device__ __forceinline__ int tri_stage_tile(const float* __restrict__ pix, const double* __restrict__ calib, int64_t B,
-                                              int V, int J, double (&sP)[kMaxViews][12], double (&sWH)[kMaxViews][2],
-                                              float (&sx)[kMaxViews][3 * kTriTile], int64_t& i0) {
-  const int tid = threadIdx.x;
-  if (tid < V) {
-    const double* c = calib + tid * 18;
-    const double fx = c[12], fy = c[13], cx = c[14], cy = c[15];
-    double Rt[3];
+// P = K [R | -R t] (row-major 3x4) and (w, h) of one [18] calibration row.
+__device__ __forceinline__ void tri_camera(const double* __restrict__ c, double (&P)[12], double (&wh)[2]) {
+  const double fx = c[12], fy = c[13], cx = c[14], cy = c[15];
+  double Rt[3];
 #pragma unroll
-    for (int r = 0; r < 3; ++r) Rt[r] = c[3 * r] * c[9] + c[3 * r + 1] * c[10] + c[3 * r + 2] * c[11];
+  for (int r = 0; r < 3; ++r) Rt[r] = c[3 * r] * c[9] + c[3 * r + 1] * c[10] + c[3 * r + 2] * c[11];
 #pragma unroll
-    for (int k = 0; k < 3; ++k) {
-      sP[tid][k] = fx * c[k] + cx * c[6 + k];
-      sP[tid][4 + k] = fy * c[3 + k] + cy * c[6 + k];
-      sP[tid][8 + k] = c[6 + k];
-    }
-    sP[tid][3] = -(fx * Rt[0] + cx * Rt[2]);
-    sP[tid][7] = -(fy * Rt[1] + cy * Rt[2]);
-    sP[tid][11] = -Rt[2];
-    sWH[tid][0] = c[16];
-    sWH[tid][1] = c[17];
+  for (int k = 0; k < 3; ++k) {
+    P[k] = fx * c[k] + cx * c[6 + k];
+    P[4 + k] = fy * c[3 + k] + cy * c[6 + k];
+    P[8 + k] = c[6 + k];
   }
-  i0 = (int64_t)blockIdx.x * kTriTile;
-  const int n = (int)(B * J - i0 < kTriTile ? B * J - i0 : kTriTile);
+  P[3] = -(fx * Rt[0] + cx * Rt[2]);
+  P[7] = -(fy * Rt[1] + cy * Rt[2]);
+  P[11] = -Rt[2];
+  wh[0] = c[16];
+  wh[1] = c[17];
+}
+
+// Per-pose calibrations (kPerPose): a tile of T consecutive items spans at most (J + T - 2) / J + 1 poses, and each needs
+// its own V projection matrices, so they go to a dynamic shared-memory table [poses][V] of P (12 doubles), then one of
+// (w, h), next to the static pixel tile.  The launch picks the largest T <= kTriTile whose table fits the 48 KB a block
+// gets without opting in (tri_pose_tile): T = kTriTile for J = 17 and every V <= 16, T = 12 for J = 1 and V = 16.
+constexpr int kTriStaticSmem = kMaxViews * (12 + 2) * 8 + kMaxViews * 3 * kTriTile * 4;   // sP, sWH, sx
+__host__ __device__ __forceinline__ int tri_tile_poses(int T, int J) { return (J + T - 2) / J + 1; }
+
+// Stages a block's tile of T (pose, joint) items: P_v = K_v [R_v | -R_v t_v] (row-major 3x4) and (w, h) per view, and per
+// view the (u, v, conf) of the tile's items.  T = kTriTile with one calibration [V, 18] for the whole batch; with per-pose
+// calibrations T = blockDim.x and pose b's are at calib + b * cstride.  Sets i0 to the tile's first item (item i = (pose i / J,
+// joint i % J)), P / WH to the V cameras of this thread's pose, and returns the number of items in the tile.  Every thread
+// of the block must call it (it ends with a barrier).
+template <bool kPerPose>
+__device__ __forceinline__ int tri_stage_tile(const float* __restrict__ pix, const double* __restrict__ calib, int64_t cstride,
+                                              int64_t B, int V, int J, double (&sP)[kMaxViews][12],
+                                              double (&sWH)[kMaxViews][2], float (&sx)[kMaxViews][3 * kTriTile], int64_t& i0,
+                                              const double (*&P)[12], const double (*&WH)[2]) {
+  const int tid = threadIdx.x;
+  if (!kPerPose && tid < V) tri_camera(calib + tid * 18, sP[tid], sWH[tid]);
+  const int T = kPerPose ? (int)blockDim.x : kTriTile;
+  i0 = (int64_t)blockIdx.x * T;
+  const int n = (int)(B * J - i0 < T ? B * J - i0 : T);
   const int row = 3 * n;
   // float f of the tile in view v is coordinate f % 3 of item i0 + f / 3 = (pose b0 + jj / J, joint jj % J), jj = j0 + f / 3
   const int64_t b0 = i0 / J;
   const int j0 = (int)(i0 - b0 * J);
-  for (int e = tid; e < V * row; e += kTriTile) {
+  if (kPerPose) {
+    extern __shared__ double tri_cams[];
+    double(*tP)[12] = reinterpret_cast<double(*)[12]>(tri_cams);
+    double(*tWH)[2] = reinterpret_cast<double(*)[2]>(tri_cams + 12 * tri_tile_poses(T, J) * V);
+    const int np = (j0 + n - 1) / J + 1;
+    for (int e = tid; e < np * V; e += T) {
+      const int p = e / V;
+      tri_camera(calib + (b0 + p) * cstride + (e - p * V) * 18, tP[e], tWH[e]);
+    }
+    P = tP + (j0 + tid) / J * V;
+    WH = tWH + (j0 + tid) / J * V;
+  } else {
+    P = sP;
+    WH = sWH;
+  }
+  for (int e = tid; e < V * row; e += T) {
     const int v = e / row, f = e - v * row;
     const int jj = j0 + f / 3, db = jj / J;
     sx[v][f] = pix[(((b0 + db) * V + v) * J + (jj - db * J)) * 3 + f % 3];
   }
   __syncthreads();
   return n;
+}
+
+// Items per block and dynamic shared memory of the per-pose triangulation kernels.
+static int tri_pose_tile(int V, int J, size_t& smem) {
+  auto bytes = [&](int t) { return (size_t)tri_tile_poses(t, J) * V * (12 + 2) * sizeof(double); };
+  int T = kTriTile;
+  while (T > 1 && bytes(T) > (size_t)(48 * 1024 - kTriStaticSmem)) T -= T > 32 ? 32 : 1;
+  smem = bytes(T);
+  return T;
 }
 
 // The view takes part iff conf > min_conf and the pixel lies strictly inside the w x h image (build_inputs_kernel's tests).
@@ -488,24 +529,27 @@ __device__ __forceinline__ void gram_null_vector(double (&G)[4][4], double (&x)[
     }
 }
 
+template <bool kPerPose>
 __global__ void __launch_bounds__(kTriTile) triangulate_kernel(const float* __restrict__ pix, const double* __restrict__ calib,
-                                                               int64_t B, int V, int J, float min_conf,
+                                                               int64_t cstride, int64_t B, int V, int J, float min_conf,
                                                                float* __restrict__ points, int32_t* __restrict__ views_used) {
   __shared__ double sP[kMaxViews][12];
   __shared__ double sWH[kMaxViews][2];
   __shared__ float sx[kMaxViews][3 * kTriTile];
   const int tid = threadIdx.x;
   int64_t i0;
-  const int n = tri_stage_tile(pix, calib, B, V, J, sP, sWH, sx, i0);
+  const double(*P)[12];
+  const double(*WH)[2];
+  const int n = tri_stage_tile<kPerPose>(pix, calib, cstride, B, V, J, sP, sWH, sx, i0, P, WH);
   if (tid >= n) return;
   // Gram matrix A^T A, upper triangle
   double G[4][4] = {{0, 0, 0, 0}, {0, 0, 0, 0}, {0, 0, 0, 0}, {0, 0, 0, 0}};
   int used = 0;
   for (int v = 0; v < V; ++v) {
     const double u = sx[v][3 * tid], w = sx[v][3 * tid + 1];
-    if (!tri_candidate(sx[v][3 * tid + 2], u, w, min_conf, sWH[v])) continue;
+    if (!tri_candidate(sx[v][3 * tid + 2], u, w, min_conf, WH[v])) continue;
     ++used;
-    gram_add_view(G, sP[v], u, w, 1.0);
+    gram_add_view(G, P[v], u, w, 1.0);
   }
   const int64_t i = i0 + tid;
   float out[3] = {__int_as_float(0x7fc00000), __int_as_float(0x7fc00000), __int_as_float(0x7fc00000)};
@@ -520,12 +564,19 @@ __global__ void __launch_bounds__(kTriTile) triangulate_kernel(const float* __re
   views_used[i] = used;
 }
 
-int launch_triangulate(const float* pix, const double* calib, int64_t B, int V, int J, float min_conf, float* points,
-                       int32_t* views_used, cudaStream_t s) {
+int launch_triangulate(const float* pix, const double* calib, int64_t calib_stride, int64_t B, int V, int J, float min_conf,
+                       float* points, int32_t* views_used, cudaStream_t s) {
   const int64_t items = B * J;
   if (items == 0) return MPL_OK;
-  triangulate_kernel<<<(unsigned)ceil_div(items, kTriTile), kTriTile, 0, s>>>(pix, calib, B, V, J, min_conf, points,
-                                                                               views_used);
+  if (calib_stride == 0) {
+    triangulate_kernel<false><<<(unsigned)ceil_div(items, kTriTile), kTriTile, 0, s>>>(pix, calib, 0, B, V, J, min_conf,
+                                                                                      points, views_used);
+  } else {
+    size_t smem;
+    const int T = tri_pose_tile(V, J, smem);
+    triangulate_kernel<true><<<(unsigned)ceil_div(items, (int64_t)T), T, smem, s>>>(pix, calib, calib_stride, B, V, J,
+                                                                                   min_conf, points, views_used);
+  }
   MPL_LAUNCH_CHECK();
   return MPL_OK;
 }
@@ -550,9 +601,10 @@ __device__ __forceinline__ double reproj_err2(const double (&P)[12], const doubl
   return du * du + dv * dv;
 }
 
+template <bool kPerPose>
 __global__ void __launch_bounds__(kTriTile) triangulate_robust_kernel(const float* __restrict__ pix,
-                                                                      const double* __restrict__ calib, int64_t B, int V,
-                                                                      int J, float min_conf, float inlier_px,
+                                                                      const double* __restrict__ calib, int64_t cstride, int64_t B,
+                                                                      int V, int J, float min_conf, float inlier_px,
                                                                       float* __restrict__ points,
                                                                       int32_t* __restrict__ inliers) {
   __shared__ double sP[kMaxViews][12];
@@ -560,11 +612,13 @@ __global__ void __launch_bounds__(kTriTile) triangulate_robust_kernel(const floa
   __shared__ float sx[kMaxViews][3 * kTriTile];
   const int tid = threadIdx.x;
   int64_t i0;
-  const int n = tri_stage_tile(pix, calib, B, V, J, sP, sWH, sx, i0);
+  const double(*P)[12];
+  const double(*WH)[2];
+  const int n = tri_stage_tile<kPerPose>(pix, calib, cstride, B, V, J, sP, sWH, sx, i0, P, WH);
   if (tid >= n) return;
   unsigned cand = 0;                                       // bit v: view v is a candidate
   for (int v = 0; v < V; ++v)
-    if (tri_candidate(sx[v][3 * tid + 2], sx[v][3 * tid], sx[v][3 * tid + 1], min_conf, sWH[v])) cand |= 1u << v;
+    if (tri_candidate(sx[v][3 * tid + 2], sx[v][3 * tid], sx[v][3 * tid + 1], min_conf, WH[v])) cand |= 1u << v;
   const double tau2 = (double)inlier_px * (double)inlier_px;
   unsigned inl = 0;
   float out[3] = {__int_as_float(0x7fc00000), __int_as_float(0x7fc00000), __int_as_float(0x7fc00000)};
@@ -575,14 +629,14 @@ __global__ void __launch_bounds__(kTriTile) triangulate_robust_kernel(const floa
       for (unsigned mb = ma & (ma - 1); mb; mb &= mb - 1) {
         const int b = __ffs(mb) - 1;
         double G[4][4] = {{0, 0, 0, 0}, {0, 0, 0, 0}, {0, 0, 0, 0}, {0, 0, 0, 0}};
-        gram_add_view(G, sP[a], sx[a][3 * tid], sx[a][3 * tid + 1], 1.0);
-        gram_add_view(G, sP[b], sx[b][3 * tid], sx[b][3 * tid + 1], 1.0);
+        gram_add_view(G, P[a], sx[a][3 * tid], sx[a][3 * tid + 1], 1.0);
+        gram_add_view(G, P[b], sx[b][3 * tid], sx[b][3 * tid + 1], 1.0);
         double x[4];
         gram_null_vector(G, x);
         double cost = 0.0;                                 // MSAC; fmin maps an infinite (or NaN) error to tau^2
         for (unsigned mc = cand; mc; mc &= mc - 1) {
           const int c = __ffs(mc) - 1;
-          cost += fmin(reproj_err2(sP[c], x, sx[c][3 * tid], sx[c][3 * tid + 1]), tau2);
+          cost += fmin(reproj_err2(P[c], x, sx[c][3 * tid], sx[c][3 * tid + 1]), tau2);
         }
         if (cost < best) {
           best = cost;
@@ -593,13 +647,13 @@ __global__ void __launch_bounds__(kTriTile) triangulate_robust_kernel(const floa
     }
     for (unsigned mc = cand; mc; mc &= mc - 1) {
       const int c = __ffs(mc) - 1;
-      if (reproj_err2(sP[c], xb, sx[c][3 * tid], sx[c][3 * tid + 1]) < tau2) inl |= 1u << c;
+      if (reproj_err2(P[c], xb, sx[c][3 * tid], sx[c][3 * tid + 1]) < tau2) inl |= 1u << c;
     }
     if (__popc(inl) >= 2) {
       // refit in triangulate_kernel's view order, rows scaled by conf (the ML weighting when the pixel noise is sigma / conf)
       double G[4][4] = {{0, 0, 0, 0}, {0, 0, 0, 0}, {0, 0, 0, 0}, {0, 0, 0, 0}};
       for (int v = 0; v < V; ++v)
-        if ((inl >> v) & 1u) gram_add_view(G, sP[v], sx[v][3 * tid], sx[v][3 * tid + 1], (double)sx[v][3 * tid + 2]);
+        if ((inl >> v) & 1u) gram_add_view(G, P[v], sx[v][3 * tid], sx[v][3 * tid + 1], (double)sx[v][3 * tid + 2]);
       double x[4];
       gram_null_vector(G, x);
 #pragma unroll
@@ -614,12 +668,19 @@ __global__ void __launch_bounds__(kTriTile) triangulate_robust_kernel(const floa
   inliers[i] = (int32_t)inl;
 }
 
-int launch_triangulate_robust(const float* pix, const double* calib, int64_t B, int V, int J, float min_conf,
-                              float inlier_px, float* points, int32_t* inliers, cudaStream_t s) {
+int launch_triangulate_robust(const float* pix, const double* calib, int64_t calib_stride, int64_t B, int V, int J,
+                              float min_conf, float inlier_px, float* points, int32_t* inliers, cudaStream_t s) {
   const int64_t items = B * J;
   if (items == 0) return MPL_OK;
-  triangulate_robust_kernel<<<(unsigned)ceil_div(items, kTriTile), kTriTile, 0, s>>>(pix, calib, B, V, J, min_conf,
-                                                                                      inlier_px, points, inliers);
+  if (calib_stride == 0) {
+    triangulate_robust_kernel<false><<<(unsigned)ceil_div(items, kTriTile), kTriTile, 0, s>>>(
+        pix, calib, 0, B, V, J, min_conf, inlier_px, points, inliers);
+  } else {
+    size_t smem;
+    const int T = tri_pose_tile(V, J, smem);
+    triangulate_robust_kernel<true><<<(unsigned)ceil_div(items, (int64_t)T), T, smem, s>>>(
+        pix, calib, calib_stride, B, V, J, min_conf, inlier_px, points, inliers);
+  }
   MPL_LAUNCH_CHECK();
   return MPL_OK;
 }
@@ -658,11 +719,14 @@ struct UniformCursor {  // sequential reader of one pose's uniform stream with a
   }
 };
 
+template <bool kPerPose>
 __global__ void __launch_bounds__(128) synth_project_kernel(uint64_t seed, int64_t start, int64_t B, int V, int J,
-                                                            const double* __restrict__ calib, const double* __restrict__ room,
-                                                            int conf_ones, float* __restrict__ pix, float* __restrict__ target) {
+                                                            const double* __restrict__ calib, int64_t cstride,
+                                                            const double* __restrict__ room, int conf_ones,
+                                                            float* __restrict__ pix, float* __restrict__ target) {
   const int64_t b = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= B) return;
+  const double* cal = kPerPose ? calib + b * cstride : calib;
   const int n = 3 * (J - 1);
   const int per_pose = 3 + 2 * n + V * J;
   const uint64_t blocks = (uint64_t)((per_pose + 3) / 4);
@@ -688,7 +752,7 @@ __global__ void __launch_bounds__(128) synth_project_kernel(uint64_t seed, int64
       tg[j * 3 + k] = (float)X[k];
     }
     for (int v = 0; v < V; ++v) {
-      const double* c = calib + v * 18;
+      const double* c = cal + v * 18;
       double xc[3];
 #pragma unroll
       for (int r = 0; r < 3; ++r)
@@ -702,10 +766,14 @@ __global__ void __launch_bounds__(128) synth_project_kernel(uint64_t seed, int64
   }
 }
 
-int launch_synth_project(uint64_t seed, int64_t start, int64_t B, int V, int J, const double* calib, const double* room,
-                         int conf_ones, float* pix, float* target, cudaStream_t s) {
+int launch_synth_project(uint64_t seed, int64_t start, int64_t B, int V, int J, const double* calib, int64_t calib_stride,
+                         const double* room, int conf_ones, float* pix, float* target, cudaStream_t s) {
   if (B == 0) return MPL_OK;
-  synth_project_kernel<<<(unsigned)ceil_div(B, 128), 128, 0, s>>>(seed, start, B, V, J, calib, room, conf_ones, pix, target);
+  const unsigned grid = (unsigned)ceil_div(B, 128);
+  if (calib_stride == 0)
+    synth_project_kernel<false><<<grid, 128, 0, s>>>(seed, start, B, V, J, calib, 0, room, conf_ones, pix, target);
+  else
+    synth_project_kernel<true><<<grid, 128, 0, s>>>(seed, start, B, V, J, calib, calib_stride, room, conf_ones, pix, target);
   MPL_LAUNCH_CHECK();
   return MPL_OK;
 }
@@ -720,8 +788,25 @@ int launch_synth_project(uint64_t seed, int64_t start, int64_t B, int V, int J, 
 //   otherwise                         -> (u, v) += sigma / conf * r (cos t, sin t), r = sqrt(-2 ln max(U1, 1e-12)), t = 2 pi U2
 // fp64 throughout, rounded once to fp32.  The outlier and threshold arithmetic is written with explicit roundings so it
 // matches numpy bit for bit.
+// Uniforms U0..U5 of record r of pose (start + b) under Philox key (seed, key1), six per record: pose i owns counter blocks
+// [i nb, (i + 1) nb), nb = ceil(6 records / 4), and slot 6 r + m is U_m.
+__device__ __forceinline__ void six_uniforms(uint64_t seed, uint64_t key1, int64_t start, int64_t b, int records, int r,
+                                             double (&U)[6]) {
+  const uint64_t base = (uint64_t)(start + b) * (uint64_t)((6 * records + 3) / 4);
+  const int s0 = 6 * r;                                    // slot of U0; s0 % 4 is 0 or 2, so U0..U5 span two blocks
+  uint64_t lo[4], hi[4];
+  philox4x64_10(base + (uint64_t)(s0 >> 2) + 1ull, seed, key1, lo);  // numpy increments the counter before generating
+  philox4x64_10(base + (uint64_t)(s0 >> 2) + 2ull, seed, key1, hi);
+  const bool al = (s0 & 3) == 0;
+  const uint64_t raw[6] = {al ? lo[0] : lo[2], al ? lo[1] : lo[3], al ? lo[2] : hi[0],
+                           al ? lo[3] : hi[1], al ? hi[0] : hi[2], al ? hi[1] : hi[3]};
+#pragma unroll
+  for (int m = 0; m < 6; ++m) U[m] = (double)(raw[m] >> 11) * (1.0 / 9007199254740992.0);
+}
+
+template <bool kPerPose>
 __global__ void __launch_bounds__(256) detector_noise_kernel(uint64_t seed, int64_t start, int64_t B, int V, int J,
-                                                             const double* __restrict__ calib, float sigma_px,
+                                                             const double* __restrict__ calib, int64_t cstride, float sigma_px,
                                                              float p_outlier, float p_miss, float* __restrict__ pix) {
   const int per = V * J;
   const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -731,24 +816,15 @@ __global__ void __launch_bounds__(256) detector_noise_kernel(uint64_t seed, int6
   if (conf == 0.0f) return;
   const int64_t b = e / per;
   const int r = (int)(e - b * per);                        // v J + j
-  const uint64_t base = (uint64_t)(start + b) * (uint64_t)((6 * per + 3) / 4);
-  const int s0 = 6 * r;                                    // slot of U0; s0 % 4 is 0 or 2, so U0..U5 span two blocks
-  uint64_t lo[4], hi[4];
-  philox4x64_10(base + (uint64_t)(s0 >> 2) + 1ull, seed, 1ull, lo);  // numpy increments the counter before generating
-  philox4x64_10(base + (uint64_t)(s0 >> 2) + 2ull, seed, 1ull, hi);
-  const bool al = (s0 & 3) == 0;
-  const uint64_t raw[6] = {al ? lo[0] : lo[2], al ? lo[1] : lo[3], al ? lo[2] : hi[0],
-                           al ? lo[3] : hi[1], al ? hi[0] : hi[2], al ? hi[1] : hi[3]};
   double U[6];
-#pragma unroll
-  for (int m = 0; m < 6; ++m) U[m] = (double)(raw[m] >> 11) * (1.0 / 9007199254740992.0);
+  six_uniforms(seed, 1ull, start, b, per, r, U);
   const double pm = (double)p_miss;
   if (U[0] < pm) {
     p[2] = 0.0f;
     return;
   }
   if (U[0] < __dadd_rn(pm, (double)p_outlier)) {
-    const double* c = calib + (r / J) * 18;
+    const double* c = (kPerPose ? calib + b * cstride : calib) + (r / J) * 18;
     p[0] = (float)__dmul_rn(U[3], c[16] - 1.0);
     p[1] = (float)__dmul_rn(U[4], c[17] - 1.0);
     p[2] = (float)__dadd_rn(0.3, __dmul_rn(0.7, U[5]));
@@ -761,21 +837,84 @@ __global__ void __launch_bounds__(256) detector_noise_kernel(uint64_t seed, int6
   p[1] = (float)((double)p[1] + s * sn);
 }
 
-int launch_detector_noise(uint64_t seed, int64_t start, int64_t B, int V, int J, const double* calib, float sigma_px,
-                          float p_outlier, float p_miss, float* pix, cudaStream_t s) {
+int launch_detector_noise(uint64_t seed, int64_t start, int64_t B, int V, int J, const double* calib, int64_t calib_stride,
+                          float sigma_px, float p_outlier, float p_miss, float* pix, cudaStream_t s) {
   const int64_t total = B * V * J;
   if (total == 0) return MPL_OK;
-  detector_noise_kernel<<<(unsigned)ceil_div(total, 256), 256, 0, s>>>(seed, start, B, V, J, calib, sigma_px, p_outlier,
-                                                                       p_miss, pix);
+  const unsigned grid = (unsigned)ceil_div(total, 256);
+  if (calib_stride == 0)
+    detector_noise_kernel<false><<<grid, 256, 0, s>>>(seed, start, B, V, J, calib, 0, sigma_px, p_outlier, p_miss, pix);
+  else
+    detector_noise_kernel<true><<<grid, 256, 0, s>>>(seed, start, B, V, J, calib, calib_stride, sigma_px, p_outlier, p_miss,
+                                                     pix);
   MPL_LAUNCH_CHECK();
   return MPL_OK;
 }
 
-int launch_build_inputs(const float* pix, const double* calib, int64_t B, int V, int J, float* poses, float* rays,
-                        float* centers, cudaStream_t s) {
+// ---- random camera setups: one thread per (pose, view), fp64 ------------------------------------------------------------
+// U0..U5 of (pose i, view v) come from the Philox4x64-10 stream of synth_project_kernel under key (seed, 2), with the slot
+// layout of the detector-noise model (pose i owns counter blocks [i nb, (i + 1) nb), nb = ceil(6 V / 4), slot 6 v + m is
+// U_m), so a pose's cameras depend only on (seed, global pose index).  openmpl_b200/synth.py (random_cameras) is the twin.
+//   azimuth a = 2 pi (v + 0.8 (U0 - 0.5)) / V + 0.3 (each camera stays in its sector), horizontal distance from the look-at
+//   point 4.5 (0.75 + 0.5 U1), height 0.9 + 1.2 U2, look-at point = room centre at height 0.9 shifted by 0.5 (U3 - 0.5) in x
+//   and 0.5 (U4 - 0.5) in y, fx = fy = f0 (0.8 + 0.4 U5), principal point at the image centre, R the look-at rotation of
+//   synth.make_rig.  Every U = 0.5 gives make_rig's camera.
+__global__ void __launch_bounds__(128) synth_cameras_kernel(uint64_t seed, int64_t start, int64_t B, int V, double f0,
+                                                            double w, double h, const double* __restrict__ room,
+                                                            double* __restrict__ calib) {
+  const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= B * V) return;
+  const int64_t b = e / V;
+  const int v = (int)(e - b * V);
+  double U[6];
+  six_uniforms(seed, 2ull, start, b, V, v, U);
+  double sn, cs;
+  sincospi(2.0 * (v + 0.8 * (U[0] - 0.5)) / V + 0.3 / 3.14159265358979323846, &sn, &cs);  // sincos's reduction needs a stack frame
+  const double dist = 4.5 * (0.75 + 0.5 * U[1]);
+  const double at[3] = {0.5 * (room[0] + room[1]) + 0.5 * (U[3] - 0.5), 0.5 * (room[2] + room[3]) + 0.5 * (U[4] - 0.5), 0.9};
+  const double pos[3] = {at[0] + dist * cs, at[1] + dist * sn, 0.9 + 1.2 * U[2]};
+  double z[3] = {at[0] - pos[0], at[1] - pos[1], at[2] - pos[2]};
+  const double zn = sqrt(z[0] * z[0] + z[1] * z[1] + z[2] * z[2]);
+#pragma unroll
+  for (int k = 0; k < 3; ++k) z[k] /= zn;
+  const double xn = sqrt(z[1] * z[1] + z[0] * z[0]);
+  const double x[3] = {z[1] / xn, -z[0] / xn, 0.0};                                    // z x (0, 0, 1)
+  const double y[3] = {z[1] * x[2] - z[2] * x[1], z[2] * x[0] - z[0] * x[2], z[0] * x[1] - z[1] * x[0]};  // z x x
+  const double f = f0 * (0.8 + 0.4 * U[5]);
+  double* c = calib + e * 18;
+#pragma unroll
+  for (int k = 0; k < 3; ++k) {
+    c[k] = x[k];
+    c[3 + k] = y[k];
+    c[6 + k] = z[k];
+    c[9 + k] = pos[k];
+  }
+  c[12] = f;
+  c[13] = f;
+  c[14] = w / 2.0;
+  c[15] = h / 2.0;
+  c[16] = w;
+  c[17] = h;
+}
+
+int launch_synth_cameras(uint64_t seed, int64_t start, int64_t B, int V, double f0, double w, double h, const double* room,
+                         double* calib, cudaStream_t s) {
+  const int64_t total = B * V;
+  if (total == 0) return MPL_OK;
+  synth_cameras_kernel<<<(unsigned)ceil_div(total, 128), 128, 0, s>>>(seed, start, B, V, f0, w, h, room, calib);
+  MPL_LAUNCH_CHECK();
+  return MPL_OK;
+}
+
+int launch_build_inputs(const float* pix, const double* calib, int64_t calib_stride, int64_t B, int V, int J, float* poses,
+                        float* rays, float* centers, cudaStream_t s) {
   const int64_t total = B * V * J;
   if (total == 0) return MPL_OK;
-  build_inputs_kernel<<<(unsigned)ceil_div(total, 256), 256, 0, s>>>(pix, calib, B, V, J, poses, rays, centers);
+  const unsigned grid = (unsigned)ceil_div(total, 256);
+  if (calib_stride == 0)
+    build_inputs_kernel<false><<<grid, 256, 0, s>>>(pix, calib, 0, B, V, J, poses, rays, centers);
+  else
+    build_inputs_kernel<true><<<grid, 256, 0, s>>>(pix, calib, calib_stride, B, V, J, poses, rays, centers);
   MPL_LAUNCH_CHECK();
   return MPL_OK;
 }

@@ -1312,77 +1312,139 @@ int mpl_pmpjpe_accumulate(const float* pred, const float* gt, int64_t batch, int
                                   reinterpret_cast<cudaStream_t>(stream));
 }
 
+// calib_stride of the *_strided entry points: 0 (one [V, 18] block for every pose) or >= 18 V (pose b at calib + b * stride)
+static bool calib_stride_ok(int64_t calib_stride, int num_views) {
+  return calib_stride == 0 || (calib_stride > 0 && calib_stride >= 18 * (int64_t)num_views);
+}
+
 int mpl_build_inputs(const float* pix, const double* calib, int64_t batch, int num_views, int num_joints, float* poses,
                      float* rays, float* centers, mpl_stream_t stream) {
-  if (batch == 0) return MPL_OK;
-  if (pix == nullptr || calib == nullptr || poses == nullptr || rays == nullptr || centers == nullptr || batch < 0) {
-    set_error("mpl_build_inputs: bad argument");
+  return mpl_build_inputs_strided(pix, calib, 0, batch, num_views, num_joints, poses, rays, centers, stream);
+}
+
+int mpl_build_inputs_strided(const float* pix, const double* calib, int64_t calib_stride, int64_t batch, int num_views,
+                             int num_joints, float* poses, float* rays, float* centers, mpl_stream_t stream) {
+  if (!calib_stride_ok(calib_stride, num_views)) {
+    set_error("mpl_build_inputs_strided: bad calib_stride %lld (0, or >= 18 * num_views)", (long long)calib_stride);
     return MPL_ERR_INVALID_ARGUMENT;
   }
-  return launch_build_inputs(pix, calib, batch, num_views, num_joints, poses, rays, centers, reinterpret_cast<cudaStream_t>(stream));
+  if (batch == 0) return MPL_OK;
+  if (pix == nullptr || calib == nullptr || poses == nullptr || rays == nullptr || centers == nullptr || batch < 0) {
+    set_error("mpl_build_inputs_strided: bad argument");
+    return MPL_ERR_INVALID_ARGUMENT;
+  }
+  return launch_build_inputs(pix, calib, calib_stride, batch, num_views, num_joints, poses, rays, centers,
+                             reinterpret_cast<cudaStream_t>(stream));
 }
 
 int mpl_synth_project(uint64_t seed, int64_t start, int64_t batch, int num_views, int num_joints, const double* calib,
                       const double* room, int conf_ones, float* pix, float* target, mpl_stream_t stream) {
+  return mpl_synth_project_strided(seed, start, batch, num_views, num_joints, calib, 0, room, conf_ones, pix, target, stream);
+}
+
+int mpl_synth_project_strided(uint64_t seed, int64_t start, int64_t batch, int num_views, int num_joints, const double* calib,
+                              int64_t calib_stride, const double* room, int conf_ones, float* pix, float* target,
+                              mpl_stream_t stream) {
+  if (!calib_stride_ok(calib_stride, num_views)) {
+    set_error("mpl_synth_project_strided: bad calib_stride %lld (0, or >= 18 * num_views)", (long long)calib_stride);
+    return MPL_ERR_INVALID_ARGUMENT;
+  }
   if (batch == 0) return MPL_OK;
   if (calib == nullptr || room == nullptr || pix == nullptr || target == nullptr || batch < 0 || start < 0 || num_views < 1 ||
       num_joints < 1) {
-    set_error("mpl_synth_project: bad argument");
+    set_error("mpl_synth_project_strided: bad argument");
     return MPL_ERR_INVALID_ARGUMENT;
   }
-  return launch_synth_project(seed, start, batch, num_views, num_joints, calib, room, conf_ones, pix, target,
+  return launch_synth_project(seed, start, batch, num_views, num_joints, calib, calib_stride, room, conf_ones, pix, target,
                               reinterpret_cast<cudaStream_t>(stream));
 }
 
 int mpl_triangulate(const float* pix, const double* calib, int64_t batch, int num_views, int num_joints, float min_conf,
                     float* points, int32_t* views_used, mpl_stream_t stream) {
-  if (batch < 0 || num_views < 1 || num_views > kMaxViews || num_joints < 1) {
-    set_error("mpl_triangulate: bad argument (batch %lld, num_views %d, num_joints %d)", (long long)batch, num_views, num_joints);
+  return mpl_triangulate_strided(pix, calib, 0, batch, num_views, num_joints, min_conf, points, views_used, stream);
+}
+
+int mpl_triangulate_strided(const float* pix, const double* calib, int64_t calib_stride, int64_t batch, int num_views,
+                            int num_joints, float min_conf, float* points, int32_t* views_used, mpl_stream_t stream) {
+  if (batch < 0 || num_views < 1 || num_views > kMaxViews || num_joints < 1 || !calib_stride_ok(calib_stride, num_views)) {
+    set_error("mpl_triangulate_strided: bad argument (batch %lld, num_views %d, num_joints %d, calib_stride %lld)",
+              (long long)batch, num_views, num_joints, (long long)calib_stride);
     return MPL_ERR_INVALID_ARGUMENT;
   }
   if (batch == 0) return MPL_OK;
   if (pix == nullptr || calib == nullptr || points == nullptr || views_used == nullptr) {
-    set_error("mpl_triangulate: null pointer");
+    set_error("mpl_triangulate_strided: null pointer");
     return MPL_ERR_INVALID_ARGUMENT;
   }
-  return launch_triangulate(pix, calib, batch, num_views, num_joints, min_conf, points, views_used,
+  return launch_triangulate(pix, calib, calib_stride, batch, num_views, num_joints, min_conf, points, views_used,
                             reinterpret_cast<cudaStream_t>(stream));
 }
 
 int mpl_triangulate_robust(const float* pix, const double* calib, int64_t batch, int num_views, int num_joints,
                            float min_conf, float inlier_px, float* points, int32_t* inliers, mpl_stream_t stream) {
-  if (batch < 0 || num_views < 1 || num_views > kMaxViews || num_joints < 1 || !std::isfinite(inlier_px) || !(inlier_px > 0.0f)) {
-    set_error("mpl_triangulate_robust: bad argument (batch %lld, num_views %d, num_joints %d, inlier_px %g)", (long long)batch,
-              num_views, num_joints, (double)inlier_px);
+  return mpl_triangulate_robust_strided(pix, calib, 0, batch, num_views, num_joints, min_conf, inlier_px, points, inliers,
+                                        stream);
+}
+
+int mpl_triangulate_robust_strided(const float* pix, const double* calib, int64_t calib_stride, int64_t batch, int num_views,
+                                   int num_joints, float min_conf, float inlier_px, float* points, int32_t* inliers,
+                                   mpl_stream_t stream) {
+  if (batch < 0 || num_views < 1 || num_views > kMaxViews || num_joints < 1 || !std::isfinite(inlier_px) || !(inlier_px > 0.0f) ||
+      !calib_stride_ok(calib_stride, num_views)) {
+    set_error("mpl_triangulate_robust_strided: bad argument (batch %lld, num_views %d, num_joints %d, inlier_px %g, "
+              "calib_stride %lld)", (long long)batch, num_views, num_joints, (double)inlier_px, (long long)calib_stride);
     return MPL_ERR_INVALID_ARGUMENT;
   }
   if (batch == 0) return MPL_OK;
   if (pix == nullptr || calib == nullptr || points == nullptr || inliers == nullptr) {
-    set_error("mpl_triangulate_robust: null pointer");
+    set_error("mpl_triangulate_robust_strided: null pointer");
     return MPL_ERR_INVALID_ARGUMENT;
   }
-  return launch_triangulate_robust(pix, calib, batch, num_views, num_joints, min_conf, inlier_px, points, inliers,
+  return launch_triangulate_robust(pix, calib, calib_stride, batch, num_views, num_joints, min_conf, inlier_px, points, inliers,
                                    reinterpret_cast<cudaStream_t>(stream));
 }
 
 int mpl_synth_detector_noise(uint64_t seed, int64_t start, int64_t batch, int num_views, int num_joints, const double* calib,
                              float sigma_px, float p_outlier, float p_miss, float* pix, mpl_stream_t stream) {
+  return mpl_synth_detector_noise_strided(seed, start, batch, num_views, num_joints, calib, 0, sigma_px, p_outlier, p_miss, pix,
+                                          stream);
+}
+
+int mpl_synth_detector_noise_strided(uint64_t seed, int64_t start, int64_t batch, int num_views, int num_joints,
+                                     const double* calib, int64_t calib_stride, float sigma_px, float p_outlier, float p_miss,
+                                     float* pix, mpl_stream_t stream) {
   // the probabilities' sum in fp64, as the kernel forms it
   if (batch < 0 || start < 0 || num_views < 1 || num_views > kMaxViews || num_joints < 1 || !std::isfinite(sigma_px) ||
       !(sigma_px >= 0.0f) || !(p_outlier >= 0.0f && p_outlier <= 1.0f) || !(p_miss >= 0.0f && p_miss <= 1.0f) ||
-      !((double)p_outlier + (double)p_miss <= 1.0)) {
-    set_error("mpl_synth_detector_noise: bad argument (batch %lld, start %lld, num_views %d, num_joints %d, sigma_px %g, "
-              "p_outlier %g, p_miss %g)", (long long)batch, (long long)start, num_views, num_joints, (double)sigma_px,
-              (double)p_outlier, (double)p_miss);
+      !((double)p_outlier + (double)p_miss <= 1.0) || !calib_stride_ok(calib_stride, num_views)) {
+    set_error("mpl_synth_detector_noise_strided: bad argument (batch %lld, start %lld, num_views %d, num_joints %d, "
+              "sigma_px %g, p_outlier %g, p_miss %g, calib_stride %lld)", (long long)batch, (long long)start, num_views,
+              num_joints, (double)sigma_px, (double)p_outlier, (double)p_miss, (long long)calib_stride);
     return MPL_ERR_INVALID_ARGUMENT;
   }
   if (batch == 0) return MPL_OK;
   if (calib == nullptr || pix == nullptr) {
-    set_error("mpl_synth_detector_noise: null pointer");
+    set_error("mpl_synth_detector_noise_strided: null pointer");
     return MPL_ERR_INVALID_ARGUMENT;
   }
-  return launch_detector_noise(seed, start, batch, num_views, num_joints, calib, sigma_px, p_outlier, p_miss, pix,
-                               reinterpret_cast<cudaStream_t>(stream));
+  return launch_detector_noise(seed, start, batch, num_views, num_joints, calib, calib_stride, sigma_px, p_outlier, p_miss,
+                               pix, reinterpret_cast<cudaStream_t>(stream));
+}
+
+int mpl_synth_cameras(uint64_t seed, int64_t start, int64_t batch, int num_views, double f0, double w, double h,
+                      const double* room, double* calib_out, mpl_stream_t stream) {
+  if (batch < 0 || start < 0 || num_views < 1 || num_views > kMaxViews || !std::isfinite(f0) || !(f0 > 0.0) ||
+      !std::isfinite(w) || !(w > 1.0) || !std::isfinite(h) || !(h > 1.0)) {
+    set_error("mpl_synth_cameras: bad argument (batch %lld, start %lld, num_views %d, f0 %g, w %g, h %g)", (long long)batch,
+              (long long)start, num_views, f0, w, h);
+    return MPL_ERR_INVALID_ARGUMENT;
+  }
+  if (batch == 0) return MPL_OK;
+  if (room == nullptr || calib_out == nullptr) {
+    set_error("mpl_synth_cameras: null pointer");
+    return MPL_ERR_INVALID_ARGUMENT;
+  }
+  return launch_synth_cameras(seed, start, batch, num_views, f0, w, h, room, calib_out, reinterpret_cast<cudaStream_t>(stream));
 }
 
 int mpl_test_gemm(const void* A, const void* W, const float* bias, void* Y, int64_t M, int N, int K, int dtype, int epilogue,

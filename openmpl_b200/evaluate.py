@@ -7,6 +7,7 @@
     python -m openmpl_b200.evaluate --arch hm0 --views 4 --triangulate                   # + the triangulation baseline
     python -m openmpl_b200.evaluate --arch hm0 --views 4 --pixel-noise 2 --outlier-rate 0.1 --triangulate \
         --triangulate-robust                                                            # noisy detections, both baselines
+    python -m openmpl_b200.evaluate --arch hm0 --views 4 --random-cameras --triangulate  # a random camera setup per pose
 
 Per micro-batch, entirely on the device: `mpl_synth_project` (3D poses from the counter-based generator keyed by the
 GLOBAL pose index, projected through the V calibrations) -> `mpl_build_inputs` (clip, confidence zeroing, screen
@@ -24,6 +25,11 @@ views; the line gains a "triangulation" entry.  Without the flag nothing of this
 index like the poses), so the lifter and the triangulations all see the same detections; the line's "data" entry records
 the three values.  `--triangulate-robust` adds a "triangulation_robust" entry for `mpl_triangulate_robust` (pair RANSAC
 with the MSAC cost at `--inlier-px`, then a confidence-weighted refit), masked where it finds fewer than two inliers.
+
+`--random-cameras` gives every pose its own camera setup: each micro-batch first generates [B, V, 18] calibrations
+(`mpl_synth_cameras`, random positions, heights, look-at points and focal lengths around the room of the rig kind, keyed
+by the global pose index), then projects, corrupts, builds inputs and triangulates through them.  The line's "data" entry
+records the camera model.  Without the flag the one rig of `--rig` serves every pose.
 """
 from __future__ import annotations
 
@@ -48,7 +54,7 @@ DEFAULT_RIG = {"hm0": "h36m", "chosen": "h36m", "kptok": "h36m", "cmu0": "cmu"}
 
 def run(arch="hm0", views=4, depth=None, poses=1 << 20, micro_batch=65536, precision="bf16", rig=None, seed=1,
         weight_seed=0, warmup=1, triangulate=False, pixel_noise=0.0, outlier_rate=0.0, miss_rate=0.0,
-        triangulate_robust=False, inlier_px=10.0):
+        triangulate_robust=False, inlier_px=10.0, random_cameras=False):
     rank, world, local = mdist.init_from_env("nccl")
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
@@ -60,7 +66,8 @@ def run(arch="hm0", views=4, depth=None, poses=1 << 20, micro_batch=65536, preci
     model.load_state_dict({k: torch.from_numpy(v) for k, v in weights.items()})
     model = model.to(dev).eval()
     mdist.broadcast_state(model)                       # replicas bit-identical (they already are: same seed)
-    the_rig = synth.make_rig(views, rig or DEFAULT_RIG[arch])
+    rig_kind = rig or DEFAULT_RIG[arch]
+    the_rig = synth.make_rig(views, rig_kind)
     start, stop = mdist.shard_range(poses, rank, world)
     acc = metric.MpjpeAccumulator(cfg.J, output_in_meter=True, device=dev)
     pacc = metric.PmpjpeAccumulator(cfg.J, output_in_meter=True, device=dev)
@@ -69,7 +76,8 @@ def run(arch="hm0", views=4, depth=None, poses=1 << 20, micro_batch=65536, preci
     noisy = pixel_noise != 0 or outlier_rate != 0 or miss_rate != 0
 
     def step(s0, n):
-        pix, target, calib = inputs.synth_project(n, the_rig, seed=seed, start=s0, device=dev)
+        cams = inputs.synth_cameras(n, views, rig_kind, seed=seed, start=s0, device=dev) if random_cameras else None
+        pix, target, calib = inputs.synth_project(n, the_rig, seed=seed, start=s0, device=dev, cameras=cams)
         if noisy:
             inputs.add_detector_noise(pix, calib, seed, s0, pixel_noise, outlier_rate, miss_rate)
         p, r, c = inputs.build_inputs(pix, calib)
@@ -125,6 +133,14 @@ def run(arch="hm0", views=4, depth=None, poses=1 << 20, micro_batch=65536, preci
                             "miss_rate": miss_rate,
                             "noise_model": "Gaussian of std pixel_noise_px / conf; outliers uniform in the image with conf "
                                            "0.3-1; misses set conf 0"}
+        if random_cameras:
+            if not isinstance(line["data"], dict):
+                line["data"] = {"source": line["data"]}
+            line["data"]["cameras"] = {
+                "model": "random per pose (mpl_synth_cameras, keyed by global pose index)", "rig_kind": rig_kind,
+                "azimuth": "2 pi (v + 0.8 (U0 - 0.5)) / V + 0.3", "distance_m": "4.5 (0.75 + 0.5 U1)",
+                "height_m": "0.9 + 1.2 U2", "look_at": "room centre at 0.9 m + 0.5 (U3 - 0.5, U4 - 0.5, 0)",
+                "focal_px": "f0 (0.8 + 0.4 U5), f0 of the rig kind"}
         if tacc is not None:
             line["triangulation"] = triangulation_summary(tacc.acc.detach().cpu().numpy(), cfg.J)
         if racc is not None:
@@ -177,10 +193,12 @@ def main(argv=None):
     p.add_argument("--outlier-rate", type=float, default=0.0, metavar="P",
                    help="detector noise: share of confident false detections")
     p.add_argument("--miss-rate", type=float, default=0.0, metavar="P", help="detector noise: share of missed detections")
+    p.add_argument("--random-cameras", action="store_true",
+                   help="a random camera setup per pose (around the room of --rig) instead of one ring for all poses")
     a = p.parse_args(argv)
     run(a.arch, a.views, a.depth, a.poses, a.micro_batch, a.precision, a.rig, a.seed, triangulate=a.triangulate,
         pixel_noise=a.pixel_noise, outlier_rate=a.outlier_rate, miss_rate=a.miss_rate,
-        triangulate_robust=a.triangulate_robust, inlier_px=a.inlier_px)
+        triangulate_robust=a.triangulate_robust, inlier_px=a.inlier_px, random_cameras=a.random_cameras)
 
 
 if __name__ == "__main__":

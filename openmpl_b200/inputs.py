@@ -12,29 +12,33 @@ from . import _lib
 
 
 def pack_calibration(R, t, f, c, image_size) -> np.ndarray:
-    """[V, 18] float64 rows: R (9, row-major world->cam), t (3), fx, fy, cx, cy, w, h."""
+    """[..., V, 18] float64 rows: R (9, row-major world->cam), t (3), fx, fy, cx, cy, w, h.
+
+    R [..., V, 3, 3], t [..., V, 3], f and c [..., V, 2]; leading batch dimensions give one calibration per pose (a
+    [B, V, 18] result is what the calibration-taking entry points accept per pose).  image_size (w, h), or any array that
+    broadcasts to [..., V, 2].
+    """
     R, t, f, c = (np.asarray(a, dtype=np.float64) for a in (R, t, f, c))
-    V = R.shape[0]
-    wh = np.tile(np.asarray(image_size, dtype=np.float64), (V, 1))
-    return np.concatenate([R.reshape(V, 9), t.reshape(V, 3), f.reshape(V, 2), c.reshape(V, 2), wh], axis=1)
+    lead = R.shape[:-2]
+    wh = np.broadcast_to(np.asarray(image_size, dtype=np.float64), lead + (2,))
+    return np.concatenate([R.reshape(lead + (9,)), t.reshape(lead + (3,)), f.reshape(lead + (2,)), c.reshape(lead + (2,)), wh],
+                          axis=-1)
 
 
 def build_inputs(pix: torch.Tensor, calib) -> tuple:
-    """pix [B, V, J, 3] fp32 (u, v, conf) pixels on the device; calib [V, 18] -> poses, rays [B,V,J,3], centers [B,V,1,3]."""
+    """pix [B, V, J, 3] fp32 (u, v, conf) pixels on the device; calib [V, 18], or [B, V, 18] with one calibration per pose
+    -> poses, rays [B,V,J,3], centers [B,V,1,3]."""
     B, V, J, _ = pix.shape
     device = pix.device
     pix = pix.to(torch.float32).contiguous()
-    if isinstance(calib, torch.Tensor):
-        calib = calib.to(device=device, dtype=torch.float64).contiguous()
-    else:
-        calib = torch.as_tensor(np.asarray(calib, dtype=np.float64)).to(device).contiguous()
+    calib, stride = _calib_arg(calib, B, V, device)
     poses = torch.empty((B, V, J, 3), dtype=torch.float32, device=device)
     rays = torch.empty_like(poses)
     centers = torch.empty((B, V, 1, 3), dtype=torch.float32, device=device)
     with torch.cuda.device(device):
         stream = torch.cuda.current_stream(device).cuda_stream
-        _lib.check(_lib.lib().mpl_build_inputs(pix.data_ptr(), calib.data_ptr(), B, V, J, poses.data_ptr(), rays.data_ptr(),
-                                               centers.data_ptr(), stream))
+        _lib.check(_lib.lib().mpl_build_inputs_strided(pix.data_ptr(), calib.data_ptr(), stride, B, V, J, poses.data_ptr(),
+                                                       rays.data_ptr(), centers.data_ptr(), stream))
     return poses, rays, centers
 
 
@@ -42,30 +46,27 @@ def triangulate(pix: torch.Tensor, calib, min_conf: float = 0.0) -> tuple:
     """Linear multi-view triangulation of raw detections (`mpl_triangulate`; the baseline of
     `MPL/lib/multiviews/triangulate.py:59-115`), enqueued on the current stream.
 
-    pix [B, V, J, 3] fp32 (u, v, conf) pixels on the device; calib [V, 18] (numpy or tensor) as for `build_inputs`.
-    A view is used for a joint iff conf > min_conf and the pixel lies strictly inside the image.  Returns
+    pix [B, V, J, 3] fp32 (u, v, conf) pixels on the device; calib [V, 18] or [B, V, 18] (numpy or tensor) as for
+    `build_inputs`.  A view is used for a joint iff conf > min_conf and the pixel lies strictly inside the image.  Returns
     (points [B, J, 3] fp32 world units, NaN where fewer than 2 views are used; views_used [B, J] int32).
     """
     B, V, J, _ = pix.shape
     device = pix.device
     pix = pix.to(torch.float32).contiguous()
-    if isinstance(calib, torch.Tensor):
-        calib = calib.to(device=device, dtype=torch.float64).contiguous()
-    else:
-        calib = torch.as_tensor(np.asarray(calib, dtype=np.float64)).to(device).contiguous()
+    calib, stride = _calib_arg(calib, B, V, device)
     points = torch.empty((B, J, 3), dtype=torch.float32, device=device)
     views_used = torch.empty((B, J), dtype=torch.int32, device=device)
     with torch.cuda.device(device):
         stream = torch.cuda.current_stream(device).cuda_stream
-        _lib.check(_lib.lib().mpl_triangulate(pix.data_ptr(), calib.data_ptr(), B, V, J, float(min_conf), points.data_ptr(),
-                                              views_used.data_ptr(), stream))
+        _lib.check(_lib.lib().mpl_triangulate_strided(pix.data_ptr(), calib.data_ptr(), stride, B, V, J, float(min_conf),
+                                                      points.data_ptr(), views_used.data_ptr(), stream))
     return points, views_used
 
 
 def triangulate_robust(pix: torch.Tensor, calib, min_conf: float = 0.0, inlier_px: float = 10.0) -> tuple:
     """Outlier-robust triangulation of raw detections (`mpl_triangulate_robust`), enqueued on the current stream.
 
-    Candidate views as in `triangulate`.  Every candidate pair gives a two-view DLT hypothesis scored by the MSAC cost
+    calib [V, 18] or [B, V, 18]; candidate views as in `triangulate`.  Every candidate pair gives a two-view DLT hypothesis scored by the MSAC cost
     sum_c min(e_c^2, inlier_px^2) over the candidates' pixel reprojection errors; the cheapest one's inliers (e_c < inlier_px)
     are refitted by a DLT with rows weighted by conf.  Returns (points [B, J, 3] fp32 world units, NaN where fewer than two
     candidates or inliers; inliers [B, J] int32 bitmask of the inlier views, bit v for view v, 0 where the point is NaN).
@@ -73,13 +74,13 @@ def triangulate_robust(pix: torch.Tensor, calib, min_conf: float = 0.0, inlier_p
     B, V, J, _ = pix.shape
     device = pix.device
     pix = pix.to(torch.float32).contiguous()
-    calib = _device_calib(calib, device)
+    calib, stride = _calib_arg(calib, B, V, device)
     points = torch.empty((B, J, 3), dtype=torch.float32, device=device)
     inliers = torch.empty((B, J), dtype=torch.int32, device=device)
     with torch.cuda.device(device):
         stream = torch.cuda.current_stream(device).cuda_stream
-        _lib.check(_lib.lib().mpl_triangulate_robust(pix.data_ptr(), calib.data_ptr(), B, V, J, float(min_conf),
-                                                     float(inlier_px), points.data_ptr(), inliers.data_ptr(), stream))
+        _lib.check(_lib.lib().mpl_triangulate_robust_strided(pix.data_ptr(), calib.data_ptr(), stride, B, V, J, float(min_conf),
+                                                             float(inlier_px), points.data_ptr(), inliers.data_ptr(), stream))
     return points, inliers
 
 
@@ -88,39 +89,56 @@ def add_detector_noise(pix: torch.Tensor, calib, seed: int, start: int, sigma_px
     """Detector-error model (`mpl_synth_detector_noise`) applied IN PLACE to raw pixels of poses [start, start + B),
     enqueued on the current stream; returns `pix`.
 
-    pix [B, V, J, 3] contiguous fp32 (u, v, conf) on the device, as `synth_project` returns it; calib [V, 18] (only w, h
-    are read).  Per entry with conf > 0: a miss (conf = 0) with probability p_miss, a confident false detection anywhere in
+    pix [B, V, J, 3] contiguous fp32 (u, v, conf) on the device, as `synth_project` returns it; calib [V, 18] or
+    [B, V, 18] (only w, h are read).  Per entry with conf > 0: a miss (conf = 0) with probability p_miss, a confident false detection anywhere in
     the image with probability p_outlier, otherwise Gaussian pixel noise of std sigma_px / conf.  The draws depend only on
     (seed, global pose index), under a key separate from `synth_project`'s; `synth.detector_noise` is the numpy twin.
     """
     if pix.dtype != torch.float32 or not pix.is_contiguous() or pix.dim() != 4 or pix.shape[-1] != 3:
         raise ValueError("add_detector_noise works in place on a contiguous float32 [B, V, J, 3] tensor")
     B, V, J, _ = pix.shape
-    calib = _device_calib(calib, pix.device)
+    calib, stride = _calib_arg(calib, B, V, pix.device)
     with torch.cuda.device(pix.device):
         stream = torch.cuda.current_stream(pix.device).cuda_stream
-        _lib.check(_lib.lib().mpl_synth_detector_noise(int(seed), int(start), B, V, J, calib.data_ptr(), float(sigma_px),
-                                                       float(p_outlier), float(p_miss), pix.data_ptr(), stream))
+        _lib.check(_lib.lib().mpl_synth_detector_noise_strided(int(seed), int(start), B, V, J, calib.data_ptr(), stride,
+                                                               float(sigma_px), float(p_outlier), float(p_miss), pix.data_ptr(),
+                                                               stream))
     return pix
 
 
-def _device_calib(calib, device) -> torch.Tensor:
+def _calib_arg(calib, B: int, V: int, device) -> tuple:
+    """(contiguous fp64 device tensor, calib_stride): [V, 18] -> stride 0 (one rig for the batch); [B, V, 18] -> 18 V."""
     if isinstance(calib, torch.Tensor):
-        return calib.to(device=device, dtype=torch.float64).contiguous()
-    return torch.as_tensor(np.asarray(calib, dtype=np.float64)).to(device).contiguous()
+        calib = calib.to(device=device, dtype=torch.float64).contiguous()
+    else:
+        calib = torch.as_tensor(np.asarray(calib, dtype=np.float64)).to(device).contiguous()
+    if calib.dim() != 3:
+        return calib, 0
+    if calib.shape[0] != B or tuple(calib.shape[1:]) != (V, 18):
+        raise ValueError(f"a per-pose calibration must be [B, V, 18] = [{B}, {V}, 18], got {list(calib.shape)}")
+    return calib, 18 * V
 
 
-def synth_project(batch: int, rig, seed: int = 0, start: int = 0, conf_mode: str = "uniform", device=None) -> tuple:
+def synth_project(batch: int, rig, seed: int = 0, start: int = 0, conf_mode: str = "uniform", device=None,
+                  cameras=None) -> tuple:
     """N3: MHP-style synthetic poses generated and projected ON THE DEVICE (`mpl_synth_project`).
 
     Pose i depends only on (seed, start + i) — the same Philox stream as `synth.make_batch` — so ranks / micro-batches
     can shard the global index range freely.  Returns (pix [B,V,17,3] raw pixels (u, v, conf), target [B,17,3] metres,
-    calib [V,18] fp64 on the device); `build_inputs(pix, calib)` turns the pixels into the model's inputs.
+    calib [V,18] fp64 on the device); `build_inputs(pix, calib)` turns the pixels into the model's inputs.  With
+    `cameras`, a [B, V, 18] calibration per pose (e.g. from `synth_cameras`), the poses are projected through those
+    instead of the rig's, and `calib` is that tensor; the 3D poses (placed in the rig's room) do not change.
     """
     from .synth import NUM_JOINTS
     device = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
     V, J = rig.num_views, NUM_JOINTS
-    calib = torch.as_tensor(pack_calibration(rig.R, rig.t, rig.f, rig.c, rig.image_size)).to(device)
+    if cameras is None:
+        calib = torch.as_tensor(pack_calibration(rig.R, rig.t, rig.f, rig.c, rig.image_size)).to(device)
+        stride = 0
+    else:
+        calib, stride = _calib_arg(cameras, batch, V, device)
+        if stride == 0:
+            raise ValueError("cameras must be a [B, V, 18] calibration per pose")
     room = torch.as_tensor(np.asarray(rig.room, dtype=np.float64)).to(device)
     pix = torch.empty((batch, V, J, 3), dtype=torch.float32, device=device)
     target = torch.empty((batch, J, 3), dtype=torch.float32, device=device)
@@ -128,6 +146,26 @@ def synth_project(batch: int, rig, seed: int = 0, start: int = 0, conf_mode: str
         raise ValueError(conf_mode)
     with torch.cuda.device(device):
         stream = torch.cuda.current_stream(device).cuda_stream
-        _lib.check(_lib.lib().mpl_synth_project(int(seed), int(start), int(batch), V, J, calib.data_ptr(), room.data_ptr(),
-                                                int(conf_mode == "ones"), pix.data_ptr(), target.data_ptr(), stream))
+        _lib.check(_lib.lib().mpl_synth_project_strided(int(seed), int(start), int(batch), V, J, calib.data_ptr(), stride,
+                                                        room.data_ptr(), int(conf_mode == "ones"), pix.data_ptr(),
+                                                        target.data_ptr(), stream))
     return pix, target, calib
+
+
+def synth_cameras(batch: int, num_views: int, kind: str = "h36m", seed: int = 0, start: int = 0, device=None) -> torch.Tensor:
+    """Random camera setups generated ON THE DEVICE (`mpl_synth_cameras`): [B, V, 18] fp64 calibrations of poses
+    [start, start + batch) around the room of rig `kind` ("h36m" or "cmu": its focal length, image size and room).  Pose
+    i's cameras depend only on (seed, start + i), under a Philox key separate from the poses' and the detector noise's;
+    `synth.random_cameras` is the numpy twin.  Feed them to `synth_project(..., cameras=...)` and every calibration-taking
+    entry point of this module.
+    """
+    from .synth import rig_kind
+    f0, (w, h), room = rig_kind(kind)
+    device = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
+    room = torch.as_tensor(np.asarray(room, dtype=np.float64)).to(device)
+    calib = torch.empty((batch, num_views, 18), dtype=torch.float64, device=device)
+    with torch.cuda.device(device):
+        stream = torch.cuda.current_stream(device).cuda_stream
+        _lib.check(_lib.lib().mpl_synth_cameras(int(seed), int(start), int(batch), int(num_views), float(f0), float(w),
+                                                float(h), room.data_ptr(), calib.data_ptr(), stream))
+    return calib

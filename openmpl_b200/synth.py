@@ -40,18 +40,25 @@ class Rig:
         return self.R.shape[0]
 
 
+# rig kind -> (focal length px, image (w, h) px, room (min_x, max_x, min_y, max_y) m)
+RIG_KINDS = {"h36m": (1145.0, (1000, 1000), (-1.0, 1.0, -1.5, 2.0)),   # hm_0 yaml:47-50,89-91
+             "cmu": (1400.0, (1920, 1080), (-2.0, 0.3, -0.8, 0.8))}     # cmu_0 yaml:85-87
+
+
+def rig_kind(kind: str) -> tuple:
+    """(f0, (w, h), room) of a rig kind."""
+    if kind not in RIG_KINDS:
+        raise ValueError(f"unknown rig kind {kind!r}")
+    return RIG_KINDS[kind]
+
+
 def make_rig(num_views: int, kind: str = "h36m") -> Rig:
     """Ring of cameras, radius 4.5 m, height 1.5 m, looking at the room centre.
 
     kind "h36m": f=1145 px, 1000x1000 image, room -1..1 x -1.5..2  (hm_0 yaml:47-50,89-91)
     kind "cmu" : f=1400 px, 1920x1080 image, room -2..0.3 x -0.8..0.8 (cmu_0 yaml:85-87)
     """
-    if kind == "h36m":
-        f0, (w, h), room = 1145.0, (1000, 1000), (-1.0, 1.0, -1.5, 2.0)
-    elif kind == "cmu":
-        f0, (w, h), room = 1400.0, (1920, 1080), (-2.0, 0.3, -0.8, 0.8)
-    else:
-        raise ValueError(f"unknown rig kind {kind!r}")
+    f0, (w, h), room = rig_kind(kind)
     centre = np.array([(room[0] + room[1]) / 2, (room[2] + room[3]) / 2, 0.9])
     Rs, ts = [], []
     for v in range(num_views):
@@ -67,6 +74,44 @@ def make_rig(num_views: int, kind: str = "h36m") -> Rig:
     V = num_views
     return Rig(R=np.stack(Rs), t=np.stack(ts), f=np.full((V, 2), f0), c=np.tile([w / 2.0, h / 2.0], (V, 1)),
                image_size=(w, h), room=room)
+
+
+def cameras_from_uniforms(U, f0: float, image_size, room) -> np.ndarray:
+    """[..., V, 18] calibrations (`inputs.pack_calibration` rows) of the camera model of `mpl_synth_cameras` from U [..., V, 6].
+
+    Azimuth 2 pi (v + 0.8 (U0 - 0.5)) / V + 0.3, horizontal distance 4.5 (0.75 + 0.5 U1) m from the look-at point, height
+    0.9 + 1.2 U2 m, look-at point the room centre at height 0.9 shifted by 0.5 (U3 - 0.5) in x and 0.5 (U4 - 0.5) in y,
+    fx = fy = f0 (0.8 + 0.4 U5), principal point at the image centre, R the look-at rotation of `make_rig`.  Every U = 0.5
+    gives `make_rig`'s camera.
+    """
+    U = np.asarray(U, dtype=np.float64)
+    V = U.shape[-2]
+    w, h = (float(x) for x in image_size)
+    v = np.arange(V, dtype=np.float64)
+    ang = 2 * math.pi * (v + 0.8 * (U[..., 0] - 0.5)) / V + 0.3
+    dist = 4.5 * (0.75 + 0.5 * U[..., 1])
+    at = np.stack([np.broadcast_to((room[0] + room[1]) / 2 + 0.5 * (U[..., 3] - 0.5), ang.shape),
+                   np.broadcast_to((room[2] + room[3]) / 2 + 0.5 * (U[..., 4] - 0.5), ang.shape),
+                   np.full(ang.shape, 0.9)], axis=-1)
+    pos = np.stack([at[..., 0] + dist * np.cos(ang), at[..., 1] + dist * np.sin(ang), 0.9 + 1.2 * U[..., 2]], axis=-1)
+    z = at - pos
+    z /= np.linalg.norm(z, axis=-1, keepdims=True)
+    x = np.cross(z, np.array([0.0, 0.0, 1.0]))
+    x /= np.linalg.norm(x, axis=-1, keepdims=True)
+    y = np.cross(z, x)
+    f = f0 * (0.8 + 0.4 * U[..., 5:6])
+    lead = U.shape[:-1]
+    return np.concatenate([x, y, z, pos, f, f, np.broadcast_to([w / 2, h / 2, w, h], lead + (4,))], axis=-1)
+
+
+def random_cameras(batch: int, num_views: int, kind: str = "h36m", seed: int = 0, start: int = 0) -> np.ndarray:
+    """Host twin of `mpl_synth_cameras`: [B, V, 18] float64 calibrations of poses [start, start + batch), random camera
+    setups around the room of rig `kind` (`cameras_from_uniforms`).  U0..U5 of (pose i, view v) come from the Philox4x64-10
+    stream under key (seed, 2) (pose i owns counter blocks [i nb, (i+1) nb), nb = ceil(6 V / 4), slot 6 v + m is U_m), so
+    pose i's cameras depend only on (seed, start + i)."""
+    f0, image_size, room = rig_kind(kind)
+    U = _uniforms(seed, start, batch, 6 * num_views, key1=2).reshape(batch, num_views, 6)
+    return cameras_from_uniforms(U, f0, image_size, room)
 
 
 def _uniforms(seed: int, start: int, count: int, per_pose: int, key1: int = 0) -> np.ndarray:
