@@ -13,9 +13,9 @@
  *   MPL/lib/dataset/joints_dataset_mpl.py:615-648,701-715,762-772,817-820,872-904
  *                                            per-sample input construction (-> mpl_build_inputs)
  *   MPL/lib/multiviews/triangulate.py:59-115 linear triangulation baseline (-> mpl_triangulate)
- * Defined here, with no counterpart in the reference: robust (RANSAC) triangulation (mpl_triangulate_robust), a
- * detector-error model for the synthetic data (mpl_synth_detector_noise) and a generator of random camera setups
- * (mpl_synth_cameras).
+ * Defined here, with no counterpart in the reference: robust (RANSAC) triangulation (mpl_triangulate_robust), nonlinear
+ * refinement of triangulated points (mpl_triangulate_refine), a detector-error model for the synthetic data
+ * (mpl_synth_detector_noise) and a generator of random camera setups (mpl_synth_cameras).
  *
  * Conventions
  *   - plain pointers and sizes only; no torch / C++ types cross this boundary;
@@ -43,7 +43,7 @@
 extern "C" {
 #endif
 
-#define MPL_ABI_VERSION 5
+#define MPL_ABI_VERSION 6
 
 typedef enum MplStatus {
   MPL_OK = 0,
@@ -282,6 +282,37 @@ int mpl_triangulate_robust(const float* pix, const double* calib, int64_t batch,
 /* mpl_triangulate_robust with a calibration per pose (see Conventions); same argument checks plus calib_stride. */
 int mpl_triangulate_robust_strided(const float* pix, const double* calib, int64_t calib_stride, int64_t batch, int num_views,
                                    int num_joints, float min_conf, float inlier_px, float* points, int32_t* inliers,
+                                   mpl_stream_t stream);
+
+/* Levenberg-Marquardt refinement of given 3D points on the confidence-weighted reprojection error (defined by this library;
+ * the reference has no refinement).  With pixel noise of std sigma / conf the maximum-likelihood point minimises the cost C
+ * below (Hartley & Zisserman section 12.3), which neither DLT above does.  Per (pose, joint) item b, j, in fp64 throughout:
+ *   - views used: view v takes part iff it is a candidate of mpl_triangulate (conf > min_conf and strictly inside the image)
+ *     and, when view_mask is not NULL, bit v of view_mask[b, j] is set (bits >= V are ignored).  Pass mpl_triangulate_robust's
+ *     inliers to refine over them, NULL for every candidate; a views_used count is not a mask;
+ *   - cost: C(X) = sum_v w_v ((p_0 / p_2 - u_v)^2 + (p_1 / p_2 - v_v)^2), w_v = conf_v^2, p = P_v [X; 1] with
+ *     P_v = K [R | -R t].  C = +inf if any used view has p_2 <= 0 or a non-finite p_2;
+ *   - X_0 = init converted to fp64.  The item is not refined when init is not finite, fewer than 2 views are used or C(X_0)
+ *     is not finite: it gets points = init bit for bit and reproj_px = NaN;
+ *   - iteration k = 1 .. max_iters: at the current X (relinearised only after an accepted step), D_v is the 2 x 3 Jacobian
+ *     of pi(P_v [X; 1]) and r_v its residual; A = sum w_v D_v^T D_v, g = sum w_v D_v^T r_v.  Before the first iteration only,
+ *     mu = 1e-3 max_i A_ii.  (A + mu I) delta = -g is solved by a 3 x 3 Cholesky; a pivot that is not finite and > 0
+ *     rejects the step (mu *= 10; there is no delta, so the stopping test below is skipped).  If C(X + delta) < C(X) the
+ *     step is accepted, X += delta and mu /= 10, otherwise rejected, mu *= 10.  The iteration stops after iteration k if
+ *     |delta|_2 <= 1e-10 (|X|_2 + 1e-10), X taken at the start of the iteration, or when k = max_iters;
+ *   - outputs: points = X rounded to fp32, reproj_px = sqrt(C(X) / sum_v w_v), the conf-weighted RMS pixel error at the
+ *     returned fp64 X.  C(X) <= C(X_0) by construction.
+ *   pix [B, V, J, 3] fp32 and calib as in mpl_triangulate, view_mask NULL or [B, J] int32, init [B, J, 3] fp32,
+ *   points [B, J, 3] fp32, reproj_px [B, J] fp32.  init may equal points (in-place refinement); no other aliasing.
+ *   1 <= V <= 16, J >= 1, 1 <= max_iters <= 100.  Deterministic and independent of how the batch is split; allocates
+ *   nothing and never synchronises (graph-capturable).  batch == 0 returns MPL_OK without touching the pointers. */
+int mpl_triangulate_refine(const float* pix, const double* calib, int64_t batch, int num_views, int num_joints,
+                           float min_conf, const int32_t* view_mask, const float* init, int max_iters, float* points,
+                           float* reproj_px, mpl_stream_t stream);
+/* mpl_triangulate_refine with a calibration per pose (see Conventions); same argument checks plus calib_stride. */
+int mpl_triangulate_refine_strided(const float* pix, const double* calib, int64_t calib_stride, int64_t batch,
+                                   int num_views, int num_joints, float min_conf, const int32_t* view_mask,
+                                   const float* init, int max_iters, float* points, float* reproj_px,
                                    mpl_stream_t stream);
 
 /* Detector-error model for the synthetic pixels of mpl_synth_project, applied in place (defined by this library; the

@@ -11,7 +11,7 @@ from ctypes import POINTER, c_char_p, c_double, c_float, c_int, c_int32, c_int64
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("MPL_B200_LIB") or os.path.join(HERE, "libmpl_b200.so")   # override: another build of the same ABI
 
-ABI_VERSION = 5
+ABI_VERSION = 6
 MPL_OK = 0
 MPL_ERR_INVALID_ARGUMENT = -1
 MPL_ERR_CONFIG_RUNTIME = -2
@@ -31,7 +31,7 @@ EXPORTS = [
     "mpl_pmpjpe_accumulate", "mpl_test_gemm_ln", "mpl_test_gemm_ln_slots", "mpl_test_gemm_emit_pitch", "mpl_set_graph_batch", "mpl_graph_stats",
     "mpl_test_qkv_attn", "mpl_triangulate", "mpl_triangulate_robust", "mpl_synth_detector_noise",
     "mpl_build_inputs_strided", "mpl_synth_project_strided", "mpl_synth_detector_noise_strided", "mpl_triangulate_strided",
-    "mpl_triangulate_robust_strided", "mpl_synth_cameras",
+    "mpl_triangulate_robust_strided", "mpl_synth_cameras", "mpl_triangulate_refine", "mpl_triangulate_refine_strided",
 ]
 
 _DESC_FLAGS = [
@@ -155,6 +155,10 @@ def lib():
                                                        c_float, c_float, c_float, c_void_p, c_void_p]
         L.mpl_synth_cameras.argtypes = [ctypes.c_uint64, c_int64, c_int64, c_int, c_double, c_double, c_double, c_void_p,
                                         c_void_p, c_void_p]
+        L.mpl_triangulate_refine.argtypes = [c_void_p, c_void_p, c_int64, c_int, c_int, c_float, c_void_p, c_void_p, c_int,
+                                             c_void_p, c_void_p, c_void_p]
+        L.mpl_triangulate_refine_strided.argtypes = [c_void_p, c_void_p, c_int64, c_int64, c_int, c_int, c_float, c_void_p,
+                                                     c_void_p, c_int, c_void_p, c_void_p, c_void_p]
         if L.mpl_abi_version() != ABI_VERSION:
             raise RuntimeError("libmpl_b200.so ABI version mismatch")
         _lib = L

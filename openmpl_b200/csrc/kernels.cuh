@@ -211,6 +211,9 @@ int launch_triangulate(const float* pix, const double* calib, int64_t calib_stri
                        float* points, int32_t* views_used, cudaStream_t s);
 int launch_triangulate_robust(const float* pix, const double* calib, int64_t calib_stride, int64_t B, int V, int J,
                               float min_conf, float inlier_px, float* points, int32_t* inliers, cudaStream_t s);
+int launch_triangulate_refine(const float* pix, const double* calib, int64_t calib_stride, int64_t B, int V, int J,
+                              float min_conf, const int32_t* view_mask, const float* init, int max_iters, float* points,
+                              float* reproj_px, cudaStream_t s);
 int launch_detector_noise(uint64_t seed, int64_t start, int64_t B, int V, int J, const double* calib, int64_t calib_stride,
                           float sigma_px, float p_outlier, float p_miss, float* pix, cudaStream_t s);
 int launch_synth_cameras(uint64_t seed, int64_t start, int64_t B, int V, double f0, double w, double h, const double* room,

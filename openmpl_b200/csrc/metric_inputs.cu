@@ -685,6 +685,152 @@ int launch_triangulate_robust(const float* pix, const double* calib, int64_t cal
   return MPL_OK;
 }
 
+// ---- Levenberg-Marquardt refinement of given points on the confidence-weighted reprojection error ------------------
+// Same items, staging and candidate views as triangulate_kernel; the views used are the candidates in the item's
+// view_mask.  C(X) = sum_v w_v |pi(P_v [X; 1]) - x_v|^2 with w_v = conf_v^2, the maximum-likelihood cost when the pixel
+// noise has std sigma / conf (Hartley & Zisserman section 12.3).  The 3 x 3 normal equations A = sum w D^T D,
+// g = sum w D^T r are rebuilt after each accepted step only, (A + mu I) delta = -g is solved by Cholesky, and the step is
+// kept iff it lowers C.  The used views are walked with __ffs on a bitmask so that P is indexed by a run-time view in shared
+// memory, never in a local array; the thread's pixels stay in the staged tile.
+
+// C(X) over the views of `used`; +inf as soon as a view sees X at a depth that is not > 0 or not finite.
+__device__ __forceinline__ double refine_cost(const double (*P)[12], const float (&sx)[kMaxViews][3 * kTriTile], int tid,
+                                              unsigned used, const double (&X)[3]) {
+  double cost = 0.0;
+  for (unsigned m = used; m; m &= m - 1) {
+    const int v = __ffs(m) - 1;
+    const double* p = P[v];
+    const double z = fma(p[8], X[0], fma(p[9], X[1], fma(p[10], X[2], p[11])));
+    if (!(z > 0.0) || isinf(z)) return __longlong_as_double(0x7ff0000000000000ll);
+    const double iz = 1.0 / z;
+    const double du = fma(p[0], X[0], fma(p[1], X[1], fma(p[2], X[2], p[3]))) * iz - (double)sx[v][3 * tid];
+    const double dv = fma(p[4], X[0], fma(p[5], X[1], fma(p[6], X[2], p[7]))) * iz - (double)sx[v][3 * tid + 1];
+    const double c = (double)sx[v][3 * tid + 2];
+    cost = fma(c * c, fma(du, du, dv * dv), cost);
+  }
+  return cost;
+}
+
+template <bool kPerPose>
+__global__ void __launch_bounds__(kTriTile) triangulate_refine_kernel(const float* __restrict__ pix,
+                                                                      const double* __restrict__ calib, int64_t cstride, int64_t B,
+                                                                      int V, int J, float min_conf,
+                                                                      const int32_t* __restrict__ view_mask, const float* init,
+                                                                      int max_iters, float* points, float* __restrict__ reproj_px) {
+  __shared__ double sP[kMaxViews][12];
+  __shared__ double sWH[kMaxViews][2];
+  __shared__ float sx[kMaxViews][3 * kTriTile];
+  const int tid = threadIdx.x;
+  int64_t i0;
+  const double(*P)[12];
+  const double(*WH)[2];
+  const int n = tri_stage_tile<kPerPose>(pix, calib, cstride, B, V, J, sP, sWH, sx, i0, P, WH);
+  if (tid >= n) return;
+  const int64_t i = i0 + tid;
+  // init may be points (in-place refinement): every read of init comes before the thread's stores
+  float out[3] = {init[i * 3], init[i * 3 + 1], init[i * 3 + 2]};
+  unsigned used = 0;
+  for (int v = 0; v < V; ++v)
+    if (tri_candidate(sx[v][3 * tid + 2], sx[v][3 * tid], sx[v][3 * tid + 1], min_conf, WH[v])) used |= 1u << v;
+  if (view_mask != nullptr) used &= (unsigned)view_mask[i];
+  double X[3] = {(double)out[0], (double)out[1], (double)out[2]};
+  float rp = __int_as_float(0x7fc00000);
+  double C = __longlong_as_double(0x7ff0000000000000ll);
+  if (isfinite(X[0]) && isfinite(X[1]) && isfinite(X[2]) && __popc(used) >= 2) C = refine_cost(P, sx, tid, used, X);
+  if (isfinite(C)) {
+    double A[6], g[3], mu = 0.0;                           // A: 00 01 02 11 12 22
+    bool relin = true;
+    for (int k = 1; k <= max_iters; ++k) {
+      if (relin) {
+#pragma unroll
+        for (int e = 0; e < 6; ++e) A[e] = 0.0;
+#pragma unroll
+        for (int e = 0; e < 3; ++e) g[e] = 0.0;
+        for (unsigned m = used; m; m &= m - 1) {
+          const int v = __ffs(m) - 1;
+          const double* p = P[v];
+          const double iz = 1.0 / fma(p[8], X[0], fma(p[9], X[1], fma(p[10], X[2], p[11])));
+          const double qu = fma(p[0], X[0], fma(p[1], X[1], fma(p[2], X[2], p[3]))) * iz;
+          const double qv = fma(p[4], X[0], fma(p[5], X[1], fma(p[6], X[2], p[7]))) * iz;
+          const double c = (double)sx[v][3 * tid + 2], w = c * c;
+          const double ru = qu - (double)sx[v][3 * tid], rv = qv - (double)sx[v][3 * tid + 1];
+          double du[3], dv[3];                              // rows of the 2 x 3 Jacobian of pi(P [X; 1])
+#pragma unroll
+          for (int a = 0; a < 3; ++a) {
+            du[a] = fma(-qu, p[8 + a], p[a]) * iz;
+            dv[a] = fma(-qv, p[8 + a], p[4 + a]) * iz;
+          }
+          int e = 0;
+#pragma unroll
+          for (int a = 0; a < 3; ++a) {
+#pragma unroll
+            for (int b = a; b < 3; ++b, ++e) A[e] = fma(w, fma(du[a], du[b], dv[a] * dv[b]), A[e]);
+            g[a] = fma(w, fma(du[a], ru, dv[a] * rv), g[a]);
+          }
+        }
+        if (k == 1) mu = 1e-3 * fmax(A[0], fmax(A[3], A[5]));
+        relin = false;
+      }
+      // Cholesky of A + mu I; a pivot that is not finite and > 0 rejects the step (there is no delta to test)
+      const double inf = __longlong_as_double(0x7ff0000000000000ll);
+      const double m00 = A[0] + mu;
+      if (!(m00 > 0.0 && m00 < inf)) { mu *= 10.0; continue; }
+      const double l00 = sqrt(m00), l10 = A[1] / l00, l20 = A[2] / l00;
+      const double m11 = A[3] + mu - l10 * l10;
+      if (!(m11 > 0.0 && m11 < inf)) { mu *= 10.0; continue; }
+      const double l11 = sqrt(m11), l21 = (A[4] - l20 * l10) / l11;
+      const double m22 = A[5] + mu - l20 * l20 - l21 * l21;
+      if (!(m22 > 0.0 && m22 < inf)) { mu *= 10.0; continue; }
+      const double l22 = sqrt(m22);
+      const double y0 = -g[0] / l00, y1 = (-g[1] - l10 * y0) / l11, y2 = (-g[2] - l20 * y0 - l21 * y1) / l22;
+      const double d2 = y2 / l22, d1 = (y1 - l21 * d2) / l11, d0 = (y0 - l10 * d1 - l20 * d2) / l00;
+      const double xnorm = sqrt(X[0] * X[0] + X[1] * X[1] + X[2] * X[2]);
+      const double dnorm = sqrt(d0 * d0 + d1 * d1 + d2 * d2);
+      const double Xn[3] = {X[0] + d0, X[1] + d1, X[2] + d2};
+      const double Cn = refine_cost(P, sx, tid, used, Xn);
+      if (Cn < C) {
+#pragma unroll
+        for (int a = 0; a < 3; ++a) X[a] = Xn[a];
+        C = Cn;
+        mu *= 0.1;
+        relin = true;
+      } else {
+        mu *= 10.0;
+      }
+      if (dnorm <= 1e-10 * (xnorm + 1e-10)) break;
+    }
+    double wsum = 0.0;
+    for (unsigned m = used; m; m &= m - 1) {
+      const double c = (double)sx[__ffs(m) - 1][3 * tid + 2];
+      wsum = fma(c, c, wsum);
+    }
+#pragma unroll
+    for (int a = 0; a < 3; ++a) out[a] = (float)X[a];
+    rp = (float)sqrt(C / wsum);
+  }
+#pragma unroll
+  for (int a = 0; a < 3; ++a) points[i * 3 + a] = out[a];
+  reproj_px[i] = rp;
+}
+
+int launch_triangulate_refine(const float* pix, const double* calib, int64_t calib_stride, int64_t B, int V, int J,
+                              float min_conf, const int32_t* view_mask, const float* init, int max_iters, float* points,
+                              float* reproj_px, cudaStream_t s) {
+  const int64_t items = B * J;
+  if (items == 0) return MPL_OK;
+  if (calib_stride == 0) {
+    triangulate_refine_kernel<false><<<(unsigned)ceil_div(items, kTriTile), kTriTile, 0, s>>>(
+        pix, calib, 0, B, V, J, min_conf, view_mask, init, max_iters, points, reproj_px);
+  } else {
+    size_t smem;
+    const int T = tri_pose_tile(V, J, smem);
+    triangulate_refine_kernel<true><<<(unsigned)ceil_div(items, (int64_t)T), T, smem, s>>>(
+        pix, calib, calib_stride, B, V, J, min_conf, view_mask, init, max_iters, points, reproj_px);
+  }
+  MPL_LAUNCH_CHECK();
+  return MPL_OK;
+}
+
 // ---------------------------------------------------------------------------------------------------------------------
 // N3: MHP-style synthetic projector.  3D poses from a counter-based generator keyed by (seed, GLOBAL pose index) --
 // any sharding of the index range over ranks / micro-batches yields the same data -- pushed through V calibrations:

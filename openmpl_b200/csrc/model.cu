@@ -1404,6 +1404,32 @@ int mpl_triangulate_robust_strided(const float* pix, const double* calib, int64_
                                    reinterpret_cast<cudaStream_t>(stream));
 }
 
+int mpl_triangulate_refine(const float* pix, const double* calib, int64_t batch, int num_views, int num_joints,
+                           float min_conf, const int32_t* view_mask, const float* init, int max_iters, float* points,
+                           float* reproj_px, mpl_stream_t stream) {
+  return mpl_triangulate_refine_strided(pix, calib, 0, batch, num_views, num_joints, min_conf, view_mask, init, max_iters,
+                                        points, reproj_px, stream);
+}
+
+int mpl_triangulate_refine_strided(const float* pix, const double* calib, int64_t calib_stride, int64_t batch,
+                                   int num_views, int num_joints, float min_conf, const int32_t* view_mask,
+                                   const float* init, int max_iters, float* points, float* reproj_px,
+                                   mpl_stream_t stream) {
+  if (batch < 0 || num_views < 1 || num_views > kMaxViews || num_joints < 1 || max_iters < 1 || max_iters > 100 ||
+      !calib_stride_ok(calib_stride, num_views)) {
+    set_error("mpl_triangulate_refine_strided: bad argument (batch %lld, num_views %d, num_joints %d, max_iters %d, "
+              "calib_stride %lld)", (long long)batch, num_views, num_joints, max_iters, (long long)calib_stride);
+    return MPL_ERR_INVALID_ARGUMENT;
+  }
+  if (batch == 0) return MPL_OK;
+  if (pix == nullptr || calib == nullptr || init == nullptr || points == nullptr || reproj_px == nullptr) {
+    set_error("mpl_triangulate_refine_strided: null pointer");
+    return MPL_ERR_INVALID_ARGUMENT;
+  }
+  return launch_triangulate_refine(pix, calib, calib_stride, batch, num_views, num_joints, min_conf, view_mask, init,
+                                   max_iters, points, reproj_px, reinterpret_cast<cudaStream_t>(stream));
+}
+
 int mpl_synth_detector_noise(uint64_t seed, int64_t start, int64_t batch, int num_views, int num_joints, const double* calib,
                              float sigma_px, float p_outlier, float p_miss, float* pix, mpl_stream_t stream) {
   return mpl_synth_detector_noise_strided(seed, start, batch, num_views, num_joints, calib, 0, sigma_px, p_outlier, p_miss, pix,

@@ -8,6 +8,8 @@
     python -m openmpl_b200.evaluate --arch hm0 --views 4 --pixel-noise 2 --outlier-rate 0.1 --triangulate \
         --triangulate-robust                                                            # noisy detections, both baselines
     python -m openmpl_b200.evaluate --arch hm0 --views 4 --random-cameras --triangulate  # a random camera setup per pose
+    python -m openmpl_b200.evaluate --arch hm0 --views 4 --pixel-noise 2 --triangulate --triangulate-robust \
+        --refine-triangulations                                                         # + nonlinear refinement of both
 
 Per micro-batch, entirely on the device: `mpl_synth_project` (3D poses from the counter-based generator keyed by the
 GLOBAL pose index, projected through the V calibrations) -> `mpl_build_inputs` (clip, confidence zeroing, screen
@@ -30,6 +32,11 @@ with the MSAC cost at `--inlier-px`, then a confidence-weighted refit), masked w
 (`mpl_synth_cameras`, random positions, heights, look-at points and focal lengths around the room of the rig kind, keyed
 by the global pose index), then projects, corrupts, builds inputs and triangulates through them.  The line's "data" entry
 records the camera model.  Without the flag the one rig of `--rig` serves every pose.
+
+`--refine-triangulations` (with `--triangulate` and / or `--triangulate-robust`) refines each triangulation's points by
+Levenberg-Marquardt on the conf^2-weighted reprojection error (`mpl_triangulate_refine`): the linear points over their
+candidate views, the robust points over their inliers.  Each triangulation entry gains a "refined" sub-entry, scored by its
+own accumulator under the parent entry's mask.  Without the flag nothing of this runs.
 """
 from __future__ import annotations
 
@@ -50,11 +57,14 @@ ARCHS = {
 }
 DEFAULT_DEPTH = {"hm0": 12, "chosen": 12, "kptok": 12, "cmu0": 2}
 DEFAULT_RIG = {"hm0": "h36m", "chosen": "h36m", "kptok": "h36m", "cmu0": "cmu"}
+REFINE_MAX_ITERS = 20
 
 
 def run(arch="hm0", views=4, depth=None, poses=1 << 20, micro_batch=65536, precision="bf16", rig=None, seed=1,
         weight_seed=0, warmup=1, triangulate=False, pixel_noise=0.0, outlier_rate=0.0, miss_rate=0.0,
-        triangulate_robust=False, inlier_px=10.0, random_cameras=False):
+        triangulate_robust=False, inlier_px=10.0, random_cameras=False, refine_triangulations=False):
+    if refine_triangulations and not (triangulate or triangulate_robust):
+        raise ValueError("refine_triangulations needs triangulate or triangulate_robust")
     rank, world, local = mdist.init_from_env("nccl")
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
@@ -73,6 +83,9 @@ def run(arch="hm0", views=4, depth=None, poses=1 << 20, micro_batch=65536, preci
     pacc = metric.PmpjpeAccumulator(cfg.J, output_in_meter=True, device=dev)
     tacc = metric.MpjpeAccumulator(cfg.J, output_in_meter=True, device=dev) if triangulate else None
     racc = metric.MpjpeAccumulator(cfg.J, output_in_meter=True, device=dev) if triangulate_robust else None
+    tfacc = metric.MpjpeAccumulator(cfg.J, output_in_meter=True, device=dev) if triangulate and refine_triangulations else None
+    rfacc = (metric.MpjpeAccumulator(cfg.J, output_in_meter=True, device=dev) if triangulate_robust and refine_triangulations
+             else None)
     noisy = pixel_noise != 0 or outlier_rate != 0 or miss_rate != 0
 
     def step(s0, n):
@@ -89,15 +102,20 @@ def run(arch="hm0", views=4, depth=None, poses=1 << 20, micro_batch=65536, preci
         if tacc is not None:
             points, used = inputs.triangulate(pix, calib)
             tacc.update(points, target, used >= 2)
+            if tfacc is not None:
+                tfacc.update(inputs.refine_triangulation(pix, calib, points, max_iters=REFINE_MAX_ITERS)[0], target, used >= 2)
         if racc is not None:
             points, inl = inputs.triangulate_robust(pix, calib, inlier_px=inlier_px)
             racc.update(points, target, inl != 0)      # popcount >= 2: a non-zero inlier mask has at least two bits
+            if rfacc is not None:
+                rfacc.update(inputs.refine_triangulation(pix, calib, points, view_mask=inl,
+                                                           max_iters=REFINE_MAX_ITERS)[0], target, inl != 0)
 
     for _ in range(warmup):                            # allocate the workspace, pack the weights
         step(start, min(micro_batch, max(stop - start, 1)))
     acc.acc.zero_()
     pacc.acc.zero_()
-    for a in (tacc, racc):
+    for a in (tacc, racc, tfacc, rfacc):
         if a is not None:
             a.acc.zero_()
     if world > 1:
@@ -109,7 +127,7 @@ def run(arch="hm0", views=4, depth=None, poses=1 << 20, micro_batch=65536, preci
         step(s0, min(micro_batch, stop - s0))
     acc.all_reduce()                                   # the only collectives of the whole job:
     pacc.all_reduce()                                  # 11 J + 1 and J + 3 doubles
-    for a in (tacc, racc):
+    for a in (tacc, racc, tfacc, rfacc):
         if a is not None:
             a.all_reduce()
     e1.record()
@@ -147,6 +165,12 @@ def run(arch="hm0", views=4, depth=None, poses=1 << 20, micro_batch=65536, preci
             line["triangulation_robust"] = triangulation_summary(
                 racc.acc.detach().cpu().numpy(), cfg.J,
                 method=f"pair RANSAC, MSAC cost at {inlier_px:g} px, conf-weighted DLT refit over the inliers")
+        for entry, a, views in (("triangulation", tfacc, "the candidate views"), ("triangulation_robust", rfacc, "the inliers")):
+            if a is not None:
+                line[entry]["refined"] = triangulation_summary(
+                    a.acc.detach().cpu().numpy(), cfg.J,
+                    method=f"Levenberg-Marquardt on the reprojection error over {views}, weights conf^2, "
+                           f"at most {REFINE_MAX_ITERS} iterations")
         print(json.dumps(line), flush=True)
     if world > 1:
         torch.distributed.barrier()
@@ -195,10 +219,16 @@ def main(argv=None):
     p.add_argument("--miss-rate", type=float, default=0.0, metavar="P", help="detector noise: share of missed detections")
     p.add_argument("--random-cameras", action="store_true",
                    help="a random camera setup per pose (around the room of --rig) instead of one ring for all poses")
+    p.add_argument("--refine-triangulations", action="store_true",
+                   help="also score each triangulation refined by Levenberg-Marquardt on the conf^2-weighted reprojection "
+                        "error (needs --triangulate or --triangulate-robust)")
     a = p.parse_args(argv)
+    if a.refine_triangulations and not (a.triangulate or a.triangulate_robust):
+        p.error("--refine-triangulations needs --triangulate or --triangulate-robust")
     run(a.arch, a.views, a.depth, a.poses, a.micro_batch, a.precision, a.rig, a.seed, triangulate=a.triangulate,
         pixel_noise=a.pixel_noise, outlier_rate=a.outlier_rate, miss_rate=a.miss_rate,
-        triangulate_robust=a.triangulate_robust, inlier_px=a.inlier_px, random_cameras=a.random_cameras)
+        triangulate_robust=a.triangulate_robust, inlier_px=a.inlier_px, random_cameras=a.random_cameras,
+        refine_triangulations=a.refine_triangulations)
 
 
 if __name__ == "__main__":

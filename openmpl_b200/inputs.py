@@ -84,6 +84,43 @@ def triangulate_robust(pix: torch.Tensor, calib, min_conf: float = 0.0, inlier_p
     return points, inliers
 
 
+def refine_triangulation(pix: torch.Tensor, calib, init: torch.Tensor, view_mask: torch.Tensor | None = None,
+                         min_conf: float = 0.0, max_iters: int = 20) -> tuple:
+    """Levenberg-Marquardt refinement of triangulated points on the confidence-weighted reprojection error
+    (`mpl_triangulate_refine`), enqueued on the current stream.
+
+    pix [B, V, J, 3] fp32 (u, v, conf) pixels on the device; calib [V, 18] or [B, V, 18] as for `build_inputs`; init
+    [B, J, 3] starting points, e.g. the points of `triangulate` or `triangulate_robust`.  Per (pose, joint), the views used
+    are the candidates of `triangulate` (conf > min_conf, strictly inside the image) whose bit is set in view_mask [B, J]
+    int32 (None: every candidate).  Pass `triangulate_robust`'s inliers as view_mask to refine over them; do NOT pass the
+    views_used count of `triangulate`, which is a number of views, not a bitmask.  Minimises
+    sum_v conf_v^2 |pi(P_v X) - x_v|^2 in fp64 (the maximum-likelihood point when the pixel noise has std sigma / conf)
+    with at most max_iters (1 to 100) iterations.  Returns (points [B, J, 3] fp32; reproj_px [B, J] fp32, the conf-weighted
+    RMS pixel error at the refined point).  Where init is not finite, fewer than two views are used or init lies behind a
+    used camera, points is init unchanged and reproj_px is NaN.
+    """
+    B, V, J, _ = pix.shape
+    device = pix.device
+    if tuple(init.shape) != (B, J, 3):
+        raise ValueError(f"init must be [B, J, 3] = [{B}, {J}, 3], got {list(init.shape)}")
+    if view_mask is not None and (tuple(view_mask.shape) != (B, J) or view_mask.dtype != torch.int32):
+        raise ValueError(f"view_mask must be a [B, J] = [{B}, {J}] int32 bitmask, got {list(view_mask.shape)} "
+                         f"{view_mask.dtype}")
+    pix = pix.to(torch.float32).contiguous()
+    init = init.to(device=device, dtype=torch.float32).contiguous()
+    mask = None if view_mask is None else view_mask.to(device).contiguous()
+    calib, stride = _calib_arg(calib, B, V, device)
+    points = torch.empty((B, J, 3), dtype=torch.float32, device=device)
+    reproj_px = torch.empty((B, J), dtype=torch.float32, device=device)
+    with torch.cuda.device(device):
+        stream = torch.cuda.current_stream(device).cuda_stream
+        _lib.check(_lib.lib().mpl_triangulate_refine_strided(
+            pix.data_ptr(), calib.data_ptr(), stride, B, V, J, float(min_conf),
+            None if mask is None else mask.data_ptr(), init.data_ptr(), int(max_iters), points.data_ptr(),
+            reproj_px.data_ptr(), stream))
+    return points, reproj_px
+
+
 def add_detector_noise(pix: torch.Tensor, calib, seed: int, start: int, sigma_px: float, p_outlier: float,
                        p_miss: float) -> torch.Tensor:
     """Detector-error model (`mpl_synth_detector_noise`) applied IN PLACE to raw pixels of poses [start, start + B),
