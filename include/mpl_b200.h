@@ -43,7 +43,7 @@
 extern "C" {
 #endif
 
-#define MPL_ABI_VERSION 6
+#define MPL_ABI_VERSION 7
 
 typedef enum MplStatus {
   MPL_OK = 0,
@@ -207,6 +207,39 @@ int mpl_mpjpe_accumulate(const float* pred, const float* gt, const float* conf3d
 #define MPL_PMETRIC_ACC_LEN(J) ((J) + 3)
 int mpl_pmpjpe_accumulate(const float* pred, const float* gt, int64_t batch, int num_joints, float unit_scale,
                           int scaling, int reflection, double* acc, mpl_stream_t stream);
+
+/* Grouped metrics (ABI 7): per-group running sums in one call, e.g. the per-action table of H36M, where a batch mixes
+ * actions.  Rules shared by the two entry points below:
+ *   - acc is [num_groups][L] doubles; pose b adds into block group[b] (a device array of batch int32).  A pose whose group
+ *     is outside [0, num_groups) adds nothing and is counted nowhere, so -1 can mark an unlabelled pose.
+ *   - group == NULL is allowed only with num_groups == 1: every pose then goes to block 0.
+ *   - MPL_ERR_INVALID_ARGUMENT, before any CUDA call: num_groups outside [1, 65536], group == NULL with num_groups > 1, a null
+ *     pred, gt or acc, batch < 0, num_joints < 1, and (P-MPJPE) reflection outside {-1, 0, 1}.  After these checks batch == 0
+ *     returns MPL_OK without touching the pointers.
+ *
+ * mpl_mpjpe_accumulate_grouped: each block has the MPL_METRIC_ACC_LEN(J) layout and the masking, root-relative and room rules
+ * of mpl_mpjpe_accumulate over the poses of its group, its [11 J] entry counting them.  With num_groups == 1 and every
+ * group 0, block 0 is mpl_mpjpe_accumulate's result up to the order of the fp64 sums, bitwise for one pose. */
+int mpl_mpjpe_accumulate_grouped(const float* pred, const float* gt, const float* conf3d, const int32_t* group,
+                                 int num_groups, int64_t batch, int num_joints, float unit_scale,
+                                 const float* room_affine, double* acc, mpl_stream_t stream);
+
+/* mpl_pmpjpe_accumulate_masked: P-MPJPE over the joints each pose marks, in groups.  mask: NULL or a device [batch, J] fp32.
+ *   - Joint j of pose b is used iff (mask == NULL or mask[b J + j] > 0) and its six coordinates (pred and gt) are finite, so
+ *     non-finite points under a zero mask, or left unmasked, cannot poison a pose.
+ *   - A pose is aligned iff it has at least 3 used joints and both centred sums of squares over them (after the unit rule)
+ *     are > 0; otherwise it is skipped.  An aligned pose runs the Procrustes of mpl_pmpjpe_accumulate (unit rule, scaling,
+ *     reflection rule, completion of a vanishing singular value) on its used joints only: the means (divided by the number
+ *     n of used joints), the norms and the cross-covariance are taken over them, in joint order.
+ *   - Per-block layout, L = MPL_PMETRIC_MASKED_ACC_LEN(J): [0, J) sum ||Z_j - gt_j|| over the aligned poses where j is used;
+ *     [J, 2J) the number of those instances; [2J] sum d; [2J+1] sum scale (1 when scaling == 0); [2J+2] aligned poses;
+ *     [2J+3] skipped poses.
+ *   - With every joint used the per-pose arithmetic is mpl_pmpjpe_accumulate's in the same order (n = J), so a one-pose call
+ *     gives bitwise its [0, J), d and scale. */
+#define MPL_PMETRIC_MASKED_ACC_LEN(J) (2 * (J) + 4)
+int mpl_pmpjpe_accumulate_masked(const float* pred, const float* gt, const float* mask, const int32_t* group,
+                                 int num_groups, int64_t batch, int num_joints, float unit_scale, int scaling,
+                                 int reflection, double* acc, mpl_stream_t stream);
 
 /* Per-sample input construction of the dataset (joints_dataset_mpl.py:615-648,701-715,762-772,817-820,872-904),
  * batched: raw detector output (u, v, conf) in pixels + per-view calibration -> the model's poses / rays / centers.

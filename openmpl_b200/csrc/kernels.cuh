@@ -198,10 +198,12 @@ int launch_fpt_kp_fused(float* tok, const void* wpack, int V, int64_t B, int dep
 
 // ---- metric + input builder -----------------------------------------------------------------------------------------
 // room_affine: host pointer to 6 floats (scale xyz, offset xyz) or null -- the room un-scaling of function_mpl.py:476-488
-int launch_mpjpe_accumulate(const float* pred, const float* gt, const float* conf3d, int64_t B, int J, float unit_scale,
-                            const float* room_affine, double* acc, cudaStream_t s);
-int launch_pmpjpe_accumulate(const float* pred, const float* gt, int64_t B, int J, float unit_scale, int scaling,
-                             int reflection, double* acc, cudaStream_t s);
+// G = 0: mpl_mpjpe_accumulate (group ignored); G >= 1: mpl_mpjpe_accumulate_grouped, acc [G][11 J + 1]
+int launch_mpjpe_accumulate(const float* pred, const float* gt, const float* conf3d, const int32_t* group, int G, int64_t B,
+                            int J, float unit_scale, const float* room_affine, double* acc, cudaStream_t s);
+// G = 0: mpl_pmpjpe_accumulate (mask, group ignored); G >= 1: mpl_pmpjpe_accumulate_masked, acc [G][2 J + 4]
+int launch_pmpjpe_accumulate(const float* pred, const float* gt, const float* mask, const int32_t* group, int G, int64_t B,
+                             int J, float unit_scale, int scaling, int reflection, double* acc, cudaStream_t s);
 // calib_stride: 0 = one calib [V, 18] for every pose; else pose b reads calib + b * calib_stride (>= 18 V, checked by the caller)
 int launch_build_inputs(const float* pix, const double* calib, int64_t calib_stride, int64_t B, int V, int J, float* poses,
                         float* rays, float* centers, cudaStream_t s);

@@ -24,12 +24,20 @@ struct RoomAffine {
   int live;
 };
 
+// kGrouped (mpl_mpjpe_accumulate_grouped): acc is [G][L] and pose b adds into block group[b] (nothing when it is outside
+// [0, G)).  Every lane of a warp works on the same pose, so the group is warp-uniform: the register partials are kept while
+// consecutive poses of the warp share a group and flushed into that group's block when it changes.  They go to a shared
+// copy of the G L block sums when ssum != 0 (flushed to acc at the end like the ungrouped kernel's), else straight to acc.
+template <bool kGrouped>
 __global__ void __launch_bounds__(256) mpjpe_kernel(const float* __restrict__ pred, const float* __restrict__ gt,
                                                     const float* __restrict__ conf, int64_t B, int J, float unit,
-                                                    const RoomAffine room, double* __restrict__ acc) {
-  extern __shared__ double sacc[];  // 11 J + 1
+                                                    const RoomAffine room, double* __restrict__ acc,
+                                                    const int32_t* __restrict__ group, int G, int ssum) {
+  extern __shared__ double sacc[];  // 11 J + 1; kGrouped: G (11 J + 1) when ssum, else unused
   const int L = 11 * J + 1;
-  for (int i = threadIdx.x; i < L; i += blockDim.x) sacc[i] = 0.0;
+  const int nsh = kGrouped ? (ssum ? G * L : 0) : L;
+  double* const dst = kGrouped && !ssum ? acc : sacc;
+  for (int i = threadIdx.x; i < nsh; i += blockDim.x) sacc[i] = 0.0;
   __syncthreads();
   const int lane = threadIdx.x & 31;
   const int warps_per_block = blockDim.x >> 5;
@@ -38,9 +46,35 @@ __global__ void __launch_bounds__(256) mpjpe_kernel(const float* __restrict__ pr
   for (int j0 = 0; j0 < J; j0 += 32) {
     const int j = j0 + lane;
     const bool live = j < J;
-    double a_abs = 0, a_rel = 0, d_abs[3] = {0, 0, 0}, d_rel[3] = {0, 0, 0}, cnt[3] = {0, 0, 0};
+    double a_abs = 0, a_rel = 0, d_abs[3] = {0, 0, 0}, d_rel[3] = {0, 0, 0}, cnt[3] = {0, 0, 0}, poses = 0;
+    int cur = -1;                                          // kGrouped: group of the partials
+    auto flush = [&](double* blk) {
+      atomicAdd(&blk[j], a_abs);
+      atomicAdd(&blk[J + j], a_rel);
+#pragma unroll
+      for (int k = 0; k < 3; ++k) {
+        atomicAdd(&blk[2 * J + j * 3 + k], d_abs[k]);
+        atomicAdd(&blk[5 * J + j * 3 + k], d_rel[k]);
+        atomicAdd(&blk[8 * J + j * 3 + k], cnt[k]);
+      }
+    };
     for (int64_t b = warp_global; b < B; b += warp_stride) {
       if (!live) continue;
+      if (kGrouped) {
+        const int g = group == nullptr ? 0 : group[b];
+        if (g != cur) {
+          if (cur >= 0) {
+            flush(dst + (size_t)cur * L);
+            if (j == 0) atomicAdd(&dst[(size_t)cur * L + L - 1], poses);
+            a_abs = a_rel = poses = 0.0;
+#pragma unroll
+            for (int k = 0; k < 3; ++k) d_abs[k] = d_rel[k] = cnt[k] = 0.0;
+          }
+          cur = g >= 0 && g < G ? g : -1;
+        }
+        if (cur < 0) continue;
+        poses += 1.0;
+      }
       const float* p = pred + (b * J + j) * 3;
       const float* g = gt + (b * J + j) * 3;
       const float* p0 = pred + b * J * 3;
@@ -71,25 +105,28 @@ __global__ void __launch_bounds__(256) mpjpe_kernel(const float* __restrict__ pr
       a_abs += sqrt(sa);
       a_rel += sqrt(sr);
     }
-    if (live) {
-      atomicAdd(&sacc[j], a_abs);
-      atomicAdd(&sacc[J + j], a_rel);
-#pragma unroll
-      for (int k = 0; k < 3; ++k) {
-        atomicAdd(&sacc[2 * J + j * 3 + k], d_abs[k]);
-        atomicAdd(&sacc[5 * J + j * 3 + k], d_rel[k]);
-        atomicAdd(&sacc[8 * J + j * 3 + k], cnt[k]);
+    if (kGrouped) {
+      if (cur >= 0) {
+        flush(dst + (size_t)cur * L);
+        if (j == 0) atomicAdd(&dst[(size_t)cur * L + L - 1], poses);
       }
+    } else if (live) {
+      flush(sacc);
     }
   }
   __syncthreads();
-  for (int i = threadIdx.x; i < L - 1; i += blockDim.x)
-    if (sacc[i] != 0.0) atomicAdd(&acc[i], sacc[i]);
-  if (blockIdx.x == 0 && threadIdx.x == 0) atomicAdd(&acc[L - 1], (double)B);
+  if (kGrouped) {
+    for (int i = threadIdx.x; i < nsh; i += blockDim.x)
+      if (sacc[i] != 0.0) atomicAdd(&acc[i], sacc[i]);
+  } else {
+    for (int i = threadIdx.x; i < L - 1; i += blockDim.x)
+      if (sacc[i] != 0.0) atomicAdd(&acc[i], sacc[i]);
+    if (blockIdx.x == 0 && threadIdx.x == 0) atomicAdd(&acc[L - 1], (double)B);
+  }
 }
 
-int launch_mpjpe_accumulate(const float* pred, const float* gt, const float* conf3d, int64_t B, int J, float unit_scale,
-                            const float* room_affine, double* acc, cudaStream_t s) {
+int launch_mpjpe_accumulate(const float* pred, const float* gt, const float* conf3d, const int32_t* group, int G, int64_t B,
+                            int J, float unit_scale, const float* room_affine, double* acc, cudaStream_t s) {
   if (B == 0) return MPL_OK;
   RoomAffine room{};
   if (room_affine != nullptr) {
@@ -98,7 +135,20 @@ int launch_mpjpe_accumulate(const float* pred, const float* gt, const float* con
   }
   const int64_t want = ceil_div(B, 8 * 16);  // 8 warps per block, ~16 poses per warp
   const unsigned grid = (unsigned)(want < 1 ? 1 : (want > 8 * kNumSMs ? 8 * kNumSMs : want));
-  mpjpe_kernel<<<grid, 256, (size_t)(11 * J + 1) * sizeof(double), s>>>(pred, gt, conf3d, B, J, unit_scale, room, acc);
+  if (G == 0) {
+    mpjpe_kernel<false><<<grid, 256, (size_t)(11 * J + 1) * sizeof(double), s>>>(pred, gt, conf3d, B, J, unit_scale, room,
+                                                                                 acc, nullptr, 0, 0);
+  } else {
+    // the G blocks go to shared memory when they fit what a block may opt into, else the flushes are global atomics
+    const size_t bytes = (size_t)G * (11 * J + 1) * sizeof(double);
+    int dev = 0, optin = 48 * 1024;
+    MPL_CUDA(cudaGetDevice(&dev));
+    MPL_CUDA(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
+    const bool ssum = bytes <= (size_t)optin;
+    if (ssum && bytes > 48 * 1024)
+      MPL_CUDA(cudaFuncSetAttribute(mpjpe_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
+    mpjpe_kernel<true><<<grid, 256, ssum ? bytes : 0, s>>>(pred, gt, conf3d, B, J, unit_scale, room, acc, group, G, (int)ssum);
+  }
   MPL_LAUNCH_CHECK();
   return MPL_OK;
 }
@@ -149,15 +199,171 @@ __device__ __forceinline__ void svd3_one_sided(double (&G)[3][3], double (&V)[3]
   }
 }
 
+// Procrustes of one pose over the joints j with use(j), n of them: on return Z_j = zs * (B_j - bm) R + am, with d and scale.
+// kMasked (mpl_pmpjpe_accumulate_masked) returns false for a skipped pose: n < 3, or a centred sum of squares not > 0.  With
+// every joint used its arithmetic is the unmasked one in the same order (n = J).  kMasked also finds imin / imax and
+// completes U without run-time indices into sig / U, which would put them in a stack frame; the unmasked kernel keeps its
+// original form, the same arithmetic.
+template <bool kMasked, typename Use>
+__device__ __forceinline__ bool procrustes_pose(const float* p, const float* g, int J, int n, double u, int scaling,
+                                                int reflection, Use use, double (&am)[3], double (&bm)[3], double (&R)[3][3],
+                                                double& zs, double& d, double& scale) {
+  if constexpr (kMasked) if (n < 3) return false;
+  for (int j = 0; j < J; ++j) {
+    if (!use(j)) continue;
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+      am[k] += (double)g[j * 3 + k] * u;
+      bm[k] += (double)p[j * 3 + k] * u;
+    }
+  }
+#pragma unroll
+  for (int k = 0; k < 3; ++k) {
+    am[k] /= (double)n;
+    bm[k] /= (double)n;
+  }
+  double ssx = 0, ssy = 0, G[3][3] = {{0, 0, 0}, {0, 0, 0}, {0, 0, 0}}, V[3][3];
+  for (int j = 0; j < J; ++j) {
+    if (!use(j)) continue;
+    double a0[3], c0[3];
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+      a0[k] = (double)g[j * 3 + k] * u - am[k];
+      c0[k] = (double)p[j * 3 + k] * u - bm[k];
+      ssx = fma(a0[k], a0[k], ssx);
+      ssy = fma(c0[k], c0[k], ssy);
+    }
+#pragma unroll
+    for (int i = 0; i < 3; ++i)
+#pragma unroll
+      for (int k = 0; k < 3; ++k) G[i][k] = fma(a0[i], c0[k], G[i][k]);
+  }
+  if constexpr (kMasked) if (!(ssx > 0.0 && ssy > 0.0)) return false;
+  const double a_norm = sqrt(ssx), b_norm = sqrt(ssy), inv = 1.0 / (a_norm * b_norm);
+#pragma unroll
+  for (int i = 0; i < 3; ++i)
+#pragma unroll
+    for (int k = 0; k < 3; ++k) G[i][k] *= inv;
+  svd3_one_sided(G, V);
+  double sig[3], U[3][3];
+  int imin = 0, imax = 0;
+  double smax = 0.0;
+  if constexpr (kMasked) {
+    double smin = 0.0;
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {
+      sig[c] = sqrt(G[0][c] * G[0][c] + G[1][c] * G[1][c] + G[2][c] * G[2][c]);
+      if (c == 0) smin = smax = sig[0];
+      if (sig[c] < smin) { imin = c; smin = sig[c]; }
+      if (sig[c] > smax) { imax = c; smax = sig[c]; }
+    }
+  } else {
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {
+      sig[c] = sqrt(G[0][c] * G[0][c] + G[1][c] * G[1][c] + G[2][c] * G[2][c]);
+      if (sig[c] < sig[imin]) imin = c;
+      if (sig[c] > sig[imax]) imax = c;
+    }
+  }
+  // left vectors; a vanishing singular value (planar / collinear prediction) gets the completion of the others
+  const double tiny = 1e-14 * (kMasked ? smax : sig[imax]);
+  int n_ok = 0;
+#pragma unroll
+  for (int c = 0; c < 3; ++c) {
+    const bool ok = sig[c] > tiny;
+    n_ok += ok;
+#pragma unroll
+    for (int i = 0; i < 3; ++i) U[i][c] = ok ? G[i][c] / sig[c] : 0.0;
+  }
+  if (n_ok == 2) {
+    if constexpr (kMasked) {
+#pragma unroll
+      for (int c = 0; c < 3; ++c)
+        if (c == imin) {
+          const int a = (c + 1) % 3, b = (c + 2) % 3;
+          U[0][c] = U[1][a] * U[2][b] - U[2][a] * U[1][b];
+          U[1][c] = U[2][a] * U[0][b] - U[0][a] * U[2][b];
+          U[2][c] = U[0][a] * U[1][b] - U[1][a] * U[0][b];
+        }
+    } else {
+      const int c = imin, a = (c + 1) % 3, b = (c + 2) % 3;
+      U[0][c] = U[1][a] * U[2][b] - U[2][a] * U[1][b];
+      U[1][c] = U[2][a] * U[0][b] - U[0][a] * U[2][b];
+      U[2][c] = U[0][a] * U[1][b] - U[1][a] * U[0][b];
+    }
+  }
+  if (reflection >= 0) {                                  // :112-120, det(R) = det(V) det(U)
+    double detR;
+    {
+      double Rt[3][3];
+#pragma unroll
+      for (int a = 0; a < 3; ++a)
+#pragma unroll
+        for (int b = 0; b < 3; ++b) Rt[a][b] = V[a][0] * U[b][0] + V[a][1] * U[b][1] + V[a][2] * U[b][2];
+      detR = Rt[0][0] * (Rt[1][1] * Rt[2][2] - Rt[1][2] * Rt[2][1]) - Rt[0][1] * (Rt[1][0] * Rt[2][2] - Rt[1][2] * Rt[2][0]) +
+             Rt[0][2] * (Rt[1][0] * Rt[2][1] - Rt[1][1] * Rt[2][0]);
+    }
+    if ((reflection != 0) != (detR < 0.0)) {
+#pragma unroll
+      for (int c = 0; c < 3; ++c)
+        if (c == imin) {
+          V[0][c] = -V[0][c];
+          V[1][c] = -V[1][c];
+          V[2][c] = -V[2][c];
+          sig[c] = -sig[c];
+        }
+    }
+  }
+#pragma unroll
+  for (int a = 0; a < 3; ++a)
+#pragma unroll
+    for (int b = 0; b < 3; ++b) R[a][b] = V[a][0] * U[b][0] + V[a][1] * U[b][1] + V[a][2] * U[b][2];
+  const double s_trace = sig[0] + sig[1] + sig[2];
+  if (scaling) {
+    scale = s_trace * a_norm / b_norm;
+    d = 1.0 - s_trace * s_trace;
+    zs = scale;                                           // a_norm * s_trace * (B0 / b_norm)
+  } else {
+    scale = 1.0;
+    d = 1.0 + ssy / ssx - 2.0 * s_trace * b_norm / a_norm;
+    zs = 1.0;                                             // b_norm * (B0 / b_norm)
+  }
+  return true;
+}
+
+// x summed over the lanes of `peers` (the lanes holding the same group), valid in the lowest lane of the set.  A log-step
+// tree over each set's members; every lane of the warp must call it.
+__device__ __forceinline__ double reduce_peers(unsigned peers, double x) {
+  const int lane = threadIdx.x & 31;
+  unsigned rel = __popc(peers & ((1u << lane) - 1u));    // my rank within the set
+  unsigned above = peers & (0xfffffffeu << lane);
+  while (__any_sync(0xffffffffu, above != 0u)) {
+    const int next = __ffs(above);
+    const double t = __shfl_sync(0xffffffffu, x, next > 0 ? next - 1 : lane);
+    if (next > 0) x += t;
+    above &= __ballot_sync(0xffffffffu, (rel & 1u) == 0u);
+    rel >>= 1;
+  }
+  return x;
+}
+
+// kMasked (mpl_pmpjpe_accumulate_masked): the mask tile [tile][J] is staged with the poses, joint j of a pose is used iff its
+// mask is > 0 (or mask is null) and its six coordinates are finite, and pose b adds into block group[b] of the
+// MPL_PMETRIC_MASKED_ACC_LEN(J) layout.  Lanes of a warp may hold different groups: each set of lanes with the same group
+// (__match_any_sync) is reduced and its lowest lane adds into acc.  The unmasked kernel keeps one shared block sum.
+template <bool kMasked>
 __global__ void __launch_bounds__(64) pmpjpe_kernel(const float* __restrict__ pred, const float* __restrict__ gt,
                                                     int64_t B, int J, float unit, int scaling, int reflection,
-                                                    double* __restrict__ acc) {
+                                                    double* __restrict__ acc, const float* __restrict__ mask,
+                                                    const int32_t* __restrict__ group, int G) {
   extern __shared__ __align__(16) unsigned char psm[];
   const int tile = blockDim.x, row = 3 * J;
-  double* sacc = reinterpret_cast<double*>(psm);                       // J + 3
-  float* sp = reinterpret_cast<float*>(sacc + (J + 3 + 1) / 2 * 2);    // [tile][3 J]
+  double* sacc = reinterpret_cast<double*>(psm);                       // J + 3 (unmasked only)
+  float* sp = reinterpret_cast<float*>(sacc + (kMasked ? 0 : (J + 3 + 1) / 2 * 2));   // [tile][3 J]
   float* sg = sp + (size_t)tile * row;
-  for (int i = threadIdx.x; i < J + 3; i += blockDim.x) sacc[i] = 0.0;
+  float* sm = sg + (size_t)tile * row;                                 // kMasked: [tile][J]
+  if (!kMasked)
+    for (int i = threadIdx.x; i < J + 3; i += blockDim.x) sacc[i] = 0.0;
   const int64_t n_tiles = (B + tile - 1) / tile;
   for (int64_t tl = blockIdx.x; tl < n_tiles; tl += gridDim.x) {
     const int64_t b0 = tl * tile;
@@ -167,110 +373,40 @@ __global__ void __launch_bounds__(64) pmpjpe_kernel(const float* __restrict__ pr
       sp[i] = pred[b0 * row + i];
       sg[i] = gt[b0 * row + i];
     }
+    if (kMasked && mask != nullptr)
+      for (int i = threadIdx.x; i < n * J; i += blockDim.x) sm[i] = mask[b0 * J + i];
     __syncthreads();
     const bool live = (int)threadIdx.x < n;
     const float* p = sp + (size_t)threadIdx.x * row;
     const float* g = sg + (size_t)threadIdx.x * row;
+    const float* m = sm + (size_t)threadIdx.x * J;
     const double u = (double)unit;
-    double am[3] = {0, 0, 0}, bm[3] = {0, 0, 0}, R[3][3], zs = 0.0, d = 0.0, scale = 0.0;
-    if (live) {
-      for (int j = 0; j < J; ++j)
-#pragma unroll
-        for (int k = 0; k < 3; ++k) {
-          am[k] += (double)g[j * 3 + k] * u;
-          bm[k] += (double)p[j * 3 + k] * u;
-        }
-#pragma unroll
-      for (int k = 0; k < 3; ++k) {
-        am[k] /= (double)J;
-        bm[k] /= (double)J;
-      }
-      double ssx = 0, ssy = 0, G[3][3] = {{0, 0, 0}, {0, 0, 0}, {0, 0, 0}}, V[3][3];
-      for (int j = 0; j < J; ++j) {
-        double a0[3], c0[3];
-#pragma unroll
-        for (int k = 0; k < 3; ++k) {
-          a0[k] = (double)g[j * 3 + k] * u - am[k];
-          c0[k] = (double)p[j * 3 + k] * u - bm[k];
-          ssx = fma(a0[k], a0[k], ssx);
-          ssy = fma(c0[k], c0[k], ssy);
-        }
-#pragma unroll
-        for (int i = 0; i < 3; ++i)
-#pragma unroll
-          for (int k = 0; k < 3; ++k) G[i][k] = fma(a0[i], c0[k], G[i][k]);
-      }
-      const double a_norm = sqrt(ssx), b_norm = sqrt(ssy), inv = 1.0 / (a_norm * b_norm);
-#pragma unroll
-      for (int i = 0; i < 3; ++i)
-#pragma unroll
-        for (int k = 0; k < 3; ++k) G[i][k] *= inv;
-      svd3_one_sided(G, V);
-      double sig[3], U[3][3];
-      int imin = 0, imax = 0;
-#pragma unroll
-      for (int c = 0; c < 3; ++c) {
-        sig[c] = sqrt(G[0][c] * G[0][c] + G[1][c] * G[1][c] + G[2][c] * G[2][c]);
-        if (sig[c] < sig[imin]) imin = c;
-        if (sig[c] > sig[imax]) imax = c;
-      }
-      // left vectors; a vanishing singular value (planar / collinear prediction) gets the completion of the others
-      const double tiny = 1e-14 * sig[imax];
-      int n_ok = 0;
-#pragma unroll
-      for (int c = 0; c < 3; ++c) {
-        const bool ok = sig[c] > tiny;
-        n_ok += ok;
-#pragma unroll
-        for (int i = 0; i < 3; ++i) U[i][c] = ok ? G[i][c] / sig[c] : 0.0;
-      }
-      if (n_ok == 2) {
-        const int c = imin, a = (c + 1) % 3, b = (c + 2) % 3;
-        U[0][c] = U[1][a] * U[2][b] - U[2][a] * U[1][b];
-        U[1][c] = U[2][a] * U[0][b] - U[0][a] * U[2][b];
-        U[2][c] = U[0][a] * U[1][b] - U[1][a] * U[0][b];
-      }
-      if (reflection >= 0) {                                  // :112-120, det(R) = det(V) det(U)
-        double detR;
-        {
-          double Rt[3][3];
-#pragma unroll
-          for (int a = 0; a < 3; ++a)
-#pragma unroll
-            for (int b = 0; b < 3; ++b) Rt[a][b] = V[a][0] * U[b][0] + V[a][1] * U[b][1] + V[a][2] * U[b][2];
-          detR = Rt[0][0] * (Rt[1][1] * Rt[2][2] - Rt[1][2] * Rt[2][1]) - Rt[0][1] * (Rt[1][0] * Rt[2][2] - Rt[1][2] * Rt[2][0]) +
-                 Rt[0][2] * (Rt[1][0] * Rt[2][1] - Rt[1][1] * Rt[2][0]);
-        }
-        if ((reflection != 0) != (detR < 0.0)) {
-#pragma unroll
-          for (int c = 0; c < 3; ++c)
-            if (c == imin) {
-              V[0][c] = -V[0][c];
-              V[1][c] = -V[1][c];
-              V[2][c] = -V[2][c];
-              sig[c] = -sig[c];
-            }
-        }
-      }
-#pragma unroll
-      for (int a = 0; a < 3; ++a)
-#pragma unroll
-        for (int b = 0; b < 3; ++b) R[a][b] = V[a][0] * U[b][0] + V[a][1] * U[b][1] + V[a][2] * U[b][2];
-      const double s_trace = sig[0] + sig[1] + sig[2];
-      if (scaling) {
-        scale = s_trace * a_norm / b_norm;
-        d = 1.0 - s_trace * s_trace;
-        zs = scale;                                           // a_norm * s_trace * (B0 / b_norm)
-      } else {
-        scale = 1.0;
-        d = 1.0 + ssy / ssx - 2.0 * s_trace * b_norm / a_norm;
-        zs = 1.0;                                             // b_norm * (B0 / b_norm)
-      }
+    auto use = [&](int j) {
+      if (!kMasked) return true;
+      return (mask == nullptr || m[j] > 0.f) && isfinite(p[j * 3]) && isfinite(p[j * 3 + 1]) && isfinite(p[j * 3 + 2]) &&
+             isfinite(g[j * 3]) && isfinite(g[j * 3 + 1]) && isfinite(g[j * 3 + 2]);
+    };
+    // kMasked: gid = the pose's block, or -1 when it adds nothing (a dead lane, or a group outside [0, G))
+    int gid = 0, nu = J;
+    if (kMasked) {
+      gid = live ? (group == nullptr ? 0 : group[b0 + threadIdx.x]) : -1;
+      if (gid >= G) gid = -1;
+      nu = 0;
+      if (gid >= 0)
+        for (int j = 0; j < J; ++j) nu += use(j);
     }
+    double am[3] = {0, 0, 0}, bm[3] = {0, 0, 0}, R[3][3], zs = 0.0, d = 0.0, scale = 0.0;
+    bool aligned = false;
+    if (kMasked ? gid >= 0 : live)
+      aligned = procrustes_pose<kMasked>(p, g, J, nu, u, scaling, reflection, use, am, bm, R, zs, d, scale);
     const int lane = threadIdx.x & 31;
+    const unsigned peers = kMasked ? __match_any_sync(0xffffffffu, gid) : 0xffffffffu;
+    const bool leader = kMasked ? gid >= 0 && lane == __ffs(peers) - 1 : lane == 0;
+    double* blk = kMasked ? acc + (size_t)(gid < 0 ? 0 : gid) * (2 * J + 4) : sacc;
     for (int j = 0; j < J; ++j) {
       double e = 0.0;
-      if (live) {
+      const bool on = kMasked ? aligned && use(j) : live;
+      if (on) {
         double c0[3], acc2 = 0.0;
 #pragma unroll
         for (int k = 0; k < 3; ++k) c0[k] = (double)p[j * 3 + k] * u - bm[k];
@@ -282,39 +418,74 @@ __global__ void __launch_bounds__(64) pmpjpe_kernel(const float* __restrict__ pr
         }
         e = sqrt(acc2);
       }
+      if (kMasked) {
+        e = reduce_peers(peers, e);
+        const int cnt = __popc(__ballot_sync(0xffffffffu, on) & peers);
+        if (leader && cnt > 0) {
+          atomicAdd(&blk[j], e);
+          atomicAdd(&blk[J + j], (double)cnt);
+        }
+      } else {
 #pragma unroll
-      for (int o = 16; o > 0; o >>= 1) e += __shfl_xor_sync(0xffffffffu, e, o);
-      if (lane == 0) atomicAdd(&sacc[j], e);
+        for (int o = 16; o > 0; o >>= 1) e += __shfl_xor_sync(0xffffffffu, e, o);
+        if (lane == 0) atomicAdd(&sacc[j], e);
+      }
     }
-    double sd = live ? d : 0.0, ssc = live ? scale : 0.0;
+    if (kMasked) {
+      const double sd = reduce_peers(peers, aligned ? d : 0.0), ssc = reduce_peers(peers, aligned ? scale : 0.0);
+      const int na = __popc(__ballot_sync(0xffffffffu, aligned) & peers);
+      const int ns = __popc(__ballot_sync(0xffffffffu, gid >= 0 && !aligned) & peers);
+      if (leader) {
+        if (na > 0) {
+          atomicAdd(&blk[2 * J], sd);
+          atomicAdd(&blk[2 * J + 1], ssc);
+          atomicAdd(&blk[2 * J + 2], (double)na);
+        }
+        if (ns > 0) atomicAdd(&blk[2 * J + 3], (double)ns);
+      }
+    } else {
+      double sd = live ? d : 0.0, ssc = live ? scale : 0.0;
 #pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-      sd += __shfl_xor_sync(0xffffffffu, sd, o);
-      ssc += __shfl_xor_sync(0xffffffffu, ssc, o);
-    }
-    if (lane == 0) {
-      atomicAdd(&sacc[J], sd);
-      atomicAdd(&sacc[J + 1], ssc);
+      for (int o = 16; o > 0; o >>= 1) {
+        sd += __shfl_xor_sync(0xffffffffu, sd, o);
+        ssc += __shfl_xor_sync(0xffffffffu, ssc, o);
+      }
+      if (lane == 0) {
+        atomicAdd(&sacc[J], sd);
+        atomicAdd(&sacc[J + 1], ssc);
+      }
     }
   }
-  __syncthreads();
-  for (int i = threadIdx.x; i < J + 2; i += blockDim.x) atomicAdd(&acc[i], sacc[i]);
-  if (blockIdx.x == 0 && threadIdx.x == 0) atomicAdd(&acc[J + 2], (double)B);
+  if (!kMasked) {
+    __syncthreads();
+    for (int i = threadIdx.x; i < J + 2; i += blockDim.x) atomicAdd(&acc[i], sacc[i]);
+    if (blockIdx.x == 0 && threadIdx.x == 0) atomicAdd(&acc[J + 2], (double)B);
+  }
 }
 
-int launch_pmpjpe_accumulate(const float* pred, const float* gt, int64_t B, int J, float unit_scale, int scaling,
-                             int reflection, double* acc, cudaStream_t s) {
+// mask == nullptr and G == 0: mpl_pmpjpe_accumulate; G >= 1: mpl_pmpjpe_accumulate_masked (mask may still be null)
+int launch_pmpjpe_accumulate(const float* pred, const float* gt, const float* mask, const int32_t* group, int G, int64_t B,
+                             int J, float unit_scale, int scaling, int reflection, double* acc, cudaStream_t s) {
   if (B == 0) return MPL_OK;
+  const bool masked = G > 0;
   int tile = 64;
-  auto smem = [&](int t) { return (size_t)((J + 3 + 1) / 2 * 2) * sizeof(double) + (size_t)2 * t * 3 * J * sizeof(float); };
+  auto smem = [&](int t) {
+    return masked ? (size_t)t * 7 * J * sizeof(float)
+                  : (size_t)((J + 3 + 1) / 2 * 2) * sizeof(double) + (size_t)2 * t * 3 * J * sizeof(float);
+  };
   if (smem(tile) > 48 * 1024) tile = 32;
   if (smem(tile) > 48 * 1024) {
-    set_error("mpl_pmpjpe_accumulate: num_joints too large for the shared-memory pose tile");
+    set_error("%s: num_joints too large for the shared-memory pose tile",
+              masked ? "mpl_pmpjpe_accumulate_masked" : "mpl_pmpjpe_accumulate");
     return MPL_ERR_INVALID_ARGUMENT;
   }
   const int64_t n_tiles = ceil_div(B, (int64_t)tile);
   const unsigned grid = (unsigned)(n_tiles > 16 * kNumSMs ? 16 * kNumSMs : n_tiles);
-  pmpjpe_kernel<<<grid, tile, smem(tile), s>>>(pred, gt, B, J, unit_scale, scaling, reflection, acc);
+  if (masked)
+    pmpjpe_kernel<true><<<grid, tile, smem(tile), s>>>(pred, gt, B, J, unit_scale, scaling, reflection, acc, mask, group, G);
+  else
+    pmpjpe_kernel<false><<<grid, tile, smem(tile), s>>>(pred, gt, B, J, unit_scale, scaling, reflection, acc, nullptr,
+                                                        nullptr, 0);
   MPL_LAUNCH_CHECK();
   return MPL_OK;
 }

@@ -1297,7 +1297,24 @@ int mpl_mpjpe_accumulate(const float* pred, const float* gt, const float* conf3d
     set_error("mpl_mpjpe_accumulate: bad argument");
     return MPL_ERR_INVALID_ARGUMENT;
   }
-  return launch_mpjpe_accumulate(pred, gt, conf3d, batch, num_joints, unit_scale, room_affine, acc,
+  return launch_mpjpe_accumulate(pred, gt, conf3d, nullptr, 0, batch, num_joints, unit_scale, room_affine, acc,
+                                 reinterpret_cast<cudaStream_t>(stream));
+}
+
+// the group rules shared by the two grouped entry points (include/mpl_b200.h)
+static bool groups_ok(const int32_t* group, int num_groups) {
+  return num_groups >= 1 && num_groups <= 65536 && (group != nullptr || num_groups == 1);
+}
+
+int mpl_mpjpe_accumulate_grouped(const float* pred, const float* gt, const float* conf3d, const int32_t* group, int num_groups,
+                                 int64_t batch, int num_joints, float unit_scale, const float* room_affine, double* acc,
+                                 mpl_stream_t stream) {
+  if (!groups_ok(group, num_groups) || pred == nullptr || gt == nullptr || acc == nullptr || batch < 0 || num_joints < 1) {
+    set_error("mpl_mpjpe_accumulate_grouped: bad argument (num_groups %d, group %s, batch %lld, num_joints %d)", num_groups,
+              group ? "set" : "null", (long long)batch, num_joints);
+    return MPL_ERR_INVALID_ARGUMENT;
+  }
+  return launch_mpjpe_accumulate(pred, gt, conf3d, group, num_groups, batch, num_joints, unit_scale, room_affine, acc,
                                  reinterpret_cast<cudaStream_t>(stream));
 }
 
@@ -1308,8 +1325,21 @@ int mpl_pmpjpe_accumulate(const float* pred, const float* gt, int64_t batch, int
     set_error("mpl_pmpjpe_accumulate: bad argument");
     return MPL_ERR_INVALID_ARGUMENT;
   }
-  return launch_pmpjpe_accumulate(pred, gt, batch, num_joints, unit_scale, scaling != 0, reflection, acc,
+  return launch_pmpjpe_accumulate(pred, gt, nullptr, nullptr, 0, batch, num_joints, unit_scale, scaling != 0, reflection, acc,
                                   reinterpret_cast<cudaStream_t>(stream));
+}
+
+int mpl_pmpjpe_accumulate_masked(const float* pred, const float* gt, const float* mask, const int32_t* group, int num_groups,
+                                 int64_t batch, int num_joints, float unit_scale, int scaling, int reflection, double* acc,
+                                 mpl_stream_t stream) {
+  if (!groups_ok(group, num_groups) || pred == nullptr || gt == nullptr || acc == nullptr || batch < 0 || num_joints < 1 ||
+      reflection < -1 || reflection > 1) {
+    set_error("mpl_pmpjpe_accumulate_masked: bad argument (num_groups %d, group %s, batch %lld, num_joints %d, reflection %d)",
+              num_groups, group ? "set" : "null", (long long)batch, num_joints, reflection);
+    return MPL_ERR_INVALID_ARGUMENT;
+  }
+  return launch_pmpjpe_accumulate(pred, gt, mask, group, num_groups, batch, num_joints, unit_scale, scaling != 0, reflection,
+                                  acc, reinterpret_cast<cudaStream_t>(stream));
 }
 
 // calib_stride of the *_strided entry points: 0 (one [V, 18] block for every pose) or >= 18 V (pose b at calib + b * stride)

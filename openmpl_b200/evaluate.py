@@ -10,6 +10,8 @@
     python -m openmpl_b200.evaluate --arch hm0 --views 4 --random-cameras --triangulate  # a random camera setup per pose
     python -m openmpl_b200.evaluate --arch hm0 --views 4 --pixel-noise 2 --triangulate --triangulate-robust \
         --refine-triangulations                                                         # + nonlinear refinement of both
+    python -m openmpl_b200.evaluate --arch hm0 --views 4 --pixel-noise 2 --triangulate --triangulate-robust \
+        --triangulation-pmpjpe                                                          # + P-MPJPE of both baselines
 
 Per micro-batch, entirely on the device: `mpl_synth_project` (3D poses from the counter-based generator keyed by the
 GLOBAL pose index, projected through the V calibrations) -> `mpl_build_inputs` (clip, confidence zeroing, screen
@@ -37,6 +39,11 @@ records the camera model.  Without the flag the one rig of `--rig` serves every 
 Levenberg-Marquardt on the conf^2-weighted reprojection error (`mpl_triangulate_refine`): the linear points over their
 candidate views, the robust points over their inliers.  Each triangulation entry gains a "refined" sub-entry, scored by its
 own accumulator under the parent entry's mask.  Without the flag nothing of this runs.
+
+`--triangulation-pmpjpe` (with `--triangulate` and / or `--triangulate-robust`) also scores each triangulation entry, and
+each "refined" sub-entry, by a masked P-MPJPE accumulator (`mpl_pmpjpe_accumulate_masked`) under that entry's own mask:
+every pose is Procrustes-aligned on its triangulated joints only.  The entry gains "procrustes_aligned".  Without the flag
+nothing of this runs.
 """
 from __future__ import annotations
 
@@ -62,9 +69,12 @@ REFINE_MAX_ITERS = 20
 
 def run(arch="hm0", views=4, depth=None, poses=1 << 20, micro_batch=65536, precision="bf16", rig=None, seed=1,
         weight_seed=0, warmup=1, triangulate=False, pixel_noise=0.0, outlier_rate=0.0, miss_rate=0.0,
-        triangulate_robust=False, inlier_px=10.0, random_cameras=False, refine_triangulations=False):
+        triangulate_robust=False, inlier_px=10.0, random_cameras=False, refine_triangulations=False,
+        triangulation_pmpjpe=False):
     if refine_triangulations and not (triangulate or triangulate_robust):
         raise ValueError("refine_triangulations needs triangulate or triangulate_robust")
+    if triangulation_pmpjpe and not (triangulate or triangulate_robust):
+        raise ValueError("triangulation_pmpjpe needs triangulate or triangulate_robust")
     rank, world, local = mdist.init_from_env("nccl")
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
@@ -86,6 +96,9 @@ def run(arch="hm0", views=4, depth=None, poses=1 << 20, micro_batch=65536, preci
     tfacc = metric.MpjpeAccumulator(cfg.J, output_in_meter=True, device=dev) if triangulate and refine_triangulations else None
     rfacc = (metric.MpjpeAccumulator(cfg.J, output_in_meter=True, device=dev) if triangulate_robust and refine_triangulations
              else None)
+    # masked P-MPJPE of each triangulation entry, keyed like the accumulators above
+    tp = {name: metric.PmpjpeAccumulator(cfg.J, output_in_meter=True, device=dev, masked=True)
+          for name, a in (("t", tacc), ("r", racc), ("tf", tfacc), ("rf", rfacc)) if triangulation_pmpjpe and a is not None}
     noisy = pixel_noise != 0 or outlier_rate != 0 or miss_rate != 0
 
     def step(s0, n):
@@ -99,23 +112,28 @@ def run(arch="hm0", views=4, depth=None, poses=1 << 20, micro_batch=65536, preci
         out = out[0] if isinstance(out, tuple) else out
         acc.update(out, target)
         pacc.update(out, target)
+        def score(key, a, points, mask):
+            a.update(points, target, mask)
+            if key in tp:
+                tp[key].update(points, target, mask)
+
         if tacc is not None:
             points, used = inputs.triangulate(pix, calib)
-            tacc.update(points, target, used >= 2)
+            score("t", tacc, points, used >= 2)
             if tfacc is not None:
-                tfacc.update(inputs.refine_triangulation(pix, calib, points, max_iters=REFINE_MAX_ITERS)[0], target, used >= 2)
+                score("tf", tfacc, inputs.refine_triangulation(pix, calib, points, max_iters=REFINE_MAX_ITERS)[0], used >= 2)
         if racc is not None:
             points, inl = inputs.triangulate_robust(pix, calib, inlier_px=inlier_px)
-            racc.update(points, target, inl != 0)      # popcount >= 2: a non-zero inlier mask has at least two bits
+            score("r", racc, points, inl != 0)         # popcount >= 2: a non-zero inlier mask has at least two bits
             if rfacc is not None:
-                rfacc.update(inputs.refine_triangulation(pix, calib, points, view_mask=inl,
-                                                           max_iters=REFINE_MAX_ITERS)[0], target, inl != 0)
+                score("rf", rfacc, inputs.refine_triangulation(pix, calib, points, view_mask=inl,
+                                                                 max_iters=REFINE_MAX_ITERS)[0], inl != 0)
 
     for _ in range(warmup):                            # allocate the workspace, pack the weights
         step(start, min(micro_batch, max(stop - start, 1)))
     acc.acc.zero_()
     pacc.acc.zero_()
-    for a in (tacc, racc, tfacc, rfacc):
+    for a in (tacc, racc, tfacc, rfacc, *tp.values()):
         if a is not None:
             a.acc.zero_()
     if world > 1:
@@ -127,7 +145,7 @@ def run(arch="hm0", views=4, depth=None, poses=1 << 20, micro_batch=65536, preci
         step(s0, min(micro_batch, stop - s0))
     acc.all_reduce()                                   # the only collectives of the whole job:
     pacc.all_reduce()                                  # 11 J + 1 and J + 3 doubles
-    for a in (tacc, racc, tfacc, rfacc):
+    for a in (tacc, racc, tfacc, rfacc, *tp.values()):
         if a is not None:
             a.all_reduce()
     e1.record()
@@ -171,6 +189,13 @@ def run(arch="hm0", views=4, depth=None, poses=1 << 20, micro_batch=65536, preci
                     a.acc.detach().cpu().numpy(), cfg.J,
                     method=f"Levenberg-Marquardt on the reprojection error over {views}, weights conf^2, "
                            f"at most {REFINE_MAX_ITERS} iterations")
+        for key, entry, sub in (("t", "triangulation", None), ("r", "triangulation_robust", None),
+                                ("tf", "triangulation", "refined"), ("rf", "triangulation_robust", "refined")):
+            if key in tp:
+                r = tp[key].result()
+                target_entry = line[entry] if sub is None else line[entry][sub]
+                target_entry["procrustes_aligned"] = {"p_mpjpe_cm": r["p_mpjpe"], "aligned_poses": r["aligned"],
+                                                      "skipped_poses": r["skipped"]}
         print(json.dumps(line), flush=True)
     if world > 1:
         torch.distributed.barrier()
@@ -183,8 +208,8 @@ def triangulation_summary(acc, J, method="linear DLT, pixel-space rows, views wi
 
     absolute / root_relative: the reference's masking convention (a masked joint adds zero error but counts as a pose).
     triangulated_joints: per joint, the error sum over its triangulated instances divided by their number (the x-count
-    of the sums), averaged over the joints triangulated at least once.  dist_rel (NaN once a root is under-determined) and
-    P-MPJPE (its accumulator takes no mask) are not reported.  For the robust triangulation the mask is "at least two
+    of the sums), averaged over the joints triangulated at least once.  dist_rel (NaN once a root is under-determined) is
+    not reported; P-MPJPE over the triangulated joints is added by run(triangulation_pmpjpe=True).  For the robust triangulation the mask is "at least two
     inliers", so under_determined_joints counts the joints it rejected as well as those seen by fewer than two views.
     """
     res = metric.finalize(acc, J)
@@ -222,13 +247,18 @@ def main(argv=None):
     p.add_argument("--refine-triangulations", action="store_true",
                    help="also score each triangulation refined by Levenberg-Marquardt on the conf^2-weighted reprojection "
                         "error (needs --triangulate or --triangulate-robust)")
+    p.add_argument("--triangulation-pmpjpe", action="store_true",
+                   help="also score each triangulation by P-MPJPE, aligned on its triangulated joints only (needs "
+                        "--triangulate or --triangulate-robust)")
     a = p.parse_args(argv)
     if a.refine_triangulations and not (a.triangulate or a.triangulate_robust):
         p.error("--refine-triangulations needs --triangulate or --triangulate-robust")
+    if a.triangulation_pmpjpe and not (a.triangulate or a.triangulate_robust):
+        p.error("--triangulation-pmpjpe needs --triangulate or --triangulate-robust")
     run(a.arch, a.views, a.depth, a.poses, a.micro_batch, a.precision, a.rig, a.seed, triangulate=a.triangulate,
         pixel_noise=a.pixel_noise, outlier_rate=a.outlier_rate, miss_rate=a.miss_rate,
         triangulate_robust=a.triangulate_robust, inlier_px=a.inlier_px, random_cameras=a.random_cameras,
-        refine_triangulations=a.refine_triangulations)
+        refine_triangulations=a.refine_triangulations, triangulation_pmpjpe=a.triangulation_pmpjpe)
 
 
 if __name__ == "__main__":
