@@ -574,8 +574,9 @@ __global__ void __launch_bounds__(256) attention_narrow_kernel(const TI* __restr
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
-// Keypoint-token attention of the FPT in bf16 mode (FPT_blocks_view_keypoint_tokens: N = V * 17 <= 136 tokens of width 32,
-// 8 heads of 4): a CTA keeps G whole token sets in shared memory as fp16 with the channels of each head PAIR interleaved
+// Keypoint-token attention of the FPT in bf16 mode where the fused FPT kernel does not apply (FPT_blocks_view_keypoint_tokens
+// with J != 17 or an MLP hidden width != 64: N = V * J <= 272 tokens of width 32, 8 heads of 4; N need not be a multiple of
+// the 17-key chunk below): a CTA keeps G whole token sets in shared memory as fp16 with the channels of each head PAIR interleaved
 // (word = (head 2p, head 2p+1) at one head-dim, q pre-scaled by scale * log2 e), exactly the staging format of the SPT
 // kernel, so the softmax of two heads runs in packed half2 arithmetic straight from 16-byte shared-memory loads.  One
 // thread per (token row, head pair), two passes over the keys (max; then exp2 / sum / PV with the scores recomputed --

@@ -251,8 +251,10 @@ __device__ __forceinline__ __half2 ex2_h2(__half2 x) {
 // rounding left is a 2^-11 operand rounding, the same class as kind::tf32's; bf16 mode takes the packed-half2 forms.
 // GROUPED: the same block stack as the keypoint-token FPT (FPT_blocks_view_keypoint_tokens: tokens = V * 17 joints of one
 // pose, width 32, one weight stack, multiview_mpl.py:261-266,416-423,496-497): `group` = V consecutive 17-row sets attend
-// together, so the whole V * J <= 136-token set of a pose lives in this CTA's shared memory for all depth + 1 block
-// applications; keys are walked in two passes (max, then exp2 / sum / PV with the scores recomputed), fp16 partial
+// together, so the whole V * J-token set of a pose lives in this CTA's shared memory for all depth + 1 block applications
+// (V <= 16: one pose of up to 238 tokens per CTA in the 14-set tile at V = 9..14, 255 / 272 tokens in the 16-set tile at
+// V = 15 / 16);
+// keys are walked in two passes (max, then exp2 / sum / PV with the scores recomputed), fp16 partial
 // sums flushed into fp32 every 17 keys.  Rows come from and go back to the fp32 token buffer in place.
 template <bool PRECISE, bool GROUPED>
 __device__ __forceinline__ void spt_fused_body(const SptArgs& args);
