@@ -15,7 +15,8 @@
  *   MPL/lib/multiviews/triangulate.py:59-115 linear triangulation baseline (-> mpl_triangulate)
  * Defined here, with no counterpart in the reference: robust (RANSAC) triangulation (mpl_triangulate_robust), nonlinear
  * refinement of triangulated points (mpl_triangulate_refine), a detector-error model for the synthetic data
- * (mpl_synth_detector_noise) and a generator of random camera setups (mpl_synth_cameras).
+ * (mpl_synth_detector_noise), a generator of random camera setups (mpl_synth_cameras) and lens distortion of pixels
+ * (mpl_distort_pixels / mpl_undistort_pixels).
  *
  * Conventions
  *   - plain pointers and sizes only; no torch / C++ types cross this boundary;
@@ -43,7 +44,7 @@
 extern "C" {
 #endif
 
-#define MPL_ABI_VERSION 7
+#define MPL_ABI_VERSION 8
 
 typedef enum MplStatus {
   MPL_OK = 0,
@@ -365,6 +366,59 @@ int mpl_synth_detector_noise(uint64_t seed, int64_t start, int64_t batch, int nu
 int mpl_synth_detector_noise_strided(uint64_t seed, int64_t start, int64_t batch, int num_views, int num_joints,
                                      const double* calib, int64_t calib_stride, float sigma_px, float p_outlier, float p_miss,
                                      float* pix, mpl_stream_t stream);
+
+/* Lens distortion (ABI 8; defined by this library, the reference's cameras are pinholes).  OpenCV's 5-coefficient
+ * Brown-Conrady model on normalised camera coordinates x = ((u - cx) / fx, (v - cy) / fy) of a pixel (u, v):
+ *   r2 = x^2 + y^2,  rho = 1 + k1 r2 + k2 r2^2 + k3 r2^3,
+ *   D(x) = (x rho + 2 p1 x y + p2 (r2 + 2 x^2),  y rho + p1 (r2 + 2 y^2) + 2 p2 x y).
+ * dist holds (k1, k2, p1, p2, k3) per view (the order of CMU Panoptic's distCoef and of OpenCV's distCoeffs), fp64:
+ * [V, 5] for the whole batch (dist_stride 0) or pose b at dist + b * dist_stride (>= 5 V; a packed [B, V, 5] tensor: 5 V).
+ * dist_stride is independent of calib_stride (the calibration convention above), so per-pose cameras can share one lens.
+ * Validity: an undistorted normalised point x is valid iff both
+ *   (a) the radial map r -> r rho(r) is increasing on [0, |x|]: g(s) = 1 + 3 k1 s + 5 k2 s^2 + 7 k3 s^3 > 0 at s = r2 and at
+ *       every root of g'(s) = 3 k1 + 10 k2 s + 21 k3 s^2 strictly inside (0, r2) (k3 != 0: the real roots
+ *       (-10 k2 -/+ sqrt(100 k2^2 - 252 k1 k3)) / (42 k3); k3 == 0, k2 != 0: -3 k1 / (10 k2)), and
+ *   (b) det J(x) > 0, J the 2 x 2 Jacobian of D.
+ * Past a fold the polynomial maps points far outside the field of view back into the image; a real camera images none.
+ * Shared rules of the two entry points below:
+ *   - pix_in / pix_out [B, V, J, 3] fp32 (u, v, conf); pix_in == pix_out (in place) is allowed, no other overlap;
+ *   - calib as in mpl_build_inputs (fx, fy, cx, cy and, for the undistortion, w and h are read); fp64 throughout, each
+ *     output pixel rounded once to fp32; entries with conf == 0 are copied unchanged;
+ *   - MPL_ERR_INVALID_ARGUMENT, before any CUDA call: batch < 0, V outside [1, 16], J < 1, a calib_stride or dist_stride
+ *     that is not 0 or >= 18 V / 5 V, a margin that is not finite or is negative; then batch == 0 returns MPL_OK without
+ *     touching the pointers (an empty tensor has no storage); then a null pointer is MPL_ERR_INVALID_ARGUMENT;
+ *   - one thread per entry; allocates nothing and never synchronises (graph-capturable); results do not depend on how the
+ *     batch is split.
+ *
+ * mpl_distort_pixels: ideal pinhole pixels (mpl_synth_project's, which are not clipped) -> the pixels a camera with this lens
+ * records: u_d = u + fx (x_d - x), v_d = v + fy (y_d - y) with (x_d, y_d) = D(x) (= fx x_d + cx up to rounding).  An entry
+ * whose x is not valid gets conf = 0 and keeps its pixel.  An entry whose five coefficients are all 0 is copied unchanged, so
+ * with a zero lens the output is the input bit for bit (non-finite pixels and -0 included).
+ * The synthetic step between mpl_synth_project and mpl_synth_detector_noise. */
+int mpl_distort_pixels(const float* pix_in, float* pix_out, const double* calib, const double* dist, int64_t batch,
+                       int num_views, int num_joints, mpl_stream_t stream);
+int mpl_distort_pixels_strided(const float* pix_in, float* pix_out, const double* calib, int64_t calib_stride,
+                               const double* dist, int64_t dist_stride, int64_t batch, int num_views, int num_joints,
+                               mpl_stream_t stream);
+
+/* mpl_undistort_pixels: detected (distorted) pixels -> the pinhole pixels of the same rays, for the triangulations, in a frame
+ * grown by margin_x / margin_y pixels on each side: pass them the calibration with cx + margin_x, cy + margin_y,
+ * w + 2 margin_x, h + 2 margin_y (DLT, reprojection errors and refinement are invariant under that shift), so undistorted
+ * pixels beyond the original frame stay candidates.  Per entry with conf != 0:
+ *   - the raw pixel not strictly inside the original frame (0 < u < w - 1 and 0 < v < h - 1, the candidate test of the
+ *     triangulations): conf = 0, pixel kept.  So the candidate sets are those of the raw pixels;
+ *   - otherwise Newton's method solves D(x) = x_d, x_d = ((u - cx) / fx, (v - cy) / fy), from x = x_d: at most 20 steps
+ *     x -= J(x)^-1 (D(x) - x_d) (Cramer's rule), stopping after a step with |dx| + |dy| not > 1e-14 (NaN included).  The
+ *     inversion succeeds iff the final x satisfies |D(x)_0 - x_d| + |D(x)_1 - y_d| <= 1e-12 and the validity rule; then
+ *     u' = u + fx (x - x_d) + margin_x, v' = v + fy (y - y_d) + margin_y (= fx x + cx + margin_x up to rounding), conf kept;
+ *     a failed inversion gives u' = v' = NaN, conf = 0.
+ * With zero coefficients and zero margins u and v are copied bit for bit (so is conf, except where the raw pixel is outside
+ * the frame, where no triangulation uses it). */
+int mpl_undistort_pixels(const float* pix_in, float* pix_out, const double* calib, const double* dist, double margin_x,
+                         double margin_y, int64_t batch, int num_views, int num_joints, mpl_stream_t stream);
+int mpl_undistort_pixels_strided(const float* pix_in, float* pix_out, const double* calib, int64_t calib_stride,
+                                 const double* dist, int64_t dist_stride, double margin_x, double margin_y, int64_t batch,
+                                 int num_views, int num_joints, mpl_stream_t stream);
 
 /* ---- unit-test hooks for the building blocks (used by tests/ only) ------------------------------------------- */
 /* Y[M,N] = epilogue(A[M,K] . W[N,K]^T): the tcgen05 projection kernel in isolation.

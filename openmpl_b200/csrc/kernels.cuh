@@ -220,5 +220,9 @@ int launch_detector_noise(uint64_t seed, int64_t start, int64_t B, int V, int J,
                           float sigma_px, float p_outlier, float p_miss, float* pix, cudaStream_t s);
 int launch_synth_cameras(uint64_t seed, int64_t start, int64_t B, int V, double f0, double w, double h, const double* room,
                          double* calib, cudaStream_t s);
+// mpl_undistort_pixels (undistort) or mpl_distort_pixels (margins ignored); strides checked by the caller
+int launch_lens_pixels(bool undistort, const float* pin, float* pout, const double* calib, int64_t calib_stride,
+                       const double* dist, int64_t dist_stride, double margin_x, double margin_y, int64_t B, int V, int J,
+                       cudaStream_t s);
 
 }  // namespace mpl

@@ -1168,6 +1168,149 @@ int launch_detector_noise(uint64_t seed, int64_t start, int64_t B, int V, int J,
   return MPL_OK;
 }
 
+// ---- lens distortion: OpenCV's 5-coefficient Brown-Conrady model, k = (k1, k2, p1, p2, k3) -------------------------------
+// One thread per (pose, view, joint) entry of pix [B, V, J, 3], fp64.  The model, the validity rule and the Newton
+// inversion are stated in include/mpl_b200.h; tests/lens_oracle.py and openmpl_b200/synth.py (distort_pixels) restate them
+// in numpy.  kPerPose: pose b reads calib + b * cstride and dist + b * dstride (either stride may be 0); otherwise every
+// pose reads the [V, 18] / [V, 5] blocks.  pix_in may equal pix_out: a thread reads its whole entry before it writes.
+constexpr int kLensMaxIters = 20;
+
+// D(x, y) and its Jacobian [[a, b], [b, d]] (the two off-diagonal derivatives are the same expression).
+__device__ __forceinline__ void lens_map(const double (&k)[5], double x, double y, double& xd, double& yd, double& a,
+                                         double& b, double& d) {
+  const double r2 = x * x + y * y;
+  const double rho = 1.0 + r2 * (k[0] + r2 * (k[1] + r2 * k[4]));
+  const double drho = k[0] + r2 * (2.0 * k[1] + r2 * (3.0 * k[4]));     // d rho / d r2
+  xd = x * rho + 2.0 * k[2] * x * y + k[3] * (r2 + 2.0 * x * x);
+  yd = y * rho + k[2] * (r2 + 2.0 * y * y) + 2.0 * k[3] * x * y;
+  a = rho + 2.0 * x * x * drho + 2.0 * k[2] * y + 6.0 * k[3] * x;
+  b = 2.0 * x * y * drho + 2.0 * k[2] * x + 2.0 * k[3] * y;
+  d = rho + 2.0 * y * y * drho + 6.0 * k[2] * y + 2.0 * k[3] * x;
+}
+
+// g(s) = 1 + 3 k1 s + 5 k2 s^2 + 7 k3 s^3 = d (r rho(r)) / dr at r^2 = s.
+__device__ __forceinline__ double lens_radial_slope(const double (&k)[5], double s) {
+  return 1.0 + s * (3.0 * k[0] + s * (5.0 * k[1] + s * (7.0 * k[4])));
+}
+
+// The validity rule of the header at (x, y), given det J there.  False for non-finite input.
+__device__ __forceinline__ bool lens_valid(const double (&k)[5], double x, double y, double det) {
+  const double r2 = x * x + y * y;
+  bool ok = det > 0.0 && lens_radial_slope(k, r2) > 0.0 && r2 < __longlong_as_double(0x7ff0000000000000ll);
+  if (k[4] != 0.0) {
+    const double disc = 100.0 * k[1] * k[1] - 252.0 * k[0] * k[4];
+    if (disc >= 0.0) {
+      const double sq = sqrt(disc);
+      const double s1 = (-10.0 * k[1] - sq) / (42.0 * k[4]), s2 = (-10.0 * k[1] + sq) / (42.0 * k[4]);
+      if (s1 > 0.0 && s1 < r2) ok = ok && lens_radial_slope(k, s1) > 0.0;
+      if (s2 > 0.0 && s2 < r2) ok = ok && lens_radial_slope(k, s2) > 0.0;
+    }
+  } else if (k[1] != 0.0) {
+    const double s1 = -3.0 * k[0] / (10.0 * k[1]);
+    if (s1 > 0.0 && s1 < r2) ok = ok && lens_radial_slope(k, s1) > 0.0;
+  }
+  return ok;
+}
+
+template <bool kPerPose>
+__global__ void __launch_bounds__(256) distort_pixels_kernel(const float* pin, float* pout, const double* __restrict__ calib,
+                                                             int64_t cstride, const double* __restrict__ dist, int64_t dstride,
+                                                             int64_t B, int V, int J) {
+  const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= B * V * J) return;
+  const float u = pin[e * 3], w = pin[e * 3 + 1], conf = pin[e * 3 + 2];
+  float ou = u, ow = w, oc = conf;
+  if (conf != 0.0f) {
+    const int64_t bv = e / J, b = bv / V;
+    const int v = (int)(bv - b * V);
+    const double* c = (kPerPose ? calib + b * cstride : calib) + v * 18;
+    const double* dd = (kPerPose ? dist + b * dstride : dist) + v * 5;
+    const double k[5] = {dd[0], dd[1], dd[2], dd[3], dd[4]};
+    const double fx = c[12], fy = c[13];
+    const double x = ((double)u - c[14]) / fx, y = ((double)w - c[15]) / fy;
+    double xd, yd, a, bb, d;
+    lens_map(k, x, y, xd, yd, a, bb, d);
+    if (k[0] == 0.0 && k[1] == 0.0 && k[2] == 0.0 && k[3] == 0.0 && k[4] == 0.0) {
+      // no lens: the entry as it is (the arithmetic below would turn -0 into +0 and zero conf at a non-finite pixel)
+    } else if (lens_valid(k, x, y, a * d - bb * bb)) {
+      ou = (float)((double)u + fx * (xd - x));
+      ow = (float)((double)w + fy * (yd - y));
+    } else {
+      oc = 0.0f;
+    }
+  }
+  pout[e * 3] = ou;
+  pout[e * 3 + 1] = ow;
+  pout[e * 3 + 2] = oc;
+}
+
+template <bool kPerPose>
+__global__ void __launch_bounds__(256) undistort_pixels_kernel(const float* pin, float* pout, const double* __restrict__ calib,
+                                                               int64_t cstride, const double* __restrict__ dist,
+                                                               int64_t dstride, double margin_x, double margin_y, int64_t B,
+                                                               int V, int J) {
+  const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= B * V * J) return;
+  const float u = pin[e * 3], w = pin[e * 3 + 1], conf = pin[e * 3 + 2];
+  float ou = u, ow = w, oc = conf;
+  if (conf != 0.0f) {
+    const int64_t bv = e / J, b = bv / V;
+    const int v = (int)(bv - b * V);
+    const double* c = (kPerPose ? calib + b * cstride : calib) + v * 18;
+    if (!(0.0 < (double)u && (double)u < c[16] - 1.0 && 0.0 < (double)w && (double)w < c[17] - 1.0)) {
+      oc = 0.0f;                                         // not a candidate of the triangulations on the raw pixels
+    } else {
+      const double* dd = (kPerPose ? dist + b * dstride : dist) + v * 5;
+      const double k[5] = {dd[0], dd[1], dd[2], dd[3], dd[4]};
+      const double fx = c[12], fy = c[13];
+      const double xd = ((double)u - c[14]) / fx, yd = ((double)w - c[15]) / fy;
+      double x = xd, y = yd, px, py, a, bb, d;
+      for (int it = 0; it < kLensMaxIters; ++it) {
+        lens_map(k, x, y, px, py, a, bb, d);
+        const double det = a * d - bb * bb, rx = px - xd, ry = py - yd;
+        const double dx = (d * rx - bb * ry) / det, dy = (a * ry - bb * rx) / det;
+        x -= dx;
+        y -= dy;
+        if (!(fabs(dx) + fabs(dy) > 1e-14)) break;
+      }
+      lens_map(k, x, y, px, py, a, bb, d);
+      if (fabs(px - xd) + fabs(py - yd) <= 1e-12 && lens_valid(k, x, y, a * d - bb * bb)) {
+        ou = (float)((double)u + fx * (x - xd) + margin_x);
+        ow = (float)((double)w + fy * (y - yd) + margin_y);
+      } else {
+        ou = ow = __int_as_float(0x7fc00000);
+        oc = 0.0f;
+      }
+    }
+  }
+  pout[e * 3] = ou;
+  pout[e * 3 + 1] = ow;
+  pout[e * 3 + 2] = oc;
+}
+
+int launch_lens_pixels(bool undistort, const float* pin, float* pout, const double* calib, int64_t calib_stride,
+                       const double* dist, int64_t dist_stride, double margin_x, double margin_y, int64_t B, int V, int J,
+                       cudaStream_t s) {
+  const int64_t total = B * V * J;
+  if (total == 0) return MPL_OK;
+  const unsigned grid = (unsigned)ceil_div(total, 256);
+  const bool per_pose = calib_stride != 0 || dist_stride != 0;
+  if (undistort) {
+    if (per_pose)
+      undistort_pixels_kernel<true><<<grid, 256, 0, s>>>(pin, pout, calib, calib_stride, dist, dist_stride, margin_x, margin_y,
+                                                         B, V, J);
+    else
+      undistort_pixels_kernel<false><<<grid, 256, 0, s>>>(pin, pout, calib, 0, dist, 0, margin_x, margin_y, B, V, J);
+  } else {
+    if (per_pose)
+      distort_pixels_kernel<true><<<grid, 256, 0, s>>>(pin, pout, calib, calib_stride, dist, dist_stride, B, V, J);
+    else
+      distort_pixels_kernel<false><<<grid, 256, 0, s>>>(pin, pout, calib, 0, dist, 0, B, V, J);
+  }
+  MPL_LAUNCH_CHECK();
+  return MPL_OK;
+}
+
 // ---- random camera setups: one thread per (pose, view), fp64 ------------------------------------------------------------
 // U0..U5 of (pose i, view v) come from the Philox4x64-10 stream of synth_project_kernel under key (seed, 2), with the slot
 // layout of the detector-noise model (pose i owns counter blocks [i nb, (i + 1) nb), nb = ceil(6 V / 4), slot 6 v + m is

@@ -1487,6 +1487,51 @@ int mpl_synth_detector_noise_strided(uint64_t seed, int64_t start, int64_t batch
                                pix, reinterpret_cast<cudaStream_t>(stream));
 }
 
+// Argument checks shared by mpl_distort_pixels_strided and mpl_undistort_pixels_strided (the distortion passes margins 0).
+static int lens_pixels(const char* name, bool undistort, const float* pix_in, float* pix_out, const double* calib,
+                       int64_t calib_stride, const double* dist, int64_t dist_stride, double margin_x, double margin_y,
+                       int64_t batch, int num_views, int num_joints, mpl_stream_t stream) {
+  const bool dist_stride_ok = dist_stride == 0 || (dist_stride > 0 && dist_stride >= 5 * (int64_t)num_views);
+  if (batch < 0 || num_views < 1 || num_views > kMaxViews || num_joints < 1 || !calib_stride_ok(calib_stride, num_views) ||
+      !dist_stride_ok || !std::isfinite(margin_x) || !(margin_x >= 0.0) || !std::isfinite(margin_y) || !(margin_y >= 0.0)) {
+    set_error("%s: bad argument (batch %lld, num_views %d, num_joints %d, calib_stride %lld, dist_stride %lld, margin %g %g)",
+              name, (long long)batch, num_views, num_joints, (long long)calib_stride, (long long)dist_stride, margin_x, margin_y);
+    return MPL_ERR_INVALID_ARGUMENT;
+  }
+  if (batch == 0) return MPL_OK;
+  if (pix_in == nullptr || pix_out == nullptr || calib == nullptr || dist == nullptr) {
+    set_error("%s: null pointer", name);
+    return MPL_ERR_INVALID_ARGUMENT;
+  }
+  return launch_lens_pixels(undistort, pix_in, pix_out, calib, calib_stride, dist, dist_stride, margin_x, margin_y, batch,
+                            num_views, num_joints, reinterpret_cast<cudaStream_t>(stream));
+}
+
+int mpl_distort_pixels(const float* pix_in, float* pix_out, const double* calib, const double* dist, int64_t batch,
+                       int num_views, int num_joints, mpl_stream_t stream) {
+  return mpl_distort_pixels_strided(pix_in, pix_out, calib, 0, dist, 0, batch, num_views, num_joints, stream);
+}
+
+int mpl_distort_pixels_strided(const float* pix_in, float* pix_out, const double* calib, int64_t calib_stride,
+                               const double* dist, int64_t dist_stride, int64_t batch, int num_views, int num_joints,
+                               mpl_stream_t stream) {
+  return lens_pixels("mpl_distort_pixels_strided", false, pix_in, pix_out, calib, calib_stride, dist, dist_stride, 0.0, 0.0,
+                     batch, num_views, num_joints, stream);
+}
+
+int mpl_undistort_pixels(const float* pix_in, float* pix_out, const double* calib, const double* dist, double margin_x,
+                         double margin_y, int64_t batch, int num_views, int num_joints, mpl_stream_t stream) {
+  return mpl_undistort_pixels_strided(pix_in, pix_out, calib, 0, dist, 0, margin_x, margin_y, batch, num_views, num_joints,
+                                      stream);
+}
+
+int mpl_undistort_pixels_strided(const float* pix_in, float* pix_out, const double* calib, int64_t calib_stride,
+                                 const double* dist, int64_t dist_stride, double margin_x, double margin_y, int64_t batch,
+                                 int num_views, int num_joints, mpl_stream_t stream) {
+  return lens_pixels("mpl_undistort_pixels_strided", true, pix_in, pix_out, calib, calib_stride, dist, dist_stride, margin_x,
+                     margin_y, batch, num_views, num_joints, stream);
+}
+
 int mpl_synth_cameras(uint64_t seed, int64_t start, int64_t batch, int num_views, double f0, double w, double h,
                       const double* room, double* calib_out, mpl_stream_t stream) {
   if (batch < 0 || start < 0 || num_views < 1 || num_views > kMaxViews || !std::isfinite(f0) || !(f0 > 0.0) ||

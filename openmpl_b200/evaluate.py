@@ -12,6 +12,8 @@
         --refine-triangulations                                                         # + nonlinear refinement of both
     python -m openmpl_b200.evaluate --arch hm0 --views 4 --pixel-noise 2 --triangulate --triangulate-robust \
         --triangulation-pmpjpe                                                          # + P-MPJPE of both baselines
+    python -m openmpl_b200.evaluate --arch hm0 --views 4 --lens-distortion=-0.207,0.248,-0.0009,-0.0016,-0.0031 \
+        --triangulate --triangulate-robust --refine-triangulations                      # cameras with a lens
 
 Per micro-batch, entirely on the device: `mpl_synth_project` (3D poses from the counter-based generator keyed by the
 GLOBAL pose index, projected through the V calibrations) -> `mpl_build_inputs` (clip, confidence zeroing, screen
@@ -44,6 +46,13 @@ own accumulator under the parent entry's mask.  Without the flag nothing of this
 each "refined" sub-entry, by a masked P-MPJPE accumulator (`mpl_pmpjpe_accumulate_masked`) under that entry's own mask:
 every pose is Procrustes-aligned on its triangulated joints only.  The entry gains "procrustes_aligned".  Without the flag
 nothing of this runs.
+
+`--lens-distortion K1,K2,P1,P2,K3` gives every view a lens of OpenCV's 5-coefficient model (`mpl_distort_pixels`): each
+micro-batch's projected pixels are distorted before the detector noise (which models errors in detector pixels), the
+lifter's inputs are built from the distorted pixels as the reference builds them from a real detector's, and every
+triangulation and refinement runs on `mpl_undistort_pixels` output (margin half the image on each side) with the shifted
+calibration it comes with.  It composes with `--random-cameras` (one lens, per-pose calibrations).  The line's "data"
+entry records the coefficients.  Without the flag nothing of this runs.
 """
 from __future__ import annotations
 
@@ -70,7 +79,11 @@ REFINE_MAX_ITERS = 20
 def run(arch="hm0", views=4, depth=None, poses=1 << 20, micro_batch=65536, precision="bf16", rig=None, seed=1,
         weight_seed=0, warmup=1, triangulate=False, pixel_noise=0.0, outlier_rate=0.0, miss_rate=0.0,
         triangulate_robust=False, inlier_px=10.0, random_cameras=False, refine_triangulations=False,
-        triangulation_pmpjpe=False):
+        triangulation_pmpjpe=False, lens_distortion=None):
+    if lens_distortion is not None:
+        lens_distortion = tuple(float(k) for k in lens_distortion)
+        if len(lens_distortion) != 5 or not all(np.isfinite(lens_distortion)):
+            raise ValueError(f"lens_distortion must be 5 finite numbers (k1, k2, p1, p2, k3), got {lens_distortion}")
     if refine_triangulations and not (triangulate or triangulate_robust):
         raise ValueError("refine_triangulations needs triangulate or triangulate_robust")
     if triangulation_pmpjpe and not (triangulate or triangulate_robust):
@@ -100,10 +113,15 @@ def run(arch="hm0", views=4, depth=None, poses=1 << 20, micro_batch=65536, preci
     tp = {name: metric.PmpjpeAccumulator(cfg.J, output_in_meter=True, device=dev, masked=True)
           for name, a in (("t", tacc), ("r", racc), ("tf", tfacc), ("rf", rfacc)) if triangulation_pmpjpe and a is not None}
     noisy = pixel_noise != 0 or outlier_rate != 0 or miss_rate != 0
+    if lens_distortion is not None:
+        lens = torch.tensor([lens_distortion] * views, dtype=torch.float64, device=dev)
+        margin = (the_rig.image_size[0] / 2.0, the_rig.image_size[1] / 2.0)   # known here: no read-back of calib
 
     def step(s0, n):
         cams = inputs.synth_cameras(n, views, rig_kind, seed=seed, start=s0, device=dev) if random_cameras else None
         pix, target, calib = inputs.synth_project(n, the_rig, seed=seed, start=s0, device=dev, cameras=cams)
+        if lens_distortion is not None:
+            inputs.distort_pixels(pix, calib, lens)
         if noisy:
             inputs.add_detector_noise(pix, calib, seed, s0, pixel_noise, outlier_rate, miss_rate)
         p, r, c = inputs.build_inputs(pix, calib)
@@ -117,6 +135,8 @@ def run(arch="hm0", views=4, depth=None, poses=1 << 20, micro_batch=65536, preci
             if key in tp:
                 tp[key].update(points, target, mask)
 
+        if lens_distortion is not None and (tacc is not None or racc is not None):
+            pix, calib = inputs.undistort_pixels(pix, calib, lens, margin=margin)
         if tacc is not None:
             points, used = inputs.triangulate(pix, calib)
             score("t", tacc, points, used >= 2)
@@ -177,6 +197,14 @@ def run(arch="hm0", views=4, depth=None, poses=1 << 20, micro_batch=65536, preci
                 "azimuth": "2 pi (v + 0.8 (U0 - 0.5)) / V + 0.3", "distance_m": "4.5 (0.75 + 0.5 U1)",
                 "height_m": "0.9 + 1.2 U2", "look_at": "room centre at 0.9 m + 0.5 (U3 - 0.5, U4 - 0.5, 0)",
                 "focal_px": "f0 (0.8 + 0.4 U5), f0 of the rig kind"}
+        if lens_distortion is not None:
+            if not isinstance(line["data"], dict):
+                line["data"] = {"source": line["data"]}
+            line["data"]["lens_distortion"] = {
+                "model": "OpenCV 5-coefficient Brown-Conrady on normalised camera coordinates, every view",
+                "coefficients": dict(zip(("k1", "k2", "p1", "p2", "k3"), lens_distortion)),
+                "pipeline": "projected pixels distorted before the detector noise; lifter inputs built from the distorted "
+                            "pixels; triangulations on the undistorted pixels (margin half the image on each side)"}
         if tacc is not None:
             line["triangulation"] = triangulation_summary(tacc.acc.detach().cpu().numpy(), cfg.J)
         if racc is not None:
@@ -250,7 +278,18 @@ def main(argv=None):
     p.add_argument("--triangulation-pmpjpe", action="store_true",
                    help="also score each triangulation by P-MPJPE, aligned on its triangulated joints only (needs "
                         "--triangulate or --triangulate-robust)")
+    p.add_argument("--lens-distortion", default=None, metavar="K1,K2,P1,P2,K3",
+                   help="a lens of OpenCV's 5-coefficient model on every view: distorted detections for the lifter, "
+                        "undistorted ones for the triangulations")
     a = p.parse_args(argv)
+    lens = None
+    if a.lens_distortion is not None:
+        try:
+            lens = tuple(float(k) for k in a.lens_distortion.split(","))
+        except ValueError:
+            lens = ()
+        if len(lens) != 5 or not all(np.isfinite(lens)):
+            p.error("--lens-distortion needs five comma-separated finite numbers K1,K2,P1,P2,K3")
     if a.refine_triangulations and not (a.triangulate or a.triangulate_robust):
         p.error("--refine-triangulations needs --triangulate or --triangulate-robust")
     if a.triangulation_pmpjpe and not (a.triangulate or a.triangulate_robust):
@@ -258,7 +297,7 @@ def main(argv=None):
     run(a.arch, a.views, a.depth, a.poses, a.micro_batch, a.precision, a.rig, a.seed, triangulate=a.triangulate,
         pixel_noise=a.pixel_noise, outlier_rate=a.outlier_rate, miss_rate=a.miss_rate,
         triangulate_robust=a.triangulate_robust, inlier_px=a.inlier_px, random_cameras=a.random_cameras,
-        refine_triangulations=a.refine_triangulations, triangulation_pmpjpe=a.triangulation_pmpjpe)
+        refine_triangulations=a.refine_triangulations, triangulation_pmpjpe=a.triangulation_pmpjpe, lens_distortion=lens)
 
 
 if __name__ == "__main__":

@@ -143,6 +143,83 @@ def add_detector_noise(pix: torch.Tensor, calib, seed: int, start: int, sigma_px
     return pix
 
 
+def distort_pixels(pix: torch.Tensor, calib, dist) -> torch.Tensor:
+    """Lens distortion (`mpl_distort_pixels`) applied IN PLACE to ideal pinhole pixels, enqueued on the current stream;
+    returns `pix`.
+
+    pix [B, V, J, 3] contiguous fp32 (u, v, conf) on the device, e.g. as `synth_project` returns it (before
+    `add_detector_noise`, which models errors in detector pixels); calib [V, 18] or [B, V, 18]; dist (k1, k2, p1, p2, k3)
+    per view, [V, 5] or [B, V, 5] (numpy or tensor; OpenCV's distCoeffs order).  Each entry with conf != 0 moves to where
+    OpenCV's 5-coefficient model images it; an entry past a fold of the model (see include/mpl_b200.h) gets conf = 0.
+    Zero coefficients leave pix bitwise unchanged.  `synth.distort_pixels` is the numpy twin.
+    """
+    if pix.dtype != torch.float32 or not pix.is_contiguous() or pix.dim() != 4 or pix.shape[-1] != 3:
+        raise ValueError("distort_pixels works in place on a contiguous float32 [B, V, J, 3] tensor")
+    B, V, J, _ = pix.shape
+    calib, cstride = _calib_arg(calib, B, V, pix.device)
+    dist, dstride = _dist_arg(dist, B, V, pix.device)
+    with torch.cuda.device(pix.device):
+        stream = torch.cuda.current_stream(pix.device).cuda_stream
+        _lib.check(_lib.lib().mpl_distort_pixels_strided(pix.data_ptr(), pix.data_ptr(), calib.data_ptr(), cstride,
+                                                         dist.data_ptr(), dstride, B, V, J, stream))
+    return pix
+
+
+def undistort_pixels(pix: torch.Tensor, calib, dist, margin=None) -> tuple:
+    """Undistortion of detected pixels for the triangulations (`mpl_undistort_pixels`), enqueued on the current stream.
+
+    pix [B, V, J, 3] fp32 (u, v, conf) raw detections on the device; calib [V, 18] or [B, V, 18]; dist [V, 5] or [B, V, 5]
+    as for `distort_pixels`.  margin: (margin_x, margin_y) pixels, or one number for both; None = half the image on each
+    side, (max w / 2, max h / 2) over the calibration's views (read from calib: a device tensor costs one synchronisation;
+    pass the margin to avoid it).  Returns (pix_u, calib_u): pix_u [B, V, J, 3] the pinhole pixels of the same rays shifted
+    by the margin, calib_u the calibration of calib's shape with cx + margin_x, cy + margin_y, w + 2 margin_x,
+    h + 2 margin_y, to pass with pix_u to `triangulate`, `triangulate_robust` and `refine_triangulation`.  Entries whose raw
+    pixel is not strictly inside the original image get conf 0 (the candidate sets stay those of the raw pixels), and so
+    do entries the Newton inversion fails on (with NaN pixels).  An undistorted pixel further than the margin outside
+    the image fails the triangulations' candidate test and is dropped.
+    """
+    if pix.dim() != 4 or pix.shape[-1] != 3:
+        raise ValueError(f"undistort_pixels takes a [B, V, J, 3] tensor, got {list(pix.shape)}")
+    B, V, J, _ = pix.shape
+    device = pix.device
+    pix = pix.to(torch.float32).contiguous()
+    calib, cstride = _calib_arg(calib, B, V, device)
+    dist, dstride = _dist_arg(dist, B, V, device)
+    if margin is None:
+        wh = calib[..., 16:18].reshape(-1, 2).amax(0).cpu() if calib.numel() else torch.zeros(2, dtype=torch.float64)
+        mx, my = float(wh[0]) / 2.0, float(wh[1]) / 2.0
+    elif np.ndim(margin) == 0:
+        mx = my = float(margin)
+    else:
+        mx, my = (float(m) for m in margin)
+    if not (np.isfinite(mx) and np.isfinite(my) and mx >= 0 and my >= 0):
+        raise ValueError(f"margin must be finite and >= 0, got ({mx}, {my})")
+    out = torch.empty_like(pix)
+    with torch.cuda.device(device):
+        stream = torch.cuda.current_stream(device).cuda_stream
+        _lib.check(_lib.lib().mpl_undistort_pixels_strided(pix.data_ptr(), out.data_ptr(), calib.data_ptr(), cstride,
+                                                           dist.data_ptr(), dstride, mx, my, B, V, J, stream))
+    calib_u = calib.clone()
+    calib_u[..., 14] += mx
+    calib_u[..., 15] += my
+    calib_u[..., 16] += 2.0 * mx
+    calib_u[..., 17] += 2.0 * my
+    return out, calib_u
+
+
+def _dist_arg(dist, B: int, V: int, device) -> tuple:
+    """(contiguous fp64 device tensor, dist_stride): [V, 5] -> stride 0 (one lens set for the batch); [B, V, 5] -> 5 V."""
+    if isinstance(dist, torch.Tensor):
+        dist = dist.to(device=device, dtype=torch.float64).contiguous()
+    else:
+        dist = torch.as_tensor(np.asarray(dist, dtype=np.float64)).to(device).contiguous()
+    if dist.dim() == 2 and tuple(dist.shape) == (V, 5):
+        return dist, 0
+    if dist.dim() == 3 and dist.shape[0] == B and tuple(dist.shape[1:]) == (V, 5):
+        return dist, 5 * V
+    raise ValueError(f"dist must be [V, 5] = [{V}, 5] or [B, V, 5] = [{B}, {V}, 5], got {list(dist.shape)}")
+
+
 def _calib_arg(calib, B: int, V: int, device) -> tuple:
     """(contiguous fp64 device tensor, calib_stride): [V, 18] -> stride 0 (one rig for the batch); [B, V, 18] -> 18 V."""
     if isinstance(calib, torch.Tensor):

@@ -203,6 +203,73 @@ def detector_noise(pix, image_size, seed: int, start: int, sigma_px: float, p_ou
     return res
 
 
+def lens_map(k, x, y) -> tuple:
+    """OpenCV's 5-coefficient model D(x, y) on normalised coordinates and its Jacobian: (xd, yd, a, b, d), J = [[a, b], [b, d]].
+    k = (k1, k2, p1, p2, k3), each broadcastable against x, y; the arithmetic of `mpl_distort_pixels` in the same order."""
+    k1, k2, p1, p2, k3 = k
+    r2 = x * x + y * y
+    rho = 1.0 + r2 * (k1 + r2 * (k2 + r2 * k3))
+    drho = k1 + r2 * (2.0 * k2 + r2 * (3.0 * k3))
+    xd = x * rho + 2.0 * p1 * x * y + p2 * (r2 + 2.0 * x * x)
+    yd = y * rho + p1 * (r2 + 2.0 * y * y) + 2.0 * p2 * x * y
+    a = rho + 2.0 * x * x * drho + 2.0 * p1 * y + 6.0 * p2 * x
+    b = 2.0 * x * y * drho + 2.0 * p1 * x + 2.0 * p2 * y
+    d = rho + 2.0 * y * y * drho + 6.0 * p1 * y + 2.0 * p2 * x
+    return xd, yd, a, b, d
+
+
+def lens_valid(k, x, y) -> np.ndarray:
+    """The validity rule of include/mpl_b200.h: det J > 0 and the radial map r -> r rho(r) increasing on [0, |x|], i.e.
+    g(s) = 1 + 3 k1 s + 5 k2 s^2 + 7 k3 s^3 > 0 at s = r^2 and at the roots of g' strictly inside (0, r^2)."""
+    k1, k2, p1, p2, k3 = (np.asarray(c, dtype=np.float64) for c in k)
+    x, y = np.asarray(x, dtype=np.float64), np.asarray(y, dtype=np.float64)
+    _, _, a, b, d = lens_map((k1, k2, p1, p2, k3), x, y)
+    r2 = x * x + y * y
+
+    def g(s):
+        return 1.0 + s * (3.0 * k1 + s * (5.0 * k2 + s * (7.0 * k3)))
+
+    with np.errstate(invalid="ignore", divide="ignore"):
+        ok = (a * d - b * b > 0.0) & (g(r2) > 0.0) & (r2 < np.inf)
+        disc = 100.0 * k2 * k2 - 252.0 * k1 * k3
+        sq = np.sqrt(np.where(disc >= 0.0, disc, 0.0))
+        cubic, quad = (k3 != 0.0) & (disc >= 0.0), (k3 == 0.0) & (k2 != 0.0)
+        roots = [np.where(cubic, (-10.0 * k2 - sq) / (42.0 * k3), np.where(quad, -3.0 * k1 / (10.0 * k2), np.nan)),
+                 np.where(cubic, (-10.0 * k2 + sq) / (42.0 * k3), np.nan)]
+        for s in roots:
+            inside = (s > 0.0) & (s < r2)
+            ok &= ~inside | (g(np.where(inside, s, 0.0)) > 0.0)
+    return ok
+
+
+def distort_pixels(pix, calib, dist) -> np.ndarray:
+    """Host twin of `mpl_distort_pixels`: ideal pinhole pixels -> those a camera with lens `dist` records.
+
+    pix [B, V, J, 3] (u, v, conf); calib [V, 18] or [B, V, 18] (`inputs.pack_calibration` rows); dist (k1, k2, p1, p2, k3)
+    per view, [V, 5] or [B, V, 5].  Returns a float32 copy: each entry with conf != 0 at x = ((u - cx) / fx, (v - cy) / fy)
+    moves to u + fx (x_d - x), v + fy (y_d - y), (x_d, y_d) = `lens_map`(x), or gets conf = 0 (pixel kept) where x fails
+    `lens_valid`.  Entries with conf == 0, and entries whose five coefficients are all 0, are kept.
+    """
+    pix = np.asarray(pix, dtype=np.float32)
+    calib = np.asarray(calib, dtype=np.float64)
+    dist = np.asarray(dist, dtype=np.float64)
+    c = calib[..., :, None, :] if calib.ndim == 3 else calib[None, :, None, :]      # [B or 1, V, 1, 18]
+    k = dist[..., :, None, :] if dist.ndim == 3 else dist[None, :, None, :]
+    k = tuple(k[..., m] for m in range(5))
+    fx, fy, cx, cy = (c[..., m] for m in range(12, 16))
+    u, v, conf = (pix[..., m].astype(np.float64) for m in range(3))
+    x, y = (u - cx) / fx, (v - cy) / fy
+    with np.errstate(invalid="ignore", over="ignore"):
+        xd, yd, _, _, _ = lens_map(k, x, y)
+        live = (conf != 0) & ~((k[0] == 0) & (k[1] == 0) & (k[2] == 0) & (k[3] == 0) & (k[4] == 0))
+        ok = live & lens_valid(k, x, y)
+        res = pix.copy()
+        res[..., 0] = np.where(ok, u + fx * (xd - x), u).astype(np.float32)
+        res[..., 1] = np.where(ok, v + fy * (yd - y), v).astype(np.float32)
+    res[..., 2] = np.where(live & ~ok, np.float32(0.0), pix[..., 2])
+    return res
+
+
 def named_weights(shapes: dict, seed: int = 0, pos_std: float = 0.02) -> dict:
     """Deterministic weights keyed by parameter NAME (order independent, numpy only).
 
