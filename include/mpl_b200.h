@@ -15,8 +15,9 @@
  *   MPL/lib/multiviews/triangulate.py:59-115 linear triangulation baseline (-> mpl_triangulate)
  * Defined here, with no counterpart in the reference: robust (RANSAC) triangulation (mpl_triangulate_robust), nonlinear
  * refinement of triangulated points (mpl_triangulate_refine), a detector-error model for the synthetic data
- * (mpl_synth_detector_noise), a generator of random camera setups (mpl_synth_cameras) and lens distortion of pixels
- * (mpl_distort_pixels / mpl_undistort_pixels).
+ * (mpl_synth_detector_noise), a generator of random camera setups (mpl_synth_cameras), lens distortion of pixels
+ * (mpl_distort_pixels / mpl_undistort_pixels), a calibration-error model (mpl_synth_calib_noise) and bundle adjustment of a
+ * rig's extrinsics from its detections (mpl_calibrate_rig).
  *
  * Conventions
  *   - plain pointers and sizes only; no torch / C++ types cross this boundary;
@@ -44,7 +45,7 @@
 extern "C" {
 #endif
 
-#define MPL_ABI_VERSION 8
+#define MPL_ABI_VERSION 9
 
 typedef enum MplStatus {
   MPL_OK = 0,
@@ -419,6 +420,65 @@ int mpl_undistort_pixels(const float* pix_in, float* pix_out, const double* cali
 int mpl_undistort_pixels_strided(const float* pix_in, float* pix_out, const double* calib, int64_t calib_stride,
                                  const double* dist, int64_t dist_stride, double margin_x, double margin_y, int64_t batch,
                                  int num_views, int num_joints, mpl_stream_t stream);
+
+/* Calibration errors and rig calibration (ABI 9; defined by this library).  Rotation vectors: Exp(w) is Rodrigues' formula
+ * I + sin t / t [w]x + (1 - cos t) / t^2 [w]x^2, t = |w|, and J_l(w) = I + (1 - cos t) / t^2 [w]x + (t - sin t) / t^3 [w]x^2
+ * its left Jacobian; below t^2 = 1e-2 the three coefficients come from their Taylor series through t^8.
+ *
+ * mpl_synth_calib_noise: calib_out [B, V, 18] packed = the calibrations of poses [start, start + B), read from calib with the
+ * calib_stride convention (0: one [V, 18] block; >= 18 V), perturbed.  Per (pose i, view v), U0..U5 come from the
+ * Philox4x64-10 stream of mpl_synth_project under key (seed, 3), in the slot layout of mpl_synth_cameras (nb = ceil(6 V / 4),
+ * slot 6 v + m is U_m), so the result depends only on (seed, global pose index).  Six standard normals by Box-Muller:
+ * n_2k = r cos(2 pi U_2k+1), n_2k+1 = r sin(2 pi U_2k+1), r = sqrt(-2 ln max(U_2k, 1e-12)), k = 0, 1, 2.  Then
+ *   R' = Exp(sigma_rot (n0, n1, n2)) R   (radians; a rotation in the camera frame, R maps world -> camera)
+ *   t' = t + sigma_pos (n3, n4, n5)       (the camera centre, world units)
+ * fx, fy, cx, cy, w, h are copied bit for bit; sigma_rot == 0 keeps R and sigma_pos == 0 keeps t bit for bit.  A fixed rig is
+ * perturbed as pose 0: batch 1, start 0, stride 0.  fp64, one thread per (pose, view); allocates nothing and never
+ * synchronises.  MPL_ERR_INVALID_ARGUMENT, before any CUDA call: V outside [1, 16], start < 0, a sigma that is not finite or
+ * is negative, a bad calib_stride, batch < 0; then batch == 0 returns MPL_OK; then a null pointer, or calib_out == calib
+ * with a stride other than 18 V, is MPL_ERR_INVALID_ARGUMENT. */
+int mpl_synth_calib_noise(uint64_t seed, int64_t start, int64_t batch, int num_views, const double* calib,
+                          int64_t calib_stride, double sigma_rot, double sigma_pos, double* calib_out, mpl_stream_t stream);
+
+/* mpl_calibrate_rig: bundle adjustment of the extrinsics of one rig calib [V, 18] (no strided variant: a rig is calibrated
+ * from many poses) from the detections pix [B, V, J, 3] of B poses, starting from the points init [B, J, 3] (e.g.
+ * mpl_triangulate's under the same calib).  fp64 throughout.
+ *   - used views of (b, j): the candidates of mpl_triangulate (conf > min_conf, strictly inside the image) whose bit is set
+ *     in view_mask[b, j] when view_mask [B, J] int32 is not NULL (the rule of mpl_triangulate_refine);
+ *   - items: the pairs (b, j) whose init is finite, with at least 2 used views, every one of which sees init at a finite
+ *     depth > 0 under calib.  The set is fixed at the start;
+ *   - parameters: per camera omega_v (R_v = Exp(omega_v) R0_v, omega_v = 0 at the start) and the centre c_v (c0_v at the
+ *     start), R0 / c0 from calib; per item X_i (init at the start).  Intrinsics are fixed;
+ *   - cost, y = R_v (X - c_v), pi(y) = (fx y0 / y2 + cx, fy y1 / y2 + cy):
+ *       C = sum_items sum_used v (conf^2 / sigma_px^2) |pi(y) - (u, v)|^2 + sum_v (|omega_v|^2 / sigma_rot^2
+ *           + |c_v - c0_v|^2 / sigma_pos^2),
+ *     +inf if a used observation has y2 <= 0 or a non-finite y2.  The prior is the distribution mpl_synth_calib_noise draws
+ *     from (so with the same sigmas this is the MAP rig) and it fixes the 7-DoF similarity gauge, hence every sigma > 0;
+ *   - Jacobians, exact: dy/domega = -[y]x J_l(omega), dy/dc = -R, dy/dX = R;
+ *   - LM: A = J^T W J and g = J^T W r over every residual, data and prior; the step solves (A + mu I) delta = -g, mu on every
+ *     camera and point parameter; mu0 = 1e-3 max diag(A) at the start.  Schur solve: per item the Cholesky factor of
+ *     M_i = A_ii + mu I, S = A_cc + mu I - sum_i A_ci M_i^-1 A_ic with the matching right-hand side, a dense Cholesky of S,
+ *     delta X_i = -M_i^-1 (g_i + A_ic delta c).  A Cholesky pivot that is not finite and > 0, in any M_i or in S, rejects the
+ *     step (mu *= 10) and skips the stop test.  If C(new) < C the step is accepted, mu /= 10; otherwise rejected, mu *= 10.
+ *     Iteration k stops the solve if the 6 V camera step satisfies |delta_cam|_2 <= 1e-10 (|c|_2 + 1e-10), c the 3 V centres
+ *     before the iteration, or when k = max_iters;
+ *   - outputs: calib_out [V, 18] = Exp(omega_v) R0_v and c_v with the other six fields copied bit for bit (R0 bit for bit
+ *     while omega_v is exactly 0); points [B, J, 3] fp32 (may be NULL, may alias init) = the refined X for items, init bit for
+ *     bit otherwise; report [8] fp64 on the device = items, observations, C at the start, C at the end, the conf-weighted
+ *     RMS pixel error sqrt(sum conf^2 e^2 / sum conf^2) at the start and at the end, iterations run, accepted steps.  With
+ *     no item calib_out is calib bit for bit, points is init and the report is all 0;
+ *   - MPL_ERR_INVALID_ARGUMENT, before any CUDA call: V outside [2, 16], J < 1, batch < 1, a sigma that is not finite or
+ *     <= 0, max_iters outside [1, 100], a null pix / calib / init / calib_out / report / workspace.  A workspace shorter
+ *     than mpl_calibrate_rig_workspace_bytes(batch, V, J) is MPL_ERR_WORKSPACE (the query returns 0 for a shape the call
+ *     rejects);
+ *   - allocates nothing and never synchronises: the LM control lives in the workspace, a fixed sequence of 4 max_iters + 3
+ *     launches is enqueued and the iterations after the stop return at once (graph-capturable).  Bitwise deterministic: no
+ *     floating-point atomics, partial sums reduced in a fixed order, their number a function of (batch, V, J) only. */
+size_t mpl_calibrate_rig_workspace_bytes(int64_t batch, int num_views, int num_joints);
+int mpl_calibrate_rig(const float* pix, const double* calib, int64_t batch, int num_views, int num_joints, float min_conf,
+                      const int32_t* view_mask, const float* init, double sigma_px, double sigma_rot, double sigma_pos,
+                      int max_iters, double* calib_out, float* points, double* report, void* workspace,
+                      size_t workspace_bytes, mpl_stream_t stream);
 
 /* ---- unit-test hooks for the building blocks (used by tests/ only) ------------------------------------------- */
 /* Y[M,N] = epilogue(A[M,K] . W[N,K]^T): the tcgen05 projection kernel in isolation.

@@ -11,7 +11,7 @@ from ctypes import POINTER, c_char_p, c_double, c_float, c_int, c_int32, c_int64
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("MPL_B200_LIB") or os.path.join(HERE, "libmpl_b200.so")   # override: another build of the same ABI
 
-ABI_VERSION = 8
+ABI_VERSION = 9
 MPL_OK = 0
 MPL_ERR_INVALID_ARGUMENT = -1
 MPL_ERR_CONFIG_RUNTIME = -2
@@ -33,7 +33,8 @@ EXPORTS = [
     "mpl_build_inputs_strided", "mpl_synth_project_strided", "mpl_synth_detector_noise_strided", "mpl_triangulate_strided",
     "mpl_triangulate_robust_strided", "mpl_synth_cameras", "mpl_triangulate_refine", "mpl_triangulate_refine_strided",
     "mpl_mpjpe_accumulate_grouped", "mpl_pmpjpe_accumulate_masked", "mpl_distort_pixels", "mpl_distort_pixels_strided",
-    "mpl_undistort_pixels", "mpl_undistort_pixels_strided",
+    "mpl_undistort_pixels", "mpl_undistort_pixels_strided", "mpl_synth_calib_noise", "mpl_calibrate_rig_workspace_bytes",
+    "mpl_calibrate_rig",
 ]
 
 _DESC_FLAGS = [
@@ -172,6 +173,12 @@ def lib():
                                            c_void_p]
         L.mpl_undistort_pixels_strided.argtypes = [c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_int64, c_double, c_double,
                                                    c_int64, c_int, c_int, c_void_p]
+        L.mpl_synth_calib_noise.argtypes = [ctypes.c_uint64, c_int64, c_int64, c_int, c_void_p, c_int64, c_double, c_double,
+                                            c_void_p, c_void_p]
+        L.mpl_calibrate_rig_workspace_bytes.argtypes = [c_int64, c_int, c_int]
+        L.mpl_calibrate_rig_workspace_bytes.restype = c_size_t
+        L.mpl_calibrate_rig.argtypes = [c_void_p, c_void_p, c_int64, c_int, c_int, c_float, c_void_p, c_void_p, c_double,
+                                        c_double, c_double, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]
         if L.mpl_abi_version() != ABI_VERSION:
             raise RuntimeError("libmpl_b200.so ABI version mismatch")
         _lib = L

@@ -15,8 +15,9 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.environ.get("MPL_B200_BUILD_LIB") or os.path.join(HERE, "libmpl_b200.so")
-SOURCES = ["model.cu", "kernels_generic.cu", "gemm_tcgen05.cu", "metric_inputs.cu", "spt_fused.cu", "io_kernels.cu"]
-HEADERS = ["common.cuh", "kernels.cuh", "ptx.cuh", os.path.join("..", "..", "include", "mpl_b200.h")]
+SOURCES = ["model.cu", "kernels_generic.cu", "gemm_tcgen05.cu", "metric_inputs.cu", "spt_fused.cu", "io_kernels.cu",
+           "calibrate_rig.cu"]
+HEADERS = ["common.cuh", "kernels.cuh", "ptx.cuh", "so3.cuh", os.path.join("..", "..", "include", "mpl_b200.h")]
 # per-file extra nvcc flags; MPL_GEMM_DEFS="-DMPL_LN_STAGES=6 ..." builds an experiment variant of the GEMM kernel
 EXTRA_FLAGS = {"gemm_tcgen05.cu": os.environ.get("MPL_GEMM_DEFS", "").split(),
                "spt_fused.cu": os.environ.get("MPL_SPT_DEFS", "").split()}

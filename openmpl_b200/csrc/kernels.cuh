@@ -221,6 +221,12 @@ int launch_detector_noise(uint64_t seed, int64_t start, int64_t B, int V, int J,
 int launch_synth_cameras(uint64_t seed, int64_t start, int64_t B, int V, double f0, double w, double h, const double* room,
                          double* calib, cudaStream_t s);
 // mpl_undistort_pixels (undistort) or mpl_distort_pixels (margins ignored); strides checked by the caller
+int launch_synth_calib_noise(uint64_t seed, int64_t start, int64_t B, int V, const double* calib, int64_t calib_stride,
+                             double sigma_rot, double sigma_pos, double* calib_out, cudaStream_t s);
+size_t rig_workspace_bytes(int64_t B, int V, int J);
+int launch_calibrate_rig(const float* pix, const double* calib, int64_t B, int V, int J, float min_conf,
+                         const int32_t* view_mask, const float* init, double sigma_px, double sigma_rot, double sigma_pos,
+                         int max_iters, double* calib_out, float* points, double* report, void* workspace, cudaStream_t s);
 int launch_lens_pixels(bool undistort, const float* pin, float* pout, const double* calib, int64_t calib_stride,
                        const double* dist, int64_t dist_stride, double margin_x, double margin_y, int64_t B, int V, int J,
                        cudaStream_t s);

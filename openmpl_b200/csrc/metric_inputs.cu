@@ -6,6 +6,7 @@
 // pixels and a generator of random camera setups (the last three have no reference counterpart).  Every kernel that reads
 // calibrations is instantiated twice: one [V, 18] block for the batch (kPerPose = false) or one per pose (true).
 #include "kernels.cuh"
+#include "so3.cuh"
 
 namespace mpl {
 
@@ -1362,6 +1363,59 @@ int launch_synth_cameras(uint64_t seed, int64_t start, int64_t B, int V, double 
   const int64_t total = B * V;
   if (total == 0) return MPL_OK;
   synth_cameras_kernel<<<(unsigned)ceil_div(total, 128), 128, 0, s>>>(seed, start, B, V, f0, w, h, room, calib);
+  MPL_LAUNCH_CHECK();
+  return MPL_OK;
+}
+
+// ---- calibration errors: one thread per (pose, view), fp64 -------------------------------------------------------------
+// U0..U5 of (pose i, view v) come from the Philox4x64-10 stream under key (seed, 3), in the slot layout of synth_cameras_kernel.
+// Six standard normals by Box-Muller on (U0, U1), (U2, U3), (U4, U5); R' = Exp(sigma_rot n0..2) R (a rotation in the camera
+// frame), t' = t + sigma_pos n3..5 (the camera centre).  openmpl_b200/synth.py (calibration_noise) is the twin.  A thread reads
+// its whole row before it writes, so calib_out may be calib when the rows coincide (stride 18 V).
+__global__ void __launch_bounds__(128) synth_calib_noise_kernel(uint64_t seed, int64_t start, int64_t B, int V,
+                                                                const double* calib, int64_t cstride, double sigma_rot,
+                                                                double sigma_pos, double* calib_out) {
+  const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= B * V) return;
+  const int64_t b = e / V;
+  const int v = (int)(e - b * V);
+  const double* c = calib + b * cstride + v * 18;
+  double row[18];
+#pragma unroll
+  for (int k = 0; k < 18; ++k) row[k] = c[k];
+  double U[6], n[6];
+  six_uniforms(seed, 3ull, start, b, V, v, U);
+#pragma unroll
+  for (int k = 0; k < 3; ++k) {
+    const double r = sqrt(-2.0 * log(fmax(U[2 * k], 1e-12)));
+    double sn, cs;
+    sincospi(2.0 * U[2 * k + 1], &sn, &cs);
+    n[2 * k] = r * cs;
+    n[2 * k + 1] = r * sn;
+  }
+  if (sigma_rot != 0.0) {
+    const double w[3] = {sigma_rot * n[0], sigma_rot * n[1], sigma_rot * n[2]};
+    double E[9], Rn[9];
+    so3_exp(w, E);
+    mat3_mul(E, row, Rn);
+#pragma unroll
+    for (int k = 0; k < 9; ++k) row[k] = Rn[k];
+  }
+  if (sigma_pos != 0.0) {
+#pragma unroll
+    for (int k = 0; k < 3; ++k) row[9 + k] += sigma_pos * n[3 + k];
+  }
+  double* o = calib_out + e * 18;
+#pragma unroll
+  for (int k = 0; k < 18; ++k) o[k] = row[k];
+}
+
+int launch_synth_calib_noise(uint64_t seed, int64_t start, int64_t B, int V, const double* calib, int64_t calib_stride,
+                             double sigma_rot, double sigma_pos, double* calib_out, cudaStream_t s) {
+  const int64_t total = B * V;
+  if (total == 0) return MPL_OK;
+  synth_calib_noise_kernel<<<(unsigned)ceil_div(total, 128), 128, 0, s>>>(seed, start, B, V, calib, calib_stride, sigma_rot,
+                                                                          sigma_pos, calib_out);
   MPL_LAUNCH_CHECK();
   return MPL_OK;
 }

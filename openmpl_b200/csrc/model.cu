@@ -1548,6 +1548,60 @@ int mpl_synth_cameras(uint64_t seed, int64_t start, int64_t batch, int num_views
   return launch_synth_cameras(seed, start, batch, num_views, f0, w, h, room, calib_out, reinterpret_cast<cudaStream_t>(stream));
 }
 
+int mpl_synth_calib_noise(uint64_t seed, int64_t start, int64_t batch, int num_views, const double* calib,
+                          int64_t calib_stride, double sigma_rot, double sigma_pos, double* calib_out, mpl_stream_t stream) {
+  if (num_views < 1 || num_views > kMaxViews || start < 0 || !std::isfinite(sigma_rot) || !(sigma_rot >= 0.0) ||
+      !std::isfinite(sigma_pos) || !(sigma_pos >= 0.0) || !calib_stride_ok(calib_stride, num_views) || batch < 0) {
+    set_error("mpl_synth_calib_noise: bad argument (batch %lld, start %lld, num_views %d, sigma_rot %g, sigma_pos %g, "
+              "calib_stride %lld)", (long long)batch, (long long)start, num_views, sigma_rot, sigma_pos,
+              (long long)calib_stride);
+    return MPL_ERR_INVALID_ARGUMENT;
+  }
+  if (batch == 0) return MPL_OK;
+  if (calib == nullptr || calib_out == nullptr) {
+    set_error("mpl_synth_calib_noise: null pointer");
+    return MPL_ERR_INVALID_ARGUMENT;
+  }
+  if (calib_out == calib && calib_stride != 18 * (int64_t)num_views) {
+    set_error("mpl_synth_calib_noise: calib_out may be calib only with calib_stride 18 * num_views");
+    return MPL_ERR_INVALID_ARGUMENT;
+  }
+  return launch_synth_calib_noise(seed, start, batch, num_views, calib, calib_stride, sigma_rot, sigma_pos, calib_out,
+                                  reinterpret_cast<cudaStream_t>(stream));
+}
+
+size_t mpl_calibrate_rig_workspace_bytes(int64_t batch, int num_views, int num_joints) {
+  if (batch < 1 || num_views < 2 || num_views > kMaxViews || num_joints < 1) return 0;
+  return rig_workspace_bytes(batch, num_views, num_joints);
+}
+
+int mpl_calibrate_rig(const float* pix, const double* calib, int64_t batch, int num_views, int num_joints, float min_conf,
+                      const int32_t* view_mask, const float* init, double sigma_px, double sigma_rot, double sigma_pos,
+                      int max_iters, double* calib_out, float* points, double* report, void* workspace,
+                      size_t workspace_bytes, mpl_stream_t stream) {
+  auto sigma_ok = [](double s) { return std::isfinite(s) && s > 0.0; };
+  if (num_views < 2 || num_views > kMaxViews || num_joints < 1 || batch < 1 || !sigma_ok(sigma_px) || !sigma_ok(sigma_rot) ||
+      !sigma_ok(sigma_pos) || max_iters < 1 || max_iters > 100) {
+    set_error("mpl_calibrate_rig: bad argument (batch %lld, num_views %d, num_joints %d, sigma_px %g, sigma_rot %g, "
+              "sigma_pos %g, max_iters %d)", (long long)batch, num_views, num_joints, sigma_px, sigma_rot, sigma_pos,
+              max_iters);
+    return MPL_ERR_INVALID_ARGUMENT;
+  }
+  if (pix == nullptr || calib == nullptr || init == nullptr || calib_out == nullptr || report == nullptr ||
+      workspace == nullptr) {
+    set_error("mpl_calibrate_rig: null pointer");
+    return MPL_ERR_INVALID_ARGUMENT;
+  }
+  const size_t need = rig_workspace_bytes(batch, num_views, num_joints);
+  if (workspace_bytes < need) {
+    set_error("mpl_calibrate_rig: workspace has %zu bytes, %zu needed", workspace_bytes, need);
+    return MPL_ERR_WORKSPACE;
+  }
+  return launch_calibrate_rig(pix, calib, batch, num_views, num_joints, min_conf, view_mask, init, sigma_px, sigma_rot,
+                              sigma_pos, max_iters, calib_out, points, report, workspace,
+                              reinterpret_cast<cudaStream_t>(stream));
+}
+
 int mpl_test_gemm(const void* A, const void* W, const float* bias, void* Y, int64_t M, int N, int K, int dtype, int epilogue,
                   int out_fp32, int cta_group, mpl_stream_t stream) {
   MPL_API_BEGIN

@@ -14,6 +14,8 @@
         --triangulation-pmpjpe                                                          # + P-MPJPE of both baselines
     python -m openmpl_b200.evaluate --arch hm0 --views 4 --lens-distortion=-0.207,0.248,-0.0009,-0.0016,-0.0031 \
         --triangulate --triangulate-robust --refine-triangulations                      # cameras with a lens
+    python -m openmpl_b200.evaluate --arch hm0 --views 4 --pixel-noise 1 --calib-noise 0.5,20 --triangulate \
+        --calibrate-rig 16384                                                           # a miscalibrated rig, recalibrated
 
 Per micro-batch, entirely on the device: `mpl_synth_project` (3D poses from the counter-based generator keyed by the
 GLOBAL pose index, projected through the V calibrations) -> `mpl_build_inputs` (clip, confidence zeroing, screen
@@ -53,6 +55,23 @@ lifter's inputs are built from the distorted pixels as the reference builds them
 triangulation and refinement runs on `mpl_undistort_pixels` output (margin half the image on each side) with the shifted
 calibration it comes with.  It composes with `--random-cameras` (one lens, per-pose calibrations).  The line's "data"
 entry records the coefficients.  Without the flag nothing of this runs.
+
+`--calib-noise ROT_DEG,POS_MM` gives every consumer of the calibration a perturbed one (`mpl_synth_calib_noise`: each
+camera rotated by a Gaussian rotation vector of std ROT_DEG degrees per axis in its own frame, its centre moved by a
+Gaussian of std POS_MM mm per axis): the lifter's inputs, the undistortion, the triangulations and the refinement all use
+it, while the synthetic pixels are still projected through the true cameras.  The rig is perturbed once (pose 0 of the
+noise stream); with `--random-cameras` every pose's cameras are perturbed under its global index.  The line's "data" entry
+records the two values.  `--calib-noise 0,0` gives the metrics of a run without the flag.
+
+`--calibrate-rig N` (with `--calib-noise`, both values > 0; not with `--random-cameras`; N <= `--micro-batch`) recalibrates
+the perturbed rig before the evaluation: every rank generates the N poses at global indices [poses, poses + N), disjoint
+from the evaluated ones, through the same data path (true projection, lens, detector noise, undistortion), triangulates
+them linearly under the perturbed rig and bundle-adjusts the rig's extrinsics and the joints (`mpl_calibrate_rig`, every
+candidate view, sigma_px = `--pixel-noise` or 1 px when it is 0, the prior of `--calib-noise`).  The refined rotations and
+centres then replace the perturbed ones for the whole evaluation (the intrinsics stay).  Every rank computes the same
+bits, so no collective is needed.  The line gains a "rig_calibration" entry: poses, items, observations, iterations,
+accepted steps, RMS pixel error before and after, per-view rotation (degrees) and centre (mm) errors of the perturbed and
+of the calibrated rig against the true one, and its own time `ms`, outside `ms_total`.
 """
 from __future__ import annotations
 
@@ -74,12 +93,24 @@ ARCHS = {
 DEFAULT_DEPTH = {"hm0": 12, "chosen": 12, "kptok": 12, "cmu0": 2}
 DEFAULT_RIG = {"hm0": "h36m", "chosen": "h36m", "kptok": "h36m", "cmu0": "cmu"}
 REFINE_MAX_ITERS = 20
+CALIBRATE_MAX_ITERS = 30
 
 
 def run(arch="hm0", views=4, depth=None, poses=1 << 20, micro_batch=65536, precision="bf16", rig=None, seed=1,
         weight_seed=0, warmup=1, triangulate=False, pixel_noise=0.0, outlier_rate=0.0, miss_rate=0.0,
         triangulate_robust=False, inlier_px=10.0, random_cameras=False, refine_triangulations=False,
-        triangulation_pmpjpe=False, lens_distortion=None):
+        triangulation_pmpjpe=False, lens_distortion=None, calib_noise=None, calibrate_rig=0):
+    if calib_noise is not None:
+        calib_noise = tuple(float(x) for x in calib_noise)
+        if len(calib_noise) != 2 or not all(np.isfinite(calib_noise)) or min(calib_noise) < 0:
+            raise ValueError(f"calib_noise must be two finite numbers >= 0 (degrees, mm), got {calib_noise}")
+    if calibrate_rig:
+        if calib_noise is None or min(calib_noise) <= 0:
+            raise ValueError("calibrate_rig needs calib_noise with both values > 0")
+        if random_cameras:
+            raise ValueError("calibrate_rig calibrates one fixed rig: not with random_cameras")
+        if not 1 <= calibrate_rig <= micro_batch:
+            raise ValueError(f"calibrate_rig must be in [1, micro_batch = {micro_batch}], got {calibrate_rig}")
     if lens_distortion is not None:
         lens_distortion = tuple(float(k) for k in lens_distortion)
         if len(lens_distortion) != 5 or not all(np.isfinite(lens_distortion)):
@@ -116,14 +147,54 @@ def run(arch="hm0", views=4, depth=None, poses=1 << 20, micro_batch=65536, preci
     if lens_distortion is not None:
         lens = torch.tensor([lens_distortion] * views, dtype=torch.float64, device=dev)
         margin = (the_rig.image_size[0] / 2.0, the_rig.image_size[1] / 2.0)   # known here: no read-back of calib
+    rig_calib = torch.as_tensor(inputs.pack_calibration(the_rig.R, the_rig.t, the_rig.f, the_rig.c, the_rig.image_size)).to(dev)
+    if calib_noise is not None:
+        sig_rot, sig_pos = np.radians(calib_noise[0]), calib_noise[1] / 1000.0
+        used_rig = inputs.calibration_noise(rig_calib, seed, 0, sig_rot, sig_pos)     # the rig as pose 0 of the noise stream
+    else:
+        used_rig = rig_calib
 
-    def step(s0, n):
-        cams = inputs.synth_cameras(n, views, rig_kind, seed=seed, start=s0, device=dev) if random_cameras else None
+    def synth_pixels(s0, n, cams):
+        """Pixels of poses [s0, s0 + n) through the true cameras, with the lens and the detector noise."""
         pix, target, calib = inputs.synth_project(n, the_rig, seed=seed, start=s0, device=dev, cameras=cams)
         if lens_distortion is not None:
             inputs.distort_pixels(pix, calib, lens)
         if noisy:
             inputs.add_detector_noise(pix, calib, seed, s0, pixel_noise, outlier_rate, miss_rate)
+        return pix, target
+
+    rig_report = None
+    if calibrate_rig:
+        ce0, ce1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        ce0.record()
+        pix, _ = synth_pixels(poses, calibrate_rig, None)
+        cal = used_rig
+        if lens_distortion is not None:
+            pix, cal = inputs.undistort_pixels(pix, cal, lens, margin=margin)
+        points, _ = inputs.triangulate(pix, cal)
+        sigma_px = pixel_noise if pixel_noise > 0 else 1.0
+        refined, _, rep = inputs.calibrate_rig(pix, cal, points, sigma_px=sigma_px, sigma_rot=sig_rot, sigma_pos=sig_pos,
+                                               max_iters=CALIBRATE_MAX_ITERS)
+        noisy_rig = used_rig
+        used_rig = used_rig.clone()
+        used_rig[:, :12] = refined[:, :12]                  # extrinsics only: the unshifted intrinsics stay
+        ce1.record()
+        torch.cuda.synchronize()
+        cals = {"noisy": noisy_rig.cpu().numpy(), "calibrated": used_rig.cpu().numpy()}
+        true_rig = rig_calib.cpu().numpy()
+        rig_report = dict(ms=ce0.elapsed_time(ce1), report=rep.cpu().numpy(), sigma_px=sigma_px,
+                          errors={k: rig_errors(c, true_rig) for k, c in cals.items()},
+                          aligned={k: rig_errors(c, true_rig, align=True) for k, c in cals.items()} if views >= 3 else None)
+
+    def step(s0, n):
+        cams = inputs.synth_cameras(n, views, rig_kind, seed=seed, start=s0, device=dev) if random_cameras else None
+        pix, target = synth_pixels(s0, n, cams)
+        if cams is None:
+            calib = used_rig
+        elif calib_noise is not None:
+            calib = inputs.calibration_noise(cams, seed, s0, sig_rot, sig_pos)
+        else:
+            calib = cams
         p, r, c = inputs.build_inputs(pix, calib)
         with torch.no_grad():
             out = model(p, rays=r, centers=c)
@@ -205,6 +276,32 @@ def run(arch="hm0", views=4, depth=None, poses=1 << 20, micro_batch=65536, preci
                 "coefficients": dict(zip(("k1", "k2", "p1", "p2", "k3"), lens_distortion)),
                 "pipeline": "projected pixels distorted before the detector noise; lifter inputs built from the distorted "
                             "pixels; triangulations on the undistorted pixels (margin half the image on each side)"}
+        if calib_noise is not None:
+            if not isinstance(line["data"], dict):
+                line["data"] = {"source": line["data"]}
+            line["data"]["calibration_noise"] = {
+                "rotation_deg": calib_noise[0], "position_mm": calib_noise[1],
+                "model": "per camera R' = Exp(w) R with w ~ N(0, rotation_deg^2 I) (camera frame), centre + N(0, "
+                         "position_mm^2 I); the pixels are projected through the true cameras, every other step uses the "
+                         "perturbed ones" + ("" if random_cameras else "; one perturbation of the rig (pose 0)")}
+        if rig_report is not None:
+            rp = rig_report["report"]
+            line["rig_calibration"] = {
+                "poses": calibrate_rig, "global_indices": [poses, poses + calibrate_rig], "items": int(rp[0]),
+                "observations": int(rp[1]), "iterations": int(rp[6]), "accepted_steps": int(rp[7]),
+                "rms_px": {"before": float(rp[4]), "after": float(rp[5])}, "sigma_px": rig_report["sigma_px"],
+                "rotation_error_deg": {k: e[0] for k, e in rig_report["errors"].items()},
+                "centre_error_mm": {k: e[1] for k, e in rig_report["errors"].items()},
+                "method": f"Levenberg-Marquardt bundle adjustment of the extrinsics and the joints, Gaussian prior of "
+                          f"--calib-noise, at most {CALIBRATE_MAX_ITERS} iterations, from the linear triangulation",
+                "ms": rig_report["ms"], "note": "ms is not part of ms_total"}
+            if rig_report["aligned"] is not None:
+                line["rig_calibration"]["after_similarity_alignment"] = {
+                    "rotation_error_deg": {k: e[0] for k, e in rig_report["aligned"].items()},
+                    "centre_error_mm": {k: e[1] for k, e in rig_report["aligned"].items()},
+                    "note": "each rig mapped into the true frame by the similarity fitting its centres to the true ones: "
+                            "the images do not observe the world frame, so the bundle adjustment leaves that similarity "
+                            "where the prior puts it"}
         if tacc is not None:
             line["triangulation"] = triangulation_summary(tacc.acc.detach().cpu().numpy(), cfg.J)
         if racc is not None:
@@ -229,6 +326,29 @@ def run(arch="hm0", views=4, depth=None, poses=1 << 20, micro_batch=65536, preci
         torch.distributed.barrier()
         torch.distributed.destroy_process_group()
     return line
+
+
+def rig_errors(calib, true_calib, align=False):
+    """Per view: rotation error (degrees, the angle of R R_true^T) and centre error (mm) of calib [V, 18] against true_calib.
+
+    align: first map calib into the true rig's frame by the similarity that best fits its centres onto the true ones
+    (Umeyama; needs V >= 3).  Images do not observe the world frame, so a bundle adjustment leaves the rig's 7-DoF
+    similarity where its prior puts it; the aligned errors measure what it can observe."""
+    if align:
+        src, dst = true_calib[:, 9:12], calib[:, 9:12]              # dst ~ s Q src + t
+        ms, md = src.mean(0), dst.mean(0)
+        U, S, Vt = np.linalg.svd((dst - md).T @ (src - ms))
+        D = np.diag([1.0, 1.0, np.sign(np.linalg.det(U @ Vt))])
+        Q = U @ D @ Vt
+        s = np.trace(np.diag(S) @ D) / ((src - ms) ** 2).sum()
+        calib = calib.copy()
+        calib[:, 9:12] = (dst - (md - s * Q @ ms)) @ Q / s
+        calib[:, :9] = (calib[:, :9].reshape(-1, 3, 3) @ Q).reshape(-1, 9)
+    R, Rt = calib[:, :9].reshape(-1, 3, 3), true_calib[:, :9].reshape(-1, 3, 3)
+    fro = np.linalg.norm((R - Rt).reshape(len(R), 9), axis=1)        # |R - R_true|_F = 2 sqrt(2) sin(angle / 2)
+    ang = np.degrees(2.0 * np.arcsin(np.minimum(fro / (2.0 * np.sqrt(2.0)), 1.0)))
+    pos = 1000.0 * np.linalg.norm(calib[:, 9:12] - true_calib[:, 9:12], axis=1)
+    return [float(a) for a in ang], [float(p) for p in pos]
 
 
 def triangulation_summary(acc, J, method="linear DLT, pixel-space rows, views with conf > 0 inside the image"):
@@ -281,7 +401,28 @@ def main(argv=None):
     p.add_argument("--lens-distortion", default=None, metavar="K1,K2,P1,P2,K3",
                    help="a lens of OpenCV's 5-coefficient model on every view: distorted detections for the lifter, "
                         "undistorted ones for the triangulations")
+    p.add_argument("--calib-noise", default=None, metavar="ROT_DEG,POS_MM",
+                   help="perturb the calibration every step but the projection uses: Gaussian rotation of std ROT_DEG "
+                        "degrees per axis and centre error of std POS_MM mm per axis, per camera")
+    p.add_argument("--calibrate-rig", type=int, default=0, metavar="N",
+                   help="recalibrate the perturbed rig's extrinsics by bundle adjustment on N extra poses before the "
+                        "evaluation (needs --calib-noise with both values > 0, not --random-cameras, N <= --micro-batch)")
     a = p.parse_args(argv)
+    cnoise = None
+    if a.calib_noise is not None:
+        try:
+            cnoise = tuple(float(x) for x in a.calib_noise.split(","))
+        except ValueError:
+            cnoise = ()
+        if len(cnoise) != 2 or not all(np.isfinite(cnoise)) or min(cnoise) < 0:
+            p.error("--calib-noise needs two comma-separated finite numbers >= 0: ROT_DEG,POS_MM")
+    if a.calibrate_rig:
+        if cnoise is None or min(cnoise) <= 0:
+            p.error("--calibrate-rig needs --calib-noise with both values > 0")
+        if a.random_cameras:
+            p.error("--calibrate-rig calibrates one fixed rig: it cannot be used with --random-cameras")
+        if not 1 <= a.calibrate_rig <= a.micro_batch:
+            p.error("--calibrate-rig N needs 1 <= N <= --micro-batch")
     lens = None
     if a.lens_distortion is not None:
         try:
@@ -297,7 +438,8 @@ def main(argv=None):
     run(a.arch, a.views, a.depth, a.poses, a.micro_batch, a.precision, a.rig, a.seed, triangulate=a.triangulate,
         pixel_noise=a.pixel_noise, outlier_rate=a.outlier_rate, miss_rate=a.miss_rate,
         triangulate_robust=a.triangulate_robust, inlier_px=a.inlier_px, random_cameras=a.random_cameras,
-        refine_triangulations=a.refine_triangulations, triangulation_pmpjpe=a.triangulation_pmpjpe, lens_distortion=lens)
+        refine_triangulations=a.refine_triangulations, triangulation_pmpjpe=a.triangulation_pmpjpe, lens_distortion=lens,
+        calib_noise=cnoise, calibrate_rig=a.calibrate_rig)
 
 
 if __name__ == "__main__":

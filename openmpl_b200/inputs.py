@@ -5,6 +5,8 @@ Replaces the per-sample numpy of `JointsDataset_MPL.__getitem__`
 """
 from __future__ import annotations
 
+import math
+
 import numpy as np
 import torch
 
@@ -205,6 +207,75 @@ def undistort_pixels(pix: torch.Tensor, calib, dist, margin=None) -> tuple:
     calib_u[..., 16] += 2.0 * mx
     calib_u[..., 17] += 2.0 * my
     return out, calib_u
+
+
+def calibration_noise(calib, seed: int, start: int, sigma_rot: float, sigma_pos: float, device=None) -> torch.Tensor:
+    """Calibration errors (`mpl_synth_calib_noise`), enqueued on the current stream; returns a new fp64 tensor.
+
+    calib [V, 18] (a fixed rig, perturbed as pose `start`) or [B, V, 18] (one calibration per pose, poses [start, start + B)),
+    numpy or tensor.  Per (pose, view): R' = Exp(sigma_rot n) R (radians, a rotation in the camera frame) and
+    t' = t + sigma_pos m (world units), n and m standard normal 3-vectors drawn under a Philox key of their own; the
+    intrinsics are copied.  The draws depend only on (seed, global pose index); `synth.calibration_noise` is the numpy twin.
+    """
+    if device is None:
+        device = calib.device if isinstance(calib, torch.Tensor) else torch.device("cuda", torch.cuda.current_device())
+    c = calib.to(device=device, dtype=torch.float64) if isinstance(calib, torch.Tensor) else \
+        torch.as_tensor(np.asarray(calib, dtype=np.float64)).to(device)
+    c = c.contiguous()
+    if c.dim() not in (2, 3) or c.shape[-1] != 18:
+        raise ValueError(f"calib must be [V, 18] or [B, V, 18], got {list(c.shape)}")
+    V = c.shape[-2]
+    B = 1 if c.dim() == 2 else c.shape[0]
+    out = torch.empty_like(c)
+    with torch.cuda.device(device):
+        stream = torch.cuda.current_stream(device).cuda_stream
+        _lib.check(_lib.lib().mpl_synth_calib_noise(int(seed), int(start), B, V, c.data_ptr(), 0 if c.dim() == 2 else 18 * V,
+                                                    float(sigma_rot), float(sigma_pos), out.data_ptr(), stream))
+    return out
+
+
+def calibrate_rig(pix: torch.Tensor, calib, init: torch.Tensor, view_mask: torch.Tensor | None = None,
+                  sigma_px: float = 1.0, sigma_rot: float = math.radians(1.0), sigma_pos: float = 0.05,
+                  min_conf: float = 0.0, max_iters: int = 30) -> tuple:
+    """Bundle adjustment of a rig's extrinsics from its detections (`mpl_calibrate_rig`), enqueued on the current stream.
+
+    pix [B, V, J, 3] fp32 (u, v, conf) pixels of B poses seen by one rig calib [V, 18]; init [B, J, 3] starting points, e.g.
+    `triangulate(pix, calib)[0]`; view_mask [B, J] int32 bitmask or None (every candidate view, as in
+    `refine_triangulation`).  Levenberg-Marquardt on sum conf^2 / sigma_px^2 |reprojection error|^2 plus the Gaussian prior
+    |omega_v|^2 / sigma_rot^2 + |c_v - c0_v|^2 / sigma_pos^2 on each camera's rotation (radians) and centre (world units),
+    the distribution `calibration_noise` draws from.  Returns (calib_refined [V, 18] fp64 with the intrinsics of calib;
+    points [B, J, 3] fp32, the refined joints where they took part and init elsewhere; report [8] fp64 = items,
+    observations, cost at the start and at the end, conf-weighted RMS pixel error at the start and at the end, iterations,
+    accepted steps), all on the device.
+    """
+    B, V, J, _ = pix.shape
+    device = pix.device
+    if tuple(init.shape) != (B, J, 3):
+        raise ValueError(f"init must be [B, J, 3] = [{B}, {J}, 3], got {list(init.shape)}")
+    if view_mask is not None and (tuple(view_mask.shape) != (B, J) or view_mask.dtype != torch.int32):
+        raise ValueError(f"view_mask must be a [B, J] = [{B}, {J}] int32 bitmask, got {list(view_mask.shape)} "
+                         f"{view_mask.dtype}")
+    pix = pix.to(torch.float32).contiguous()
+    init = init.to(device=device, dtype=torch.float32).contiguous()
+    mask = None if view_mask is None else view_mask.to(device).contiguous()
+    calib, stride = _calib_arg(calib, B, V, device)
+    if stride != 0 or tuple(calib.shape) != (V, 18):
+        raise ValueError(f"calibrate_rig takes one rig calib [V, 18] = [{V}, 18], got {list(calib.shape)}")
+    L = _lib.lib()
+    nbytes = L.mpl_calibrate_rig_workspace_bytes(B, V, J)
+    if nbytes == 0:
+        raise ValueError(f"calibrate_rig: unsupported shape B={B} V={V} J={J} (2 <= V <= 16, B >= 1, J >= 1)")
+    ws = torch.empty(nbytes, dtype=torch.uint8, device=device)
+    calib_out = torch.empty_like(calib)
+    points = torch.empty((B, J, 3), dtype=torch.float32, device=device)
+    report = torch.empty(8, dtype=torch.float64, device=device)
+    with torch.cuda.device(device):
+        stream = torch.cuda.current_stream(device).cuda_stream
+        _lib.check(L.mpl_calibrate_rig(pix.data_ptr(), calib.data_ptr(), B, V, J, float(min_conf),
+                                       None if mask is None else mask.data_ptr(), init.data_ptr(), float(sigma_px),
+                                       float(sigma_rot), float(sigma_pos), int(max_iters), calib_out.data_ptr(),
+                                       points.data_ptr(), report.data_ptr(), ws.data_ptr(), nbytes, stream))
+    return calib_out, points, report
 
 
 def _dist_arg(dist, B: int, V: int, device) -> tuple:

@@ -114,6 +114,47 @@ def random_cameras(batch: int, num_views: int, kind: str = "h36m", seed: int = 0
     return cameras_from_uniforms(U, f0, image_size, room)
 
 
+def so3_exp(w) -> np.ndarray:
+    """Rodrigues' formula Exp(w) = I + sin t / t [w]x + (1 - cos t) / t^2 [w]x^2, t = |w|, for w [..., 3] -> [..., 3, 3]; below
+    t^2 = 1e-2 the coefficients come from their Taylor series through t^8, as on the device."""
+    w = np.asarray(w, dtype=np.float64)
+    t2 = (w * w).sum(-1)
+    small = t2 < 1e-2
+    with np.errstate(invalid="ignore", divide="ignore"):
+        t = np.sqrt(t2)
+        a = np.where(small, 1.0 - t2 / 6.0 * (1.0 - t2 / 20.0 * (1.0 - t2 / 42.0 * (1.0 - t2 / 72.0))), np.sin(t) / t)
+        b = np.where(small, 0.5 * (1.0 - t2 / 12.0 * (1.0 - t2 / 30.0 * (1.0 - t2 / 56.0 * (1.0 - t2 / 90.0)))),
+                     (1.0 - np.cos(t)) / t2)
+    K = np.zeros(w.shape[:-1] + (3, 3))
+    K[..., 0, 1], K[..., 0, 2], K[..., 1, 2] = -w[..., 2], w[..., 1], -w[..., 0]
+    K[..., 1, 0], K[..., 2, 0], K[..., 2, 1] = w[..., 2], -w[..., 1], w[..., 0]
+    K2 = w[..., :, None] * w[..., None, :] - t2[..., None, None] * np.eye(3)
+    return np.eye(3) + a[..., None, None] * K + b[..., None, None] * K2
+
+
+def calibration_noise(calib, seed: int, start: int, sigma_rot: float, sigma_pos: float) -> np.ndarray:
+    """Host twin of `mpl_synth_calib_noise`: calib [V, 18] (a fixed rig, drawn as pose `start`) or [B, V, 18] (poses
+    [start, start + B)) perturbed.  U0..U5 of (pose i, view v) come from the Philox4x64-10 stream under key (seed, 3)
+    (slot layout of `random_cameras`); Box-Muller gives n_2k = r cos(2 pi U_2k+1), n_2k+1 = r sin(2 pi U_2k+1),
+    r = sqrt(-2 ln max(U_2k, 1e-12)); R' = Exp(sigma_rot n0..2) R and t' = t + sigma_pos n3..5.  The intrinsics are copied, and a
+    zero sigma keeps its field bit for bit."""
+    calib = np.asarray(calib, dtype=np.float64)
+    rig = calib.ndim == 2
+    c = calib[None] if rig else calib
+    B, V = c.shape[:2]
+    U = _uniforms(seed, start, B, 6 * V, key1=3).reshape(B, V, 6)
+    r = np.sqrt(-2.0 * np.log(np.maximum(U[..., 0::2], 1e-12)))
+    th = 2 * math.pi * U[..., 1::2]
+    n = np.empty((B, V, 6))
+    n[..., 0::2], n[..., 1::2] = r * np.cos(th), r * np.sin(th)
+    out = c.copy()
+    if sigma_rot != 0:
+        out[..., 0:9] = (so3_exp(sigma_rot * n[..., 0:3]) @ c[..., 0:9].reshape(B, V, 3, 3)).reshape(B, V, 9)
+    if sigma_pos != 0:
+        out[..., 9:12] = c[..., 9:12] + sigma_pos * n[..., 3:6]
+    return out[0] if rig else out
+
+
 def _uniforms(seed: int, start: int, count: int, per_pose: int, key1: int = 0) -> np.ndarray:
     """[count, per_pose] uniforms in [0,1); row i depends only on (seed, start+i).  Philox key (seed, key1)."""
     blocks = (per_pose + 3) // 4                      # Philox4x64: 4 outputs per counter step
