@@ -45,7 +45,7 @@
 extern "C" {
 #endif
 
-#define MPL_ABI_VERSION 9
+#define MPL_ABI_VERSION 10
 
 typedef enum MplStatus {
   MPL_OK = 0,
@@ -104,16 +104,15 @@ typedef struct MplDesc {
                              non-zero (make_desc default: 1) = fused: the GEMM that updates the residual stream also emits
                              the next GEMM's operand and per-row (sum, sum^2); the next GEMM multiplies the raw rows by
                              W diag(gamma) and applies (mean, rstd) in its epilogue */
-  int32_t gemm_cta_group; /* 0 / 2: CTA pair per 256x256 tile (cta_group::2, cluster 2x1x1); 1: one CTA per 128x256 tile */
+  int32_t gemm_cta_group; /* must be 0 or 2: every projection GEMM tile is 256x256 on a CTA pair (cta_group::2, cluster
+                             2x1x1).  Kept so that the struct layout stays; any other value is MPL_ERR_INVALID_ARGUMENT */
   int32_t spt_hidden, fpt_hidden; /* int(width * mlp_ratio) of the SPT / FPT Mlp as the reference's float64 arithmetic gives it
                                      (0 = derive from the float mlp_ratio above) */
   int32_t qkv_attn_fusion; /* bf16 LayerNorm-fused mode, view tokens, 136-wide heads (or an even number of 68-wide ones), 2 to 8 views: QKV projection and
                               cross-view attention run as ONE kernel (no q|k|v tensor).  0 = two kernels, non-zero (make_desc
                               default: 1) = fused where the shape allows */
-  int32_t chunk_streams;  /* 0 / 1: one pose chunk at a time on the caller's stream (default).  2: batches of >= 16384 poses
-                             run as two interleaved pose chunks on two internal streams (forked from / joined to the
-                             caller's stream) so that kernels of one chunk may overlap those of the other; the
-                             workspace doubles.  Same results; measured neutral on B200 (profiles/r2_experiments.md) */
+  int32_t chunk_streams;  /* must be 0 or 1: the pose chunks of a forward run one at a time on the caller's stream.  Kept
+                             so that the struct layout stays; any other value is MPL_ERR_INVALID_ARGUMENT */
 } MplDesc;
 
 typedef struct MplModel MplModel;          /* opaque host-side handle */
@@ -179,9 +178,8 @@ int64_t mpl_last_launch_count(const MplModel* m);
 /* Optional per-launch timing with CUDA events on the caller's stream (the reference's only profiling hook is an
  * unsynchronised time.time() around the model call, core/function_mpl.py:346-351).  While enabled, every kernel
  * launch of mpl_forward is bracketed by two events; mpl_profile_collect waits for the last forward's events and
- * returns milliseconds and launch counts per kernel category (mpl_profile_category_name).  enabled = 1 profiles the
- * production schedule (two chunks in flight: launches of the two streams overlap, so the per-category times sum to more
- * than the step); enabled = 2 additionally runs one chunk at a time, so the times add up to the (slower) serial step. */
+ * returns milliseconds and launch counts per kernel category (mpl_profile_category_name).  Any non-zero `enabled`
+ * profiles; the launches run one after the other on the caller's stream, so the per-category times add up to the step. */
 int mpl_set_profile(MplModel* m, int enabled);
 int mpl_profile_categories(void);
 const char* mpl_profile_category_name(int category);
@@ -484,10 +482,9 @@ int mpl_calibrate_rig(const float* pix, const double* calib, int64_t batch, int 
 /* Y[M,N] = epilogue(A[M,K] . W[N,K]^T): the tcgen05 projection kernel in isolation.
  *   dtype: MPL_PREC_BF16 (A, W bf16) or MPL_PREC_TF32 (split mode: A = [2][M][K], W = [2][N][K] bf16 planes hi, lo)
  *   epilogue: 0 bias -> operand format (bf16, or two planes [2][M][N]) / fp32 per `out_fp32`; 1 bias+GELU;
- *             2 bias + residual(fp32, in place in Y)
- *   cta_group: 1 or 2 (see MplDesc.gemm_cta_group). */
+ *             2 bias + residual(fp32, in place in Y) */
 int mpl_test_gemm(const void* A, const void* W, const float* bias, void* Y, int64_t M, int N, int K, int dtype,
-                  int epilogue, int out_fp32, int cta_group, mpl_stream_t stream);
+                  int epilogue, int out_fp32, mpl_stream_t stream);
 
 /* The LayerNorm-fused epilogues of the bf16 mode in isolation (DESIGN.md section 4).
  *   epilogue 4 / 5 (LayerNorm-apply, QKV / fc1): Y[M,N] (bf16, or fp16 when out_fp16) = act(rstd * (A W'^T - mu * colsum) + bias),
@@ -498,12 +495,12 @@ int mpl_test_gemm(const void* A, const void* W, const float* bias, void* Y, int6
  *       ab_fp16: A and W hold fp16 instead of bf16. */
 int mpl_test_gemm_ln(const void* A, const void* W, const float* bias, void* Y, int64_t M, int N, int K, int epilogue,
                      const float* colsum, const void* stats_in, int slots_in, void* stats_out, void* x_lo, float eps,
-                     int ab_fp16, int out_fp16, int cta_group, mpl_stream_t stream);
+                     int ab_fp16, int out_fp16, mpl_stream_t stream);
 int mpl_test_gemm_ln_slots(int N);
 /* Epilogue 6 on the first N columns of residual planes whose rows are `ldy` >= N elements apart (the last fc2 of the stack
  * updates the pose half of the channel-permuted residual stream only, DESIGN.md section 3); the other columns stay. */
 int mpl_test_gemm_emit_pitch(const void* A, const void* W, const float* bias, void* Y, int64_t M, int N, int K, void* stats_out,
-                             void* x_lo, int ab_fp16, int ldy, int cta_group, mpl_stream_t stream);
+                             void* x_lo, int ab_fp16, int ldy, mpl_stream_t stream);
 /* The fused QKV projection + cross-view attention kernel (multiview_mpl.py:48-64 behind the folded norm1) in isolation:
  *   xb [M, D] bf16 raw residual rows, W [3D, D] / bias [3D] (or NULL) / gamma, beta [D] fp32 on the device, stats as above,
  *   att [M, D] bf16 out; M = poses * V rows, D = H * 136 (or H * 68, H even), 2 <= V <= 8.

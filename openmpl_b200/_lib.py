@@ -11,7 +11,7 @@ from ctypes import POINTER, c_char_p, c_double, c_float, c_int, c_int32, c_int64
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("MPL_B200_LIB") or os.path.join(HERE, "libmpl_b200.so")   # override: another build of the same ABI
 
-ABI_VERSION = 9
+ABI_VERSION = 10
 MPL_OK = 0
 MPL_ERR_INVALID_ARGUMENT = -1
 MPL_ERR_CONFIG_RUNTIME = -2
@@ -57,8 +57,7 @@ class MplDesc(ctypes.Structure):
                                                          ("chunk_streams", c_int32)])
 
 
-def make_desc(kw: dict, precision: str, ln_fusion: bool = True, gemm_cta_group: int = 2, chunk_streams: int = 1,
-              qkv_attn_fusion: bool = True) -> MplDesc:
+def make_desc(kw: dict, precision: str, ln_fusion: bool = True, qkv_attn_fusion: bool = True) -> MplDesc:
     """Constructor kwargs of MultiView_MPL (multiview_mpl.py:95-117) -> MplDesc."""
     if precision not in PRECISIONS:
         raise ValueError(f"precision must be one of {sorted(PRECISIONS)}, got {precision!r}")
@@ -72,8 +71,6 @@ def make_desc(kw: dict, precision: str, ln_fusion: bool = True, gemm_cta_group: 
         setattr(d, f, int(bool(kw[f])))
     d.precision = PRECISIONS[precision]
     d.ln_fusion = int(bool(ln_fusion))
-    d.gemm_cta_group = int(gemm_cta_group)
-    d.chunk_streams = int(chunk_streams)
     d.qkv_attn_fusion = int(bool(qkv_attn_fusion))
     # the Mlp widths as Python's float64 int(dim * ratio) gives them (the float32 ratio in the struct can round differently)
     from .spec import make_config
@@ -125,12 +122,12 @@ def lib():
         L.mpl_pmpjpe_accumulate.argtypes = [c_void_p, c_void_p, c_int64, c_int, c_float, c_int, c_int, c_void_p, c_void_p]
         L.mpl_build_inputs.argtypes = [c_void_p, c_void_p, c_int64, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p]
         L.mpl_test_gemm.argtypes = [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int, c_int, c_int, c_int, c_int,
-                                    c_int, c_void_p]
+                                    c_void_p]
         L.mpl_test_gemm_ln.argtypes = [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int, c_int, c_int, c_void_p, c_void_p,
-                                       c_int, c_void_p, c_void_p, c_float, c_int, c_int, c_int, c_void_p]
+                                       c_int, c_void_p, c_void_p, c_float, c_int, c_int, c_void_p]
         L.mpl_test_gemm_ln_slots.argtypes = [c_int]
         L.mpl_test_gemm_emit_pitch.argtypes = [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int, c_int, c_void_p, c_void_p,
-                                               c_int, c_int, c_int, c_void_p]
+                                               c_int, c_int, c_void_p]
         L.mpl_test_qkv_attn.argtypes = [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_float, c_float, c_void_p,
                                         c_int64, c_int, c_int, c_int, c_void_p, c_size_t, c_void_p]
         L.mpl_set_graph_batch.argtypes = [c_void_p, c_int64]

@@ -15,8 +15,8 @@
 //                             residual-emit epilogues (EPI 6 / 7) for proj / fc2, see GemmLn below.
 //   warp 3     residual producer (EPI 6 / 7 only): TMA-loads the old residual boxes (two bf16 planes) into a ring of
 //                             shared-memory slots, running ahead of the epilogue warps across tile boundaries
-// CG = 1: one CTA per 128 x 256 output tile.  CG = 2: a CTA pair (cluster 2x1x1, cta_group::2) per 256 x 256 tile, each
-// CTA staging half of A and half of W, which halves the shared-memory and L2 operand traffic per MMA.
+// A CTA pair (cluster 2x1x1, cta_group::2) computes each 256 x 256 output tile, each CTA staging half of A and half of W,
+// which halves the shared-memory and L2 operand traffic per MMA.
 // Every FPT width is a multiple of 17 (D = 1088 = 17*64): ragged N tiles use a narrower UMMA N (multiple of 16) and
 // the K tail is zero-filled by TMA, so no padding copies are needed.
 #include <cuda.h>
@@ -34,13 +34,14 @@ namespace mpl {
 
 namespace {
 
+constexpr int CG = 2;            // CTAs per output tile (a CTA pair)
 constexpr int BM = 128;          // accumulator rows per CTA (TMEM lanes)
 constexpr int BN = 256;          // accumulator columns per tile
 constexpr int KB_BYTES = 128;    // bytes of K per stage row = one 128B swizzle span
 constexpr int UMMA_K_BYTES = 32; // bytes of K per tcgen05.mma
-// Shared-memory budget of the LayerNorm-fused bf16 kernels (CTA pairs).  Defaults: all of shared memory.  The smaller settings
-// (5 / 1 / 4: ~193 KB, leaving room for CTAs of a light kernel of another stream beside the persistent GEMM CTA) were measured
-// together with two pose chunks in flight on two streams (MplDesc.chunk_streams = 2): no gain, see profiles/r2_experiments.md.
+// Shared-memory budget of the LayerNorm-fused bf16 kernels.  Defaults: all of shared memory.  The smaller settings (5 / 1 / 4:
+// ~193 KB, room for CTAs of a light kernel beside the persistent GEMM CTA) were measured with an experimental schedule, since
+// removed, that ran two pose chunks on two streams: no gain, see profiles/r2_experiments.md.
 #ifndef MPL_LN_STAGES
 #define MPL_LN_STAGES 6      // QKV / fc1 operand stages
 #endif
@@ -53,13 +54,13 @@ constexpr int UMMA_K_BYTES = 32; // bytes of K per tcgen05.mma
 constexpr int NUM_EPI_WARPS = 8;   // two per TMEM lane quarter: even / odd 64-column groups
 constexpr int TMEM_COLS = 512;
 
-template <int CG, int EPI = 0, int KIND = 0>
+template <int EPI = 0, int KIND = 0>
 struct Cfg {
   static constexpr int OPS = (KIND == 1) ? 2 : 1;           // operand planes per matrix (split mode: hi + lo)
   static constexpr int A_BYTES = BM * KB_BYTES;             // 16 KB
   static constexpr int B_ROWS = BN / CG;                    // W rows staged per CTA
-  static constexpr int B_BYTES = B_ROWS * KB_BYTES;         // 32 KB / 16 KB
-  static constexpr int STAGE_BYTES = OPS * (A_BYTES + B_BYTES);  // 48 KB / 32 KB (split: 96 KB / 64 KB)
+  static constexpr int B_BYTES = B_ROWS * KB_BYTES;         // 16 KB
+  static constexpr int STAGE_BYTES = OPS * (A_BYTES + B_BYTES);  // 32 KB (split: 64 KB)
   // The residual-emit epilogues keep the old residual in TMA-fed shared-memory slots of 8 KB (a 32-row x 64-column box of each
   // bf16 plane) that are updated in place and stored back from the same slot.  Slots are PRIVATE to an epilogue warp (its
   // mbarrier phases are then observed in order by construction -- a shared ring lets a warp wait for generation n + 1 of a
@@ -70,9 +71,10 @@ struct Cfg {
   static constexpr bool RESID = (KIND == 0) && (EPI == 6 || EPI == 7);
   static constexpr int EPI_WARPS = NUM_EPI_WARPS;
   static constexpr int THREADS = (4 + EPI_WARPS) * 32;
-  // Register cap.  The LayerNorm-fused bf16 kernels (the bench path) need no more than 112 registers (no spills): 42 k of the
-  // SM's 64 k, which leaves room for CTAs of a light kernel from another stream beside the persistent GEMM CTA; the other
-  // instantiations take what a single CTA per SM may use.
+  // Register cap.  The LayerNorm-fused bf16 kernels (the bench path) need no more than 112 registers (no spills).  The cap
+  // (42 k of the SM's 64 k) was set for a since removed two-stream chunk schedule, to leave room for CTAs of a light kernel
+  // beside the persistent GEMM CTA, and is kept because the shipped build is measured with it.  The other instantiations
+  // take what a single CTA per SM may use.
 #ifndef MPL_LN_MAXREG
 #define MPL_LN_MAXREG 112
 #endif
@@ -81,9 +83,7 @@ struct Cfg {
   static constexpr int RING_SLOTS = !RESID ? 0 : 4 * SLOTS_EVEN + 4;
   static constexpr int SLOT_BYTES = 8192;
   static constexpr int RING_BYTES = RING_SLOTS * SLOT_BYTES;
-  static constexpr int STAGES = (KIND == 1) ? ((CG == 1) ? 2 : 3)
-                                : (EPI == 6) ? ((CG == 1) ? 2 : 4) : (EPI == 7) ? ((CG == 1) ? 3 : MPL_E7_STAGES)
-                                : ((CG == 1) ? 4 : (EPI >= 4 ? MPL_LN_STAGES : 6));
+  static constexpr int STAGES = (KIND == 1) ? 3 : (EPI == 6) ? 4 : (EPI == 7) ? MPL_E7_STAGES : (EPI >= 4 ? MPL_LN_STAGES : 6);
   static constexpr int STAGING_BYTES = RESID ? 0 : EPI_WARPS * 4096;  // per epilogue warp: one 32-row x 128-byte output box
   // slot and mbarrier phase of the n-th residual box (n = 0, 1, ...) of epilogue warp (lane quarter q, group parity `odd`)
   static constexpr uint32_t SE = SLOTS_EVEN ? SLOTS_EVEN : 1;
@@ -234,15 +234,15 @@ __device__ __forceinline__ void stage_row_f16(uint32_t box, int lane, int j0, co
   }
 }
 
-template <int CG, int KIND, int EPI>
-__global__ void __maxnreg__((Cfg<CG, EPI, KIND>::MAXREG))
+template <int KIND, int EPI>
+__global__ void __maxnreg__((Cfg<EPI, KIND>::MAXREG))
 gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                     const __grid_constant__ CUtensorMap tmY, const __grid_constant__ CUtensorMap tmA2,
                     const __grid_constant__ CUtensorMap tmB2, const __grid_constant__ CUtensorMap tmY2,
                     const float* __restrict__ bias, int64_t M, int N, int K, const TileSplit ts, const GemmLn ln) {
   // tmA2 / tmY2: the lo planes of the split mode (KIND 1) and of the residual stream (EPI 6 / 7).  tmB2: the lo plane of W in
   // split mode; otherwise the W box of the narrow tiles (q groups; tmB serves the wide ones, q + 1 groups)
-  using C = Cfg<CG, EPI, KIND>;
+  using C = Cfg<EPI, KIND>;
   constexpr bool SPLIT = (KIND == 1);
   constexpr bool RESID = C::RESID;
   constexpr int BK = KB_BYTES / 2;  // K elements per stage (16-bit operands)
@@ -265,7 +265,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
       smem_gen + C::STAGES * C::STAGE_BYTES + C::STAGING_BYTES + C::RING_BYTES + 8 * (2 * C::STAGES + 4));
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const uint32_t cta_rank = (CG == 2) ? ptx::cluster_ctarank() : 0u;
+  const uint32_t cta_rank = ptx::cluster_ctarank();
   const bool is_leader = cta_rank == 0;
 
   if (warp == 0 && lane == 0) {
@@ -294,11 +294,11 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
     ptx::fence_barrier_init();
   }
   if (warp == 2) {
-    ptx::tmem_alloc<CG>(tmem_slot, TMEM_COLS);
-    ptx::tmem_relinquish<CG>();
+    ptx::tmem_alloc(tmem_slot, TMEM_COLS);
+    ptx::tmem_relinquish();
   }
   ptx::tc_fence_before();
-  if constexpr (CG == 2) ptx::cluster_sync(); else __syncthreads();
+  ptx::cluster_sync();
   ptx::tc_fence_after();
   const uint32_t tmem_base = *tmem_slot_ptr;
 
@@ -317,7 +317,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
     if (lane == 0) {
       int stage = 0;
       uint32_t phase = 0;
-      const uint32_t leader_full0 = (CG == 2) ? ptx::mapa(full_bar(0), 0) : 0u;
+      const uint32_t leader_full0 = ptx::mapa(full_bar(0), 0);
       for (int64_t tile = first_tile; tile < total_tiles; tile += tile_stride) {
         const int64_t m_blk = tile / n_tiles;
         const int n_blk = (int)(tile % n_tiles);
@@ -343,24 +343,14 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
           ptx::mbar_wait(empty_bar(stage), phase ^ 1u);
           const uint32_t a_dst = smem_base + stage * C::STAGE_BYTES;  // [A hi][A lo][W hi][W lo] in split mode
           const uint32_t b_dst = a_dst + C::OPS * C::A_BYTES;
-          if constexpr (CG == 1) {
-            ptx::mbar_arrive_expect_tx(full_bar(stage), stage_tx);
-            ptx::tma_load_2d(a_dst, &tmA, full_bar(stage), kb * BK, m0);
-            ptx::tma_load_2d(b_dst, tb, full_bar(stage), kb * BK, n0);
-            if constexpr (SPLIT) {
-              ptx::tma_load_2d(a_dst + C::A_BYTES, &tmA2, full_bar(stage), kb * BK, m0);
-              ptx::tma_load_2d(b_dst + C::B_BYTES, &tmB2, full_bar(stage), kb * BK, n0);
-            }
-          } else {
-            const uint32_t lbar = leader_full0 + 8u * stage;
-            // the peer's bytes may land before this expect_tx: the phase still cannot complete without this arrive
-            if (is_leader) ptx::mbar_arrive_expect_tx(full_bar(stage), 2 * stage_tx);
-            ptx::tma_load_2d_pair(a_dst, &tmA, lbar, kb * BK, m0);
-            ptx::tma_load_2d_pair(b_dst, tb, lbar, kb * BK, n0);
-            if constexpr (SPLIT) {
-              ptx::tma_load_2d_pair(a_dst + C::A_BYTES, &tmA2, lbar, kb * BK, m0);
-              ptx::tma_load_2d_pair(b_dst + C::B_BYTES, &tmB2, lbar, kb * BK, n0);
-            }
+          const uint32_t lbar = leader_full0 + 8u * stage;
+          // the peer's bytes may land before this expect_tx: the phase still cannot complete without this arrive
+          if (is_leader) ptx::mbar_arrive_expect_tx(full_bar(stage), 2 * stage_tx);
+          ptx::tma_load_2d_pair(a_dst, &tmA, lbar, kb * BK, m0);
+          ptx::tma_load_2d_pair(b_dst, tb, lbar, kb * BK, n0);
+          if constexpr (SPLIT) {
+            ptx::tma_load_2d_pair(a_dst + C::A_BYTES, &tmA2, lbar, kb * BK, m0);
+            ptx::tma_load_2d_pair(b_dst + C::B_BYTES, &tmB2, lbar, kb * BK, n0);
           }
           if (++stage == C::STAGES) { stage = 0; phase ^= 1u; }
         }
@@ -401,19 +391,15 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
                 // small cross terms first, the hi.hi product last (the lo.lo term, 2^-18 relative, is dropped)
                 const uint64_t adesc2 = adesc + (uint64_t)(C::A_BYTES >> 4);
                 const uint64_t bdesc2 = bdesc + (uint64_t)(C::B_BYTES >> 4);
-                ptx::umma<CG, 0>(d_tmem, adesc, bdesc2, idesc, (kb | k) != 0 ? 1u : 0u);
-                ptx::umma<CG, 0>(d_tmem, adesc2, bdesc, idesc, 1u);
-                ptx::umma<CG, 0>(d_tmem, adesc, bdesc, idesc, 1u);
+                ptx::umma<0>(d_tmem, adesc, bdesc2, idesc, (kb | k) != 0 ? 1u : 0u);
+                ptx::umma<0>(d_tmem, adesc2, bdesc, idesc, 1u);
+                ptx::umma<0>(d_tmem, adesc, bdesc, idesc, 1u);
               } else {
-                ptx::umma<CG, 0>(d_tmem, adesc, bdesc, idesc, (kb | k) != 0 ? 1u : 0u);
+                ptx::umma<0>(d_tmem, adesc, bdesc, idesc, (kb | k) != 0 ? 1u : 0u);
               }
             }
-            if constexpr (CG == 1) ptx::umma_commit(empty_bar(stage));
-            else ptx::umma_commit_pair(empty_bar(stage), 0x3);
-            if (kb == num_kb - 1) {
-              if constexpr (CG == 1) ptx::umma_commit(tfull_bar(acc));
-              else ptx::umma_commit_pair(tfull_bar(acc), 0x3);
-            }
+            ptx::umma_commit_pair(empty_bar(stage), 0x3);
+            if (kb == num_kb - 1) ptx::umma_commit_pair(tfull_bar(acc), 0x3);
           }
           __syncwarp();
           if (++stage == C::STAGES) { stage = 0; phase ^= 1u; }
@@ -466,7 +452,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
     const uint32_t box = staging_base + (uint32_t)(warp - 4) * 4096u;
     int acc = 0;
     uint32_t acc_phase = 0;
-    const uint32_t leader_tempty0 = (CG == 2) ? ptx::mapa(tempty_bar(0), 0) : 0u;
+    const uint32_t leader_tempty0 = ptx::mapa(tempty_bar(0), 0);
     uint32_t box_count = 0;  // RESID: residual boxes this warp has consumed so far (selects its slot and mbarrier phase)
     int held_slot = -1;      // RESID: slot whose TMA stores may still be reading shared memory
     for (int64_t tile = first_tile; tile < total_tiles; tile += tile_stride) {
@@ -583,10 +569,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
         ln.stats_out[(2 * n_blk + half) * ln.stats_ld + my_row] = make_float2(s1.x + s1.y, s2.x + s2.y);
         ptx::tc_fence_before();
         __syncwarp();
-        if (lane == 0) {
-          if constexpr (CG == 1) ptx::mbar_arrive(tempty_bar(acc));
-          else ptx::mbar_arrive_cluster(leader_tempty0 + 8u * acc);
-        }
+        if (lane == 0) ptx::mbar_arrive_cluster(leader_tempty0 + 8u * acc);
         if (++acc == 2) { acc = 0; acc_phase ^= 1u; }
         continue;
       }
@@ -596,7 +579,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
       for (int c = half * 64; c < n_size; c += 128) {
         if constexpr (OUT_BF16) {
           // one 64-column bf16 box per step, filled in two 32-column halves (one accumulator chunk in registers at a time:
-          // ~100 registers per thread, which leaves room for CTAs of other kernels on the SM -- see mpl_forward)
+          // ~100 registers per thread, see Cfg::MAXREG)
           constexpr bool GELU = (EPI == 1 || EPI == 5);
           const bool f16_out = (ln.flags & 4) != 0;
           if (lane == 0) ptx::bulk_wait_read<0>();  // the previous store has finished reading the box
@@ -668,10 +651,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
       }
       ptx::tc_fence_before();
       __syncwarp();
-      if (lane == 0) {
-        if constexpr (CG == 1) ptx::mbar_arrive(tempty_bar(acc));
-        else ptx::mbar_arrive_cluster(leader_tempty0 + 8u * acc);
-      }
+      if (lane == 0) ptx::mbar_arrive_cluster(leader_tempty0 + 8u * acc);
       if (++acc == 2) { acc = 0; acc_phase ^= 1u; }
     }
     if (lane == 0) ptx::bulk_wait_all();  // every output tile has landed before the CTA retires
@@ -679,10 +659,10 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
   }
 
   ptx::tc_fence_before();
-  if constexpr (CG == 2) ptx::cluster_sync(); else __syncthreads();
+  ptx::cluster_sync();
   if (warp == 2) {
     ptx::tc_fence_after();
-    ptx::tmem_dealloc<CG>(tmem_base, TMEM_COLS);
+    ptx::tmem_dealloc(tmem_base, TMEM_COLS);
   }
 }
 
@@ -783,8 +763,8 @@ qkv_attn_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
     ptx::fence_barrier_init();
   }
   if (warp == 2) {
-    ptx::tmem_alloc<2>(tmem_slot, TMEM_COLS);
-    ptx::tmem_relinquish<2>();
+    ptx::tmem_alloc(tmem_slot, TMEM_COLS);
+    ptx::tmem_relinquish();
   }
   ptx::tc_fence_before();
   ptx::cluster_sync();
@@ -845,9 +825,9 @@ qkv_attn_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
             for (int k = 0; k < KB_BYTES / UMMA_K_BYTES; ++k) {
 #pragma unroll
               for (int u = 0; u < 2; ++u)  // W rows [104 u, 104 u + 104) of both CTAs = accumulator columns [208 u, 208 u + 208)
-                ptx::umma<2, 0>(tmem_base + (uint32_t)(u * FA_UW), adesc0 + (uint64_t)(k * (UMMA_K_BYTES >> 4)),
-                                bdesc0 + (uint64_t)(k * (UMMA_K_BYTES >> 4) + u * ((FA_UW / 2 * KB_BYTES) >> 4)), idesc,
-                                (kb | k) != 0 ? 1u : 0u);
+                ptx::umma<0>(tmem_base + (uint32_t)(u * FA_UW), adesc0 + (uint64_t)(k * (UMMA_K_BYTES >> 4)),
+                             bdesc0 + (uint64_t)(k * (UMMA_K_BYTES >> 4) + u * ((FA_UW / 2 * KB_BYTES) >> 4)), idesc,
+                             (kb | k) != 0 ? 1u : 0u);
             }
             ptx::umma_commit_pair(empty_bar(stage), 0x3);
             if (kb == num_kb - 1) ptx::umma_commit_pair(tfull_bar, 0x3);
@@ -1083,7 +1063,7 @@ qkv_attn_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
   ptx::cluster_sync();
   if (warp == 2) {
     ptx::tc_fence_after();
-    ptx::tmem_dealloc<2>(tmem_base, TMEM_COLS);
+    ptx::tmem_dealloc(tmem_base, TMEM_COLS);
   }
 }
 
@@ -1175,11 +1155,11 @@ struct GemmMaps {
   CUtensorMap a, b, y, a2, b2, y2;
 };
 
-template <int CG, int KIND, int EPI>
+template <int KIND, int EPI>
 int launch_one(const GemmMaps& tm, const float* bias, int64_t M, int N, int K, const TileSplit& ts, const GemmLn& ln,
                cudaStream_t s) {
-  using C = Cfg<CG, EPI, KIND>;
-  auto kern = gemm_tcgen05_kernel<CG, KIND, EPI>;
+  using C = Cfg<EPI, KIND>;
+  auto kern = gemm_tcgen05_kernel<KIND, EPI>;
   // per instantiation and device (function attributes live in the device's context); a benign race: two threads may both set it
   static std::atomic<unsigned char> attr_set[64];
   int dev = 0;
@@ -1208,22 +1188,22 @@ int launch_one(const GemmMaps& tm, const float* bias, int64_t M, int N, int K, c
   return MPL_OK;
 }
 
-template <int CG, int KIND>
+template <int KIND>
 int launch_epi(int epi, const GemmMaps& tm, const float* bias, int64_t M, int N, int K, const TileSplit& bn, const GemmLn& ln,
                cudaStream_t s) {
   switch (epi) {
-    case 0: return launch_one<CG, KIND, 0>(tm, bias, M, N, K, bn, ln, s);
-    case 1: return launch_one<CG, KIND, 1>(tm, bias, M, N, K, bn, ln, s);
-    case 2: return launch_one<CG, KIND, 2>(tm, bias, M, N, K, bn, ln, s);
-    case 3: return launch_one<CG, KIND, 3>(tm, bias, M, N, K, bn, ln, s);
+    case 0: return launch_one<KIND, 0>(tm, bias, M, N, K, bn, ln, s);
+    case 1: return launch_one<KIND, 1>(tm, bias, M, N, K, bn, ln, s);
+    case 2: return launch_one<KIND, 2>(tm, bias, M, N, K, bn, ln, s);
+    case 3: return launch_one<KIND, 3>(tm, bias, M, N, K, bn, ln, s);
     default: break;
   }
   if constexpr (KIND == 0) {  // the LayerNorm-fused epilogues exist for single-plane bf16 / fp16 operands only
     switch (epi) {
-      case 4: return launch_one<CG, KIND, 4>(tm, bias, M, N, K, bn, ln, s);
-      case 5: return launch_one<CG, KIND, 5>(tm, bias, M, N, K, bn, ln, s);
-      case 6: return launch_one<CG, KIND, 6>(tm, bias, M, N, K, bn, ln, s);
-      case 7: return launch_one<CG, KIND, 7>(tm, bias, M, N, K, bn, ln, s);
+      case 4: return launch_one<KIND, 4>(tm, bias, M, N, K, bn, ln, s);
+      case 5: return launch_one<KIND, 5>(tm, bias, M, N, K, bn, ln, s);
+      case 6: return launch_one<KIND, 6>(tm, bias, M, N, K, bn, ln, s);
+      case 7: return launch_one<KIND, 7>(tm, bias, M, N, K, bn, ln, s);
       default: break;
     }
   }
@@ -1330,7 +1310,7 @@ bool gemm_tcgen05_supports(int N, int K, int dtype) {
 int gemm_ln_slots(int N) { return 2 * split_tiles(N).T; }  // one slot per (tile, epilogue warp of a lane quarter)
 
 int launch_gemm_tcgen05(const void* A, const void* W, const float* bias, void* Y, int64_t M, int N, int K, int dtype,
-                        int epilogue, int out_fp32, cudaStream_t s, const GemmLnArgs* lnargs, int cta_group) {
+                        int epilogue, int out_fp32, cudaStream_t s, const GemmLnArgs* lnargs) {
   if (M == 0) return MPL_OK;
   GemmLn ln{};
   if (epilogue >= EPI_LN_BIAS) {
@@ -1368,7 +1348,6 @@ int launch_gemm_tcgen05(const void* A, const void* W, const float* bias, void* Y
     set_error("launch_gemm_tcgen05: bias must not be null");
     return MPL_ERR_INVALID_ARGUMENT;
   }
-  const int cg = (cta_group == 1) ? 1 : 2;  // CTA pairs by default: half the operand traffic per SM (measured faster on every FPT shape)
   const bool split = dtype == MPL_PREC_TF32;  // the fp32-grade mode: operands are two bf16 planes (hi, lo), [2][rows][K]
   int epi = epilogue;
   if (epilogue == EPI_BIAS && out_fp32) epi = 3;
@@ -1379,7 +1358,7 @@ int launch_gemm_tcgen05(const void* A, const void* W, const float* bias, void* Y
   const bool resid = epi == 6 || epi == 7;
   const bool out_bf16 = epi == 0 || epi == 1 || epi == 4 || epi == 5 || resid;
   const TileSplit ts = split_tiles(N);
-  const int wide_rows = 64 * (ts.q + (ts.r > 0 ? 1 : 0)) / cg, narrow_rows = 64 * ts.q / cg;
+  const int wide_rows = 64 * (ts.q + (ts.r > 0 ? 1 : 0)) / CG, narrow_rows = 64 * ts.q / CG;
   GemmMaps tm;
   MPL_TRY(make_tmap(&tm.a, A, M, K, 2, BM));
   MPL_TRY(make_tmap(&tm.b, W, N, K, 2, wide_rows));
@@ -1399,10 +1378,7 @@ int launch_gemm_tcgen05(const void* A, const void* W, const float* bias, void* Y
     MPL_TRY(make_tmap(&tm.b2, W, N, K, 2, narrow_rows));  // the W box of the narrow tiles
     if (resid) MPL_TRY(make_tmap(&tm.y2, lnargs->x_lo, M, N, 2, 32, 64, true, ldy));  // Y = the hi plane, x_lo = the lo plane
   }
-  if (cg == 1) {
-    return split ? launch_epi<1, 1>(epi, tm, bias, M, N, K, ts, ln, s) : launch_epi<1, 0>(epi, tm, bias, M, N, K, ts, ln, s);
-  }
-  return split ? launch_epi<2, 1>(epi, tm, bias, M, N, K, ts, ln, s) : launch_epi<2, 0>(epi, tm, bias, M, N, K, ts, ln, s);
+  return split ? launch_epi<1>(epi, tm, bias, M, N, K, ts, ln, s) : launch_epi<0>(epi, tm, bias, M, N, K, ts, ln, s);
 }
 
 }  // namespace mpl

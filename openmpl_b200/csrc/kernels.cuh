@@ -156,9 +156,8 @@ int gemm_ln_slots(int N);
 // "split" mode): every matrix is TWO bf16 planes, [2][rows][K] = hi = bf16(x) then lo = bf16(x - hi), and the kernel
 // accumulates hi.hi + hi.lo + lo.hi.  EPI_BIAS / EPI_BIAS_GELU write Y [M,N] in the operand format (bf16, or two planes
 // [2][M][N]) or fp32 if out_fp32; EPI_BIAS_RESIDUAL does Y(fp32) += A W^T + bias in place.
-// cta_group: 1 = one CTA per 128 x 256 tile, anything else = CTA pairs per 256 x 256 tile (the default).
 int launch_gemm_tcgen05(const void* A, const void* W, const float* bias, void* Y, int64_t M, int N, int K, int dtype,
-                        int epilogue, int out_fp32, cudaStream_t s, const GemmLnArgs* ln = nullptr, int cta_group = 2);
+                        int epilogue, int out_fp32, cudaStream_t s, const GemmLnArgs* ln = nullptr);
 bool gemm_tcgen05_supports(int N, int K, int dtype);
 
 // QKV projection + cross-view attention fused (bf16 mode, LayerNorm folded; D = H * 136 or H * 68 with H even, 2 <= V <= 8): att [M, D] bf16 straight

@@ -75,7 +75,6 @@ struct MplModel {
   bool qkv_attn;      // bf16 LN-fused mode, view tokens, D = H * 136 (or H * 68), 2 <= V <= 8: QKV GEMM + cross-view attention are one kernel
   bool fpt_kp_fused;  // bf16 mode, keypoint-token FPT (width 32, 8 heads, J = 17): the whole FPT stack is one kernel launch
   int ln_slots;    // statistics slots per row written by the residual-emit GEMMs
-  int cta_group;   // 1: one CTA per 128 x 256 GEMM tile, 2: CTA pairs per 256 x 256 tile (default)
   std::vector<ParamInfo> params;
   std::unordered_map<std::string, int> index;
   std::vector<Derived> derived;
@@ -98,10 +97,6 @@ struct MplModel {
     uint64_t last_used;
   };
   std::vector<GraphEntry> graphs;
-  // large batches: two pose chunks in flight on two internal streams (see plan_chunks)
-  int chunk_streams = 1;
-  cudaStream_t lane_stream[2] = {nullptr, nullptr};
-  cudaEvent_t ev_fork = nullptr, ev_join[2] = {nullptr, nullptr};
   int64_t graph_max_batch = 0;   // 0: off (mpl_set_graph_batch)
   cudaStream_t cap_stream = nullptr;
   uint64_t graph_clock = 0;
@@ -111,7 +106,6 @@ struct MplModel {
   std::vector<mpl::BlockW> fpt_blocks;
   // optional per-launch CUDA-event profiling (bench.py's roofline numbers come from here)
   bool profile = false;
-  bool profile_serial = false;  // profiling with one chunk at a time: per-launch times that add up to the step
   struct ProfRec { int cat; cudaEvent_t e0, e1; };
   std::vector<ProfRec> prof;
   std::vector<cudaEvent_t> ev_pool;
@@ -492,7 +486,6 @@ static int block_tc(MplModel* m, const BlockW& w, float* x, int64_t rows, int64_
                     void* xn, void* xl, void* qkv, void* att, void* hid, void* stats, bool last, cudaStream_t s) {
   const int prec = m->d.precision;
   const int hd = C / m->H;
-  const int cg = m->cta_group;
   if (m->ln_fused) {
     // The residual stream lives in two bf16 planes: xn = hi (also the A operand of QKV / fc1), xl = lo; `stats` holds its
     // per-row (sum, sum^2) partials.  All three are rewritten by every residual-emit epilogue (launch_ln_prep makes them from
@@ -509,41 +502,41 @@ static int block_tc(MplModel* m, const BlockW& w, float* x, int64_t rows, int64_
       LC(CAT_FPT_QKV, launch_qkv_attn(xn, w.qa_w, w.qa_b, w.qa_cs, stats, m->ln_slots, 1e-6f, att, rows, C, m->H, N, s));
     } else {
       app.colsum = w.qkv_cs;
-      LC(CAT_FPT_QKV, launch_gemm_tcgen05(xn, w.qkvw_tc, w.qkv_bf, qkv, rows, 3 * C, C, prec, EPI_LN_BIAS, 0, s, &app, cg));
+      LC(CAT_FPT_QKV, launch_gemm_tcgen05(xn, w.qkvw_tc, w.qkv_bf, qkv, rows, 3 * C, C, prec, EPI_LN_BIAS, 0, s, &app));
       LC(CAT_FPT_ATTN, launch_attention_bf16((const __nv_bfloat16*)qkv, (__nv_bfloat16*)att, sets, N, m->H, hd, scale, s));
     }
-    LC(CAT_FPT_PROJ, launch_gemm_tcgen05(att, w.projw_tc, w.projb, xn, rows, C, C, prec, EPI_RESIDUAL_EMIT, 0, s, &emit, cg));
+    LC(CAT_FPT_PROJ, launch_gemm_tcgen05(att, w.projw_tc, w.projb, xn, rows, C, C, prec, EPI_RESIDUAL_EMIT, 0, s, &emit));
     app.colsum = w.fc1_cs;
     app.out_fp16 = 1;   // hidden activations in fp16 (GELU in packed half2), fc2 runs kind::f16 on fp16 operands
-    LC(CAT_FPT_FC1, launch_gemm_tcgen05(xn, w.fc1w_tc, w.fc1_bf, hid, rows, hidden, C, prec, EPI_LN_BIAS_GELU, 0, s, &app, cg));
+    LC(CAT_FPT_FC1, launch_gemm_tcgen05(xn, w.fc1w_tc, w.fc1_bf, hid, rows, hidden, C, prec, EPI_LN_BIAS_GELU, 0, s, &app));
     emit.ab_fp16 = 1;
     // channel-permuted stream: the head reads the first E = J * d channels only, so the last fc2 of the stack leaves the ray
     // half of the residual as it is (half the MMAs, half the residual traffic of that launch)
     const int n_fc2 = (last && m->perm) ? m->E : C;
     emit.ldy = C;
-    LC(CAT_FPT_FC2, launch_gemm_tcgen05(hid, w.fc2w_tc, w.fc2b, xn, rows, n_fc2, hidden, prec, EPI_RESIDUAL_EMIT, 0, s, &emit, cg));
+    LC(CAT_FPT_FC2, launch_gemm_tcgen05(hid, w.fc2w_tc, w.fc2b, xn, rows, n_fc2, hidden, prec, EPI_RESIDUAL_EMIT, 0, s, &emit));
     return MPL_OK;
   }
   if (prec == MPL_PREC_BF16) {
     LC(CAT_FPT_LN, launch_layernorm_bf16(x, C, w.n1w, w.n1b, 1e-6f, (__nv_bfloat16*)xn, C, rows, C, s));
-    LC(CAT_FPT_QKV, launch_gemm_tcgen05(xn, w.qkvw_tc, w.qkvb, qkv, rows, 3 * C, C, prec, EPI_BIAS, 0, s, nullptr, cg));
+    LC(CAT_FPT_QKV, launch_gemm_tcgen05(xn, w.qkvw_tc, w.qkvb, qkv, rows, 3 * C, C, prec, EPI_BIAS, 0, s, nullptr));
     LC(CAT_FPT_ATTN, launch_attention_bf16((const __nv_bfloat16*)qkv, (__nv_bfloat16*)att, sets, N, m->H, hd, scale, s));
-    LC(CAT_FPT_PROJ, launch_gemm_tcgen05(att, w.projw_tc, w.projb, x, rows, C, C, prec, EPI_BIAS_RESIDUAL, 1, s, nullptr, cg));
+    LC(CAT_FPT_PROJ, launch_gemm_tcgen05(att, w.projw_tc, w.projb, x, rows, C, C, prec, EPI_BIAS_RESIDUAL, 1, s, nullptr));
     LC(CAT_FPT_LN, launch_layernorm_bf16(x, C, w.n2w, w.n2b, 1e-6f, (__nv_bfloat16*)xn, C, rows, C, s));
-    LC(CAT_FPT_FC1, launch_gemm_tcgen05(xn, w.fc1w_tc, w.fc1b, hid, rows, hidden, C, prec, EPI_BIAS_GELU, 0, s, nullptr, cg));
-    LC(CAT_FPT_FC2, launch_gemm_tcgen05(hid, w.fc2w_tc, w.fc2b, x, rows, C, hidden, prec, EPI_BIAS_RESIDUAL, 1, s, nullptr, cg));
+    LC(CAT_FPT_FC1, launch_gemm_tcgen05(xn, w.fc1w_tc, w.fc1b, hid, rows, hidden, C, prec, EPI_BIAS_GELU, 0, s, nullptr));
+    LC(CAT_FPT_FC2, launch_gemm_tcgen05(hid, w.fc2w_tc, w.fc2b, x, rows, C, hidden, prec, EPI_BIAS_RESIDUAL, 1, s, nullptr));
   } else {
     // split planes: xn / att [2][rows][C], hid [2][rows][hidden] bf16; qkv [rows][3C] fp32 (the attention arithmetic is fp32).
     // xn is free between the QKV GEMM and the second LayerNorm: it doubles as the fp32 scratch of the attention fallback.
     __nv_bfloat16* xnp = (__nv_bfloat16*)xn;
     __nv_bfloat16* attp = (__nv_bfloat16*)att;
     LC(CAT_FPT_LN, launch_layernorm_split(x, C, w.n1w, w.n1b, 1e-6f, xnp, C, rows * C, rows, C, s));
-    LC(CAT_FPT_QKV, launch_gemm_tcgen05(xn, w.qkvw_tc, w.qkvb, qkv, rows, 3 * C, C, prec, EPI_BIAS, 1, s, nullptr, cg));
+    LC(CAT_FPT_QKV, launch_gemm_tcgen05(xn, w.qkvw_tc, w.qkvb, qkv, rows, 3 * C, C, prec, EPI_BIAS, 1, s, nullptr));
     LC(CAT_FPT_ATTN, launch_attention_split((const float*)qkv, attp, rows * C, (float*)xn, sets, N, m->H, hd, scale, s));
-    LC(CAT_FPT_PROJ, launch_gemm_tcgen05(att, w.projw_tc, w.projb, x, rows, C, C, prec, EPI_BIAS_RESIDUAL, 1, s, nullptr, cg));
+    LC(CAT_FPT_PROJ, launch_gemm_tcgen05(att, w.projw_tc, w.projb, x, rows, C, C, prec, EPI_BIAS_RESIDUAL, 1, s, nullptr));
     LC(CAT_FPT_LN, launch_layernorm_split(x, C, w.n2w, w.n2b, 1e-6f, xnp, C, rows * C, rows, C, s));
-    LC(CAT_FPT_FC1, launch_gemm_tcgen05(xn, w.fc1w_tc, w.fc1b, hid, rows, hidden, C, prec, EPI_BIAS_GELU, 0, s, nullptr, cg));
-    LC(CAT_FPT_FC2, launch_gemm_tcgen05(hid, w.fc2w_tc, w.fc2b, x, rows, C, hidden, prec, EPI_BIAS_RESIDUAL, 1, s, nullptr, cg));
+    LC(CAT_FPT_FC1, launch_gemm_tcgen05(xn, w.fc1w_tc, w.fc1b, hid, rows, hidden, C, prec, EPI_BIAS_GELU, 0, s, nullptr));
+    LC(CAT_FPT_FC2, launch_gemm_tcgen05(hid, w.fc2w_tc, w.fc2b, x, rows, C, hidden, prec, EPI_BIAS_RESIDUAL, 1, s, nullptr));
   }
   return MPL_OK;
 }
@@ -806,8 +799,12 @@ int mpl_create(const MplDesc* desc, MplModel** out) {
     set_error("mpl_create: unknown precision %d", desc->precision);
     return MPL_ERR_INVALID_ARGUMENT;
   }
-  if (desc->gemm_cta_group < 0 || desc->gemm_cta_group > 2) {
-    set_error("mpl_create: gemm_cta_group must be 0 (default), 1 or 2");
+  if (desc->gemm_cta_group != 0 && desc->gemm_cta_group != 2) {
+    set_error("mpl_create: gemm_cta_group must be 0 or 2 (CTA pairs), got %d", desc->gemm_cta_group);
+    return MPL_ERR_INVALID_ARGUMENT;
+  }
+  if (desc->chunk_streams != 0 && desc->chunk_streams != 1) {
+    set_error("mpl_create: chunk_streams must be 0 or 1 (the caller's stream), got %d", desc->chunk_streams);
     return MPL_ERR_INVALID_ARGUMENT;
   }
   *out = nullptr;
@@ -858,10 +855,8 @@ int mpl_create(const MplDesc* desc, MplModel** out) {
   }
   // LayerNorm fusion: the residual-emit epilogue works on whole 32-column chunks, launch_ln_prep on float4 rows
   m->ln_fused = m->fpt_tc && d.precision == MPL_PREC_BF16 && d.ln_fusion != 0 && m->fpt_dim % 32 == 0 && m->fpt_dim <= 32 * 4 * 17;
-  m->cta_group = (d.gemm_cta_group == 1) ? 1 : 2;
-  m->chunk_streams = (d.chunk_streams == 2) ? 2 : 1;
   m->ln_slots = m->ln_fused ? gemm_ln_slots(m->fpt_dim) : 0;
-  m->qkv_attn = m->ln_fused && d.qkv_attn_fusion != 0 && m->cta_group == 2 && qkv_attn_supports(m->fpt_dim, m->H, m->fpt_tokens);
+  m->qkv_attn = m->ln_fused && d.qkv_attn_fusion != 0 && qkv_attn_supports(m->fpt_dim, m->H, m->fpt_tokens);
   {
     // channel-permuted residual stream (see MplModel::perm): every producer and consumer of the planes must be one that
     // knows the permutation -- the SPT epilogue, the LN-fused GEMMs and the K5 head reading the planes
@@ -888,11 +883,6 @@ void mpl_destroy(MplModel* m) {
   if (m == nullptr) return;
   for (auto& e : m->graphs) cudaGraphExecDestroy(e.exec);
   if (m->cap_stream) cudaStreamDestroy(m->cap_stream);
-  for (int k = 0; k < 2; ++k) {
-    if (m->lane_stream[k]) cudaStreamDestroy(m->lane_stream[k]);
-    if (m->ev_join[k]) cudaEventDestroy(m->ev_join[k]);
-  }
-  if (m->ev_fork) cudaEventDestroy(m->ev_fork);
   for (cudaEvent_t e : m->ev_pool) cudaEventDestroy(e);
   delete m;
 }
@@ -903,7 +893,6 @@ int mpl_set_profile(MplModel* m, int enabled) {
     return MPL_ERR_INVALID_ARGUMENT;
   }
   m->profile = enabled != 0;
-  m->profile_serial = enabled == 2;  // 2: also run the chunks one after the other (times that add up); 1: as in production
   m->prof.clear();
   m->ev_used = 0;
   return MPL_OK;
@@ -1099,30 +1088,10 @@ int mpl_set_chunk_poses(MplModel* m, int64_t chunk) {
   return MPL_OK;
 }
 
-// How a batch is cut into chunks.  Every pose is independent, so a batch may be processed in any number of chunks without
-// changing a result.  Large batches run as TWO interleaved chunk sequences on two internal streams: while one chunk is
-// inside a tensor-bound GEMM (one persistent CTA per SM, registers and shared memory capped so that more fits), the HBM-bound
-// kernels of the other chunk (view attention, ln_prep, head) become resident beside it, and the next GEMM's CTAs start on
-// SMs the previous one has already left -- the tail of every launch overlaps the head of the next.
-constexpr int64_t kDualMinBatch = 16384;
-struct ChunkPlan {
-  int64_t chunk;
-  int lanes;
-};
-static ChunkPlan plan_chunks(const MplModel* m, int64_t batch) {
-  ChunkPlan p{std::min<int64_t>(std::max<int64_t>(batch, 1), m->chunk), 1};
-  if (m->chunk_streams == 2 && batch >= kDualMinBatch && !m->profile_serial) {
-    if (batch <= m->chunk) p.chunk = (batch + 1) / 2;  // one chunk's worth of poses: two halves
-    p.lanes = 2;
-  }
-  return p;
-}
-
 size_t mpl_workspace_bytes(const MplModel* m, int64_t max_batch) {
   if (m == nullptr || max_batch < 0) return 0;
   const int64_t Bc = std::min<int64_t>(std::max<int64_t>(max_batch, 1), m->chunk);
-  const int lanes = (m->chunk_streams == 2 && max_batch >= kDualMinBatch) ? 2 : 1;  // an upper bound for every smaller batch
-  return lanes * layout_workspace(m, Bc, nullptr).bytes;
+  return layout_workspace(m, Bc, nullptr).bytes;
 }
 
 int mpl_forward(MplModel* m, const void* packed, const float* const* poses, const float* const* rays,
@@ -1160,16 +1129,14 @@ int mpl_forward(MplModel* m, const void* packed, const float* const* poses, cons
   m->launches = 0;
   if (m->profile) { m->prof.clear(); m->ev_used = 0; }
   if (batch == 0) return MPL_OK;
-  const ChunkPlan plan = plan_chunks(m, batch);
-  const int64_t Bc_max = plan.chunk;
-  const size_t lane_bytes = layout_workspace(m, Bc_max, nullptr).bytes;
-  const size_t need = plan.lanes * lane_bytes;
+  // Every pose is independent: the batch runs as chunks of at most m->chunk poses, one after the other on the caller's stream
+  const int64_t Bc_max = std::min<int64_t>(std::max<int64_t>(batch, 1), m->chunk);
+  const size_t need = layout_workspace(m, Bc_max, nullptr).bytes;
   if (workspace == nullptr || workspace_bytes < need) {
     set_error("mpl_forward: workspace has %zu bytes, %zu needed for batch %lld", workspace_bytes, need, (long long)batch);
     return MPL_ERR_WORKSPACE;
   }
-  const Workspace wl[2] = {layout_workspace(m, Bc_max, reinterpret_cast<uint8_t*>(workspace)),
-                           layout_workspace(m, Bc_max, reinterpret_cast<uint8_t*>(workspace) + (plan.lanes == 2 ? lane_bytes : 0))};
+  const Workspace w = layout_workspace(m, Bc_max, reinterpret_cast<uint8_t*>(workspace));
   Packed P{m, reinterpret_cast<const uint8_t*>(packed)};
   cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
   const int out_dim = 3 * m->J;
@@ -1223,29 +1190,8 @@ int mpl_forward(MplModel* m, const void* packed, const float* const* poses, cons
     MPL_CUDA(cudaGraphLaunch(exec, reinterpret_cast<cudaStream_t>(stream)));
     return MPL_OK;
   };
-  cudaStream_t lane_s[2] = {s, s};
-  if (plan.lanes == 2) {
-    // fork: both lane streams wait for everything enqueued on the caller's stream so far
-    for (int k = 0; k < 2; ++k) {
-      if (m->lane_stream[k] == nullptr) MPL_CUDA(cudaStreamCreateWithFlags(&m->lane_stream[k], cudaStreamNonBlocking));
-      if (m->ev_join[k] == nullptr) MPL_CUDA(cudaEventCreateWithFlags(&m->ev_join[k], cudaEventDisableTiming));
-      lane_s[k] = m->lane_stream[k];
-    }
-    if (m->ev_fork == nullptr) MPL_CUDA(cudaEventCreateWithFlags(&m->ev_fork, cudaEventDisableTiming));
-    MPL_CUDA(cudaEventRecord(m->ev_fork, s));
-    for (int k = 0; k < 2; ++k) MPL_CUDA(cudaStreamWaitEvent(lane_s[k], m->ev_fork, 0));
-  }
-  auto join = [&]() -> int {  // the caller's stream continues after both lanes
-    if (plan.lanes == 2)
-      for (int k = 0; k < 2; ++k) {
-        MPL_CUDA(cudaEventRecord(m->ev_join[k], lane_s[k]));
-        MPL_CUDA(cudaStreamWaitEvent(s, m->ev_join[k], 0));
-      }
-    return MPL_OK;
-  };
-  int lane = 0;
-  for (int64_t b0 = 0; b0 < batch; b0 += plan.chunk, lane ^= 1) {
-    const int64_t Bc = std::min<int64_t>(plan.chunk, batch - b0);
+  for (int64_t b0 = 0; b0 < batch; b0 += Bc_max) {
+    const int64_t Bc = std::min<int64_t>(Bc_max, batch - b0);
     const float* pp[kMaxViews];
     const float* rp[kMaxViews];
     const float* cp[kMaxViews];
@@ -1256,14 +1202,9 @@ int mpl_forward(MplModel* m, const void* packed, const float* const* poses, cons
     }
     const int st = forward_chunk(m, P, pp, rays ? rp : nullptr, centers ? cp : nullptr, pose_stride, center_stride,
                                  out + b0 * out_dim, aux1 ? aux1 + b0 * out_dim : nullptr, aux2 ? aux2 + b0 * out_dim : nullptr, Bc,
-                                 wl[plan.lanes == 2 ? lane : 0], lane_s[plan.lanes == 2 ? lane : 0]);
-    if (st != MPL_OK) {
-      join();
-      return try_graph ? end_capture(st) : st;
-    }
+                                 w, s);
+    if (st != MPL_OK) return try_graph ? end_capture(st) : st;
   }
-  const int jst = join();
-  if (jst != MPL_OK) return try_graph ? end_capture(jst) : jst;
   return try_graph ? end_capture(MPL_OK) : MPL_OK;
   MPL_API_END
 }
@@ -1603,17 +1544,16 @@ int mpl_calibrate_rig(const float* pix, const double* calib, int64_t batch, int 
 }
 
 int mpl_test_gemm(const void* A, const void* W, const float* bias, void* Y, int64_t M, int N, int K, int dtype, int epilogue,
-                  int out_fp32, int cta_group, mpl_stream_t stream) {
+                  int out_fp32, mpl_stream_t stream) {
   MPL_API_BEGIN
-  return launch_gemm_tcgen05(A, W, bias, Y, M, N, K, dtype, epilogue, out_fp32, reinterpret_cast<cudaStream_t>(stream), nullptr,
-                             cta_group);
+  return launch_gemm_tcgen05(A, W, bias, Y, M, N, K, dtype, epilogue, out_fp32, reinterpret_cast<cudaStream_t>(stream));
   MPL_API_END
 }
 
 /* The LayerNorm-fused epilogues of the same kernel in isolation (tests/test_gemm_ln_gpu.py). */
 int mpl_test_gemm_ln(const void* A, const void* W, const float* bias, void* Y, int64_t M, int N, int K, int epilogue,
                      const float* colsum, const void* stats_in, int slots_in, void* stats_out, void* x_lo, float eps,
-                     int ab_fp16, int out_fp16, int cta_group, mpl_stream_t stream) {
+                     int ab_fp16, int out_fp16, mpl_stream_t stream) {
   MPL_API_BEGIN
   GemmLnArgs a{};
   a.colsum = colsum;
@@ -1624,22 +1564,20 @@ int mpl_test_gemm_ln(const void* A, const void* W, const float* bias, void* Y, i
   a.eps = eps;
   a.ab_fp16 = ab_fp16;
   a.out_fp16 = out_fp16;
-  return launch_gemm_tcgen05(A, W, bias, Y, M, N, K, MPL_PREC_BF16, epilogue, 0, reinterpret_cast<cudaStream_t>(stream), &a,
-                             cta_group);
+  return launch_gemm_tcgen05(A, W, bias, Y, M, N, K, MPL_PREC_BF16, epilogue, 0, reinterpret_cast<cudaStream_t>(stream), &a);
   MPL_API_END
 }
 int mpl_test_gemm_ln_slots(int N) { return gemm_ln_slots(N); }
 
 int mpl_test_gemm_emit_pitch(const void* A, const void* W, const float* bias, void* Y, int64_t M, int N, int K, void* stats_out,
-                             void* x_lo, int ab_fp16, int ldy, int cta_group, mpl_stream_t stream) {
+                             void* x_lo, int ab_fp16, int ldy, mpl_stream_t stream) {
   MPL_API_BEGIN
   GemmLnArgs a{};
   a.stats_out = stats_out;
   a.x_lo = x_lo;
   a.ab_fp16 = ab_fp16;
   a.ldy = ldy;
-  return launch_gemm_tcgen05(A, W, bias, Y, M, N, K, MPL_PREC_BF16, EPI_RESIDUAL_EMIT, 0, reinterpret_cast<cudaStream_t>(stream), &a,
-                             cta_group);
+  return launch_gemm_tcgen05(A, W, bias, Y, M, N, K, MPL_PREC_BF16, EPI_RESIDUAL_EMIT, 0, reinterpret_cast<cudaStream_t>(stream), &a);
   MPL_API_END
 }
 

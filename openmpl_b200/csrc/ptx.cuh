@@ -126,52 +126,32 @@ __device__ __forceinline__ void st_shared_v2(uint32_t addr, uint32_t a, uint32_t
 }
 
 // ---- tcgen05 ----------------------------------------------------------------------------------------------------------
-template <int CG>
+// Every tensor-core kernel runs as CTA pairs (cluster 2x1x1): allocation, MMA and commit are the cta_group::2 forms.
 __device__ __forceinline__ void tmem_alloc(uint32_t dst_smem, uint32_t ncols) {
-  if constexpr (CG == 1)
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(dst_smem), "r"(ncols) : "memory");
-  else
-    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(dst_smem), "r"(ncols) : "memory");
+  asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(dst_smem), "r"(ncols) : "memory");
 }
-template <int CG>
 __device__ __forceinline__ void tmem_relinquish() {
-  if constexpr (CG == 1)
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  else
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
+  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
 }
-template <int CG>
 __device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t ncols) {
-  if constexpr (CG == 1)
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
-  else
-    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
+  asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
 }
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
 
 // D[tmem] (+)= A[smem desc] * B[smem desc];  KIND 0: kind::f16 (bf16/fp16 operands), 1: kind::tf32
-template <int CG, int KIND>
+template <int KIND>
 __device__ __forceinline__ void umma(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accumulate) {
-  if constexpr (CG == 1 && KIND == 0)
-    asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\ttcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}\n"
-                 ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate) : "memory");
-  else if constexpr (CG == 2 && KIND == 0)
+  if constexpr (KIND == 0)
     asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\ttcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}\n"
-                 ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate) : "memory");
-  else if constexpr (CG == 1 && KIND == 1)
-    asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\ttcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}\n"
                  ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate) : "memory");
   else
     asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\ttcgen05.mma.cta_group::2.kind::tf32 [%0], %1, %2, %3, p;\n\t}\n"
                  ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate) : "memory");
 }
 
-// all previously issued tcgen05.mma of this thread arrive on `bar` when complete (implies fence::before_thread_sync)
-__device__ __forceinline__ void umma_commit(uint32_t bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-// pair version: arrives on the barrier at the same offset in every CTA of `cta_mask`
+// all previously issued tcgen05.mma of this thread arrive on the barrier at offset `bar` in every CTA of `cta_mask` when
+// complete (implies fence::before_thread_sync)
 __device__ __forceinline__ void umma_commit_pair(uint32_t bar, uint16_t cta_mask) {
   asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
                ::"r"(bar), "h"(cta_mask) : "memory");

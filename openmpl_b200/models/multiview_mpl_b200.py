@@ -115,21 +115,18 @@ class MultiView_MPL(nn.Module):
                  deep_head=False,
                  head_kadkhod=False,
                  hidden_dim=1024,
-                 FPT_blocks_view_keypoint_tokens=False, *, precision=None, ln_fusion=True, gemm_cta_group=2,
-                 graph_batch=2048, chunk_streams=1, qkv_attn_fusion=True):
+                 FPT_blocks_view_keypoint_tokens=False, *, precision=None, ln_fusion=True, graph_batch=2048,
+                 qkv_attn_fusion=True):
         super().__init__()
         kw = {k: v for k, v in locals().items() if k in CTOR_DEFAULTS}
         self.cfg = make_config(**kw)
         self.precision = precision or DEFAULT_PRECISION
-        # implementation switches (MplDesc.ln_fusion / gemm_cta_group): bf16 mode folds the FPT LayerNorms into the GEMMs
-        # unless ln_fusion=False (checkpoints whose residual rows have |mean| >> std, see DESIGN.md section 5)
-        self.ln_fusion, self.gemm_cta_group = bool(ln_fusion), int(gemm_cta_group)
+        # implementation switch (MplDesc.ln_fusion): bf16 mode folds the FPT LayerNorms into the GEMMs unless
+        # ln_fusion=False (checkpoints whose residual rows have |mean| >> std, see DESIGN.md section 5)
+        self.ln_fusion = bool(ln_fusion)
         # batches of at most `graph_batch` poses (the reference runner's 256, valid_mpl.py:205-210) replay one captured CUDA
         # graph per batch size instead of ~130 kernel launches (mpl_set_graph_batch); 0 = always launch kernel by kernel
         self.graph_batch = int(graph_batch)
-        # chunk_streams=2: batches of >= 16384 poses run as two interleaved pose chunks on two internal streams
-        # (MplDesc.chunk_streams; measured neutral on B200, profiles/r2_experiments.md, hence off by default)
-        self.chunk_streams = int(chunk_streams)
         # bf16 mode: QKV projection + cross-view attention as one kernel where the shape allows (MplDesc.qkv_attn_fusion)
         self.qkv_attn_fusion = bool(qkv_attn_fusion)
         # host inputs spanning more than one forward chunk are copied piece by piece on a side stream under the kernels of
@@ -156,8 +153,7 @@ class MultiView_MPL(nn.Module):
             index = torch.cuda.current_device() if torch.cuda.is_available() else -1
         if index not in self._h.ptrs:
             L = _lib.lib()
-            desc = _lib.make_desc(self.cfg.kw, self.precision, self.ln_fusion, self.gemm_cta_group, self.chunk_streams,
-                                  self.qkv_attn_fusion)
+            desc = _lib.make_desc(self.cfg.kw, self.precision, self.ln_fusion, self.qkv_attn_fusion)
             h = ctypes.c_void_p()
             _lib.check(L.mpl_create(ctypes.byref(desc), ctypes.byref(h)))
             n = L.mpl_num_params(h)
@@ -255,9 +251,10 @@ class MultiView_MPL(nn.Module):
         return int(_lib.lib().mpl_chunk_poses(self._get_handle()))
 
     def set_profile(self, enabled, serial: bool = False):
-        """Bracket every kernel launch of the next forwards with CUDA events (see `profile()`).  serial=True also runs the
-        pose chunks one after the other instead of two in flight, so that the per-category times add up."""
-        _lib.check(_lib.lib().mpl_set_profile(self._get_handle(), (2 if serial else 1) if enabled else 0))
+        """Bracket every kernel launch of the next forwards with CUDA events (see `profile()`).  The pose chunks always run
+        one after the other, so the per-category times add up to the step; `serial` is accepted for old callers and changes
+        nothing."""
+        _lib.check(_lib.lib().mpl_set_profile(self._get_handle(), 1 if enabled else 0))
 
     def profile(self) -> dict:
         """{category: (milliseconds, launches)} of the last forward run with profiling enabled."""
@@ -595,9 +592,7 @@ class MultiView_MPL_G(nn.Module):
             FPT_blocks_view_keypoint_tokens=net.TRANSFORMER_FPT_BLOCKS_VIEW_KEYPOINT_TOKENS,
             precision=kwargs.get("precision"),
             ln_fusion=kwargs.get("ln_fusion", True),
-            gemm_cta_group=kwargs.get("gemm_cta_group", 2),
             graph_batch=kwargs.get("graph_batch", 2048),
-            chunk_streams=kwargs.get("chunk_streams", 1),
             qkv_attn_fusion=kwargs.get("qkv_attn_fusion", True),
         )
 

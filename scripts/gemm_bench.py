@@ -1,6 +1,6 @@
 """Microbenchmark of the tcgen05 projection kernel on the four FPT shapes (CUDA events, L2-cold inputs by size).
 
-    python scripts/gemm_bench.py [--cg 1|2] [--dtype bf16|tf32] [--rows 131072] [--iters 10] [--shapes qkv,proj,fc1,fc2]
+    python scripts/gemm_bench.py [--dtype bf16|tf32] [--rows 131072] [--iters 10] [--shapes qkv,proj,fc1,fc2]
 """
 import argparse
 import os
@@ -12,7 +12,6 @@ import torch  # noqa: E402
 from openmpl_b200 import _lib  # noqa: E402
 
 p = argparse.ArgumentParser()
-p.add_argument("--cg", type=int, default=2)
 p.add_argument("--dtype", default="bf16")
 p.add_argument("--rows", type=int, default=131072)
 p.add_argument("--iters", type=int, default=10)
@@ -32,7 +31,7 @@ for name in a.shapes.split(","):
     bias = torch.randn(N, device="cuda")
     Y = torch.zeros(M, N, device="cuda", dtype=torch.float32) if out_fp32 else torch.zeros((2 if split else 1) * M, N, device="cuda", dtype=torch.bfloat16)
     run = lambda: _lib.check(L.mpl_test_gemm(A.data_ptr(), W.data_ptr(), bias.data_ptr(), Y.data_ptr(), M, N, K,
-                                             _lib.PRECISIONS[a.dtype], epi, out_fp32, a.cg, stream))
+                                             _lib.PRECISIONS[a.dtype], epi, out_fp32, stream))
     for _ in range(3):
         run()
     torch.cuda.synchronize()
@@ -43,4 +42,4 @@ for name in a.shapes.split(","):
     e1.record()
     torch.cuda.synchronize()
     ms = e0.elapsed_time(e1) / a.iters
-    print(f"cg{a.cg} {a.dtype} {name:5s} M={M} N={N} K={K} epi={epi}: {ms:.3f} ms  {2.0 * M * N * K / ms / 1e9:.1f} TFLOP/s", flush=True)
+    print(f"{a.dtype} {name:5s} M={M} N={N} K={K} epi={epi}: {ms:.3f} ms  {2.0 * M * N * K / ms / 1e9:.1f} TFLOP/s", flush=True)

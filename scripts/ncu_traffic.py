@@ -38,7 +38,7 @@ def main():
         if "qkv_attn_kernel" in name:
             key = "qkv_attention_fused"
         elif "gemm_tcgen05_kernel" in name:
-            epi = name.split("gemm_tcgen05_kernel<")[1].split(">")[0].replace("(int)", "").split(",")[2].strip()
+            epi = name.split("gemm_tcgen05_kernel<")[1].split(">")[0].replace("(int)", "").split(",")[-1].strip()
             key = NAMES.get(epi, "epi" + epi)
         else:
             continue

@@ -91,26 +91,26 @@ def kernel_path(kw, precision):
     p["spt"] = not kw.get("no_transformer_spt") and depth > 0
     p["fpt"] = not kw.get("no_transformer_fpt") and depth > 0
     p["stacks"] = V if kw.get("multiple_spatial_blocks") else 1
-    # model.cu:666-667 (spt_fused.cu:366 in the fused SPT): one more SPT block application per layer for the
+    # model.cu:659-660 (spt_fused.cu:366 in the fused SPT): one more SPT block application per layer for the
     # confidence-weighted pass
     p["spt_apps"] = p["reps"] + (depth if kw.get("confidence_as_attention_uncertainty_weight") else 0)
-    # model.cu:840-841 + spt_fused.cu:851: the single-kernel SPT needs J = 17, d = 32, H = 8, hidden 64 and a tensor-core mode
+    # model.cu:837-838 + spt_fused.cu:851: the single-kernel SPT needs J = 17, d = 32, H = 8, hidden 64 and a tensor-core mode
     p["spt_fused"] = precision != "fp32" and p["spt"] and J == 17 and d == 32 and H == 8 and c.spt_hidden == 64
-    # model.cu:843-844: the keypoint-token FPT stack as one kernel (bf16, V <= 16, same block shape as the SPT)
+    # model.cu:840-841: the keypoint-token FPT stack as one kernel (bf16, V <= 16, same block shape as the SPT)
     p["kp_fused"] = (precision == "bf16" and p["kp"] and p["fpt"] and V <= 16 and J == 17 and D == 32 and H == 8
                      and p["hidden"] == 64)
-    # model.cu:846 + 860: LayerNorm-fused bf16 mode, residual stream in two bf16 planes (model.cu:632: `planes`)
+    # model.cu:843 + 857: LayerNorm-fused bf16 mode, residual stream in two bf16 planes (model.cu:625: `planes`)
     p["ln_fused"] = precision == "bf16" and p["fpt"] and not p["kp_fused"] and D % 32 == 0 and D <= 32 * 4 * 17
-    # model.cu:864 + gemm_tcgen05.cu:1250-1253: fused QKV + attention for 136- or 68-wide heads and 2 <= V <= 8
+    # model.cu:859 + gemm_tcgen05.cu:1230-1233: fused QKV + attention for 136- or 68-wide heads and 2 <= V <= 8
     p["qkv_attn"] = p["ln_fused"] and (D == H * 136 or (D == H * 68 and H % 2 == 0)) and 2 <= N <= 8
-    # model.cu:628: the SPT kernel computes the embedding unless the 3D position is Linear(normalize(ray)) (model.cu:584)
+    # model.cu:621: the SPT kernel computes the embedding unless the 3D position is Linear(normalize(ray)) (model.cu:577)
     p["pos_mode2"] = bool(kw.get("add_3D_pos_encoding_in_Spatial")) and not kw.get("pose_3d_emb_learnable")
     p["fuse_embed"] = p["spt_fused"] and not p["pos_mode2"]
-    # model.cu:707: the K5 head (head_fused / head_block_kernel) serves the default head only
+    # model.cu:700: the K5 head (head_fused / head_block_kernel) serves the default head only
     p["fused_head"] = not (kw.get("linear_weighted_mean") or kw.get("deep_head") or kw.get("head_kadkhod"))
-    # model.cu:870-872: channel-permuted planes need the interleaved ray layout, the fused SPT and the K5 head
+    # model.cu:865-867: channel-permuted planes need the interleaved ray layout, the fused SPT and the K5 head
     p["perm"] = (p["ln_fused"] and c.ray_layout == "interleave" and p["spt_fused"] and D == 2 * E and p["fused_head"])
-    # model.cu:711-716: every head but the K5 one reading the planes refills the fp32 tokens from them
+    # model.cu:704-709: every head but the K5 one reading the planes refills the fp32 tokens from them
     p["join_planes"] = p["ln_fused"] and not p["fused_head"]
     return p
 
@@ -161,7 +161,7 @@ def expected_kernels(kw, precision):
             if precision == "tf32":
                 must["to_split_kernel"] = (None, None)                           # kernels_generic.cu:972-980
     else:
-        # no FPT (model.cu:679): the only attention left is the SPT's
+        # no FPT (model.cu:672): the only attention left is the SPT's
         never += ["qkv_attn_kernel", "attention_views_kernel", "attention_kernel<", "attention_kp_h4_kernel",
                   "spt_fused_kernel_fast<true>"]
         if spt_narrow:
@@ -173,21 +173,21 @@ def expected_kernels(kw, precision):
             never += ["attention_narrow_kernel"]         # the SPT is the only narrow-head attention of view tokens
     else:
         never += ["spt_fused_kernel_fast<false>", "spt_fused_kernel_precise"]
-    # model.cu:684-685 / 632-633: ln_prep converts the fp32 tokens into the planes unless the fused SPT wrote them
+    # model.cu:677-678 / 625-626: ln_prep converts the fp32 tokens into the planes unless the fused SPT wrote them
     if p["ln_fused"]:
         if p["spt_fused"]:
             never += ["ln_prep_kernel"]
         else:
             must["ln_prep_kernel"] = (1, None)
     if p["fused_head"]:
-        # head: model.cu:704-705 (ray-layout rows are read as 32-channel segments at stride 64 unless the planes are channel-
-        # permuted, model.cu:871-872), model.cu:632 + 711-714 (planes are read directly), io_kernels.cu:447 (instantiation)
+        # head: model.cu:697-698 (ray-layout rows are read as 32-channel segments at stride 64 unless the planes are channel-
+        # permuted, model.cu:866-867), model.cu:625 + 704-707 (planes are read directly), io_kernels.cu:447 (instantiation)
         stride = 64 if (p["ray_layout"] == "interleave" and not p["perm"]) else 32
         E = p["E"]
         nk = f"9, {stride}, 17" if E == 544 else ("9, 0, 0" if E > 320 else "5, 0, 0")
         must[f"head_block_kernel<{nk}, {'true' if p['ln_fused'] else 'false'}>"] = (1, 256)
     else:
-        # model.cu:732-773: LayerNorm / view mean or Linear / (BN-folded) Linear chain on the fp32 tokens
+        # model.cu:725-766: LayerNorm / view mean or Linear / (BN-folded) Linear chain on the fp32 tokens
         never += ["head_block_kernel", "head_fused_kernel"]
     return must, never
 

@@ -78,6 +78,18 @@ def test_bad_struct_size_and_precision_are_rejected():
     desc = _lib.make_desc(dict(spec.CTOR_DEFAULTS), "fp32")
     desc.precision = 9
     assert L.mpl_create(ctypes.byref(desc), ctypes.byref(h)) == _lib.MPL_ERR_INVALID_ARGUMENT
+    # fields kept for the struct layout: each accepts 0 and the one schedule that exists (CTA pairs, the caller's stream)
+    for field, good, bad in (("gemm_cta_group", (0, 2), (1, 3)), ("chunk_streams", (0, 1), (2, -1))):
+        for value in good + bad:
+            desc = _lib.make_desc(dict(spec.CTOR_DEFAULTS), "fp32")
+            setattr(desc, field, value)
+            status = L.mpl_create(ctypes.byref(desc), ctypes.byref(h))
+            if value in good:
+                assert status == 0, (field, value)
+                L.mpl_destroy(h)
+            else:
+                assert status == _lib.MPL_ERR_INVALID_ARGUMENT, (field, value)
+                assert field in L.mpl_last_error().decode()
     # tensor-core modes refuse widths the tcgen05 kernel cannot tile instead of silently falling back
     kw = dict(spec.CTOR_DEFAULTS, num_joints=13, embed_dim_ratio=8, num_heads=2, num_views=3)     # D = 104
     desc = _lib.make_desc(kw, "bf16")

@@ -2,7 +2,7 @@
 
 The flag goldens (oracle/cases.py, `flag_*`) are built at d = 16, H = 4, where no tensor-core mode runs the kernels that
 serve the flags in production: the single-kernel SPT needs J = 17, d = 32, H = 8, hidden 64 (spt_fused.cu:851) and the
-LayerNorm-fused bf16 FPT needs a width that is a multiple of 32 (model.cu:860).  Here every flag case of the goldens
+LayerNorm-fused bf16 FPT needs a width that is a multiple of 32 (model.cu:857).  Here every flag case of the goldens
 (tests/flag_matrix.py) runs at d = 32, H = 8, J = 17, depth 2, B = 37 (ragged CTA tiles everywhere), V = 4 (and V = 5
 where the FPT runs on D = 544 / 1088 view tokens), in fp32, tf32 and bf16, against the fp64 oracle on the same seeded
 weights and batch.  One traced forward per case proves which kernels ran.  Run on the B200 with `-m gpu`."""
@@ -71,26 +71,26 @@ def _flag_expected(kw, precision):
     must, never = expected_kernels(kw, precision)
     p = kernel_path(kw, precision)
     if p["spt_fused"]:
-        # model.cu:645-652: one launch for the whole SPT stack of every view; PRECISE in tf32, fast<false> in bf16
+        # model.cu:638-645: one launch for the whole SPT stack of every view; PRECISE in tf32, fast<false> in bf16
         must["spt_fused_kernel_precise" if precision == "tf32" else "spt_fused_kernel_fast<false>"] = (1, None)
         never += ["spt_fused_kernel_fast<false>" if precision == "tf32" else "spt_fused_kernel_precise"]
-        never += ["token_build"]                          # model.cu:629 + 675: its epilogue writes the FPT tokens
+        never += ["token_build"]                          # model.cu:622 + 668: its epilogue writes the FPT tokens
     else:
-        must["token_build"] = (1, 256)                    # model.cu:675 (token_build_vec_kernel or token_build_kernel)
+        must["token_build"] = (1, 256)                    # model.cu:668 (token_build_vec_kernel or token_build_kernel)
         if not p["kp"]:
             if p["spt"]:
-                # model.cu:657-669: generic SPT, N = J = 17, hd = 4 -> attention_narrow_kernel once per block application
+                # model.cu:650-662: generic SPT, N = J = 17, hd = 4 -> attention_narrow_kernel once per block application
                 # (the confidence-weighted pass included) and stack; the FPT of view tokens has no narrow heads
                 must["attention_narrow_kernel<float, float, 4>"] = (p["spt_apps"] * p["stacks"], 256)
             else:
                 never += ["attention_narrow_kernel"]
-    # model.cu:628 + 642: a stand-alone embed kernel unless the fused SPT computes the embedding in its prologue, which it
-    # does for every spatial position mode but Linear(normalize(ray)) (spatial_pos_mode 2, model.cu:584)
+    # model.cu:621 + 635: a stand-alone embed kernel unless the fused SPT computes the embedding in its prologue, which it
+    # does for every spatial position mode but Linear(normalize(ray)) (spatial_pos_mode 2, model.cu:577)
     if p["fuse_embed"]:
         never += ["embed_"]
     else:
         must["embed_"] = (1, 256)                         # embed_vec_kernel or embed_kernel
-    # model.cu:711-716: non-K5 heads behind the bf16 planes refill the fp32 tokens once
+    # model.cu:704-709: non-K5 heads behind the bf16 planes refill the fp32 tokens once
     if p["join_planes"]:
         must["join_planes_kernel"] = (1, None)
     else:

@@ -2,8 +2,8 @@
 through the C-ABI test hook, against fp64 references built from the same rounded operands:
   LN-apply (EPI 4 / 5):      Y = act(rstd * (bf16(x) W'^T - mu * colsum(W')) + b')            (QKV, fc1)
   residual-emit (EPI 6 / 7): x (two bf16 planes) += A W^T + bias, plus per-row (sum, sum^2)   (proj, fc2)
-Covers M that is not a multiple of the 256-row tile, N = 544 (half group at the end) and 1088 / 2176 / 3264, both
-CTA-group modes, bf16 and fp16 operands / outputs."""
+Covers M that is not a multiple of the 256-row tile, N = 544 (half group at the end) and 1088 / 2176 / 3264, bf16
+and fp16 operands / outputs."""
 import numpy as np
 import pytest
 import torch
@@ -23,11 +23,10 @@ def _pad256(m):
     return (m + 255) // 256 * 256
 
 
-@pytest.mark.parametrize("cg", [1, 2])
 @pytest.mark.parametrize("M,N,K,gelu,out_fp16", [(1000, 3264, 1088, False, False), (777, 2176, 1088, True, True),
                                                   (513, 1632, 544, False, False), (300, 1088, 544, True, True),
                                                   (260, 1088, 544, True, False), (64, 96, 32, False, False)])
-def test_layernorm_apply_epilogue(M, N, K, gelu, out_fp16, cg):
+def test_layernorm_apply_epilogue(M, N, K, gelu, out_fp16):
     L = _lib.lib()
     g = torch.Generator(device="cuda").manual_seed(M + 3 * N + 7 * K)
     x = torch.randn(M, K, device="cuda", generator=g) * 0.8 + 0.05 * torch.randn(M, 1, device="cuda", generator=g)
@@ -49,7 +48,7 @@ def test_layernorm_apply_epilogue(M, N, K, gelu, out_fp16, cg):
     Y = torch.empty(M, N, device="cuda", dtype=torch.float16 if out_fp16 else torch.bfloat16)
     stream = torch.cuda.current_stream().cuda_stream
     _lib.check(L.mpl_test_gemm_ln(xb.data_ptr(), Wf.data_ptr(), biasf.data_ptr(), Y.data_ptr(), M, N, K, 5 if gelu else 4,
-                                  colsum.data_ptr(), stats.data_ptr(), slots, None, None, eps, 0, int(out_fp16), cg, stream))
+                                  colsum.data_ptr(), stats.data_ptr(), slots, None, None, eps, 0, int(out_fp16), stream))
     torch.cuda.synchronize()
     s1 = (stats[:, :M, 0].double()).sum(0); s2 = (stats[:, :M, 1].double()).sum(0)
     mu = s1 / K
@@ -63,18 +62,17 @@ def test_layernorm_apply_epilogue(M, N, K, gelu, out_fp16, cg):
         true = 0.5 * true * (1.0 + torch.erf(true / np.sqrt(2.0)))
     scale = ref.abs().max().item()
     err = (Y.double() - ref).abs().max().item() / scale
-    assert err <= 6e-3, f"M={M} N={N} K={K} gelu={gelu} fp16={out_fp16} cg={cg}: {err:.3e} vs rounded-operand reference"
+    assert err <= 6e-3, f"M={M} N={N} K={K} gelu={gelu} fp16={out_fp16}: {err:.3e} vs rounded-operand reference"
     err_true = (Y.double() - true).abs().max().item() / true.abs().max().item()
     assert err_true <= 2e-2, f"vs LayerNorm + Linear in fp64: {err_true:.3e}"
 
 
-@pytest.mark.parametrize("cg", [1, 2])
 @pytest.mark.parametrize("M,N,K,fp16", [(1000, 1088, 1088, False), (777, 1088, 2176, True), (513, 544, 544, False),
                                          (300, 544, 1088, True), (2049, 1088, 1088, False), (100, 32, 64, False),
                                          (4100, 544, 2176, False),
                                          # many tiles per CTA: the residual slots and their mbarrier phases wrap many times
                                          (40000, 1088, 1088, False), (36000, 1088, 2176, True), (50000, 544, 544, False)])
-def test_residual_emit_epilogue(M, N, K, fp16, cg):
+def test_residual_emit_epilogue(M, N, K, fp16):
     L = _lib.lib()
     g = torch.Generator(device="cuda").manual_seed(2 * M + N + K)
     dt = torch.float16 if fp16 else torch.bfloat16
@@ -89,13 +87,13 @@ def test_residual_emit_epilogue(M, N, K, fp16, cg):
     stats = torch.full((slots, Mp, 2), float("nan"), device="cuda")
     stream = torch.cuda.current_stream().cuda_stream
     _lib.check(L.mpl_test_gemm_ln(A.data_ptr(), W.data_ptr(), bias.data_ptr(), hi.data_ptr(), M, N, K, 6, None, None, 0,
-                                  stats.data_ptr(), lo.data_ptr(), 0.0, int(fp16), 0, cg, stream))
+                                  stats.data_ptr(), lo.data_ptr(), 0.0, int(fp16), 0, stream))
     torch.cuda.synchronize()
     ref = x_old_planes + A.double() @ W.double().T + bias.double()
     got = hi.double() + lo.double()
     scale = ref.abs().max().item()
     err = (got - ref).abs().max().item() / scale
-    assert err <= 2e-5, f"M={M} N={N} K={K} fp16={fp16} cg={cg}: residual {err:.3e}"
+    assert err <= 2e-5, f"M={M} N={N} K={K} fp16={fp16}: residual {err:.3e}"
     # hi is the bf16 rounding of the value, lo the remainder: |lo| <= half an ulp of hi
     assert (lo.float().abs() <= hi.float().abs() * 2.0 ** -8 + 1e-30).all()
     s = stats[:, :M].double().sum(0)
@@ -121,7 +119,7 @@ def test_residual_emit_on_the_leading_columns_of_wider_planes(M, N, K, ldy, fp16
     hi0, lo0 = hi.clone(), lo.clone()
     stats = torch.full((L.mpl_test_gemm_ln_slots(N), _pad256(M), 2), float("nan"), device="cuda")
     _lib.check(L.mpl_test_gemm_emit_pitch(A.data_ptr(), W.data_ptr(), bias.data_ptr(), hi.data_ptr(), M, N, K, stats.data_ptr(),
-                                          lo.data_ptr(), int(fp16), ldy, 2, torch.cuda.current_stream().cuda_stream))
+                                          lo.data_ptr(), int(fp16), ldy, torch.cuda.current_stream().cuda_stream))
     torch.cuda.synchronize()
     ref = (hi0.double() + lo0.double())[:, :N] + A.double() @ W.double().T + bias.double()
     got = (hi.double() + lo.double())[:, :N]
@@ -131,7 +129,7 @@ def test_residual_emit_on_the_leading_columns_of_wider_planes(M, N, K, ldy, fp16
     s = stats[:, :M].double().sum(0)
     assert (s[:, 0] - ref.sum(1)).abs().max().item() / ref.abs().sum(1).max().item() <= 1e-5
     L2 = L.mpl_test_gemm_emit_pitch(A.data_ptr(), W.data_ptr(), bias.data_ptr(), hi.data_ptr(), M, N, K, stats.data_ptr(),
-                                    lo.data_ptr(), int(fp16), N - 16, 2, None)
+                                    lo.data_ptr(), int(fp16), N - 16, None)
     assert L2 == _lib.MPL_ERR_INVALID_ARGUMENT                      # a pitch below N is refused
 
 
@@ -156,7 +154,7 @@ def test_folded_layernorm_error_grows_with_row_mean_over_std(mean_over_std, boun
     stats[0, :M, 0] = x.sum(1); stats[0, :M, 1] = (x ** 2).sum(1)
     Y = torch.empty(M, N, device="cuda", dtype=torch.bfloat16)
     _lib.check(L.mpl_test_gemm_ln(xb.data_ptr(), Wf.data_ptr(), b.data_ptr(), Y.data_ptr(), M, N, K, 4, colsum.data_ptr(),
-                                  stats.data_ptr(), 1, None, None, 1e-6, 0, 0, 2, torch.cuda.current_stream().cuda_stream))
+                                  stats.data_ptr(), 1, None, None, 1e-6, 0, 0, torch.cuda.current_stream().cuda_stream))
     torch.cuda.synchronize()
     ln = torch.nn.functional.layer_norm(x.double(), (K,), gamma.double(), beta.double(), 1e-6)
     true = ln @ W.double().T

@@ -194,24 +194,6 @@ def test_layernorm_fusion_on_and_off_agree_with_the_reference(name):
     assert rel_err(outs[1], outs[0].astype(np.float64)) <= TOL["bf16"]
 
 
-@pytest.mark.parametrize("name,precision", [("hm0_v4_d12", "bf16"), ("cmu_v5_d2_hm0flags", "bf16"), ("chosen_v4_d12", "bf16"),
-                                            ("cmu0_v2_d2", "tf32")])
-def test_single_cta_gemm_path_meets_the_same_bounds(name, precision):
-    """`gemm_cta_group=1` (MplDesc.gemm_cta_group): the projections run as single-CTA tcgen05 tiles instead of CTA pairs, the
-    QKV projection and the view attention stay two kernels (the fused kernel is a CTA-pair kernel) -- every other piece is the
-    same: folded LayerNorms, channel-permuted residual planes, the last fc2 on the pose half only.  Same bounds, and a
-    3000-pose batch agrees with the CTA-pair build."""
-    case = CASES[name]
-    g = load_golden(name)
-    cfg, weights, batch = make_inputs(case)
-    m1 = build_module(case["kw"], weights, precision, gemm_cta_group=1)
-    assert rel_err(run_module(m1, batch)[0], g["out64_0"]) <= TOL[precision]
-    big = synth.make_batch(3000, synth.make_rig(cfg.V, case["rig"]), seed=5)
-    a = run_module(m1, big, packed=True)[0]
-    b = run_module(build_module(case["kw"], weights, precision), big, packed=True)[0]
-    assert np.isfinite(a).all() and rel_err(a, b.astype(np.float64)) <= TOL[precision]
-
-
 @pytest.mark.parametrize("precision", ["fp32", "tf32", "bf16"])
 def test_cuda_graph_small_batch_path_equals_the_plain_path(precision):
     """Batches up to `graph_batch` poses (the reference runner's TEST.BATCH_SIZE = 256) are captured once per batch size as a

@@ -186,7 +186,7 @@ def test_bf16_keypoint_tokens_off_the_fused_kernel(J, mlp_ratio, V, tmp_path):
 @pytest.mark.parametrize("precision", PRECISIONS)
 def test_hm0_flags_with_thirteen_joints(precision, V, tmp_path):
     """J = 13 (E = 416, D = 832): the head is head_block_kernel<9, 0, 0, PL> (bf16 reads unpermuted planes: the permutation
-    needs the fused SPT, model.cu:871), and the SPT leaves the fused kernel for the generic path plus ln_prep."""
+    needs the fused SPT, model.cu:866), and the SPT leaves the fused kernel for the generic path plus ln_prep."""
     kw, cfg, weights, batch, ref = _case("hm0", V, 13)
     m = build_module(kw, weights, precision, graph_batch=0)
     out, kernels = traced_forward(m, batch, tmp_path)
