@@ -17,7 +17,8 @@
  * refinement of triangulated points (mpl_triangulate_refine), a detector-error model for the synthetic data
  * (mpl_synth_detector_noise), a generator of random camera setups (mpl_synth_cameras), lens distortion of pixels
  * (mpl_distort_pixels / mpl_undistort_pixels), a calibration-error model (mpl_synth_calib_noise) and bundle adjustment of a
- * rig's extrinsics from its detections (mpl_calibrate_rig).
+ * rig's extrinsics from its detections (mpl_calibrate_rig), and multi-person scenes with the association of detections
+ * across views (mpl_synth_people, mpl_associate_people, mpl_gather_people, mpl_association_score).
  *
  * Conventions
  *   - plain pointers and sizes only; no torch / C++ types cross this boundary;
@@ -45,7 +46,7 @@
 extern "C" {
 #endif
 
-#define MPL_ABI_VERSION 10
+#define MPL_ABI_VERSION 11
 
 typedef enum MplStatus {
   MPL_OK = 0,
@@ -477,6 +478,79 @@ int mpl_calibrate_rig(const float* pix, const double* calib, int64_t batch, int 
                       const int32_t* view_mask, const float* init, double sigma_px, double sigma_rot, double sigma_pos,
                       int max_iters, double* calib_out, float* points, double* report, void* workspace,
                       size_t workspace_bytes, mpl_stream_t stream);
+
+/* Multi-person association across views (ABI 11; defined by this library: the reference's datasets give which detection of
+ * each view belongs to which person).  Every other entry point takes pix [B, V, J, 3] with row b of every view one person;
+ * the calls below get that grouping from the detections.
+ *
+ * Scene layout: a frame holds P detection slots per view.  scene [F, P, V, J, 3] fp32 (u, v, conf): entry (f, s, v) is slot s
+ * of view v; slots of different views are unrelated.  Detection (s, v) has the flat index m = s V + v.  Viewed as
+ * [F P, V, J, 3] a scene has the [B, V, J, 3] shape, so the lens and input-builder entry points apply to it unchanged.
+ *
+ * mpl_synth_people: scenes out of person-ordered pixels.  pix [F P, V, J, 3] holds person p of frame f in row f P + p (e.g.
+ * mpl_synth_project of poses [start P, (start + F) P) with lens and detector noise); perm [F, V, P] int32 gets, for frame f
+ * and view v, the person in each slot, and scene[f, s, v] = pix[f P + perm[f, v, s], v], copied bit for bit.  The draw:
+ * global frame i = start + f owns the counter blocks [i nb, (i + 1) nb), nb = ceil(V P / 4), of the Philox4x64-10 stream of
+ * mpl_synth_project under key (seed, 4); slot v P + s of those is U_s of view v, and perm[f, v] is the stable ascending
+ * argsort of U_0 .. U_{P-1} (openmpl_b200/synth.py synth_people is the twin).  MPL_ERR_INVALID_ARGUMENT, before any CUDA
+ * call: frames < 0, start < 0, V outside [1, 16], P < 1, P V > 128, J < 1; then frames == 0 returns MPL_OK; then a null
+ * pointer or scene == pix is MPL_ERR_INVALID_ARGUMENT.
+ *
+ * mpl_associate_people(_strided): groups the detections of each frame into people, fp64 throughout.  Frame f reads the
+ * calibration calib + f calib_stride (the calib_stride convention with frames in place of poses).
+ *   - candidate joint: conf > min_conf and strictly inside the w x h image (the rule of mpl_triangulate);
+ *   - active detection: at least min_joints candidate joints;
+ *   - ray of a candidate joint of view v: origin c_v (calib t), direction d = R^T ((u - cx) / fx, (v - cy) / fy, 1).  The
+ *     model is a pinhole: undistort first (mpl_undistort_pixels), as for the triangulations;
+ *   - joint distance of two rays: the distance of the two lines, |(c2 - c1) . n| / |n| with n = d1 x d2; where
+ *     |n|^2 <= 1e-24 |d1|^2 |d2|^2, |(c2 - c1) x d1| / |d1|;
+ *   - pair cost of active (s, v) and (t, w), v < w (member 1 in the lower view): the median of the joint distances over the
+ *     joints that are candidates in both (the mean of the two middle values for an even count); +inf when fewer than
+ *     min_joints joints are shared.  The median keeps a few confident false detections from hiding a true pair;
+ *   - greedy complete linkage: every active detection starts as its own cluster.  The pairs with cost <= max_dist, sorted by
+ *     (cost, key) ascending with key = m1 P V + m2 (m1 the member in the lower view), are taken in order; each merges its
+ *     two clusters unless they are already one, they share a view, or some cross pair of their members has a cost that is
+ *     not <= max_dist;
+ *   - people: the clusters with >= 2 members, ranked by member count descending, then smallest member m ascending;
+ *   - outputs: members [F, K, V] int32, the slot of view v in the person of rank k, or -1 (rows past the last person all
+ *     -1); labels [F, P, V] int32, the rank of the detection's person if that rank is < K, -1 for an active detection in no
+ *     output person, -2 for an inactive one; people [F] int32, the number of people (may exceed K);
+ *   - MPL_ERR_INVALID_ARGUMENT, before any CUDA call: frames < 0, V outside [2, 16], P < 1, P V > 128 (at most 8128 pairs
+ *     per frame), J outside [1, 32], min_joints outside [1, J], max_dist not finite or not > 0, K < 1, a bad calib_stride;
+ *     then frames == 0 returns MPL_OK; then a null pointer is MPL_ERR_INVALID_ARGUMENT;
+ *   - one CTA per frame; no floating-point atomics; results independent of how the frames are split; allocates nothing and
+ *     never synchronises (graph-capturable).
+ *
+ * mpl_gather_people: out [F, K, V, J, 3] fp32, out[f, k, v] = scene[f, members[f, k, v], v] bit for bit, zeros (u = v =
+ * conf = 0) where the member is -1 (or any value outside [0, P)).  Viewed as [F K, V, J, 3] it is a batch of people for the
+ * input builder, the forward, the triangulations and the refinement; with a lens, gather from the raw scene for the lifter
+ * and from the undistorted scene for the triangulations.  MPL_ERR_INVALID_ARGUMENT, before any CUDA call: frames < 0, P < 1,
+ * K < 1, V outside [1, 16], J < 1; then frames == 0 returns MPL_OK; then a null pointer.
+ *
+ * mpl_association_score: scores members / labels (of mpl_associate_people) against the true slots perm (of
+ * mpl_synth_people).  The true person of detection (s, v) is perm[f, v, s]; a detection is active iff its label is not -2.
+ *   owner [F, K] int32: the true person with the most members in row k, ties to the smaller person index; -1 for an empty row;
+ *   acc [MPL_ASSOC_ACC_LEN] fp64 running sums (added to, so ranks combine with one all-reduce):
+ *     [0] frames; [1] associable people (true persons with >= 2 active detections); [2] non-empty rows; [3] pure rows (every
+ *     member belongs to one person); [4] complete rows (pure, and holding every active detection of that person);
+ *     [5] predicted linked pairs (member pairs within rows); [6] correct linked pairs (of the same person); [7] true pairs
+ *     (pairs of active detections of one person, in different views).
+ *   Integer counts reduced in a fixed order, added once per call.  MPL_ERR_INVALID_ARGUMENT, before any CUDA call: frames < 0,
+ *   V outside [1, 16], P < 1, P V > 128, K < 1; then frames == 0 returns MPL_OK (acc untouched); then a null pointer. */
+#define MPL_ASSOC_ACC_LEN 8
+int mpl_synth_people(uint64_t seed, int64_t start, int64_t frames, int people, int num_views, int num_joints, const float* pix,
+                     float* scene, int32_t* perm, mpl_stream_t stream);
+int mpl_associate_people(const float* scene, const double* calib, int64_t frames, int people, int num_views, int num_joints,
+                         float min_conf, int min_joints, double max_dist, int max_people, int32_t* members, int32_t* labels,
+                         int32_t* num_people, mpl_stream_t stream);
+int mpl_associate_people_strided(const float* scene, const double* calib, int64_t calib_stride, int64_t frames, int people,
+                                 int num_views, int num_joints, float min_conf, int min_joints, double max_dist,
+                                 int max_people, int32_t* members, int32_t* labels, int32_t* num_people,
+                                 mpl_stream_t stream);
+int mpl_gather_people(const float* scene, const int32_t* members, int64_t frames, int people, int max_people, int num_views,
+                      int num_joints, float* out, mpl_stream_t stream);
+int mpl_association_score(const int32_t* members, const int32_t* labels, const int32_t* perm, int64_t frames, int people,
+                          int max_people, int num_views, int32_t* owner, double* acc, mpl_stream_t stream);
 
 /* ---- unit-test hooks for the building blocks (used by tests/ only) ------------------------------------------- */
 /* Y[M,N] = epilogue(A[M,K] . W[N,K]^T): the tcgen05 projection kernel in isolation.

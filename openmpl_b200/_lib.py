@@ -11,7 +11,7 @@ from ctypes import POINTER, c_char_p, c_double, c_float, c_int, c_int32, c_int64
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("MPL_B200_LIB") or os.path.join(HERE, "libmpl_b200.so")   # override: another build of the same ABI
 
-ABI_VERSION = 10
+ABI_VERSION = 11
 MPL_OK = 0
 MPL_ERR_INVALID_ARGUMENT = -1
 MPL_ERR_CONFIG_RUNTIME = -2
@@ -34,8 +34,10 @@ EXPORTS = [
     "mpl_triangulate_robust_strided", "mpl_synth_cameras", "mpl_triangulate_refine", "mpl_triangulate_refine_strided",
     "mpl_mpjpe_accumulate_grouped", "mpl_pmpjpe_accumulate_masked", "mpl_distort_pixels", "mpl_distort_pixels_strided",
     "mpl_undistort_pixels", "mpl_undistort_pixels_strided", "mpl_synth_calib_noise", "mpl_calibrate_rig_workspace_bytes",
-    "mpl_calibrate_rig",
+    "mpl_calibrate_rig", "mpl_synth_people", "mpl_associate_people", "mpl_associate_people_strided", "mpl_gather_people",
+    "mpl_association_score",
 ]
+ASSOC_ACC_LEN = 8   # MPL_ASSOC_ACC_LEN
 
 _DESC_FLAGS = [
     "qkv_bias", "add_confidence_input", "mult_confidence_emb", "concat_confidence_emb", "confidence_input_as_third",
@@ -176,6 +178,15 @@ def lib():
         L.mpl_calibrate_rig_workspace_bytes.restype = c_size_t
         L.mpl_calibrate_rig.argtypes = [c_void_p, c_void_p, c_int64, c_int, c_int, c_float, c_void_p, c_void_p, c_double,
                                         c_double, c_double, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]
+        L.mpl_synth_people.argtypes = [ctypes.c_uint64, c_int64, c_int64, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p,
+                                       c_void_p]
+        L.mpl_associate_people.argtypes = [c_void_p, c_void_p, c_int64, c_int, c_int, c_int, c_float, c_int, c_double, c_int,
+                                           c_void_p, c_void_p, c_void_p, c_void_p]
+        L.mpl_associate_people_strided.argtypes = [c_void_p, c_void_p, c_int64, c_int64, c_int, c_int, c_int, c_float, c_int,
+                                                   c_double, c_int, c_void_p, c_void_p, c_void_p, c_void_p]
+        L.mpl_gather_people.argtypes = [c_void_p, c_void_p, c_int64, c_int, c_int, c_int, c_int, c_void_p, c_void_p]
+        L.mpl_association_score.argtypes = [c_void_p, c_void_p, c_void_p, c_int64, c_int, c_int, c_int, c_void_p, c_void_p,
+                                            c_void_p]
         if L.mpl_abi_version() != ABI_VERSION:
             raise RuntimeError("libmpl_b200.so ABI version mismatch")
         _lib = L

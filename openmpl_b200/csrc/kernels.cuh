@@ -229,5 +229,15 @@ int launch_calibrate_rig(const float* pix, const double* calib, int64_t B, int V
 int launch_lens_pixels(bool undistort, const float* pin, float* pout, const double* calib, int64_t calib_stride,
                        const double* dist, int64_t dist_stride, double margin_x, double margin_y, int64_t B, int V, int J,
                        cudaStream_t s);
+// associate.cu: multi-person scenes, association, gathering and scoring (argument checks in model.cu)
+int launch_synth_people(uint64_t seed, int64_t start, int64_t F, int P, int V, int J, const float* pix, float* scene,
+                        int32_t* perm, cudaStream_t s);
+int launch_associate_people(const float* scene, const double* calib, int64_t calib_stride, int64_t F, int P, int V, int J,
+                            float min_conf, int min_joints, double max_dist, int K, int32_t* members, int32_t* labels,
+                            int32_t* people, cudaStream_t s);
+int launch_gather_people(const float* scene, const int32_t* members, int64_t F, int P, int K, int V, int J, float* out,
+                         cudaStream_t s);
+int launch_association_score(const int32_t* members, const int32_t* labels, const int32_t* perm, int64_t F, int P, int K,
+                             int V, int32_t* owner, double* acc, cudaStream_t s);
 
 }  // namespace mpl

@@ -6,6 +6,7 @@
 // pixels and a generator of random camera setups (the last three have no reference counterpart).  Every kernel that reads
 // calibrations is instantiated twice: one [V, 18] block for the batch (kPerPose = false) or one per pose (true).
 #include "kernels.cuh"
+#include "shared.cuh"
 #include "so3.cuh"
 
 namespace mpl {
@@ -664,11 +665,6 @@ static int tri_pose_tile(int V, int J, size_t& smem) {
   return T;
 }
 
-// The view takes part iff conf > min_conf and the pixel lies strictly inside the w x h image (build_inputs_kernel's tests).
-__device__ __forceinline__ bool tri_candidate(float conf, double u, double w, float min_conf, const double (&wh)[2]) {
-  return conf > min_conf && 0.0 < u && u < wh[0] - 1.0 && 0.0 < w && w < wh[1] - 1.0;
-}
-
 // Adds the DLT rows s (u P3 - P1) and s (w P3 - P2) of one view into the Gram matrix G (upper triangle).  s = 1 is an
 // exact multiply, so the unweighted sum has the same bits with or without it.
 __device__ __forceinline__ void gram_add_view(double (&G)[4][4], const double (&P)[12], double u, double w, double s) {
@@ -1009,20 +1005,8 @@ int launch_triangulate_refine(const float* pix, const double* calib, int64_t cal
 // x_cam = R (X - t), u = f x_cam / z + c (MPL/lib/utils/calib.py:42-77).  Emits raw detector-style pixels (u, v, conf)
 // for mpl_build_inputs and the 3D target.  The generator is numpy's Philox4x64-10 stream, bit for bit (openmpl_b200/
 // synth.py draws the same uniforms on the host), so the device data can be checked against the host generator.
+// philox4x64_10 is in shared.cuh.
 // ---------------------------------------------------------------------------------------------------------------------
-__device__ __forceinline__ void philox4x64_10(uint64_t n, uint64_t key0, uint64_t key1, uint64_t (&out)[4]) {
-  uint64_t c0 = n, c1 = 0, c2 = 0, c3 = 0, k0 = key0, k1 = key1;
-#pragma unroll
-  for (int r = 0; r < 10; ++r) {
-    if (r > 0) { k0 += 0x9E3779B97F4A7C15ull; k1 += 0xBB67AE8584CAA73Bull; }
-    const uint64_t hi0 = __umul64hi(0xD2E7470EE14C6C93ull, c0), lo0 = 0xD2E7470EE14C6C93ull * c0;
-    const uint64_t hi1 = __umul64hi(0xCA5A826395121157ull, c2), lo1 = 0xCA5A826395121157ull * c2;
-    const uint64_t n0 = hi1 ^ c1 ^ k0, n2 = hi0 ^ c3 ^ k1;
-    c0 = n0; c1 = lo1; c2 = n2; c3 = lo0;
-  }
-  out[0] = c0; out[1] = c1; out[2] = c2; out[3] = c3;
-}
-
 struct UniformCursor {  // sequential reader of one pose's uniform stream with a one-block cache
   uint64_t v[4];
   int64_t blk;

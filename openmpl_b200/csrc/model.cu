@@ -1543,6 +1543,87 @@ int mpl_calibrate_rig(const float* pix, const double* calib, int64_t batch, int 
                               reinterpret_cast<cudaStream_t>(stream));
 }
 
+// Shape rules of the association entry points: V views, P slots per view, J joints (include/mpl_b200.h).
+static bool people_shape_ok(int P, int V, int J, int min_views) {
+  return V >= min_views && V <= kMaxViews && P >= 1 && P * V <= 128 && J >= 1;
+}
+
+int mpl_synth_people(uint64_t seed, int64_t start, int64_t frames, int people, int num_views, int num_joints, const float* pix,
+                     float* scene, int32_t* perm, mpl_stream_t stream) {
+  if (frames < 0 || start < 0 || !people_shape_ok(people, num_views, num_joints, 1)) {
+    set_error("mpl_synth_people: bad argument (frames %lld, start %lld, people %d, num_views %d, num_joints %d)",
+              (long long)frames, (long long)start, people, num_views, num_joints);
+    return MPL_ERR_INVALID_ARGUMENT;
+  }
+  if (frames == 0) return MPL_OK;
+  if (pix == nullptr || scene == nullptr || perm == nullptr || (const void*)pix == (const void*)scene) {
+    set_error("mpl_synth_people: null pointer, or scene == pix");
+    return MPL_ERR_INVALID_ARGUMENT;
+  }
+  return launch_synth_people(seed, start, frames, people, num_views, num_joints, pix, scene, perm,
+                             reinterpret_cast<cudaStream_t>(stream));
+}
+
+int mpl_associate_people(const float* scene, const double* calib, int64_t frames, int people, int num_views, int num_joints,
+                         float min_conf, int min_joints, double max_dist, int max_people, int32_t* members, int32_t* labels,
+                         int32_t* num_people, mpl_stream_t stream) {
+  return mpl_associate_people_strided(scene, calib, 0, frames, people, num_views, num_joints, min_conf, min_joints, max_dist,
+                                      max_people, members, labels, num_people, stream);
+}
+
+int mpl_associate_people_strided(const float* scene, const double* calib, int64_t calib_stride, int64_t frames, int people,
+                                 int num_views, int num_joints, float min_conf, int min_joints, double max_dist,
+                                 int max_people, int32_t* members, int32_t* labels, int32_t* num_people,
+                                 mpl_stream_t stream) {
+  if (frames < 0 || !people_shape_ok(people, num_views, num_joints, 2) || num_joints > 32 || min_joints < 1 ||
+      min_joints > num_joints || !std::isfinite(max_dist) || !(max_dist > 0.0) || max_people < 1 ||
+      !calib_stride_ok(calib_stride, num_views)) {
+    set_error("mpl_associate_people_strided: bad argument (frames %lld, people %d, num_views %d, num_joints %d, min_joints %d, "
+              "max_dist %g, K %d, calib_stride %lld)", (long long)frames, people, num_views, num_joints, min_joints, max_dist,
+              max_people, (long long)calib_stride);
+    return MPL_ERR_INVALID_ARGUMENT;
+  }
+  if (frames == 0) return MPL_OK;
+  if (scene == nullptr || calib == nullptr || members == nullptr || labels == nullptr || num_people == nullptr) {
+    set_error("mpl_associate_people_strided: null pointer");
+    return MPL_ERR_INVALID_ARGUMENT;
+  }
+  return launch_associate_people(scene, calib, calib_stride, frames, people, num_views, num_joints, min_conf, min_joints,
+                                 max_dist, max_people, members, labels, num_people, reinterpret_cast<cudaStream_t>(stream));
+}
+
+int mpl_gather_people(const float* scene, const int32_t* members, int64_t frames, int people, int max_people, int num_views,
+                      int num_joints, float* out, mpl_stream_t stream) {
+  if (frames < 0 || people < 1 || max_people < 1 || num_views < 1 || num_views > kMaxViews || num_joints < 1) {
+    set_error("mpl_gather_people: bad argument (frames %lld, people %d, K %d, num_views %d, num_joints %d)", (long long)frames,
+              people, max_people, num_views, num_joints);
+    return MPL_ERR_INVALID_ARGUMENT;
+  }
+  if (frames == 0) return MPL_OK;
+  if (scene == nullptr || members == nullptr || out == nullptr) {
+    set_error("mpl_gather_people: null pointer");
+    return MPL_ERR_INVALID_ARGUMENT;
+  }
+  return launch_gather_people(scene, members, frames, people, max_people, num_views, num_joints, out,
+                              reinterpret_cast<cudaStream_t>(stream));
+}
+
+int mpl_association_score(const int32_t* members, const int32_t* labels, const int32_t* perm, int64_t frames, int people,
+                          int max_people, int num_views, int32_t* owner, double* acc, mpl_stream_t stream) {
+  if (frames < 0 || !people_shape_ok(people, num_views, 1, 1) || max_people < 1) {
+    set_error("mpl_association_score: bad argument (frames %lld, people %d, K %d, num_views %d)", (long long)frames, people,
+              max_people, num_views);
+    return MPL_ERR_INVALID_ARGUMENT;
+  }
+  if (frames == 0) return MPL_OK;
+  if (members == nullptr || labels == nullptr || perm == nullptr || owner == nullptr || acc == nullptr) {
+    set_error("mpl_association_score: null pointer");
+    return MPL_ERR_INVALID_ARGUMENT;
+  }
+  return launch_association_score(members, labels, perm, frames, people, max_people, num_views, owner, acc,
+                                  reinterpret_cast<cudaStream_t>(stream));
+}
+
 int mpl_test_gemm(const void* A, const void* W, const float* bias, void* Y, int64_t M, int N, int K, int dtype, int epilogue,
                   int out_fp32, mpl_stream_t stream) {
   MPL_API_BEGIN

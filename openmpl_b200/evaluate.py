@@ -16,6 +16,8 @@
         --triangulate --triangulate-robust --refine-triangulations                      # cameras with a lens
     python -m openmpl_b200.evaluate --arch hm0 --views 4 --pixel-noise 1 --calib-noise 0.5,20 --triangulate \
         --calibrate-rig 16384                                                           # a miscalibrated rig, recalibrated
+    python -m openmpl_b200.evaluate --arch cmu0 --views 5 --people 4 --pixel-noise 2 --outlier-rate 0.1 --triangulate \
+        --triangulate-robust                                                            # 4 people per frame, associated
 
 Per micro-batch, entirely on the device: `mpl_synth_project` (3D poses from the counter-based generator keyed by the
 GLOBAL pose index, projected through the V calibrations) -> `mpl_build_inputs` (clip, confidence zeroing, screen
@@ -72,6 +74,19 @@ centres then replace the perturbed ones for the whole evaluation (the intrinsics
 bits, so no collective is needed.  The line gains a "rig_calibration" entry: poses, items, observations, iterations,
 accepted steps, RMS pixel error before and after, per-view rotation (degrees) and centre (mm) errors of the perturbed and
 of the calibrated rig against the true one, and its own time `ms`, outside `ms_total`.
+
+`--people P` (P >= 2; not with `--calibrate-rig`) evaluates multi-person frames whose grouping is not given: `--poses`
+counts persons, frame f holds the persons of global indices [f P, (f + 1) P), and each micro-batch is micro_batch // P
+frames.  Per micro-batch: the persons are generated and projected with the lens and detector noise as above, put into
+random detection slots per view (`mpl_synth_people`), associated across views (`mpl_associate_people`: rays of the
+candidate joints, median line distance per cross-view pair at most `--assoc-max-dist` world units over at least
+`--assoc-min-joints` shared joints, greedy complete linkage), on the undistorted scene with the shifted calibration when
+there is a lens, and gathered into K = P person rows (`mpl_gather_people`, once from the raw scene for the lifter and once
+from the undistorted one for the triangulations).  Every metric of the line scores the person rows against the target of
+their owner, the true person with the most members in the row; rows without an owner add nothing.  `--random-cameras`
+draws the cameras per frame (keyed by the global frame index) and `--calib-noise` applies as above.  The line gains an
+"association" entry (`mpl_association_score`): the counts, pair precision and recall, the pure and complete fractions, the
+people dropped past K and the parameters.  Without the flag nothing of this runs.
 """
 from __future__ import annotations
 
@@ -99,7 +114,21 @@ CALIBRATE_MAX_ITERS = 30
 def run(arch="hm0", views=4, depth=None, poses=1 << 20, micro_batch=65536, precision="bf16", rig=None, seed=1,
         weight_seed=0, warmup=1, triangulate=False, pixel_noise=0.0, outlier_rate=0.0, miss_rate=0.0,
         triangulate_robust=False, inlier_px=10.0, random_cameras=False, refine_triangulations=False,
-        triangulation_pmpjpe=False, lens_distortion=None, calib_noise=None, calibrate_rig=0):
+        triangulation_pmpjpe=False, lens_distortion=None, calib_noise=None, calibrate_rig=0, people=0,
+        assoc_max_dist=0.1, assoc_min_joints=3):
+    if people:
+        if people < 2:
+            raise ValueError(f"people must be >= 2, got {people}")
+        if people * views > 128:
+            raise ValueError(f"people * views must be <= 128 (the detections of one frame), got {people} * {views}")
+        if calibrate_rig:
+            raise ValueError("calibrate_rig calibrates from single-person poses: not with people")
+        if not (np.isfinite(assoc_max_dist) and assoc_max_dist > 0):
+            raise ValueError(f"assoc_max_dist must be finite and > 0, got {assoc_max_dist}")
+        if not 1 <= assoc_min_joints <= 17:
+            raise ValueError(f"assoc_min_joints must be in [1, 17], got {assoc_min_joints}")
+        if micro_batch < people:
+            raise ValueError(f"micro_batch must hold at least one frame of {people} people, got {micro_batch}")
     if calib_noise is not None:
         calib_noise = tuple(float(x) for x in calib_noise)
         if len(calib_noise) != 2 or not all(np.isfinite(calib_noise)) or min(calib_noise) < 0:
@@ -132,16 +161,25 @@ def run(arch="hm0", views=4, depth=None, poses=1 << 20, micro_batch=65536, preci
     mdist.broadcast_state(model)                       # replicas bit-identical (they already are: same seed)
     rig_kind = rig or DEFAULT_RIG[arch]
     the_rig = synth.make_rig(views, rig_kind)
-    start, stop = mdist.shard_range(poses, rank, world)
-    acc = metric.MpjpeAccumulator(cfg.J, output_in_meter=True, device=dev)
-    pacc = metric.PmpjpeAccumulator(cfg.J, output_in_meter=True, device=dev)
-    tacc = metric.MpjpeAccumulator(cfg.J, output_in_meter=True, device=dev) if triangulate else None
-    racc = metric.MpjpeAccumulator(cfg.J, output_in_meter=True, device=dev) if triangulate_robust else None
-    tfacc = metric.MpjpeAccumulator(cfg.J, output_in_meter=True, device=dev) if triangulate and refine_triangulations else None
-    rfacc = (metric.MpjpeAccumulator(cfg.J, output_in_meter=True, device=dev) if triangulate_robust and refine_triangulations
-             else None)
+    if people:                                         # frames of `people` persons: the index range counts frames
+        frames = poses // people
+        poses = frames * people
+        micro_batch //= people
+        start, stop = mdist.shard_range(frames, rank, world)
+    else:
+        start, stop = mdist.shard_range(poses, rank, world)
+    # with people, a person row adds into group 0 and a row without an owner into none (-1)
+    grouped = dict(num_groups=1) if people else {}
+    acc = metric.MpjpeAccumulator(cfg.J, output_in_meter=True, device=dev, **grouped)
+    pacc = metric.PmpjpeAccumulator(cfg.J, output_in_meter=True, device=dev, **grouped)
+    tacc = metric.MpjpeAccumulator(cfg.J, output_in_meter=True, device=dev, **grouped) if triangulate else None
+    racc = metric.MpjpeAccumulator(cfg.J, output_in_meter=True, device=dev, **grouped) if triangulate_robust else None
+    tfacc = (metric.MpjpeAccumulator(cfg.J, output_in_meter=True, device=dev, **grouped)
+             if triangulate and refine_triangulations else None)
+    rfacc = (metric.MpjpeAccumulator(cfg.J, output_in_meter=True, device=dev, **grouped)
+             if triangulate_robust and refine_triangulations else None)
     # masked P-MPJPE of each triangulation entry, keyed like the accumulators above
-    tp = {name: metric.PmpjpeAccumulator(cfg.J, output_in_meter=True, device=dev, masked=True)
+    tp = {name: metric.PmpjpeAccumulator(cfg.J, output_in_meter=True, device=dev, masked=True, **grouped)
           for name, a in (("t", tacc), ("r", racc), ("tf", tfacc), ("rf", rfacc)) if triangulation_pmpjpe and a is not None}
     noisy = pixel_noise != 0 or outlier_rate != 0 or miss_rate != 0
     if lens_distortion is not None:
@@ -186,27 +224,67 @@ def run(arch="hm0", views=4, depth=None, poses=1 << 20, micro_batch=65536, preci
                           errors={k: rig_errors(c, true_rig) for k, c in cals.items()},
                           aligned={k: rig_errors(c, true_rig, align=True) for k, c in cals.items()} if views >= 3 else None)
 
-    def step(s0, n):
-        cams = inputs.synth_cameras(n, views, rig_kind, seed=seed, start=s0, device=dev) if random_cameras else None
-        pix, target = synth_pixels(s0, n, cams)
+    assoc_acc = torch.zeros(8, dtype=torch.float64, device=dev) if people else None
+    dropped = torch.zeros(1, dtype=torch.float64, device=dev) if people else None
+
+    def person_rows(f0, nf):
+        """The person rows of frames [f0, f0 + nf): (pixels and calibration for the lifter, the same for the triangulations,
+        the owners' targets, the group of each row: 0 with an owner, -1 without)."""
+        P = people
+        cams = inputs.synth_cameras(nf, views, rig_kind, seed=seed, start=f0, device=dev) if random_cameras else None
         if cams is None:
             calib = used_rig
         elif calib_noise is not None:
-            calib = inputs.calibration_noise(cams, seed, s0, sig_rot, sig_pos)
+            calib = inputs.calibration_noise(cams, seed, f0, sig_rot, sig_pos)
         else:
             calib = cams
+        pix, target = synth_pixels(f0 * P, nf * P, None if cams is None else cams.repeat_interleave(P, 0))
+        scene, perm = inputs.synth_people(pix, P, seed, f0)
+        rows_calib = calib if calib.dim() == 2 else calib.repeat_interleave(P, 0)   # frame f's cameras for its slots and rows
+        scene_t, tri_calib = scene, rows_calib
+        if lens_distortion is not None:
+            u, tri_calib = inputs.undistort_pixels(scene.view(nf * P, views, cfg.J, 3), rows_calib, lens, margin=margin)
+            scene_t = u.view(scene.shape)
+        members, labels, npeople = inputs.associate_people(
+            scene_t, tri_calib if tri_calib.dim() == 2 else tri_calib[::P], min_joints=assoc_min_joints,
+            max_dist=assoc_max_dist, max_people=P)
+        owner, _ = inputs.association_score(members, labels, perm, assoc_acc)
+        dropped.add_((npeople - P).clamp(min=0).sum().to(torch.float64))
+        rows = inputs.gather_people(scene, members).view(nf * P, views, cfg.J, 3)
+        rows_t = rows if scene_t is scene else inputs.gather_people(scene_t, members).view(nf * P, views, cfg.J, 3)
+        idx = owner.clamp(min=0).long()[:, :, None, None].expand(nf, P, cfg.J, 3)
+        target = target.view(nf, P, cfg.J, 3).gather(1, idx).view(nf * P, cfg.J, 3)
+        group = torch.where(owner >= 0, 0, -1).to(torch.int32).view(-1)
+        return rows, rows_calib, (rows_t, tri_calib), target, group
+
+    def step(s0, n):
+        g, tri = {}, None
+        if people:
+            pix, calib, tri, target, group = person_rows(s0, n)
+            g = {"group": group}
+        else:
+            cams = inputs.synth_cameras(n, views, rig_kind, seed=seed, start=s0, device=dev) if random_cameras else None
+            pix, target = synth_pixels(s0, n, cams)
+            if cams is None:
+                calib = used_rig
+            elif calib_noise is not None:
+                calib = inputs.calibration_noise(cams, seed, s0, sig_rot, sig_pos)
+            else:
+                calib = cams
         p, r, c = inputs.build_inputs(pix, calib)
         with torch.no_grad():
             out = model(p, rays=r, centers=c)
         out = out[0] if isinstance(out, tuple) else out
-        acc.update(out, target)
-        pacc.update(out, target)
+        acc.update(out, target, **g)
+        pacc.update(out, target, **g)
         def score(key, a, points, mask):
-            a.update(points, target, mask)
+            a.update(points, target, mask, **g)
             if key in tp:
-                tp[key].update(points, target, mask)
+                tp[key].update(points, target, mask, **g)
 
-        if lens_distortion is not None and (tacc is not None or racc is not None):
+        if tri is not None:
+            pix, calib = tri
+        elif lens_distortion is not None and (tacc is not None or racc is not None):
             pix, calib = inputs.undistort_pixels(pix, calib, lens, margin=margin)
         if tacc is not None:
             points, used = inputs.triangulate(pix, calib)
@@ -227,6 +305,9 @@ def run(arch="hm0", views=4, depth=None, poses=1 << 20, micro_batch=65536, preci
     for a in (tacc, racc, tfacc, rfacc, *tp.values()):
         if a is not None:
             a.acc.zero_()
+    if people:
+        assoc_acc.zero_()
+        dropped.zero_()
     if world > 1:
         torch.distributed.barrier()
     torch.cuda.synchronize()
@@ -239,6 +320,9 @@ def run(arch="hm0", views=4, depth=None, poses=1 << 20, micro_batch=65536, preci
     for a in (tacc, racc, tfacc, rfacc, *tp.values()):
         if a is not None:
             a.all_reduce()
+    if people and world > 1:
+        torch.distributed.all_reduce(assoc_acc)
+        torch.distributed.all_reduce(dropped)
     e1.record()
     torch.cuda.synchronize()
     ms = mdist.max_over_ranks(e0.elapsed_time(e1), dev)
@@ -302,16 +386,20 @@ def run(arch="hm0", views=4, depth=None, poses=1 << 20, micro_batch=65536, preci
                     "note": "each rig mapped into the true frame by the similarity fitting its centres to the true ones: "
                             "the images do not observe the world frame, so the bundle adjustment leaves that similarity "
                             "where the prior puts it"}
+        if people:
+            line["association"] = association_summary(assoc_acc.cpu().numpy(), float(dropped.item()), res["n"], people,
+                                                      assoc_max_dist, assoc_min_joints)
+        # .reshape(-1): the sums of the one group with people
         if tacc is not None:
-            line["triangulation"] = triangulation_summary(tacc.acc.detach().cpu().numpy(), cfg.J)
+            line["triangulation"] = triangulation_summary(tacc.acc.detach().cpu().numpy().reshape(-1), cfg.J)
         if racc is not None:
             line["triangulation_robust"] = triangulation_summary(
-                racc.acc.detach().cpu().numpy(), cfg.J,
+                racc.acc.detach().cpu().numpy().reshape(-1), cfg.J,
                 method=f"pair RANSAC, MSAC cost at {inlier_px:g} px, conf-weighted DLT refit over the inliers")
         for entry, a, views in (("triangulation", tfacc, "the candidate views"), ("triangulation_robust", rfacc, "the inliers")):
             if a is not None:
                 line[entry]["refined"] = triangulation_summary(
-                    a.acc.detach().cpu().numpy(), cfg.J,
+                    a.acc.detach().cpu().numpy().reshape(-1), cfg.J,
                     method=f"Levenberg-Marquardt on the reprojection error over {views}, weights conf^2, "
                            f"at most {REFINE_MAX_ITERS} iterations")
         for key, entry, sub in (("t", "triangulation", None), ("r", "triangulation_robust", None),
@@ -349,6 +437,24 @@ def rig_errors(calib, true_calib, align=False):
     ang = np.degrees(2.0 * np.arcsin(np.minimum(fro / (2.0 * np.sqrt(2.0)), 1.0)))
     pos = 1000.0 * np.linalg.norm(calib[:, 9:12] - true_calib[:, 9:12], axis=1)
     return [float(a) for a in ang], [float(p) for p in pos]
+
+
+def association_summary(acc, dropped, scored_rows, people, max_dist, min_joints):
+    """The association entry of the JSON line from the 8 sums of mpl_association_score."""
+    def ratio(a, b):
+        return float(a / b) if b > 0 else float("nan")
+
+    names = ("frames", "associable_people", "rows", "pure_rows", "complete_rows", "predicted_pairs", "correct_pairs",
+             "true_pairs")
+    out = {k: int(round(float(v))) for k, v in zip(names, acc)}
+    out.update(pair_precision=ratio(acc[6], acc[5]), pair_recall=ratio(acc[6], acc[7]), pure_fraction=ratio(acc[3], acc[2]),
+               complete_fraction=ratio(acc[4], acc[1]), dropped_past_k=int(round(dropped)), scored_rows=scored_rows,
+               parameters={"people_per_frame": people, "K": people, "max_dist_m": max_dist, "min_joints": min_joints,
+                           "min_conf": 0.0},
+               method="median line distance of the candidate joints' rays per cross-view pair, greedy complete linkage",
+               note="pure_fraction: pure rows over rows; complete_fraction: complete rows over associable people; rows "
+                    "without an owner add nothing to the metrics")
+    return out
 
 
 def triangulation_summary(acc, J, method="linear DLT, pixel-space rows, views with conf > 0 inside the image"):
@@ -407,7 +513,27 @@ def main(argv=None):
     p.add_argument("--calibrate-rig", type=int, default=0, metavar="N",
                    help="recalibrate the perturbed rig's extrinsics by bundle adjustment on N extra poses before the "
                         "evaluation (needs --calib-noise with both values > 0, not --random-cameras, N <= --micro-batch)")
+    p.add_argument("--people", type=int, default=0, metavar="P",
+                   help="P >= 2 people per frame in random detection slots, associated across views before every metric "
+                        "(not with --calibrate-rig)")
+    p.add_argument("--assoc-max-dist", type=float, default=0.1, metavar="M",
+                   help="association: largest median ray distance of a linked pair, world units (m)")
+    p.add_argument("--assoc-min-joints", type=int, default=3, metavar="N",
+                   help="association: candidate joints a detection needs, and joints a pair must share")
     a = p.parse_args(argv)
+    if a.people:
+        if a.people < 2:
+            p.error("--people needs P >= 2")
+        if a.people * a.views > 128:
+            p.error("--people P needs P * --views <= 128")
+        if a.calibrate_rig:
+            p.error("--calibrate-rig cannot be used with --people")
+        if not (np.isfinite(a.assoc_max_dist) and a.assoc_max_dist > 0):
+            p.error("--assoc-max-dist needs a finite value > 0")
+        if not 1 <= a.assoc_min_joints <= 17:
+            p.error("--assoc-min-joints needs 1 <= N <= 17")
+        if a.micro_batch < a.people:
+            p.error("--micro-batch must hold at least one frame of --people persons")
     cnoise = None
     if a.calib_noise is not None:
         try:
@@ -439,7 +565,8 @@ def main(argv=None):
         pixel_noise=a.pixel_noise, outlier_rate=a.outlier_rate, miss_rate=a.miss_rate,
         triangulate_robust=a.triangulate_robust, inlier_px=a.inlier_px, random_cameras=a.random_cameras,
         refine_triangulations=a.refine_triangulations, triangulation_pmpjpe=a.triangulation_pmpjpe, lens_distortion=lens,
-        calib_noise=cnoise, calibrate_rig=a.calibrate_rig)
+        calib_noise=cnoise, calibrate_rig=a.calibrate_rig, people=a.people, assoc_max_dist=a.assoc_max_dist,
+        assoc_min_joints=a.assoc_min_joints)
 
 
 if __name__ == "__main__":

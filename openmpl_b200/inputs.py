@@ -278,6 +278,111 @@ def calibrate_rig(pix: torch.Tensor, calib, init: torch.Tensor, view_mask: torch
     return calib_out, points, report
 
 
+def synth_people(pix: torch.Tensor, people: int, seed: int, start: int) -> tuple:
+    """Multi-person scenes out of person-ordered pixels (`mpl_synth_people`), enqueued on the current stream.
+
+    pix [F P, V, J, 3] fp32 on the device holds person p of frame f in row f P + p, e.g. `synth_project` of poses
+    [start P, (start + F) P) with lens and detector noise.  Each view's P detections are put into its P slots in a random
+    order drawn per (seed, global frame index start + f) under a Philox key of their own.  Returns (scene [F, P, V, J, 3],
+    scene[f, s, v] = pix[f P + perm[f, v, s], v] bit for bit; perm [F, V, P] int32, the person in each slot).
+    `synth.synth_people` is the numpy twin.
+    """
+    if pix.dim() != 4 or pix.shape[-1] != 3 or pix.shape[0] % people:
+        raise ValueError(f"pix must be [F P, V, J, 3] with P = {people}, got {list(pix.shape)}")
+    B, V, J, _ = pix.shape
+    F = B // people
+    pix = pix.to(torch.float32).contiguous()
+    scene = torch.empty((F, people, V, J, 3), dtype=torch.float32, device=pix.device)
+    perm = torch.empty((F, V, people), dtype=torch.int32, device=pix.device)
+    with torch.cuda.device(pix.device):
+        stream = torch.cuda.current_stream(pix.device).cuda_stream
+        _lib.check(_lib.lib().mpl_synth_people(int(seed), int(start), F, int(people), V, J, pix.data_ptr(), scene.data_ptr(),
+                                               perm.data_ptr(), stream))
+    return scene, perm
+
+
+def associate_people(scene: torch.Tensor, calib, min_conf: float = 0.0, min_joints: int = 3, max_dist: float = 0.1,
+                     max_people: int | None = None) -> tuple:
+    """Cross-view association of the detections of multi-person scenes (`mpl_associate_people`), enqueued on the current
+    stream.
+
+    scene [F, P, V, J, 3] fp32 (u, v, conf) pinhole pixels (undistort first when the cameras have a lens); calib [V, 18] or
+    [F, V, 18] (one calibration per frame).  A detection is active with at least min_joints candidate joints (conf >
+    min_conf, strictly inside the image); the cost of two active detections of different views is the median, over their
+    shared candidate joints, of the distance between their rays (world units); pairs with cost <= max_dist are merged
+    greedily, cheapest first, into clusters with at most one detection per view whose member pairs all pass the threshold.
+    Clusters of >= 2 detections are people, ranked by size, then by their first detection.  Returns (members [F, K, V]
+    int32 slots or -1, K = max_people (default P); labels [F, P, V] int32: the detection's person rank if < K, -1 when
+    active but in no such person, -2 when inactive; people [F] int32, the number of people, which may exceed K).
+    """
+    if scene.dim() != 5 or scene.shape[-1] != 3:
+        raise ValueError(f"scene must be [F, P, V, J, 3], got {list(scene.shape)}")
+    F, P, V, J, _ = scene.shape
+    K = P if max_people is None else int(max_people)
+    device = scene.device
+    scene = scene.to(torch.float32).contiguous()
+    calib, stride = _calib_arg(calib, F, V, device)
+    members = torch.empty((F, K, V), dtype=torch.int32, device=device)
+    labels = torch.empty((F, P, V), dtype=torch.int32, device=device)
+    people = torch.empty((F,), dtype=torch.int32, device=device)
+    with torch.cuda.device(device):
+        stream = torch.cuda.current_stream(device).cuda_stream
+        _lib.check(_lib.lib().mpl_associate_people_strided(
+            scene.data_ptr(), calib.data_ptr(), stride, F, P, V, J, float(min_conf), int(min_joints), float(max_dist), K,
+            members.data_ptr(), labels.data_ptr(), people.data_ptr(), stream))
+    return members, labels, people
+
+
+def gather_people(scene: torch.Tensor, members: torch.Tensor) -> torch.Tensor:
+    """The detections of each associated person (`mpl_gather_people`), enqueued on the current stream: out [F, K, V, J, 3],
+    out[f, k, v] = scene[f, members[f, k, v], v] bit for bit, zeros where the member is -1.  `out.view(F * K, V, J, 3)` is a
+    batch of people for `build_inputs`, the model and the triangulations."""
+    if scene.dim() != 5 or scene.shape[-1] != 3:
+        raise ValueError(f"scene must be [F, P, V, J, 3], got {list(scene.shape)}")
+    F, P, V, J, _ = scene.shape
+    if members.dim() != 3 or members.shape[0] != F or members.shape[2] != V or members.dtype != torch.int32:
+        raise ValueError(f"members must be an int32 [F, K, V] = [{F}, K, {V}] tensor, got {list(members.shape)} {members.dtype}")
+    K = members.shape[1]
+    scene = scene.to(torch.float32).contiguous()
+    members = members.to(scene.device).contiguous()
+    out = torch.empty((F, K, V, J, 3), dtype=torch.float32, device=scene.device)
+    with torch.cuda.device(scene.device):
+        stream = torch.cuda.current_stream(scene.device).cuda_stream
+        _lib.check(_lib.lib().mpl_gather_people(scene.data_ptr(), members.data_ptr(), F, P, K, V, J, out.data_ptr(), stream))
+    return out
+
+
+def association_score(members: torch.Tensor, labels: torch.Tensor, perm: torch.Tensor, acc: torch.Tensor | None = None) -> tuple:
+    """Scores an association against the true slots (`mpl_association_score`), enqueued on the current stream.
+
+    members [F, K, V] and labels [F, P, V] of `associate_people`, perm [F, V, P] of `synth_people`.  Returns (owner [F, K]
+    int32: the true person with the most members in each row, ties to the smaller index, -1 for an empty row; acc [8] fp64,
+    the running sums of include/mpl_b200.h added into `acc` when given: frames, associable people, non-empty rows, pure
+    rows, complete rows, predicted linked pairs, correct linked pairs, true pairs)."""
+    if members.dim() != 3 or labels.dim() != 3 or perm.dim() != 3:
+        raise ValueError("members [F, K, V], labels [F, P, V] and perm [F, V, P] must be 3-dimensional")
+    F, K, V = members.shape
+    P = labels.shape[1]
+    if tuple(labels.shape) != (F, P, V) or tuple(perm.shape) != (F, V, P):
+        raise ValueError(f"labels must be [F, P, V] and perm [F, V, P] for members {list(members.shape)}, got "
+                         f"{list(labels.shape)} and {list(perm.shape)}")
+    for name, t in (("members", members), ("labels", labels), ("perm", perm)):
+        if t.dtype != torch.int32:
+            raise ValueError(f"{name} must be int32, got {t.dtype}")
+    device = members.device
+    if acc is None:
+        acc = torch.zeros(_lib.ASSOC_ACC_LEN, dtype=torch.float64, device=device)
+    elif acc.dtype != torch.float64 or tuple(acc.shape) != (_lib.ASSOC_ACC_LEN,) or not acc.is_contiguous():
+        raise ValueError(f"acc must be a contiguous float64 [{_lib.ASSOC_ACC_LEN}] tensor")
+    members, labels, perm = (t.to(device).contiguous() for t in (members, labels, perm))
+    owner = torch.empty((F, K), dtype=torch.int32, device=device)
+    with torch.cuda.device(device):
+        stream = torch.cuda.current_stream(device).cuda_stream
+        _lib.check(_lib.lib().mpl_association_score(members.data_ptr(), labels.data_ptr(), perm.data_ptr(), F, P, K, V,
+                                                    owner.data_ptr(), acc.data_ptr(), stream))
+    return owner, acc
+
+
 def _dist_arg(dist, B: int, V: int, device) -> tuple:
     """(contiguous fp64 device tensor, dist_stride): [V, 5] -> stride 0 (one lens set for the batch); [B, V, 5] -> 5 V."""
     if isinstance(dist, torch.Tensor):

@@ -155,6 +155,26 @@ def calibration_noise(calib, seed: int, start: int, sigma_rot: float, sigma_pos:
     return out[0] if rig else out
 
 
+def people_permutations(seed: int, start: int, frames: int, people: int, num_views: int) -> np.ndarray:
+    """perm [F, V, P] int32 of `mpl_synth_people`: for frame start + f and view v, the person in each detection slot.  Frame
+    i owns the counter blocks [i nb, (i + 1) nb), nb = ceil(V P / 4), of the Philox4x64-10 stream under key (seed, 4), and
+    perm[f, v] is the stable ascending argsort of its uniforms in slots v P .. v P + P - 1."""
+    U = _uniforms(seed, start, frames, num_views * people, key1=4).reshape(frames, num_views, people)
+    return np.argsort(U, axis=-1, kind="stable").astype(np.int32)
+
+
+def synth_people(pix, people: int, seed: int, start: int) -> tuple:
+    """Host twin of `mpl_synth_people`: pix [F P, V, J, 3] with person p of frame f in row f P + p -> (scene [F, P, V, J, 3]
+    with scene[f, s, v] = pix[f P + perm[f, v, s], v], perm [F, V, P] of `people_permutations`)."""
+    pix = np.asarray(pix)
+    B, V = pix.shape[:2]
+    F = B // people
+    perm = people_permutations(seed, start, F, people, V)
+    rows = np.arange(F)[:, None, None] * people + perm                  # [F, V, P]
+    scene = pix[rows, np.arange(V)[None, :, None]]                       # [F, V, P, J, 3]
+    return np.ascontiguousarray(scene.transpose(0, 2, 1, 3, 4)), perm
+
+
 def _uniforms(seed: int, start: int, count: int, per_pose: int, key1: int = 0) -> np.ndarray:
     """[count, per_pose] uniforms in [0,1); row i depends only on (seed, start+i).  Philox key (seed, key1)."""
     blocks = (per_pose + 3) // 4                      # Philox4x64: 4 outputs per counter step
