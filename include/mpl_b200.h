@@ -18,7 +18,8 @@
  * (mpl_synth_detector_noise), a generator of random camera setups (mpl_synth_cameras), lens distortion of pixels
  * (mpl_distort_pixels / mpl_undistort_pixels), a calibration-error model (mpl_synth_calib_noise) and bundle adjustment of a
  * rig's extrinsics from its detections (mpl_calibrate_rig), and multi-person scenes with the association of detections
- * across views (mpl_synth_people, mpl_associate_people, mpl_gather_people, mpl_association_score).
+ * across views (mpl_synth_people, mpl_associate_people, mpl_gather_people, mpl_association_score), and people that move
+ * with the tracking of person rows across frames (mpl_synth_motion, mpl_track_people, mpl_tracking_score).
  *
  * Conventions
  *   - plain pointers and sizes only; no torch / C++ types cross this boundary;
@@ -551,6 +552,82 @@ int mpl_gather_people(const float* scene, const int32_t* members, int64_t frames
                       int num_joints, float* out, mpl_stream_t stream);
 int mpl_association_score(const int32_t* members, const int32_t* labels, const int32_t* perm, int64_t frames, int people,
                           int max_people, int num_views, int32_t* owner, double* acc, mpl_stream_t stream);
+
+/* Multi-person tracking across frames (additions to ABI 11: new entry points only, so a caller built against ABI 11 is
+ * unaffected; defined by this library).  A sequence is T consecutive frames of one scene; the calls below give each person
+ * row of a frame a track id that persists from frame to frame.
+ *
+ * mpl_synth_motion: S sequences of T frames of P people that move, for sequences [start, start + S).  Row
+ * r = ((start + s) T + t) P + p (local row b = (s T + t) P + p) holds person p in frame t of global sequence i = start + s:
+ * target [S T P, J, 3] fp32 (metres) and pix [S T P, V, J, 3] fp32 (u, v, conf), the formats of mpl_synth_project.  Viewed as
+ * [F P, ...] with F = S T frames the rows feed mpl_distort_pixels, mpl_synth_detector_noise (start index r) and
+ * mpl_synth_people (frame index (start + s) T + t) unchanged.  The motion of (i, p) is drawn from the Philox4x64-10 stream of
+ * mpl_synth_project under key (seed, 5): g = i P + p owns the counter blocks [g nb, (g + 1) nb), nb = ceil((9 + 6 (J - 1)) /
+ * 4), with uniform slots U0 .. U8 and the body pairs (u1_m, u2_m) in slots 9 + m and 9 + 3 (J - 1) + m, m = 3 (j - 1) + k.
+ * With tau = t / fps seconds, room (x0, x1, y0, y1), w_x = x1 - x0 and w_y = y1 - y0:
+ *   - root x = (x0 + x1) / 2 + a_x sin(2 pi f_x tau + 2 pi U4), a_x = (0.25 + 0.25 U0) w_x, f_x = 0.03 + 0.07 U2 Hz; y likewise
+ *     with U1, U3, U5 and w_y (so the root stays in the room and moves at most 2 pi 0.1 0.5 |(w_x, w_y)| m/s);
+ *     z = 0.8 + 0.2 U6, constant;
+ *   - heading theta = 2 pi U7 + (U8 - 0.5) tau rad (at most 0.5 rad/s);
+ *   - body o_0 = 0, o_j[k] = 0.25 sqrt(-2 ln max(u1_m, 1e-12)) cos(2 pi u2_m) (mpl_synth_project's Box-Muller), fixed in time;
+ *   - joints X_j = root + Rz(theta) o_j, fp64, so the motion of (i, p, t) depends only on (seed, i, p, t, J, fps, room);
+ *   - pixels: mpl_synth_project's camera model (x_cam = R (X - t), u = f x_cam / z + c, no clipping, conf 0 behind the
+ *     camera) through calib + b calib_stride (the calib_stride convention with rows in place of poses), and conf = 1 with
+ *     conf_ones, otherwise 0.3 + 0.7 U from mpl_synth_project's confidence slots of pose index r (key (seed, 0)): a row's
+ *     confidences are those mpl_synth_project gives pose r.
+ * openmpl_b200/synth.py synth_motion is the numpy twin.  MPL_ERR_INVALID_ARGUMENT, before any CUDA call: sequences < 0,
+ * start < 0, frames < 1, people < 1, V outside [1, 16], J < 1, fps not finite or not > 0, a bad calib_stride; then
+ * sequences == 0 returns MPL_OK; then a null pointer.
+ *
+ * mpl_track_people: online tracking of person rows, sequence by sequence; the state carries the tracks across calls.
+ *   points [S, T, K, J, 3] fp32: per frame, K rows of 3D joints (e.g. mpl_triangulate_robust of mpl_gather_people rows, or
+ *     the lifter's output); NaN joints are allowed.  joint_mask NULL or [S, T, K, J] fp32.
+ *   state: per sequence mpl_track_state_bytes(max_tracks, J) bytes, opaque, 4-byte aligned, sequence s at s times that size;
+ *     all-zero bytes are a fresh sequence.  mpl_track_state_bytes returns 0 for a shape the call rejects (max_tracks
+ *     outside [1, 128], J outside [1, 32]).
+ *   track_id [S, T, K] int32 output.  The rules, frame by frame in order:
+ *   - used joint: its three coordinates are finite and joint_mask is NULL or > 0; a row with >= min_joints used joints is a
+ *     detection;
+ *   - a track remembers, per joint, the last observed position (fp32, bit for bit) and whether it has one, its id and its
+ *     count of consecutive missed frames.  No prediction (zero velocity);
+ *   - cost of (track, row), fp64: the median over the joints used in the row and remembered by the track of the joint
+ *     distance sqrt((dx dx + dy dy) + dz dz), each product and sum rounded (no fused multiply-add); the mean of the two
+ *     middle values for an even count; +inf with fewer than min_joints such joints;
+ *   - matching: the pairs with cost <= max_dist, sorted by (cost, key) ascending with key = id K + k, are taken in order; a
+ *     pair matches unless its track or its row is already matched.  A matched track overwrites the joints the row uses,
+ *     keeps the others and resets its misses to 0;
+ *   - ageing: every unmatched live track increments its misses and is freed when they exceed max_age;
+ *   - births: every unmatched detection, in row order, starts a track with the sequence's next id (0, 1, 2, ...) while
+ *     fewer than max_tracks tracks are live; otherwise its id is -1;
+ *   - track_id: the id the row was matched to or born as; -1 for a row that is not a detection or found no free track.
+ *   Sequences are independent; frames [0, T1) then [T1, T) on the same state give bitwise the ids of one call on [0, T).
+ *   MPL_ERR_INVALID_ARGUMENT, before any CUDA call: sequences < 0, frames < 0 or > INT32_MAX, K outside [1, 64], J outside
+ *   [1, 32], min_joints outside [1, J], max_dist not finite or not > 0, max_age < 0, max_tracks outside [1, 128]; then
+ *   sequences == 0 or frames == 0 returns MPL_OK; then a null points / state / track_id or a misaligned state.  One CTA per
+ *   sequence with its state in shared memory; no floating-point atomics; allocates nothing and never synchronises
+ *   (graph-capturable).
+ *
+ * mpl_tracking_score: CLEAR-MOT style counts of track_id [S, T, K] (of mpl_track_people from a zeroed state, whole
+ * sequences) against the rows' true persons owner [S, T, K] (e.g. mpl_association_score's owner; -1 for none) of P persons,
+ * each present in every frame (T P objects per sequence).  The match of person q in frame t is the smallest row k with
+ * owner == q and track_id >= 0, its id the hypothesis.  acc [MPL_TRACK_ACC_LEN] fp64 running sums (added to):
+ *   [0] sequences; [1] frames; [2] objects; [3] matches; [4] misses (objects - matches); [5] false positives (rows with
+ *   track_id >= 0 that are no match); [6] ID switches (a match whose hypothesis differs from q's previous match in the
+ *   sequence); [7] fragmentations (a match after a frame without one, following an earlier match); [8] mostly tracked
+ *   (persons matched in >= 80 % of the frames); [9] mostly lost (< 20 %); [10] tracks (1 + the largest id per sequence).
+ *   Integer counts reduced in a fixed order, added once per call.  MPL_ERR_INVALID_ARGUMENT, before any CUDA call:
+ *   sequences < 0, frames < 0 or > INT32_MAX, K < 1, P < 1; then sequences == 0 or frames == 0 returns MPL_OK (acc untouched);
+ *   then a null pointer. */
+#define MPL_TRACK_ACC_LEN 11
+int mpl_synth_motion(uint64_t seed, int64_t start, int64_t sequences, int frames, int people, int num_views, int num_joints,
+                     const double* calib, int64_t calib_stride, const double* room, double fps, int conf_ones, float* pix,
+                     float* target, mpl_stream_t stream);
+size_t mpl_track_state_bytes(int max_tracks, int num_joints);
+int mpl_track_people(const float* points, const float* joint_mask, int64_t sequences, int64_t frames, int max_rows,
+                     int num_joints, int min_joints, double max_dist, int max_age, int max_tracks, void* state,
+                     int32_t* track_id, mpl_stream_t stream);
+int mpl_tracking_score(const int32_t* track_id, const int32_t* owner, int64_t sequences, int64_t frames, int max_rows,
+                       int people, double* acc, mpl_stream_t stream);
 
 /* ---- unit-test hooks for the building blocks (used by tests/ only) ------------------------------------------- */
 /* Y[M,N] = epilogue(A[M,K] . W[N,K]^T): the tcgen05 projection kernel in isolation.

@@ -35,9 +35,10 @@ EXPORTS = [
     "mpl_mpjpe_accumulate_grouped", "mpl_pmpjpe_accumulate_masked", "mpl_distort_pixels", "mpl_distort_pixels_strided",
     "mpl_undistort_pixels", "mpl_undistort_pixels_strided", "mpl_synth_calib_noise", "mpl_calibrate_rig_workspace_bytes",
     "mpl_calibrate_rig", "mpl_synth_people", "mpl_associate_people", "mpl_associate_people_strided", "mpl_gather_people",
-    "mpl_association_score",
+    "mpl_association_score", "mpl_synth_motion", "mpl_track_state_bytes", "mpl_track_people", "mpl_tracking_score",
 ]
 ASSOC_ACC_LEN = 8   # MPL_ASSOC_ACC_LEN
+TRACK_ACC_LEN = 11  # MPL_TRACK_ACC_LEN
 
 _DESC_FLAGS = [
     "qkv_bias", "add_confidence_input", "mult_confidence_emb", "concat_confidence_emb", "confidence_input_as_third",
@@ -187,6 +188,13 @@ def lib():
         L.mpl_gather_people.argtypes = [c_void_p, c_void_p, c_int64, c_int, c_int, c_int, c_int, c_void_p, c_void_p]
         L.mpl_association_score.argtypes = [c_void_p, c_void_p, c_void_p, c_int64, c_int, c_int, c_int, c_void_p, c_void_p,
                                             c_void_p]
+        L.mpl_synth_motion.argtypes = [ctypes.c_uint64, c_int64, c_int64, c_int, c_int, c_int, c_int, c_void_p, c_int64,
+                                       c_void_p, c_double, c_int, c_void_p, c_void_p, c_void_p]
+        L.mpl_track_state_bytes.argtypes = [c_int, c_int]
+        L.mpl_track_state_bytes.restype = c_size_t
+        L.mpl_track_people.argtypes = [c_void_p, c_void_p, c_int64, c_int64, c_int, c_int, c_int, c_double, c_int, c_int,
+                                       c_void_p, c_void_p, c_void_p]
+        L.mpl_tracking_score.argtypes = [c_void_p, c_void_p, c_int64, c_int64, c_int, c_int, c_void_p, c_void_p]
         if L.mpl_abi_version() != ABI_VERSION:
             raise RuntimeError("libmpl_b200.so ABI version mismatch")
         _lib = L

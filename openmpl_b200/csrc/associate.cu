@@ -313,12 +313,6 @@ int launch_gather_people(const float* scene, const int32_t* members, int64_t F, 
 }
 
 // ---- score: one warp per frame, integer counts per lane, one fixed-order reduction, then acc += the counts ---------------
-__device__ __forceinline__ long long warp_sum_ll(long long v) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-  return v;
-}
-
 __global__ void __launch_bounds__(kScoreWarps * 32, 1) association_score_kernel(const int32_t* __restrict__ members,
                                                                              const int32_t* __restrict__ labels,
                                                                              const int32_t* __restrict__ perm, int64_t F,

@@ -239,5 +239,14 @@ int launch_gather_people(const float* scene, const int32_t* members, int64_t F, 
                          cudaStream_t s);
 int launch_association_score(const int32_t* members, const int32_t* labels, const int32_t* perm, int64_t F, int P, int K,
                              int V, int32_t* owner, double* acc, cudaStream_t s);
+// track.cu: people that move, tracking of person rows across frames and its score (argument checks in model.cu)
+int launch_synth_motion(uint64_t seed, int64_t start, int64_t S, int T, int P, int V, int J, const double* calib,
+                        int64_t calib_stride, const double* room, double fps, int conf_ones, float* pix, float* target,
+                        cudaStream_t s);
+size_t track_state_bytes(int max_tracks, int J);
+int launch_track_people(const float* points, const float* joint_mask, int64_t S, int64_t T, int K, int J, int min_joints,
+                        double max_dist, int max_age, int max_tracks, void* state, int32_t* track_id, cudaStream_t s);
+int launch_tracking_score(const int32_t* track_id, const int32_t* owner, int64_t S, int64_t T, int K, int P, double* acc,
+                          cudaStream_t s);
 
 }  // namespace mpl

@@ -1005,22 +1005,8 @@ int launch_triangulate_refine(const float* pix, const double* calib, int64_t cal
 // x_cam = R (X - t), u = f x_cam / z + c (MPL/lib/utils/calib.py:42-77).  Emits raw detector-style pixels (u, v, conf)
 // for mpl_build_inputs and the 3D target.  The generator is numpy's Philox4x64-10 stream, bit for bit (openmpl_b200/
 // synth.py draws the same uniforms on the host), so the device data can be checked against the host generator.
-// philox4x64_10 is in shared.cuh.
+// philox4x64_10, UniformCursor and project_pixel are in shared.cuh (track.cu's mpl_synth_motion uses them too).
 // ---------------------------------------------------------------------------------------------------------------------
-struct UniformCursor {  // sequential reader of one pose's uniform stream with a one-block cache
-  uint64_t v[4];
-  int64_t blk;
-  uint64_t base, key;
-  __device__ UniformCursor(uint64_t base_, uint64_t key_) : blk(-1), base(base_), key(key_) {}
-  __device__ double get(int i) {
-    const int64_t b = i >> 2;
-    if (b != blk) { philox4x64_10(base + (uint64_t)b + 1ull, key, 0ull, v); blk = b; }  // numpy increments the counter before generating
-    const int k = i & 3;
-    const uint64_t raw = k == 0 ? v[0] : (k == 1 ? v[1] : (k == 2 ? v[2] : v[3]));
-    return (double)(raw >> 11) * (1.0 / 9007199254740992.0);
-  }
-};
-
 template <bool kPerPose>
 __global__ void __launch_bounds__(128) synth_project_kernel(uint64_t seed, int64_t start, int64_t B, int V, int J,
                                                             const double* __restrict__ calib, int64_t cstride,
@@ -1053,18 +1039,8 @@ __global__ void __launch_bounds__(128) synth_project_kernel(uint64_t seed, int64
       }
       tg[j * 3 + k] = (float)X[k];
     }
-    for (int v = 0; v < V; ++v) {
-      const double* c = cal + v * 18;
-      double xc[3];
-#pragma unroll
-      for (int r = 0; r < 3; ++r)
-        xc[r] = c[3 * r] * (X[0] - c[9]) + c[3 * r + 1] * (X[1] - c[10]) + c[3 * r + 2] * (X[2] - c[11]);
-      const double u = xc[0] / xc[2] * c[12] + c[14], w = xc[1] / xc[2] * c[13] + c[15];
-      double conf = conf_ones ? 1.0 : 0.3 + 0.7 * cc.get(3 + 2 * n + v * J + j);
-      if (!(xc[2] > 0.0)) conf = 0.0;  // behind the camera: never a detection
-      float* o = px + (v * J + j) * 3;
-      o[0] = (float)u; o[1] = (float)w; o[2] = (float)conf;
-    }
+    for (int v = 0; v < V; ++v)
+      project_pixel(cal + v * 18, X, conf_ones ? 1.0 : 0.3 + 0.7 * cc.get(3 + 2 * n + v * J + j), px + (v * J + j) * 3);
   }
 }
 

@@ -1624,6 +1624,69 @@ int mpl_association_score(const int32_t* members, const int32_t* labels, const i
                                   reinterpret_cast<cudaStream_t>(stream));
 }
 
+// Shape rules of the tracking entry points (include/mpl_b200.h): K rows per frame, J joints, max_tracks track slots.
+static bool track_shape_ok(int K, int J, int max_tracks) {
+  return K >= 1 && K <= 64 && J >= 1 && J <= 32 && max_tracks >= 1 && max_tracks <= 128;
+}
+
+int mpl_synth_motion(uint64_t seed, int64_t start, int64_t sequences, int frames, int people, int num_views, int num_joints,
+                     const double* calib, int64_t calib_stride, const double* room, double fps, int conf_ones, float* pix,
+                     float* target, mpl_stream_t stream) {
+  if (sequences < 0 || start < 0 || frames < 1 || people < 1 || num_views < 1 || num_views > kMaxViews || num_joints < 1 ||
+      !std::isfinite(fps) || !(fps > 0.0) || !calib_stride_ok(calib_stride, num_views)) {
+    set_error("mpl_synth_motion: bad argument (sequences %lld, start %lld, frames %d, people %d, num_views %d, num_joints %d, "
+              "fps %g, calib_stride %lld)", (long long)sequences, (long long)start, frames, people, num_views, num_joints, fps,
+              (long long)calib_stride);
+    return MPL_ERR_INVALID_ARGUMENT;
+  }
+  if (sequences == 0) return MPL_OK;
+  if (calib == nullptr || room == nullptr || pix == nullptr || target == nullptr) {
+    set_error("mpl_synth_motion: null pointer");
+    return MPL_ERR_INVALID_ARGUMENT;
+  }
+  return launch_synth_motion(seed, start, sequences, frames, people, num_views, num_joints, calib, calib_stride, room, fps,
+                             conf_ones, pix, target, reinterpret_cast<cudaStream_t>(stream));
+}
+
+size_t mpl_track_state_bytes(int max_tracks, int num_joints) {
+  return track_shape_ok(1, num_joints, max_tracks) ? track_state_bytes(max_tracks, num_joints) : 0;
+}
+
+int mpl_track_people(const float* points, const float* joint_mask, int64_t sequences, int64_t frames, int max_rows,
+                     int num_joints, int min_joints, double max_dist, int max_age, int max_tracks, void* state,
+                     int32_t* track_id, mpl_stream_t stream) {
+  if (sequences < 0 || frames < 0 || frames > INT32_MAX || !track_shape_ok(max_rows, num_joints, max_tracks) ||
+      min_joints < 1 || min_joints > num_joints || !std::isfinite(max_dist) || !(max_dist > 0.0) || max_age < 0) {
+    set_error("mpl_track_people: bad argument (sequences %lld, frames %lld, K %d, num_joints %d, min_joints %d, max_dist %g, "
+              "max_age %d, max_tracks %d)", (long long)sequences, (long long)frames, max_rows, num_joints, min_joints, max_dist,
+              max_age, max_tracks);
+    return MPL_ERR_INVALID_ARGUMENT;
+  }
+  if (sequences == 0 || frames == 0) return MPL_OK;
+  if (points == nullptr || state == nullptr || track_id == nullptr || (reinterpret_cast<uintptr_t>(state) & 3u) != 0) {
+    set_error("mpl_track_people: null pointer, or state not 4-byte aligned");
+    return MPL_ERR_INVALID_ARGUMENT;
+  }
+  return launch_track_people(points, joint_mask, sequences, frames, max_rows, num_joints, min_joints, max_dist, max_age,
+                             max_tracks, state, track_id, reinterpret_cast<cudaStream_t>(stream));
+}
+
+int mpl_tracking_score(const int32_t* track_id, const int32_t* owner, int64_t sequences, int64_t frames, int max_rows,
+                       int people, double* acc, mpl_stream_t stream) {
+  if (sequences < 0 || frames < 0 || frames > INT32_MAX || max_rows < 1 || people < 1) {
+    set_error("mpl_tracking_score: bad argument (sequences %lld, frames %lld, K %d, people %d)", (long long)sequences,
+              (long long)frames, max_rows, people);
+    return MPL_ERR_INVALID_ARGUMENT;
+  }
+  if (sequences == 0 || frames == 0) return MPL_OK;
+  if (track_id == nullptr || owner == nullptr || acc == nullptr) {
+    set_error("mpl_tracking_score: null pointer");
+    return MPL_ERR_INVALID_ARGUMENT;
+  }
+  return launch_tracking_score(track_id, owner, sequences, frames, max_rows, people, acc,
+                               reinterpret_cast<cudaStream_t>(stream));
+}
+
 int mpl_test_gemm(const void* A, const void* W, const float* bias, void* Y, int64_t M, int N, int K, int dtype, int epilogue,
                   int out_fp32, mpl_stream_t stream) {
   MPL_API_BEGIN

@@ -18,6 +18,8 @@
         --calibrate-rig 16384                                                           # a miscalibrated rig, recalibrated
     python -m openmpl_b200.evaluate --arch cmu0 --views 5 --people 4 --pixel-noise 2 --outlier-rate 0.1 --triangulate \
         --triangulate-robust                                                            # 4 people per frame, associated
+    python -m openmpl_b200.evaluate --arch cmu0 --views 5 --people 4 --frames 64 --pixel-noise 2 --outlier-rate 0.1 \
+        --triangulate-robust                                                            # sequences of 64 frames, tracked
 
 Per micro-batch, entirely on the device: `mpl_synth_project` (3D poses from the counter-based generator keyed by the
 GLOBAL pose index, projected through the V calibrations) -> `mpl_build_inputs` (clip, confidence zeroing, screen
@@ -87,6 +89,17 @@ their owner, the true person with the most members in the row; rows without an o
 draws the cameras per frame (keyed by the global frame index) and `--calib-noise` applies as above.  The line gains an
 "association" entry (`mpl_association_score`): the counts, pair precision and recall, the pure and complete fractions, the
 people dropped past K and the parameters.  Without the flag nothing of this runs.
+
+`--frames T` (with `--people P`, T >= 2) evaluates sequences of T frames of P people that move (`mpl_synth_motion`, FPS
+frames per second): `--poses` counts person-frames, sequence i holds the frames [i T, (i + 1) T), ranks shard whole
+sequences and a micro-batch holds micro_batch // (T P) of them (micro_batch >= T P).  The persons are generated by the
+motion model instead of `mpl_synth_project`; the lens, detector noise, slots, association, gathering and every metric run as
+with `--people` alone.  The person rows are then triangulated robustly (`mpl_triangulate_robust` at `--inlier-px`) and
+tracked from a fresh state per sequence (`mpl_track_people`: `--track-max-dist`, `--track-max-age`, min_joints of
+`--assoc-min-joints`, max_tracks = 2 P), and scored against the rows' owners (`mpl_tracking_score`).  `--random-cameras`
+draws the cameras per sequence (keyed by the global sequence index), the same for all its frames.  The line gains a
+"tracking" entry: the counts, MOTA = 1 - (misses + false positives + ID switches) / objects, the mostly tracked / lost
+fractions, tracks per person, the parameters and the time of the tracking calls.  Without the flag nothing of this runs.
 """
 from __future__ import annotations
 
@@ -108,6 +121,7 @@ ARCHS = {
 DEFAULT_DEPTH = {"hm0": 12, "chosen": 12, "kptok": 12, "cmu0": 2}
 DEFAULT_RIG = {"hm0": "h36m", "chosen": "h36m", "kptok": "h36m", "cmu0": "cmu"}
 REFINE_MAX_ITERS = 20
+FPS = 30.0                                             # frame rate of the --frames sequences
 CALIBRATE_MAX_ITERS = 30
 
 
@@ -115,7 +129,21 @@ def run(arch="hm0", views=4, depth=None, poses=1 << 20, micro_batch=65536, preci
         weight_seed=0, warmup=1, triangulate=False, pixel_noise=0.0, outlier_rate=0.0, miss_rate=0.0,
         triangulate_robust=False, inlier_px=10.0, random_cameras=False, refine_triangulations=False,
         triangulation_pmpjpe=False, lens_distortion=None, calib_noise=None, calibrate_rig=0, people=0,
-        assoc_max_dist=0.1, assoc_min_joints=3):
+        assoc_max_dist=0.1, assoc_min_joints=3, frames=0, track_max_dist=0.2, track_max_age=5):
+    if frames:
+        if not people:
+            raise ValueError("frames needs people")
+        if frames < 2:
+            raise ValueError(f"frames must be >= 2, got {frames}")
+        if micro_batch < frames * people:
+            raise ValueError(f"micro_batch must hold at least one sequence of {frames} x {people} person-frames, got "
+                             f"{micro_batch}")
+        if poses < frames * people:
+            raise ValueError(f"poses must hold at least one sequence of {frames} x {people} person-frames, got {poses}")
+        if not (np.isfinite(track_max_dist) and track_max_dist > 0):
+            raise ValueError(f"track_max_dist must be finite and > 0, got {track_max_dist}")
+        if track_max_age < 0:
+            raise ValueError(f"track_max_age must be >= 0, got {track_max_age}")
     if people:
         if people < 2:
             raise ValueError(f"people must be >= 2, got {people}")
@@ -161,11 +189,16 @@ def run(arch="hm0", views=4, depth=None, poses=1 << 20, micro_batch=65536, preci
     mdist.broadcast_state(model)                       # replicas bit-identical (they already are: same seed)
     rig_kind = rig or DEFAULT_RIG[arch]
     the_rig = synth.make_rig(views, rig_kind)
-    if people:                                         # frames of `people` persons: the index range counts frames
-        frames = poses // people
-        poses = frames * people
+    if frames:                                         # sequences of frames of `people` persons: the range counts sequences
+        sequences = poses // (frames * people)
+        poses = sequences * frames * people
+        micro_batch //= frames * people
+        start, stop = mdist.shard_range(sequences, rank, world)
+    elif people:                                       # frames of `people` persons: the index range counts frames
+        nframes = poses // people
+        poses = nframes * people
         micro_batch //= people
-        start, stop = mdist.shard_range(frames, rank, world)
+        start, stop = mdist.shard_range(nframes, rank, world)
     else:
         start, stop = mdist.shard_range(poses, rank, world)
     # with people, a person row adds into group 0 and a row without an owner into none (-1)
@@ -192,9 +225,14 @@ def run(arch="hm0", views=4, depth=None, poses=1 << 20, micro_batch=65536, preci
     else:
         used_rig = rig_calib
 
-    def synth_pixels(s0, n, cams):
-        """Pixels of poses [s0, s0 + n) through the true cameras, with the lens and the detector noise."""
-        pix, target, calib = inputs.synth_project(n, the_rig, seed=seed, start=s0, device=dev, cameras=cams)
+    def synth_pixels(s0, n, cams, seqs=None):
+        """Pixels of poses [s0, s0 + n) through the true cameras, with the lens and the detector noise; with seqs =
+        (first sequence, sequences), the rows of those sequences of people that move."""
+        if seqs is None:
+            pix, target, calib = inputs.synth_project(n, the_rig, seed=seed, start=s0, device=dev, cameras=cams)
+        else:
+            pix, target, calib = inputs.synth_motion(seqs[1], frames, people, the_rig, seed=seed, start=seqs[0], fps=FPS,
+                                                     device=dev, cameras=cams)
         if lens_distortion is not None:
             inputs.distort_pixels(pix, calib, lens)
         if noisy:
@@ -226,19 +264,25 @@ def run(arch="hm0", views=4, depth=None, poses=1 << 20, micro_batch=65536, preci
 
     assoc_acc = torch.zeros(8, dtype=torch.float64, device=dev) if people else None
     dropped = torch.zeros(1, dtype=torch.float64, device=dev) if people else None
+    track_acc = torch.zeros(11, dtype=torch.float64, device=dev) if frames else None
+    track_events = []                                  # (start, end) events around each micro-batch's tracking calls
 
-    def person_rows(f0, nf):
+    def person_rows(f0, nf, seqs=None):
         """The person rows of frames [f0, f0 + nf): (pixels and calibration for the lifter, the same for the triangulations,
-        the owners' targets, the group of each row: 0 with an owner, -1 without)."""
+        the owners' targets, the group of each row: 0 with an owner, -1 without).  With seqs = (first sequence, sequences),
+        the frames of those sequences, whose rows are also tracked and scored."""
         P = people
-        cams = inputs.synth_cameras(nf, views, rig_kind, seed=seed, start=f0, device=dev) if random_cameras else None
+        u0, nu, per = (f0, nf, 1) if seqs is None else (seqs[0], seqs[1], frames)     # cameras per frame or per sequence
+        cams = inputs.synth_cameras(nu, views, rig_kind, seed=seed, start=u0, device=dev) if random_cameras else None
         if cams is None:
             calib = used_rig
         elif calib_noise is not None:
-            calib = inputs.calibration_noise(cams, seed, f0, sig_rot, sig_pos)
+            calib = inputs.calibration_noise(cams, seed, u0, sig_rot, sig_pos)
         else:
             calib = cams
-        pix, target = synth_pixels(f0 * P, nf * P, None if cams is None else cams.repeat_interleave(P, 0))
+        if cams is not None and per > 1:
+            cams, calib = cams.repeat_interleave(per, 0), calib.repeat_interleave(per, 0)
+        pix, target = synth_pixels(f0 * P, nf * P, None if cams is None else cams.repeat_interleave(P, 0), seqs)
         scene, perm = inputs.synth_people(pix, P, seed, f0)
         rows_calib = calib if calib.dim() == 2 else calib.repeat_interleave(P, 0)   # frame f's cameras for its slots and rows
         scene_t, tri_calib = scene, rows_calib
@@ -255,11 +299,23 @@ def run(arch="hm0", views=4, depth=None, poses=1 << 20, micro_batch=65536, preci
         idx = owner.clamp(min=0).long()[:, :, None, None].expand(nf, P, cfg.J, 3)
         target = target.view(nf, P, cfg.J, 3).gather(1, idx).view(nf * P, cfg.J, 3)
         group = torch.where(owner >= 0, 0, -1).to(torch.int32).view(-1)
+        if seqs is not None:
+            points, _ = inputs.triangulate_robust(rows_t, tri_calib, inlier_px=inlier_px)
+            ev = (torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True))
+            ev[0].record()
+            ids, _ = inputs.track_people(points.view(seqs[1], frames, P, cfg.J, 3), min_joints=assoc_min_joints,
+                                         max_dist=track_max_dist, max_age=track_max_age, max_tracks=2 * P)
+            inputs.tracking_score(ids, owner.view(seqs[1], frames, P), P, track_acc)
+            ev[1].record()
+            track_events.append(ev)
         return rows, rows_calib, (rows_t, tri_calib), target, group
 
     def step(s0, n):
         g, tri = {}, None
-        if people:
+        if frames:
+            pix, calib, tri, target, group = person_rows(s0 * frames, n * frames, (s0, n))
+            g = {"group": group}
+        elif people:
             pix, calib, tri, target, group = person_rows(s0, n)
             g = {"group": group}
         else:
@@ -308,6 +364,9 @@ def run(arch="hm0", views=4, depth=None, poses=1 << 20, micro_batch=65536, preci
     if people:
         assoc_acc.zero_()
         dropped.zero_()
+    if frames:
+        track_acc.zero_()
+        track_events.clear()
     if world > 1:
         torch.distributed.barrier()
     torch.cuda.synchronize()
@@ -323,6 +382,8 @@ def run(arch="hm0", views=4, depth=None, poses=1 << 20, micro_batch=65536, preci
     if people and world > 1:
         torch.distributed.all_reduce(assoc_acc)
         torch.distributed.all_reduce(dropped)
+        if frames:
+            torch.distributed.all_reduce(track_acc)
     e1.record()
     torch.cuda.synchronize()
     ms = mdist.max_over_ranks(e0.elapsed_time(e1), dev)
@@ -348,7 +409,8 @@ def run(arch="hm0", views=4, depth=None, poses=1 << 20, micro_batch=65536, preci
             if not isinstance(line["data"], dict):
                 line["data"] = {"source": line["data"]}
             line["data"]["cameras"] = {
-                "model": "random per pose (mpl_synth_cameras, keyed by global pose index)", "rig_kind": rig_kind,
+                "model": "random per sequence (mpl_synth_cameras, keyed by global sequence index)" if frames else
+                         "random per pose (mpl_synth_cameras, keyed by global pose index)", "rig_kind": rig_kind,
                 "azimuth": "2 pi (v + 0.8 (U0 - 0.5)) / V + 0.3", "distance_m": "4.5 (0.75 + 0.5 U1)",
                 "height_m": "0.9 + 1.2 U2", "look_at": "room centre at 0.9 m + 0.5 (U3 - 0.5, U4 - 0.5, 0)",
                 "focal_px": "f0 (0.8 + 0.4 U5), f0 of the rig kind"}
@@ -389,6 +451,9 @@ def run(arch="hm0", views=4, depth=None, poses=1 << 20, micro_batch=65536, preci
         if people:
             line["association"] = association_summary(assoc_acc.cpu().numpy(), float(dropped.item()), res["n"], people,
                                                       assoc_max_dist, assoc_min_joints)
+        if frames:
+            line["tracking"] = tracking_summary(track_acc.cpu().numpy(), sum(a.elapsed_time(b) for a, b in track_events),
+                                                people, frames, track_max_dist, track_max_age, assoc_min_joints, inlier_px)
         # .reshape(-1): the sums of the one group with people
         if tacc is not None:
             line["triangulation"] = triangulation_summary(tacc.acc.detach().cpu().numpy().reshape(-1), cfg.J)
@@ -457,6 +522,28 @@ def association_summary(acc, dropped, scored_rows, people, max_dist, min_joints)
     return out
 
 
+def tracking_summary(acc, ms, people, frames, max_dist, max_age, min_joints, inlier_px):
+    """The tracking entry of the JSON line from the 11 sums of mpl_tracking_score."""
+    def ratio(a, b):
+        return float(a / b) if b > 0 else float("nan")
+
+    names = ("sequences", "frames", "objects", "matches", "misses", "false_positives", "id_switches", "fragmentations",
+             "mostly_tracked", "mostly_lost", "tracks")
+    out = {k: int(round(float(v))) for k, v in zip(names, acc)}
+    persons = acc[0] * people
+    out.update(mota=1.0 - ratio(acc[4] + acc[5] + acc[6], acc[2]), mostly_tracked_fraction=ratio(acc[8], persons),
+               mostly_lost_fraction=ratio(acc[9], persons), tracks_per_person=ratio(acc[10], persons),
+               parameters={"frames_per_sequence": frames, "fps": FPS, "people": people, "max_dist_m": max_dist,
+                           "max_age_frames": max_age, "min_joints": min_joints, "max_tracks": 2 * people},
+               motion="per person: root on a sinusoid in x and y inside the room (0.03-0.1 Hz), fixed height, heading "
+                      "turning at most 0.5 rad/s, fixed body (mpl_synth_motion)",
+               method=f"robust triangulation of the person rows (inlier {inlier_px:g} px), then greedy matching of the "
+                      f"median joint distance to each track's last observed joints, from a fresh state per sequence",
+               ms=ms, note="ms: device time of mpl_track_people and mpl_tracking_score (with the state's zeroing); ms_total "
+                           "includes it and the triangulation for the tracker")
+    return out
+
+
 def triangulation_summary(acc, J, method="linear DLT, pixel-space rows, views with conf > 0 inside the image"):
     """The triangulation entry of the JSON line from the MPJPE sums of triangulated points masked by views_used >= 2.
 
@@ -520,7 +607,25 @@ def main(argv=None):
                    help="association: largest median ray distance of a linked pair, world units (m)")
     p.add_argument("--assoc-min-joints", type=int, default=3, metavar="N",
                    help="association: candidate joints a detection needs, and joints a pair must share")
+    p.add_argument("--frames", type=int, default=0, metavar="T",
+                   help="sequences of T >= 2 frames of people that move, tracked across frames (needs --people; "
+                        "--micro-batch >= T P)")
+    p.add_argument("--track-max-dist", type=float, default=0.2, metavar="M",
+                   help="tracking: largest median joint distance of a track and a row it matches, world units (m)")
+    p.add_argument("--track-max-age", type=int, default=5, metavar="N",
+                   help="tracking: missed frames after which a track is dropped")
     a = p.parse_args(argv)
+    if a.frames:
+        if not a.people:
+            p.error("--frames needs --people")
+        if a.frames < 2:
+            p.error("--frames needs T >= 2")
+        if a.micro_batch < a.frames * a.people:
+            p.error("--micro-batch must hold at least one sequence of --frames x --people person-frames")
+        if not (np.isfinite(a.track_max_dist) and a.track_max_dist > 0):
+            p.error("--track-max-dist needs a finite value > 0")
+        if a.track_max_age < 0:
+            p.error("--track-max-age needs N >= 0")
     if a.people:
         if a.people < 2:
             p.error("--people needs P >= 2")
@@ -566,7 +671,8 @@ def main(argv=None):
         triangulate_robust=a.triangulate_robust, inlier_px=a.inlier_px, random_cameras=a.random_cameras,
         refine_triangulations=a.refine_triangulations, triangulation_pmpjpe=a.triangulation_pmpjpe, lens_distortion=lens,
         calib_noise=cnoise, calibrate_rig=a.calibrate_rig, people=a.people, assoc_max_dist=a.assoc_max_dist,
-        assoc_min_joints=a.assoc_min_joints)
+        assoc_min_joints=a.assoc_min_joints, frames=a.frames, track_max_dist=a.track_max_dist,
+        track_max_age=a.track_max_age)
 
 
 if __name__ == "__main__":

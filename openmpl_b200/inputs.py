@@ -383,6 +383,114 @@ def association_score(members: torch.Tensor, labels: torch.Tensor, perm: torch.T
     return owner, acc
 
 
+def synth_motion(sequences: int, frames: int, people: int, rig, seed: int = 0, start: int = 0, fps: float = 30.0,
+                 conf_mode: str = "uniform", device=None, cameras=None) -> tuple:
+    """Sequences of people that move, generated and projected ON THE DEVICE (`mpl_synth_motion`).
+
+    Row ((start + s) T + t) P + p is person p in frame t of global sequence start + s: a body of synth_project's shape
+    walking a closed-form path in the rig's room and turning slowly (include/mpl_b200.h states the model), so person p of a
+    sequence depends only on (seed, sequence, p, t).  Returns (pix [S T P, V, 17, 3] raw pixels (u, v, conf), target
+    [S T P, 17, 3] metres, calib) as `synth_project` does: the rig's [V, 18] calibration, or `cameras`, a [S T P, V, 18]
+    calibration per row.  Viewed as [F P, ...] with F = S T frames, pass frame (start + s) T + t to `synth_people` and row
+    index r to `add_detector_noise`.  `synth.synth_motion` is the numpy twin.
+    """
+    from .synth import NUM_JOINTS
+    device = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
+    V, J = rig.num_views, NUM_JOINTS
+    rows = sequences * frames * people
+    if cameras is None:
+        calib = torch.as_tensor(pack_calibration(rig.R, rig.t, rig.f, rig.c, rig.image_size)).to(device)
+        stride = 0
+    else:
+        calib, stride = _calib_arg(cameras, rows, V, device)
+        if stride == 0:
+            raise ValueError("cameras must be a [S T P, V, 18] calibration per row")
+    if conf_mode not in ("uniform", "ones"):
+        raise ValueError(conf_mode)
+    room = torch.as_tensor(np.asarray(rig.room, dtype=np.float64)).to(device)
+    pix = torch.empty((rows, V, J, 3), dtype=torch.float32, device=device)
+    target = torch.empty((rows, J, 3), dtype=torch.float32, device=device)
+    with torch.cuda.device(device):
+        stream = torch.cuda.current_stream(device).cuda_stream
+        _lib.check(_lib.lib().mpl_synth_motion(int(seed), int(start), int(sequences), int(frames), int(people), V, J,
+                                               calib.data_ptr(), stride, room.data_ptr(), float(fps),
+                                               int(conf_mode == "ones"), pix.data_ptr(), target.data_ptr(), stream))
+    return pix, target, calib
+
+
+def track_state(sequences: int, max_tracks: int, num_joints: int, device=None) -> torch.Tensor:
+    """A zeroed tracker state for `track_people`: [S, mpl_track_state_bytes(max_tracks, J)] uint8, fresh sequences."""
+    nbytes = _lib.lib().mpl_track_state_bytes(int(max_tracks), int(num_joints))
+    if nbytes == 0:
+        raise ValueError(f"unsupported tracker shape max_tracks={max_tracks} J={num_joints} (1 <= max_tracks <= 128, "
+                         f"1 <= J <= 32)")
+    device = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
+    return torch.zeros((sequences, nbytes), dtype=torch.uint8, device=device)
+
+
+def track_people(points: torch.Tensor, joint_mask: torch.Tensor | None = None, state: torch.Tensor | None = None,
+                 min_joints: int = 3, max_dist: float = 0.2, max_age: int = 5, max_tracks: int | None = None) -> tuple:
+    """Online tracking of person rows across frames (`mpl_track_people`), enqueued on the current stream.
+
+    points [S, T, K, J, 3] fp32 on the device: per frame of S independent sequences, K rows of 3D joints (e.g. the robust
+    triangulation of `gather_people` rows); NaN joints are not used.  joint_mask [S, T, K, J] (> 0: use the joint) or None.
+    state: the [S, nbytes] uint8 tensor of `track_state` for the same max_tracks (default 2 K), updated in place, so frames
+    can be fed in chunks; None: a fresh one.  A row with at least min_joints used joints is a detection; each frame, (track, row) pairs
+    whose median joint distance is at most max_dist (world units) are matched greedily, cheapest first; unmatched tracks die
+    after max_age missed frames, and unmatched detections start new tracks with the sequence's next id.  Returns (track_id
+    [S, T, K] int32, -1 for rows without a track; state).
+    """
+    if points.dim() != 5 or points.shape[-1] != 3:
+        raise ValueError(f"points must be [S, T, K, J, 3], got {list(points.shape)}")
+    S, T, K, J, _ = points.shape
+    device = points.device
+    points = points.to(torch.float32).contiguous()
+    mask = None
+    if joint_mask is not None:
+        if tuple(joint_mask.shape) != (S, T, K, J):
+            raise ValueError(f"joint_mask must be [S, T, K, J] = [{S}, {T}, {K}, {J}], got {list(joint_mask.shape)}")
+        mask = joint_mask.to(device=device, dtype=torch.float32).contiguous()
+    max_tracks = 2 * K if max_tracks is None else int(max_tracks)
+    if state is None:
+        state = track_state(S, max_tracks, J, device)
+    nbytes = _lib.lib().mpl_track_state_bytes(max_tracks, J)
+    if state.dim() != 2 or tuple(state.shape) != (S, nbytes) or state.dtype != torch.uint8 or not state.is_contiguous() or \
+            nbytes == 0:
+        raise ValueError(f"state must be a contiguous uint8 [S, mpl_track_state_bytes(max_tracks, J)] tensor for S={S}, "
+                         f"max_tracks={max_tracks}, J={J}, got {list(state.shape)} {state.dtype}")
+    track_id = torch.empty((S, T, K), dtype=torch.int32, device=device)
+    with torch.cuda.device(device):
+        stream = torch.cuda.current_stream(device).cuda_stream
+        _lib.check(_lib.lib().mpl_track_people(points.data_ptr(), None if mask is None else mask.data_ptr(), S, T, K, J,
+                                               int(min_joints), float(max_dist), int(max_age), max_tracks,
+                                               state.data_ptr(), track_id.data_ptr(), stream))
+    return track_id, state
+
+
+def tracking_score(track_id: torch.Tensor, owner: torch.Tensor, people: int, acc: torch.Tensor | None = None) -> torch.Tensor:
+    """CLEAR-MOT style counts of a tracking against the rows' true persons (`mpl_tracking_score`), enqueued on the current
+    stream.  track_id [S, T, K] of `track_people` (whole sequences from a fresh state), owner [S, T, K] int32 (the true
+    person of each row, -1 for none, e.g. `association_score`'s owner), people P per frame.  Returns acc [11] fp64, the
+    running sums of include/mpl_b200.h added into `acc` when given: sequences, frames, objects, matches, misses, false
+    positives, ID switches, fragmentations, mostly tracked, mostly lost, tracks."""
+    if track_id.dim() != 3 or tuple(owner.shape) != tuple(track_id.shape):
+        raise ValueError(f"track_id and owner must both be [S, T, K], got {list(track_id.shape)} and {list(owner.shape)}")
+    if track_id.dtype != torch.int32 or owner.dtype != torch.int32:
+        raise ValueError("track_id and owner must be int32")
+    S, T, K = track_id.shape
+    device = track_id.device
+    if acc is None:
+        acc = torch.zeros(_lib.TRACK_ACC_LEN, dtype=torch.float64, device=device)
+    elif acc.dtype != torch.float64 or tuple(acc.shape) != (_lib.TRACK_ACC_LEN,) or not acc.is_contiguous():
+        raise ValueError(f"acc must be a contiguous float64 [{_lib.TRACK_ACC_LEN}] tensor")
+    track_id, owner = (t.to(device).contiguous() for t in (track_id, owner))
+    with torch.cuda.device(device):
+        stream = torch.cuda.current_stream(device).cuda_stream
+        _lib.check(_lib.lib().mpl_tracking_score(track_id.data_ptr(), owner.data_ptr(), S, T, K, int(people), acc.data_ptr(),
+                                                 stream))
+    return acc
+
+
 def _dist_arg(dist, B: int, V: int, device) -> tuple:
     """(contiguous fp64 device tensor, dist_stride): [V, 5] -> stride 0 (one lens set for the batch); [B, V, 5] -> 5 V."""
     if isinstance(dist, torch.Tensor):

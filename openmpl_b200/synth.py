@@ -175,6 +175,71 @@ def synth_people(pix, people: int, seed: int, start: int) -> tuple:
     return np.ascontiguousarray(scene.transpose(0, 2, 1, 3, 4)), perm
 
 
+def motion_joints(seed: int, start: int, sequences: int, frames: int, people: int, room, fps: float = 30.0,
+                  num_joints: int = NUM_JOINTS) -> np.ndarray:
+    """The 3D joints of `mpl_synth_motion`, fp64 [S, T, P, J, 3], for sequences [start, start + S).
+
+    (sequence i, person p) owns the counter blocks of g = i P + p in the Philox4x64-10 stream under key (seed, 5), uniform
+    slots U0..U8 then the Box-Muller pairs (u1_m, u2_m) at 9 + m and 9 + 3 (J - 1) + m.  With tau = t / fps:
+    root x = (x0 + x1) / 2 + (0.25 + 0.25 U0) w_x sin(2 pi (0.03 + 0.07 U2) tau + 2 pi U4), y likewise with U1, U3, U5,
+    z = 0.8 + 0.2 U6; heading theta = 2 pi U7 + (U8 - 0.5) tau; X_j = root + Rz(theta) o_j with synth_project's body o_j."""
+    J = num_joints
+    n = 3 * (J - 1)
+    U = _uniforms(seed, start * people, sequences * people, 9 + 2 * n, key1=5).reshape(sequences, 1, people, 9 + 2 * n)
+    x0, x1, y0, y1 = (float(r) for r in room)
+    tau = (np.arange(frames, dtype=np.float64) / fps)[None, :, None]
+    two_pi = 2 * math.pi
+    ax, ay = (0.25 + 0.25 * U[..., 0]) * (x1 - x0), (0.25 + 0.25 * U[..., 1]) * (y1 - y0)
+    fx, fy = 0.03 + 0.07 * U[..., 2], 0.03 + 0.07 * U[..., 3]
+    px0, py0 = two_pi * U[..., 4], two_pi * U[..., 5]
+    rx = 0.5 * (x0 + x1) + ax * np.sin(two_pi * fx * tau + px0)                      # [S, T, P]
+    ry = 0.5 * (y0 + y1) + ay * np.sin(two_pi * fy * tau + py0)
+    rz = np.broadcast_to(0.8 + 0.2 * U[..., 6], rx.shape)
+    theta = two_pi * U[..., 7] + (U[..., 8] - 0.5) * tau
+    c, s = np.cos(theta)[..., None], np.sin(theta)[..., None]
+    u1 = np.maximum(U[..., 9:9 + n], 1e-12)
+    u2 = U[..., 9 + n:9 + 2 * n]
+    o = np.concatenate([np.zeros(U.shape[:-1] + (3,)), 0.25 * (np.sqrt(-2.0 * np.log(u1)) * np.cos(two_pi * u2))], axis=-1)
+    o = o.reshape(U.shape[:-1] + (J, 3))                                              # [S, 1, P, J, 3]
+    X = np.empty((sequences, frames, people, J, 3))
+    X[..., 0] = rx[..., None] + (c * o[..., 0] - s * o[..., 1])
+    X[..., 1] = ry[..., None] + (s * o[..., 0] + c * o[..., 1])
+    X[..., 2] = rz[..., None] + o[..., 2]
+    return X
+
+
+def synth_motion(seed: int, start: int, sequences: int, frames: int, people: int, calib, room, fps: float = 30.0,
+                 conf_mode: str = "uniform", num_joints: int = NUM_JOINTS) -> tuple:
+    """Host twin of `mpl_synth_motion` -> (pix [S T P, V, J, 3] fp32, target [S T P, J, 3] fp32).
+
+    Row r = ((start + s) T + t) P + p holds person p in frame t of sequence start + s (`motion_joints`), projected like
+    `mpl_synth_project` through calib [V, 18] or one calibration per row [S T P, V, 18] (x_cam = R (X - t),
+    u = f x_cam / z + c, no clipping, conf 0 behind the camera); conf 1 with conf_mode "ones", otherwise 0.3 + 0.7 U of
+    `mpl_synth_project`'s confidence slots of pose r."""
+    J = num_joints
+    X = motion_joints(seed, start, sequences, frames, people, room, fps, J).reshape(-1, J, 3)
+    B = len(X)
+    calib = np.asarray(calib, dtype=np.float64)
+    c = calib[None] if calib.ndim == 2 else calib                                     # [1 or B, V, 18]
+    V = c.shape[1]
+    R, t = c[..., :9].reshape(c.shape[0], V, 3, 3), c[..., 9:12]
+    d = X[:, None, :, :] - t[:, :, None, :]                                           # [B, V, J, 3]
+    xc = [R[:, :, None, r, 0] * d[..., 0] + R[:, :, None, r, 1] * d[..., 1] + R[:, :, None, r, 2] * d[..., 2] for r in range(3)]
+    with np.errstate(divide="ignore", invalid="ignore"):
+        u = xc[0] / xc[2] * c[:, :, None, 12] + c[:, :, None, 14]
+        w = xc[1] / xc[2] * c[:, :, None, 13] + c[:, :, None, 15]
+    if conf_mode == "ones":
+        conf = np.ones((B, V, J))
+    elif conf_mode == "uniform":
+        n = 3 * (J - 1)
+        conf = 0.3 + 0.7 * _uniforms(seed, start * frames * people, B, 3 + 2 * n + V * J)[:, 3 + 2 * n:].reshape(B, V, J)
+    else:
+        raise ValueError(conf_mode)
+    conf = np.where(xc[2] > 0.0, conf, 0.0)
+    pix = np.stack([u, w, conf], axis=-1).astype(np.float32)
+    return pix, X.astype(np.float32)
+
+
 def _uniforms(seed: int, start: int, count: int, per_pose: int, key1: int = 0) -> np.ndarray:
     """[count, per_pose] uniforms in [0,1); row i depends only on (seed, start+i).  Philox key (seed, key1)."""
     blocks = (per_pose + 3) // 4                      # Philox4x64: 4 outputs per counter step
